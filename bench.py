@@ -2,7 +2,7 @@
 """Benchmark of the SimplyP daily mass-balance integration path on B200.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config 2|3|4|5]
-                    [--members M] [--period 2004|full]
+                    [--members M] [--period 2004|full] [--dump-outputs DIR]
 
 One "step" = one pass of the whole workload over its whole period.  Metric (BASELINE.json): member-sub-catchment-days
 per second, whole job.  Workloads = BASELINE.json `configs` (SURVEY.md §8d):
@@ -21,6 +21,8 @@ Members are sharded over ranks with no data-path collective; the only collective
 statistics (configs 2 and 4).  Prints ONE JSON line (rank 0).  See DESIGN.md §5 for how each field is obtained.
 `--impl reference` times the reference's own CPU algorithm (oracle port: per-day scipy odeint/LSODA at the reference's
 rtol=0.01) on all host cores, on a bounded sample of the same workload.
+`--dump-outputs DIR` writes what the last timed step returned (see dump_outputs) so that two builds can be compared
+output for output: every input is generated from fixed seeds, so the same arguments give the same inputs.
 """
 import argparse
 import json
@@ -39,6 +41,8 @@ UNIT = "member-SC-days/s"
 F_RHS, F_STEP_EXTRA, F_DAY = 140.0, 700.0, 120.0      # SURVEY.md §8(d) algorithmic flop counts
 B_DAY = 200.0                                         # SURVEY.md §8(d): bytes written per member-SC-day (full output)
 FP64_DFMA_PER_SM_CLK = 64                             # B200: 64 DFMA per SM per clock (nominal)
+DUMP_BYTES = 64 * 10 ** 6                             # --dump-outputs: all files together
+ST_SPEARMAN = 8                                       # SIMPLYP_ST_SPEARMAN: first stats slot after SIMPLYP_ST_SSE
 
 
 def parse_args():
@@ -58,7 +62,13 @@ def parse_args():
                     help="configs 3 and 5: members of the end-to-end leg (default: as many as fit 48 GB of pinned host memory)")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=24.0, help="sizes the cpu_baseline samples (about this many seconds of CPU work in total)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float64, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs: the reference arm keeps no outputs")
     if args.members is None:
         args.members = {2: 10000, 3: 64, 4: 1000000, 5: 8}[args.config]
     return args
@@ -300,6 +310,24 @@ def _pinned(a):
     return torch.from_numpy(np.ascontiguousarray(a)).pin_memory().numpy()
 
 
+def dump_outputs(dirname, outputs):
+    """Write each tensor of `outputs` (name -> tensor, last axis = one row) as DIR/<name>.npy in float64.
+    A tensor larger than its share of DUMP_BYTES (the full daily output of configs 3 and 5 is tens of GB) is written as
+    a sample of its rows, drawn with seed 0 from its shape alone, with the flat row indices in DIR/<name>_rows.npy:
+    runs with the same arguments write the same rows."""
+    import torch
+    os.makedirs(dirname, exist_ok=True)
+    share = DUMP_BYTES // len(outputs) - 1024         # an equal share per output, less its two .npy headers
+    for name, t in outputs.items():
+        rows = t.reshape(-1, t.shape[-1])
+        n_keep = share // (8 * (rows.shape[1] + 1))   # a sampled row costs its values and its index
+        if rows.shape[0] > n_keep:
+            pick = np.sort(np.random.default_rng(0).choice(rows.shape[0], n_keep, replace=False))
+            np.save(os.path.join(dirname, name + "_rows.npy"), pick.astype(np.float64))
+            t = rows.index_select(0, torch.from_numpy(pick).to(rows.device))
+        np.save(os.path.join(dirname, name + ".npy"), t.cpu().numpy().astype(np.float64))
+
+
 def run_ours(args):
     import torch
     import torch.distributed as dist
@@ -410,12 +438,19 @@ def run_ours(args):
     for k in range(args.steps):
         flush.zero_()                      # L2 flush between timed iterations (outside the events)
         ev[k][0].record()
-        step(mid[k])
+        result = step(mid[k])
         ev[k][1].record()
     barrier()
     t_wall = time.perf_counter() - t_wall0
     launches = _cabi.launch_count() - launches0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:   # what a caller of the step receives; diag is this rank's
+        if calibration:
+            # the statistics the call computes: Spearman's r (slot 8) is a NaN placeholder unless opt.rank_stats is
+            # set, and the last slot is reserved (include/simplyp_b200.h, SIMPLYP_ST_*)
+            result = result[..., :ST_SPEARMAN + 1 if opt.rank_stats else ST_SPEARMAN]
+        dump_outputs(args.dump_outputs, {"stats" if calibration else "out": result, "diag": diag})
+    del result                            # configs 3 and 5: `out` must be freed before the end-to-end leg
     step_ms = [a.elapsed_time(b) for a, b in ev]
     total_ms = torch.tensor([float(sum(step_ms))], dtype=torch.float64, device=eng.device)
     if world > 1:

@@ -25,9 +25,12 @@ from oracle import parallel as opar, simplyp_oracle as orc      # noqa: E402
 from simplyp_b200 import packing as pk, synthetic                # noqa: E402
 
 WINDOW = {3: 730, 5: 120}
+# points of the spread per config.  Config 3 (730 days) keeps its fixture under 1 MB with 4: run-order indices 0, 84,
+# 169 and 254, of which 254 is already a deepest reach, so 8 reaches in all.  Config 5: 6 points, 12 reaches in all.
+SPREAD = {3: 4, 5: 6}
 
 
-def sampled_reaches(w, n_extra=6):
+def sampled_reaches(w, n_extra):
     """Run-order indices: outlet, 3 stiffest by the nominal rate estimate, 2 deepest non-outlet, a spread."""
     topo, sc, member = w["topo"], w["sc"][0], w["member"][0]
     S = topo.n_sc
@@ -59,7 +62,7 @@ def main():
         raw = opar.run_network_parallel(met["P"].to_numpy(), met["PET"].to_numpy(), met.index.dayofyear.to_numpy(), p, lu,
                                         sc, ups, run_mode="cal", dynamic_EPC0=True, dynamic_erodibility=True,
                                         rtol=1e-10, atol=1e-13, mxstep=500000)
-        sel, lvl, rate = sampled_reaches(w)
+        sel, lvl, rate = sampled_reaches(w, SPREAD[cfg])
         full = np.concatenate([raw["ode"], raw["nonode"]], axis=2)          # [S][D][25]
         path = os.path.join(HERE, "ref_config%d.npz" % cfg)
         np.savez_compressed(path, reaches=np.array(sel, dtype=np.int32), raw=full[sel], levels=lvl[sel],

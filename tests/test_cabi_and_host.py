@@ -137,7 +137,11 @@ def test_ensemble_packing_and_sharding(tarland_2004_static):
 
 # ------------------------------------------------------------------------------------------ inputs
 def _write_xlsx(path, sheets):
-    """Minimal .xlsx writer (inline strings + numbers) used to round-trip the stdlib reader."""
+    """Minimal .xlsx writer laid out as a spreadsheet application saves a workbook, used to round-trip the stdlib
+    reader: strings in the shared-string table (every other one as two rich-text runs), a styles part, floats under a
+    number format, datetimes as day serials (origin 1899-12-30) under a custom and a builtin date format, rows
+    alternating, and the styles / shared strings listed among the workbook's relationships."""
+    import datetime
     import zipfile
     from xml.sax.saxutils import escape
 
@@ -149,15 +153,18 @@ def _write_xlsx(path, sheets):
             s = chr(65 + r) + s
         return s
 
+    ns = 'xmlns="http://schemas.openxmlformats.org/spreadsheetml/2006/main"'
+    rel = "http://schemas.openxmlformats.org/officeDocument/2006/relationships/"
+    strings = {}
     with zipfile.ZipFile(path, "w") as z:
         z.writestr("[Content_Types].xml", '<?xml version="1.0"?><Types xmlns="http://schemas.openxmlformats.org/package/2006/content-types"><Default Extension="rels" ContentType="application/vnd.openxmlformats-package.relationships+xml"/><Default Extension="xml" ContentType="application/xml"/></Types>')
-        z.writestr("_rels/.rels", '<?xml version="1.0"?><Relationships xmlns="http://schemas.openxmlformats.org/package/2006/relationships"><Relationship Id="rId1" Type="http://schemas.openxmlformats.org/officeDocument/2006/relationships/officeDocument" Target="xl/workbook.xml"/></Relationships>')
-        wb = ['<?xml version="1.0"?><workbook xmlns="http://schemas.openxmlformats.org/spreadsheetml/2006/main" xmlns:r="http://schemas.openxmlformats.org/officeDocument/2006/relationships"><sheets>']
+        z.writestr("_rels/.rels", '<?xml version="1.0"?><Relationships xmlns="http://schemas.openxmlformats.org/package/2006/relationships"><Relationship Id="rId1" Type="%sofficeDocument" Target="xl/workbook.xml"/></Relationships>' % rel)
+        wb = ['<?xml version="1.0"?><workbook %s xmlns:r="http://schemas.openxmlformats.org/officeDocument/2006/relationships"><sheets>' % ns]
         rels = ['<?xml version="1.0"?><Relationships xmlns="http://schemas.openxmlformats.org/package/2006/relationships">']
         for k, (name, rows) in enumerate(sheets.items(), 1):
             wb.append('<sheet name="%s" sheetId="%d" r:id="rId%d"/>' % (escape(name), k, k))
-            rels.append('<Relationship Id="rId%d" Type="http://schemas.openxmlformats.org/officeDocument/2006/relationships/worksheet" Target="worksheets/sheet%d.xml"/>' % (k, k))
-            xml = ['<?xml version="1.0"?><worksheet xmlns="http://schemas.openxmlformats.org/spreadsheetml/2006/main"><sheetData>']
+            rels.append('<Relationship Id="rId%d" Type="%sworksheet" Target="worksheets/sheet%d.xml"/>' % (k, rel, k))
+            xml = ['<?xml version="1.0"?><worksheet %s><sheetData>' % ns]
             for r, row in enumerate(rows, 1):
                 xml.append('<row r="%d">' % r)
                 for c, v in enumerate(row):
@@ -165,54 +172,88 @@ def _write_xlsx(path, sheets):
                         continue
                     ref = "%s%d" % (col(c), r)
                     if isinstance(v, str):
-                        xml.append('<c r="%s" t="inlineStr"><is><t>%s</t></is></c>' % (ref, escape(v)))
+                        xml.append('<c r="%s" t="s"><v>%d</v></c>' % (ref, strings.setdefault(v, len(strings))))
+                    elif isinstance(v, datetime.datetime):
+                        days = (v - datetime.datetime(1899, 12, 30)).days
+                        xml.append('<c r="%s" s="%d"><v>%d</v></c>' % (ref, 2 + r % 2, days))
+                    elif isinstance(v, float):
+                        xml.append('<c r="%s" s="1"><v>%r</v></c>' % (ref, v))
                     else:
-                        xml.append('<c r="%s"><v>%r</v></c>' % (ref, v))
+                        xml.append('<c r="%s"><v>%d</v></c>' % (ref, v))
                 xml.append("</row>")
             xml.append("</sheetData></worksheet>")
             z.writestr("xl/worksheets/sheet%d.xml" % k, "".join(xml))
         wb.append("</sheets></workbook>")
+        n = len(sheets)
+        rels.append('<Relationship Id="rId%d" Type="%sstyles" Target="styles.xml"/>' % (n + 1, rel))
+        rels.append('<Relationship Id="rId%d" Type="%ssharedStrings" Target="sharedStrings.xml"/>' % (n + 2, rel))
         rels.append("</Relationships>")
         z.writestr("xl/workbook.xml", "".join(wb))
         z.writestr("xl/_rels/workbook.xml.rels", "".join(rels))
+        z.writestr("xl/styles.xml", '<?xml version="1.0"?><styleSheet %s><numFmts count="1"><numFmt numFmtId="164" formatCode="dd/mm/yyyy;@"/></numFmts><cellXfs count="4"><xf numFmtId="0"/><xf numFmtId="2" applyNumberFormat="1"/><xf numFmtId="164" applyNumberFormat="1"/><xf numFmtId="14" applyNumberFormat="1"/></cellXfs></styleSheet>' % ns)
+        sst = ['<?xml version="1.0"?><sst %s count="%d" uniqueCount="%d">' % (ns, len(strings), len(strings))]
+        for i, text in enumerate(sorted(strings, key=strings.get)):
+            if i % 2 == 0 and len(text) > 1:
+                h = len(text) // 2
+                sst.append('<si><r><t xml:space="preserve">%s</t></r><r><rPr><b/></rPr><t xml:space="preserve">%s</t></r></si>'
+                           % (escape(text[:h]), escape(text[h:])))
+            else:
+                sst.append('<si><t xml:space="preserve">%s</t></si>' % escape(text))
+        sst.append("</sst>")
+        z.writestr("xl/sharedStrings.xml", "".join(sst))
 
 
-def test_read_input_data_roundtrip(tmp_path, golden_dir):
-    """Write the Tarland set-up as a workbook in the reference's sheet layout + met CSV + obs workbooks,
-    read it back with read_input_data, and get the same objects as the fixture loader."""
+def test_read_input_data_roundtrip(tmp_path, monkeypatch):
+    """Write the Tarland set-up in the original project's layout — the parameter workbook in Current_Release/v0-2A,
+    naming the met CSV and the two observation workbooks by its own Windows-style relative paths — as workbooks saved
+    the way a spreadsheet application saves them (_write_xlsx), read it back with read_input_data from the workbook's
+    directory, and get the same objects as the fixture loader."""
+    import datetime
     import simplyp_b200 as sp
-    from simplyp_b200 import tarland
+    from simplyp_b200 import _xlsx, tarland
     p_SU, dyn, p, p_LU, p_SC, p_struc, met, obs = tarland.load(dynamic="n")
+    wb_dir = tmp_path / "Current_Release" / "v0-2A"
+    wb_dir.mkdir(parents=True)
+
+    def place(rel_path):
+        path = os.path.normpath(os.path.join(str(wb_dir), rel_path.replace("\\", "/")))
+        os.makedirs(os.path.dirname(path), exist_ok=True)
+        return path
+
     z = np.load(os.path.join(tarland.DATA_DIR, "tarland_met.npz"))
     idx = pd.date_range(str(z["day0"]), periods=int(z["n"]), freq="D")
     sel = (idx >= "2003-12-01") & (idx <= "2005-01-31")
-    with open(tmp_path / "met.csv", "w") as f:
+    with open(place(p_SU["metdata_fpath"]), "w") as f:
         f.write("Date,T_air,PET,Precipitation\n")
         for d, t, e, pr in zip(idx[sel], z["T_air"][sel], z["PET"][sel], z["Precipitation"][sel]):
             f.write("%s,%r,%r,%r\n" % (d.strftime("%d/%m/%Y"), float(t), float(e), float(pr)))
     o = obs[1]
+    # discharge dates as date-formatted cells, chemistry dates as plain day serials
     serial = [(d - pd.Timestamp("1899-12-30")).days for d in o.index]
-    q_rows = [["Date", "Q"]] + [[s, None if np.isnan(v) else float(v)] for s, v in zip(serial, o["Q"])]
+    q_rows = [["Date", "Q"]] + [[d.to_pydatetime(), None if np.isnan(v) else float(v)] for d, v in zip(o.index, o["Q"])]
     chem_cols = ["SRP", "SS", "TDP", "TP", "PP"]
     c_rows = [["Date"] + chem_cols] + [[s] + [None if np.isnan(o[c].iloc[i]) else float(o[c].iloc[i]) for c in chem_cols]
                                       for i, s in enumerate(serial)]
-    _write_xlsx(tmp_path / "q.xlsx", {"1": q_rows})
-    _write_xlsx(tmp_path / "chem.xlsx", {"1": c_rows})
-    setup = dict(p_SU)
-    setup.update(metdata_fpath=str(tmp_path / "met.csv"), Qobsdata_fpath=str(tmp_path / "q.xlsx"),
-                 chemObsData_fpath=str(tmp_path / "chem.xlsx"))
+    # the original workbook's two observation paths are swapped (Qobsdata_fpath names the chemistry workbook)
+    _write_xlsx(place(p_SU["chemObsData_fpath"]), {"1": q_rows})
+    q_cells = _xlsx.Workbook(place(p_SU["chemObsData_fpath"])).cells("1")
+    assert all(isinstance(q_cells[(r, 0)], datetime.datetime) for r in (1, 2))     # both date formats recognised
+    _write_xlsx(place(p_SU["Qobsdata_fpath"]), {"1": c_rows})
     sheets = {
         "Readme": [["nothing here"]],
-        "Setup": [["Param", "Description", "Value"]] + [[k, "", (v if isinstance(v, str) else float(v))] for k, v in setup.items()],
+        "Setup": [["Param", "Description", "Value"]] + [[k, "", (v if isinstance(v, str) else float(v))] for k, v in p_SU.items()],
         "Reach_structure": [["Reach", "Upstream", "Final"], [1, None, None]],
         "LU": [["", "Param", "", "", "A", "S", "IG", "NC"]] + [["", r, "", ""] + [None if np.isnan(p_LU.loc[r, c]) else float(p_LU.loc[r, c]) for c in ["A", "S", "IG", "NC"]] for r in p_LU.index],
         "SC_reach": [["", "Param", "", "", 1]] + [["", r, "", "", float(p_SC.loc[r, 1])] for r in p_SC.index],
         "Constant": [["", "Param", "", "", "Value"]] + [["", k, "", "", float(v)] for k, v in p.items() if k != "SC_list"],
     }
-    _write_xlsx(tmp_path / "params.xlsx", sheets)
-    got = sp.read_input_data(str(tmp_path / "params.xlsx"))
+    _write_xlsx(str(wb_dir / "Parameters_v0-2A_Tarland.xlsx"), sheets)
+    monkeypatch.chdir(wb_dir)
+    got = sp.read_input_data("Parameters_v0-2A_Tarland.xlsx")
     g_SU, g_dyn, g_p, g_LU, g_SC, g_struc, g_met, g_obs = got
-    assert g_SU["run_mode"] == "cal" and int(g_SU["n_SC"]) == 1
+    for k, v in p_SU.items():
+        assert g_SU[k] == v, k
+    assert g_SU["st_dt"] == "2004-01-01" and g_SU["Dynamic_EPC0"] == "n" and g_struc.shape == (1, 2)
     for k in p.index:
         if k != "SC_list":
             assert float(g_p[k]) == float(p[k]), k
@@ -221,26 +262,9 @@ def test_read_input_data_roundtrip(tmp_path, golden_dir):
     assert np.array_equal(g_SC.loc[p_SC.index, 1].to_numpy(float), p_SC[1].to_numpy(float))
     assert len(g_met) == 366 and np.array_equal(g_met["P"].to_numpy(), met["P"].to_numpy())
     assert np.array_equal(g_met["D_snow_end"].to_numpy(), met["D_snow_end"].to_numpy())
-    for c in ["Q"] + chem_cols:
+    assert list(g_obs[1].columns) == list(o.columns) and g_obs[1].index.equals(o.index)
+    for c in o.columns:
         assert np.array_equal(g_obs[1][c].to_numpy(), o[c].to_numpy(), equal_nan=True), c
-
-
-@pytest.mark.skipif(not os.path.isdir("/root/reference"), reason="reference workbook not available here")
-def test_read_input_data_on_the_reference_workbook():
-    import simplyp_b200 as sp
-    from simplyp_b200 import tarland
-    cwd = os.getcwd()
-    os.chdir("/root/reference/Current_Release/v0-2A")
-    try:
-        got = sp.read_input_data("Parameters_v0-2A_Tarland.xlsx")
-    finally:
-        os.chdir(cwd)
-    want = tarland.load(dynamic="n")
-    assert got[0]["st_dt"] == "2004-01-01" and got[0]["Dynamic_EPC0"] == "n"
-    assert np.array_equal(got[6]["P"].to_numpy(), want[6]["P"].to_numpy())
-    assert np.array_equal(got[7][1]["Q"].to_numpy(), want[7][1]["Q"].to_numpy(), equal_nan=True)
-    assert np.allclose(got[3].to_numpy(float), want[3].to_numpy(float), equal_nan=True)
-    assert float(got[2]["fc"]) == 290.0 and got[5].shape == (1, 2)
 
 
 def test_snow_module_vs_oracle_and_golden(golden_dir):
