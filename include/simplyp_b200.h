@@ -292,6 +292,68 @@ int simplyp_thornthwaite_pet_device(int32_t n_days, int32_t n_months, const doub
                                     const int32_t* month_start, const int32_t* year_is_leap, double latitude_deg,
                                     double* pet, int32_t pet_stride, void* stream);
 
+/* ---- ensemble MCMC over the fused log-likelihood -------------------------------------------------
+ * The affine-invariant stretch move (Goodman & Weare 2010; emcee's EnsembleSampler with its default StretchMove)
+ * with a uniform prior box, for the calibration the reference does with emcee in Development/2016/MCMC.ipynb.
+ * The W walkers are two contiguous halves of W/2; one iteration is, for half 0 and then half 1:
+ *   simplyp_mcmc_propose_device  -> the free columns of that half's member_params (and sc_params) rows;
+ *   zero that half's diag, then simplyp_calibrate_device on that half's rows;
+ *   simplyp_mcmc_accept_device   -> Metropolis-Hastings test, walkers / lp / accepted updated (half 1: chain slot
+ *                                   stored when (t+1) % thin == 0, then the iteration counter t is incremented).
+ * Random words: Philox4x32-10 keyed by the seed, counter (walker, t low word, t high word, block), block 0 = partner
+ * and stretch factor, block 1 = acceptance; t lives in device memory, so one captured iteration replays unchanged.
+ * A proposal outside the box is flagged and its rows get the walker's CURRENT values (the integrator never sees an
+ * out-of-box parameter); the accept step rejects it from the flag.
+ * lp of a member = sum over its series of stats[.][v][SIMPLYP_ST_LOGLIK], or -inf if a diag status word of the member
+ * is non-zero; the box prior adds 0 inside. */
+#define SIMPLYP_MCMC_MAX_FREE 64
+enum {
+  SIMPLYP_MCMC_MEMBER = 0,  /* member_params[.][index]                                   */
+  SIMPLYP_MCMC_SC_ALL,      /* sc_params[.][s][index] for every sub-catchment s          */
+  SIMPLYP_MCMC_SC_AT        /* sc_params[.][pos][index], pos = position in the run order */
+};
+
+typedef struct {
+  int32_t kind, index, pos, reserved;
+  double  lo, hi;           /* prior box, lo < hi, both finite */
+} SimplypMcmcParam;
+
+typedef struct {
+  int32_t n_walkers;        /* W: even, >= 2 * n_free */
+  int32_t n_free;           /* K: 1..SIMPLYP_MCMC_MAX_FREE */
+  int32_t n_sc;             /* S of the calibration runs */
+  int32_t n_obs_series;     /* V of the calibration runs */
+  int32_t sc_per_member;    /* sc_params is [W][S][NP_SC] (required by the SC targets) rather than [1][S][NP_SC] */
+  int32_t thin;             /* chain slot stored every `thin` iterations */
+  uint64_t seed;            /* Philox key: (low word, high word) */
+  double  stretch;          /* a > 1 (emcee's default 2) */
+  SimplypMcmcParam param[SIMPLYP_MCMC_MAX_FREE];
+} SimplypMcmc;
+
+typedef struct {            /* device pointers */
+  double*  walkers;         /* [W][K] current states */
+  double*  lp;              /* [W] their log-probabilities */
+  double*  proposals;       /* [W/2][K] proposals of the active half */
+  double*  log_z;           /* [W/2] ln z of those proposals */
+  int32_t* out_of_box;      /* [W/2] 1: proposal outside the box */
+  int64_t* iteration;       /* [1] t, the iteration in progress */
+  int64_t* accepted;        /* [W] accepted proposals per walker */
+  double*  chain;           /* [n_saved][W][K] */
+  double*  chain_lp;        /* [n_saved][W] */
+  int64_t  n_saved;         /* slots of chain / chain_lp */
+  int64_t  chain_base;      /* iteration t stores slot (t+1)/thin - 1 - chain_base (floor(t_start/thin) of the run) */
+} SimplypMcmcState;
+
+/* member_params [W][NP_MEMBER], sc_params [1 or W][S][NP_SC]: the ensemble's rows; half = 0 or 1. */
+int simplyp_mcmc_propose_device(const SimplypMcmc* mc, const SimplypMcmcState* state, int half,
+                                double* member_params, double* sc_params, void* stream);
+/* stats [W/2][V][NSTAT] and diag [W/2][S][NDIAG]: what simplyp_calibrate_device wrote for the active half's rows. */
+int simplyp_mcmc_accept_device(const SimplypMcmc* mc, const SimplypMcmcState* state, int half,
+                               const double* stats, const int64_t* diag, void* stream);
+/* lp [W] of the current walkers from one calibration run of all W rows: stats [W][V][NSTAT], diag [W][S][NDIAG]. */
+int simplyp_mcmc_init_device(const SimplypMcmc* mc, const SimplypMcmcState* state, const double* stats,
+                             const int64_t* diag, void* stream);
+
 /* Host-buffer forms: same arguments as HOST pointers; the library stages them through its own
  * (cached) device buffers on `device`, runs and copies the result back before returning. */
 int simplyp_run_host(int device, const SimplypDims* dims, const SimplypOptions* opt,

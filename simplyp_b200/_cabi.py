@@ -24,7 +24,8 @@ EXPORTS = [
     "simplyp_release_cache", "simplyp_launch_count", "simplyp_measure_fp64_peak",
     "simplyp_measure_fp64_latency", "simplyp_sum_to_waterbody_device", "simplyp_thornthwaite_pet_device",
     "simplyp_calibrate_gather_device", "simplyp_peer_alloc", "simplyp_peer_free", "simplyp_ipc_export",
-    "simplyp_ipc_import", "simplyp_ipc_close",
+    "simplyp_ipc_import", "simplyp_ipc_close", "simplyp_mcmc_propose_device", "simplyp_mcmc_accept_device",
+    "simplyp_mcmc_init_device",
 ]
 MAX_RANKS = 8
 
@@ -46,6 +47,27 @@ class SimplypPeerGather(C.Structure):
     _fields_ = [("n_ranks", C.c_int32), ("rank", C.c_int32), ("member_offset", C.c_int64),
                 ("n_members_total", C.c_int64), ("step", C.c_int64), ("stats_bufs", C.c_void_p * MAX_RANKS),
                 ("flag_bufs", C.c_void_p * MAX_RANKS)]
+
+
+MCMC_MAX_FREE = 64
+MCMC_MEMBER, MCMC_SC_ALL, MCMC_SC_AT = 0, 1, 2
+
+
+class SimplypMcmcParam(C.Structure):
+    _fields_ = [("kind", C.c_int32), ("index", C.c_int32), ("pos", C.c_int32), ("reserved", C.c_int32),
+                ("lo", C.c_double), ("hi", C.c_double)]
+
+
+class SimplypMcmc(C.Structure):
+    _fields_ = [("n_walkers", C.c_int32), ("n_free", C.c_int32), ("n_sc", C.c_int32), ("n_obs_series", C.c_int32),
+                ("sc_per_member", C.c_int32), ("thin", C.c_int32), ("seed", C.c_uint64), ("stretch", C.c_double),
+                ("param", SimplypMcmcParam * MCMC_MAX_FREE)]
+
+
+class SimplypMcmcState(C.Structure):
+    _fields_ = [("walkers", C.c_void_p), ("lp", C.c_void_p), ("proposals", C.c_void_p), ("log_z", C.c_void_p),
+                ("out_of_box", C.c_void_p), ("iteration", C.c_void_p), ("accepted", C.c_void_p),
+                ("chain", C.c_void_p), ("chain_lp", C.c_void_p), ("n_saved", C.c_int64), ("chain_base", C.c_int64)]
 
 
 class SimplypError(RuntimeError):
@@ -111,6 +133,13 @@ def load():
     lib.simplyp_ipc_import.restype = C.c_int
     lib.simplyp_ipc_close.argtypes = [vp]
     lib.simplyp_ipc_close.restype = C.c_int
+    mp, sp = C.POINTER(SimplypMcmc), C.POINTER(SimplypMcmcState)
+    lib.simplyp_mcmc_propose_device.argtypes = [mp, sp, C.c_int, vp, vp, vp]
+    lib.simplyp_mcmc_propose_device.restype = C.c_int
+    lib.simplyp_mcmc_accept_device.argtypes = [mp, sp, C.c_int, vp, vp, vp]
+    lib.simplyp_mcmc_accept_device.restype = C.c_int
+    lib.simplyp_mcmc_init_device.argtypes = [mp, sp, vp, vp, vp]
+    lib.simplyp_mcmc_init_device.restype = C.c_int
     if lib.simplyp_abi_version() != 4:
         raise SimplypError("ABI version mismatch")
     _lib = lib
@@ -305,6 +334,49 @@ def thornthwaite_pet_device(n_days, n_months, t_air_ptr, t_stride, month_start_p
                                                   C.c_void_p(month_start_ptr), C.c_void_p(year_is_leap_ptr),
                                                   float(latitude_deg), C.c_void_p(pet_ptr), int(pet_stride),
                                                   C.c_void_p(stream_ptr)))
+
+
+def make_mcmc(n_walkers, targets, lo, hi, n_sc, n_obs_series, sc_per_member=False, thin=1, seed=0, stretch=2.0):
+    """SimplypMcmc for ``targets`` [(kind, index, pos)] (``MCMC_MEMBER`` / ``MCMC_SC_ALL`` / ``MCMC_SC_AT``) with the
+    prior box ``[lo[k], hi[k]]``."""
+    if not 1 <= len(targets) <= MCMC_MAX_FREE:
+        raise ValueError("1..%d free parameters" % MCMC_MAX_FREE)
+    mc = SimplypMcmc()
+    mc.n_walkers, mc.n_free, mc.n_sc, mc.n_obs_series = int(n_walkers), len(targets), int(n_sc), int(n_obs_series)
+    mc.sc_per_member, mc.thin = 1 if sc_per_member else 0, int(thin)
+    mc.seed, mc.stretch = int(seed) & 0xFFFFFFFFFFFFFFFF, float(stretch)
+    for k, (kind, index, pos) in enumerate(targets):
+        p = mc.param[k]
+        p.kind, p.index, p.pos, p.lo, p.hi = int(kind), int(index), int(pos), float(lo[k]), float(hi[k])
+    return mc
+
+
+def make_mcmc_state(walkers, lp, proposals, log_z, out_of_box, iteration, accepted, chain, chain_lp, n_saved,
+                    chain_base=0):
+    """SimplypMcmcState from device pointers (torch ``.data_ptr()`` integers)."""
+    st = SimplypMcmcState()
+    st.walkers, st.lp, st.proposals, st.log_z = walkers, lp, proposals, log_z
+    st.out_of_box, st.iteration, st.accepted = out_of_box, iteration, accepted
+    st.chain, st.chain_lp, st.n_saved, st.chain_base = chain, chain_lp, int(n_saved), int(chain_base)
+    return st
+
+
+def mcmc_propose_device(mc, state, half, member_ptr, sc_ptr, stream_ptr):
+    """Proposals of walker half ``half`` into its member (and SC) rows; asynchronous on ``stream_ptr``."""
+    lib = require_device()
+    _check(lib.simplyp_mcmc_propose_device(C.byref(mc), C.byref(state), int(half), member_ptr, sc_ptr, stream_ptr))
+
+
+def mcmc_accept_device(mc, state, half, stats_ptr, diag_ptr, stream_ptr):
+    """Metropolis-Hastings step of half ``half`` from its calibration statistics; asynchronous on ``stream_ptr``."""
+    lib = require_device()
+    _check(lib.simplyp_mcmc_accept_device(C.byref(mc), C.byref(state), int(half), stats_ptr, diag_ptr, stream_ptr))
+
+
+def mcmc_init_device(mc, state, stats_ptr, diag_ptr, stream_ptr):
+    """lp of the current walkers from the statistics of one run of all W rows; asynchronous on ``stream_ptr``."""
+    lib = require_device()
+    _check(lib.simplyp_mcmc_init_device(C.byref(mc), C.byref(state), stats_ptr, diag_ptr, stream_ptr))
 
 
 def workspace_bytes(dims, calibrate, rank_stats=False):

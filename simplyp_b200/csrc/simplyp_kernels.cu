@@ -13,6 +13,8 @@
 //   waterbody_kernel                sum_to_waterbody (model.py:851-900)
 //   thornthwaite_kernel             daily_PET (inputs.py:232-312)
 //   fp64_peak_kernel, fp64_latency_kernel  DFMA throughput / latency probes for the roofline denominator
+//   mcmc_propose_kernel, mcmc_accept_kernel, mcmc_advance_kernel, mcmc_init_kernel  ensemble sampler (stretch move,
+//                                   arithmetic in simplyp_mcmc.cuh) over the fused log-likelihood
 //
 // There is deliberately no host implementation of the integration in this library.
 #include <cuda_runtime.h>
@@ -29,6 +31,7 @@
 
 #include "simplyp_quad.cuh"
 #include "simplyp_plan.cuh"
+#include "simplyp_mcmc.cuh"
 
 using namespace simplyp;
 
@@ -1560,6 +1563,93 @@ int check_device_index(int device) {
   return SIMPLYP_OK;
 }
 
+// ------------------------------------------------------------------------------------------ ensemble sampler
+// One thread per walker of the active half (simplyp_mcmc.cuh holds the arithmetic).
+__global__ void mcmc_propose_kernel(const SimplypMcmc mc, const SimplypMcmcState st, int half, double* member_params,
+                                    double* sc_params) {
+  const int H = mc.n_walkers / 2, K = mc.n_free, S = mc.n_sc;
+  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= H) return;
+  const long long t = *st.iteration;
+  double* prop = st.proposals + (size_t)k * K;
+  const int out = mcmc_propose_walker(mc, st.walkers, t, half, k, prop, st.log_z + k);
+  st.out_of_box[k] = out;
+  const int w = half * H + k;
+  const double* src = out ? st.walkers + (size_t)w * K : prop;
+  double* mrow = member_params + (size_t)w * SIMPLYP_NP_MEMBER;
+  double* srow = sc_params + (mc.sc_per_member ? (size_t)w * S * SIMPLYP_NP_SC : 0);
+  for (int i = 0; i < K; ++i) {
+    const SimplypMcmcParam& p = mc.param[i];
+    if (p.kind == SIMPLYP_MCMC_MEMBER) {
+      mrow[p.index] = src[i];
+    } else if (p.kind == SIMPLYP_MCMC_SC_AT) {
+      srow[(size_t)p.pos * SIMPLYP_NP_SC + p.index] = src[i];
+    } else {
+      for (int s = 0; s < S; ++s) srow[(size_t)s * SIMPLYP_NP_SC + p.index] = src[i];
+    }
+  }
+}
+
+// Half 1 also stores the chain slot of the iteration: thread k writes walker k (half 0, final since the half-0
+// accept) and walker H + k (its own).  The counter is advanced by mcmc_advance_kernel after every thread has read it.
+__global__ void mcmc_accept_kernel(const SimplypMcmc mc, const SimplypMcmcState st, int half, const double* stats,
+                                   const int64_t* diag) {
+  const int H = mc.n_walkers / 2, K = mc.n_free, V = mc.n_obs_series, S = mc.n_sc;
+  const int k = blockIdx.x * blockDim.x + threadIdx.x;
+  if (k >= H) return;
+  const long long t = *st.iteration;
+  const double lp_new = st.out_of_box[k]
+                            ? -INFINITY
+                            : mcmc_member_lp(stats + (size_t)k * V * SIMPLYP_NSTAT, V, diag + (size_t)k * S * SIMPLYP_NDIAG, S);
+  mcmc_accept_walker(mc, t, half, k, lp_new, st.log_z[k], st.proposals + (size_t)k * K, st.walkers, st.lp, st.accepted);
+  if (half == 1 && (t + 1) % mc.thin == 0) {
+    const long long slot = (t + 1) / mc.thin - 1 - st.chain_base;
+    if (slot < 0 || slot >= st.n_saved) return;
+    for (int w = k; w < 2 * H; w += H) {
+      for (int i = 0; i < K; ++i)
+        st.chain[((size_t)slot * mc.n_walkers + w) * K + i] = st.walkers[(size_t)w * K + i];
+      st.chain_lp[(size_t)slot * mc.n_walkers + w] = st.lp[w];
+    }
+  }
+}
+
+__global__ void mcmc_advance_kernel(int64_t* iteration) { *iteration += 1; }
+
+__global__ void mcmc_init_kernel(const SimplypMcmc mc, const SimplypMcmcState st, const double* stats,
+                                 const int64_t* diag) {
+  const int w = blockIdx.x * blockDim.x + threadIdx.x;
+  if (w >= mc.n_walkers) return;
+  st.lp[w] = mcmc_member_lp(stats + (size_t)w * mc.n_obs_series * SIMPLYP_NSTAT, mc.n_obs_series,
+                            diag + (size_t)w * mc.n_sc * SIMPLYP_NDIAG, mc.n_sc);
+}
+
+int check_mcmc(const SimplypMcmc* mc, const SimplypMcmcState* st) {
+  if (!mc || !st) return fail(SIMPLYP_EINVAL, "mcmc: null argument%s");
+  const int K = mc->n_free;
+  if (K < 1 || K > SIMPLYP_MCMC_MAX_FREE) return fail(SIMPLYP_EINVAL, "mcmc: 1..SIMPLYP_MCMC_MAX_FREE free parameters%s");
+  if (mc->n_walkers < 2 * K || mc->n_walkers % 2 != 0) return fail(SIMPLYP_EINVAL, "mcmc: an even number of walkers >= 2 K%s");
+  if (mc->n_sc < 1 || mc->n_obs_series < 0 || mc->thin < 1) return fail(SIMPLYP_EINVAL, "mcmc: bad n_sc / n_obs_series / thin%s");
+  if (!(mc->stretch > 1.0 && mc->stretch < INFINITY)) return fail(SIMPLYP_EINVAL, "mcmc: stretch scale must be > 1%s");
+  for (int i = 0; i < K; ++i) {
+    const SimplypMcmcParam& p = mc->param[i];
+    if (!(p.lo < p.hi) || !std::isfinite(p.lo) || !std::isfinite(p.hi)) return fail(SIMPLYP_EINVAL, "mcmc: need finite lo < hi%s");
+    if (p.kind == SIMPLYP_MCMC_MEMBER) {
+      if (p.index < 0 || p.index >= SIMPLYP_NP_MEMBER) return fail(SIMPLYP_EINVAL, "mcmc: member column out of range%s");
+    } else if (p.kind == SIMPLYP_MCMC_SC_ALL || p.kind == SIMPLYP_MCMC_SC_AT) {
+      if (p.index < 0 || p.index >= SIMPLYP_NP_SC) return fail(SIMPLYP_EINVAL, "mcmc: SC row out of range%s");
+      if (p.kind == SIMPLYP_MCMC_SC_AT && (p.pos < 0 || p.pos >= mc->n_sc)) return fail(SIMPLYP_EINVAL, "mcmc: SC position out of range%s");
+      if (!mc->sc_per_member) return fail(SIMPLYP_EINVAL, "mcmc: SC targets need per-member sc_params%s");
+    } else {
+      return fail(SIMPLYP_EINVAL, "mcmc: unknown target kind%s");
+    }
+  }
+  if (!st->walkers || !st->lp || !st->proposals || !st->log_z || !st->out_of_box || !st->iteration || !st->accepted)
+    return fail(SIMPLYP_EINVAL, "mcmc: null state pointer%s");
+  if (st->n_saved < 0 || (st->n_saved > 0 && (!st->chain || !st->chain_lp))) return fail(SIMPLYP_EINVAL, "mcmc: null chain%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  return SIMPLYP_OK;
+}
+
 }  // namespace
 
 // ============================================================================================ C-ABI
@@ -1901,6 +1991,51 @@ int simplyp_thornthwaite_pet_device(int32_t n_days, int32_t n_months, const doub
   if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
   thornthwaite_kernel<<<1, 256, sizeof(double) * 2 * (size_t)n_months, static_cast<cudaStream_t>(stream)>>>(
       n_days, n_months, t_air, t_stride, month_start, year_is_leap, latitude_deg * (M_PI / 180.0), pet, pet_stride);
+  g_launches.fetch_add(1);
+  SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
+int simplyp_mcmc_propose_device(const SimplypMcmc* mc, const SimplypMcmcState* state, int half,
+                                double* member_params, double* sc_params, void* stream) {
+  int rc = check_mcmc(mc, state);
+  if (rc) return rc;
+  if (half != 0 && half != 1) return fail(SIMPLYP_EINVAL, "mcmc: half must be 0 or 1%s");
+  if (!member_params || !sc_params) return fail(SIMPLYP_EINVAL, "mcmc: null parameter rows%s");
+  const int H = mc->n_walkers / 2;
+  mcmc_propose_kernel<<<(H + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(*mc, *state, half,
+                                                                                       member_params, sc_params);
+  g_launches.fetch_add(1);
+  SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
+int simplyp_mcmc_accept_device(const SimplypMcmc* mc, const SimplypMcmcState* state, int half,
+                               const double* stats, const int64_t* diag, void* stream) {
+  int rc = check_mcmc(mc, state);
+  if (rc) return rc;
+  if (half != 0 && half != 1) return fail(SIMPLYP_EINVAL, "mcmc: half must be 0 or 1%s");
+  if (!diag || (mc->n_obs_series > 0 && !stats)) return fail(SIMPLYP_EINVAL, "mcmc: null statistics%s");
+  const int H = mc->n_walkers / 2;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  mcmc_accept_kernel<<<(H + 127) / 128, 128, 0, st>>>(*mc, *state, half, stats, diag);
+  g_launches.fetch_add(1);
+  SP_CUDA(cudaGetLastError());
+  if (half == 1) {
+    mcmc_advance_kernel<<<1, 1, 0, st>>>(state->iteration);
+    g_launches.fetch_add(1);
+    SP_CUDA(cudaGetLastError());
+  }
+  return SIMPLYP_OK;
+}
+
+int simplyp_mcmc_init_device(const SimplypMcmc* mc, const SimplypMcmcState* state, const double* stats,
+                             const int64_t* diag, void* stream) {
+  int rc = check_mcmc(mc, state);
+  if (rc) return rc;
+  if (!diag || (mc->n_obs_series > 0 && !stats)) return fail(SIMPLYP_EINVAL, "mcmc: null statistics%s");
+  mcmc_init_kernel<<<(mc->n_walkers + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(*mc, *state, stats,
+                                                                                               diag);
   g_launches.fetch_add(1);
   SP_CUDA(cudaGetLastError());
   return SIMPLYP_OK;
