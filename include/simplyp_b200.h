@@ -225,7 +225,10 @@ int simplyp_run_device(const SimplypDims* dims, const SimplypOptions* opt,
 /* Calibration mode: same integration, nothing written per day; instead fit statistics against
  * observed series are reduced on the fly.
  *   obs[V][D]     : observed value or NaN, aligned with forcing days
- *   obs_desc[V][2]: (sub-catchment index 0..S-1, series kind SIMPLYP_V_*)
+ *   obs_desc[V][2]: (sub-catchment index 0..S-1, series kind SIMPLYP_V_*); simplyp_calibrate_host refuses any other
+ *                   row with SIMPLYP_EINVAL before device work.  The _device entry points take valid rows as a
+ *                   precondition: checking rows in device memory would need a synchronising copy, which breaks
+ *                   graph capture.  An invalid row there gives undefined statistics for that series.
  *   stats[M][V][SIMPLYP_NSTAT] */
 int simplyp_calibrate_device(const SimplypDims* dims, const SimplypOptions* opt,
                              const double* forcing, const double* member_params, const double* sc_params,

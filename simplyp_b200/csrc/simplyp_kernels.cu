@@ -93,7 +93,7 @@ struct KArgs {
   // The pilot is the FIRST PART of the run: the same kernel integrates days [0, pilot days) in member order, stores
   // every member's midnight state (carry) and its step attempts (cost); the main launch continues at day_begin.
   QuadCarry* carry;             // [M] or null
-  double* carry_stats;          // cal: [M][STAT_SLOTS * 8] shared-memory fit-statistic sums at the hand-over, or null
+  double* carry_stats;          // cal: [M][STAT_SLOTS * RS_COUNT] shared-memory fit-statistic sums at the hand-over, or null
   int day_begin;                // first day this launch integrates (main launch after a pilot), else 0
   int day_end;                  // one past the last day this launch integrates (D, or the pilot's days); D stays the
                                 // length of the record, i.e. the stride of forcing / obs / out
@@ -127,8 +127,10 @@ constexpr int PLAN_SM_LIST = PLAN_SM_ARR + PLAN_MAX_SM;         // [PLAN_MAX_SM]
 constexpr int PLAN_CLAIMED = PLAN_SM_LIST + PLAN_MAX_SM;        // [3 * PLAN_MAX_SM] list taken?
 constexpr int PLAN_INTS = PLAN_CLAIMED + 3 * PLAN_MAX_SM;       // zeroed before every launch
 
-// raw sums kept in stats[][][] while a calibration kernel runs (finalised in place at the end)
-enum { RS_N = 0, RS_SSE, RS_SSE_LOG, RS_LL, RS_S1, RS_S2, RS_SOS, RS_SABS };
+// raw sums kept in stats[][][] while a calibration kernel runs (finalised in place at the end).  S1, S2 and SOS are
+// taken about RS_SHIFT, the simulated value of the series' first observed day (fixed there, carried with the sums).
+enum { RS_N = 0, RS_SSE, RS_SSE_LOG, RS_LL, RS_S1, RS_S2, RS_SOS, RS_SABS, RS_SHIFT, RS_COUNT };
+static_assert((int)RS_COUNT <= (int)SIMPLYP_NSTAT, "the raw sums of a series beyond STAT_SLOTS live in its stats row");
 // obs_const[V][8]
 enum { OC_N = 0, OC_MEAN, OC_SS, OC_MEAN_LOG, OC_SS_LOG, OC_SUM, OC_STD, OC_SS_RANK };
 
@@ -343,14 +345,20 @@ struct RunIO : IOBase<ROUTED> {
 // read-modify-write of eight sums per series in global memory was the largest stall of the day-boundary code.
 // Series beyond STAT_SLOTS on one reach, and the one-thread-per-item kernel, accumulate in stats[][][] directly.
 constexpr int STAT_SLOTS = 6;
-constexpr int STAT_STRIDE = STAT_SLOTS * 8 + 1;      // doubles per item; odd: the 8 quad leaders of a warp hit distinct banks
+constexpr int STAT_STRIDE = STAT_SLOTS * RS_COUNT + 1;   // doubles per item; odd: the 8 quad leaders of a warp hit distinct banks
+static_assert(STAT_SLOTS * RS_COUNT % 2 == 0, "the accumulators are zeroed / restored in pairs");
+// The calibration launches of simplyp_quad_kernel (32 quads a block) do not opt in to more than the default 48 KB of
+// shared memory a block: quad state, forcing ring and these accumulators (dynamic) plus the exp2 table (static).
+static_assert(32 * sizeof(QuadMem) + sizeof(ForcingRing) + 32 * STAT_STRIDE * sizeof(double) +
+                  EXP_TAB * sizeof(double) + 2 * sizeof(int) <= 48 * 1024,
+              "calibration shared memory above 48 KB a block: opt in with cudaFuncAttributeMaxDynamicSharedMemorySize");
 
 template <bool ROUTED>
 struct CalIO : IOBase<ROUTED> {
   using B = IOBase<ROUTED>;
   using B::a; using B::m; using B::s; using B::scp_member;
   double f_TDP;
-  double* sacc;     // shared-memory accumulators of this item [STAT_SLOTS][8], or null
+  double* sacc;     // shared-memory accumulators of this item [STAT_SLOTS][RS_COUNT], or null
   __device__ CalIO(const KArgs& a_, int m_, int s_, ForcingRing* ring_, double f_TDP_, double* sacc_ = nullptr)
       : B(a_, m_, s_, ring_), f_TDP(f_TDP_), sacc(sacc_) {}
 
@@ -418,10 +426,15 @@ struct CalIO : IOBase<ROUTED> {
       const double lsg = (sg > 0.0) ? sp_log(sg) : NAN;
       const double dl = lo - ls;
       const double rsg = sp_rcp(sg);
-      const double ds = sim - mo;
-      double* rs = (sacc != nullptr && k < STAT_SLOTS) ? sacc + 8 * k
+      double* rs = (sacc != nullptr && k < STAT_SLOTS) ? sacc + RS_COUNT * k
                                                        : a.stats + ((size_t)m * a.V + v) * SIMPLYP_NSTAT;
-      rs[RS_N] += 1.0;
+      // the simulated-side sums about a shift near the simulated series, not about mean(obs): S2 - S1^2/n then keeps
+      // its digits when the two means are far apart (observations in other units, a flat offset member)
+      const double n0 = rs[RS_N];
+      const double shift = (n0 == 0.0) ? sim : rs[RS_SHIFT];
+      rs[RS_SHIFT] = shift;
+      const double ds = sim - shift;
+      rs[RS_N] = n0 + 1.0;
       rs[RS_SSE] += d * d;
       rs[RS_SSE_LOG] += dl * dl;
       rs[RS_LL] += -0.91893853320467274178 - lsg - 0.5 * (d * rsg) * (d * rsg);   // MCMC.ipynb:233-236
@@ -439,9 +452,9 @@ struct CalIO : IOBase<ROUTED> {
       const int k = slot++;
       const double* oc = a.obs_const + 8 * v;
       double* rs = a.stats + ((size_t)m * a.V + v) * SIMPLYP_NSTAT;
-      const double* src = (sacc != nullptr && k < STAT_SLOTS) ? sacc + 8 * k : rs;
+      const double* src = (sacc != nullptr && k < STAT_SLOTS) ? sacc + RS_COUNT * k : rs;
       const double n = src[RS_N], sse = src[RS_SSE], ssel = src[RS_SSE_LOG], ll = src[RS_LL];
-      const double s1 = src[RS_S1], s2 = src[RS_S2], sos = src[RS_SOS], sabs = src[RS_SABS];
+      const double s1 = src[RS_S1], s2 = src[RS_S2], sos = src[RS_SOS], sabs = src[RS_SABS], shift = src[RS_SHIFT];
       const double ss_o = oc[OC_SS], ss_lo = oc[OC_SS_LOG], sum_o = oc[OC_SUM], std_o = oc[OC_STD];
       const double var_s = s2 - s1 * s1 / n;
       rs[SIMPLYP_ST_N] = n;
@@ -449,7 +462,7 @@ struct CalIO : IOBase<ROUTED> {
       rs[SIMPLYP_ST_LOG_NSE] = 1.0 - ssel / ss_lo;
       rs[SIMPLYP_ST_LOGLIK] = (ll == ll) ? ll : -INFINITY;       // NaN -> -inf, MCMC.ipynb:238-240
       rs[SIMPLYP_ST_R2] = (sos * sos) / (ss_o * var_s);
-      rs[SIMPLYP_ST_PBIAS] = 100.0 * (s1 + n * oc[OC_MEAN] - sum_o) / sum_o;
+      rs[SIMPLYP_ST_PBIAS] = 100.0 * (s1 + n * shift - sum_o) / sum_o;
       rs[SIMPLYP_ST_NRMSD] = 100.0 * (sabs / n) / std_o;
       rs[SIMPLYP_ST_SSE] = sse;
       rs[SIMPLYP_ST_SPEARMAN] = NAN;            // filled by spearman_kernel when rank statistics are on
@@ -651,8 +664,9 @@ __global__ void __launch_bounds__(128, MINB) simplyp_quad_kernel(const KArgs a) 
     if (MODE == MODE_CAL) {
       sacc = reinterpret_cast<double*>(ring + 1) + (size_t)(threadIdx.x >> 2) * STAT_STRIDE;
       if ((threadIdx.x & 3) == 0) {
-        const double* src = resume ? a.carry_stats + ci * (STAT_SLOTS * 8) : nullptr;
-        for (int i = 0; i < STAT_SLOTS * 8; ++i) sacc[i] = src ? src[i] : 0.0;
+        const double* src = resume ? a.carry_stats + ci * (STAT_SLOTS * RS_COUNT) : nullptr;
+        // (in pairs: the 2- and 3-blocks-per-SM builds then keep the register allocation they had with 8 sums a series)
+        for (int i = 0; i < STAT_SLOTS * RS_COUNT; i += 2) { sacc[i] = src ? src[i] : 0.0; sacc[i + 1] = src ? src[i + 1] : 0.0; }
       }
       __syncwarp();
     }
@@ -666,8 +680,8 @@ __global__ void __launch_bounds__(128, MINB) simplyp_quad_kernel(const KArgs a) 
       run_quad<STIFF>(q, mp, sp, A_qr0, nc_last, a.topt, day_end, valid, qm, io, cnt, day_begin, cin, cout, resume, hand_over);
       if (valid && q.ql == 0) {
         if (hand_over) {
-          double* dst = a.carry_stats + ci * (STAT_SLOTS * 8);
-          for (int i = 0; i < STAT_SLOTS * 8; ++i) dst[i] = sacc[i];
+          double* dst = a.carry_stats + ci * (STAT_SLOTS * RS_COUNT);
+          for (int i = 0; i < STAT_SLOTS * RS_COUNT; ++i) dst[i] = sacc[i];
         } else {
           io.finalise();
         }
@@ -1163,7 +1177,7 @@ WsLayout ws_layout(const SimplypDims& d, int n_edges, bool cal, bool ranks = fal
   L.off_carry = o;
   o = align_up(o + sizeof(QuadCarry) * n_carry);
   L.off_carry_stats = o;
-  if (cal) o = align_up(o + sizeof(double) * STAT_SLOTS * 8 * n_carry);
+  if (cal) o = align_up(o + sizeof(double) * STAT_SLOTS * RS_COUNT * n_carry);
   L.off_ticket = o; o = align_up(o + sizeof(int));
   L.off_progress = o;
   if (d.n_sc > 1) o = align_up(o + sizeof(int) * (size_t)d.n_members * d.n_sc);
@@ -1927,6 +1941,17 @@ int simplyp_calibrate_host(int device, const SimplypDims* dims, const SimplypOpt
   if (rc) return rc;
   if (dims->n_obs_series <= 0 || !obs || !obs_desc || !stats)
     return fail(SIMPLYP_EINVAL, "observations and statistics buffers required%s");
+  // the rows are in host memory here, so they are checked before any device work (the device entry points take them
+  // as a precondition: a reach outside 0..S-1 is never finalised, a kind outside 0..5 reads another parameter)
+  for (int v = 0; v < dims->n_obs_series; ++v) {
+    const int32_t sc = obs_desc[2 * v], kind = obs_desc[2 * v + 1];
+    if (sc < 0 || sc >= dims->n_sc || kind < 0 || kind >= SIMPLYP_NVARKIND) {
+      char row[160];
+      snprintf(row, sizeof(row), "obs_desc row %d = (%d, %d): reach must be in 0..%d and kind in 0..%d", v, (int)sc,
+               (int)kind, dims->n_sc - 1, SIMPLYP_NVARKIND - 1);
+      return fail(SIMPLYP_EINVAL, "%s", row);
+    }
+  }
   rc = check_device_index(device);
   if (rc) return rc;
   HostCache& hc = g_cache[device];
