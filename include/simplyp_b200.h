@@ -357,6 +357,35 @@ int simplyp_mcmc_accept_device(const SimplypMcmc* mc, const SimplypMcmcState* st
 int simplyp_mcmc_init_device(const SimplypMcmc* mc, const SimplypMcmcState* state, const double* stats,
                              const int64_t* diag, void* stream);
 
+/* ---- posterior predictive bands -----------------------------------------------------------------------------------
+ * Quantiles over an ensemble of the simulated series the fused statistics see (SIMPLYP_V_* kinds of a reach), with or
+ * without the likelihood's error model N(o; s, (m s)^2), m = member_params[.][SIMPLYP_P_ERR_M0 + kind].
+ *
+ * simplyp_predictive_draws_device: for a chunk of M members (dims: M, S, D, Msc = 1 or M) of a full-output run,
+ *   out[M][S][D][25], member_params[M][NP_MEMBER], sc_params[Msc][S][NP_SC], diag[M][S][NDIAG], and
+ *   series_desc[n_series][2] = (run-order reach 0..S-1, kind 0..5) on the device (a device-side precondition, like
+ *   obs_desc), writes draws[n_series][D][n_members_total] at columns member_offset .. member_offset + M - 1:
+ *     y = sim                        (obs_error = 0)
+ *     y = sim + (m sim) eps          (obs_error = 1; eps standard normal by Box-Muller from Philox4x32-10 keyed by
+ *                                     `seed` with counter (member_offset + m, day, series, 2): a pure function of
+ *                                     (seed, member, day, series), whatever the chunking)
+ *   A member with a non-zero SIMPLYP_DG_STATUS word at any reach draws NaN everywhere.
+ * simplyp_nanquantile_device: for every row of x[n_rows][n_cols], exactly np.nanquantile(row, q, method='linear')
+ *   (NaNs dropped; an all-NaN row gives NaN) into quantiles[n_q][n_rows], the mean of the non-NaN entries into
+ *   mean[n_rows] and their count into count[n_rows].  q[n_q] is a HOST array of values in [0, 1], n_q <= SIMPLYP_NQ_MAX,
+ *   passed to the kernels by value.  Rows longer than one block's shared memory holds (about 29k entries on B200) need
+ *   simplyp_nanquantile_workspace_bytes(n_rows, n_cols) bytes of device workspace (0 otherwise).
+ * Both only enqueue work on `stream` (no allocation, no synchronisation), so they can be captured into a graph. */
+#define SIMPLYP_NQ_MAX 16
+int simplyp_predictive_draws_device(const SimplypDims* dims, const double* out, const double* member_params,
+                                    const double* sc_params, const int64_t* diag, const int32_t* series_desc,
+                                    int32_t n_series, double* draws, int64_t n_members_total, int64_t member_offset,
+                                    int32_t obs_error, uint64_t seed, void* stream);
+int64_t simplyp_nanquantile_workspace_bytes(int64_t n_rows, int64_t n_cols);
+int simplyp_nanquantile_device(const double* x, int64_t n_rows, int64_t n_cols, const double* q, int32_t n_q,
+                               double* quantiles, double* mean, int64_t* count, void* workspace,
+                               int64_t workspace_bytes, void* stream);
+
 /* Host-buffer forms: same arguments as HOST pointers; the library stages them through its own
  * (cached) device buffers on `device`, runs and copies the result back before returning. */
 int simplyp_run_host(int device, const SimplypDims* dims, const SimplypOptions* opt,

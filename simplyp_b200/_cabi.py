@@ -25,7 +25,8 @@ EXPORTS = [
     "simplyp_measure_fp64_latency", "simplyp_sum_to_waterbody_device", "simplyp_thornthwaite_pet_device",
     "simplyp_calibrate_gather_device", "simplyp_peer_alloc", "simplyp_peer_free", "simplyp_ipc_export",
     "simplyp_ipc_import", "simplyp_ipc_close", "simplyp_mcmc_propose_device", "simplyp_mcmc_accept_device",
-    "simplyp_mcmc_init_device",
+    "simplyp_mcmc_init_device", "simplyp_predictive_draws_device", "simplyp_nanquantile_workspace_bytes",
+    "simplyp_nanquantile_device",
 ]
 MAX_RANKS = 8
 
@@ -50,6 +51,7 @@ class SimplypPeerGather(C.Structure):
 
 
 MCMC_MAX_FREE = 64
+NQ_MAX = 16
 MCMC_MEMBER, MCMC_SC_ALL, MCMC_SC_AT = 0, 1, 2
 
 
@@ -140,6 +142,13 @@ def load():
     lib.simplyp_mcmc_accept_device.restype = C.c_int
     lib.simplyp_mcmc_init_device.argtypes = [mp, sp, vp, vp, vp]
     lib.simplyp_mcmc_init_device.restype = C.c_int
+    lib.simplyp_predictive_draws_device.argtypes = [C.POINTER(SimplypDims), vp, vp, vp, vp, vp, C.c_int32, vp,
+                                                    C.c_int64, C.c_int64, C.c_int32, C.c_uint64, vp]
+    lib.simplyp_predictive_draws_device.restype = C.c_int
+    lib.simplyp_nanquantile_workspace_bytes.argtypes = [C.c_int64, C.c_int64]
+    lib.simplyp_nanquantile_workspace_bytes.restype = C.c_int64
+    lib.simplyp_nanquantile_device.argtypes = [vp, C.c_int64, C.c_int64, dp, C.c_int32, vp, vp, vp, vp, C.c_int64, vp]
+    lib.simplyp_nanquantile_device.restype = C.c_int
     if lib.simplyp_abi_version() != 4:
         raise SimplypError("ABI version mismatch")
     _lib = lib
@@ -377,6 +386,32 @@ def mcmc_init_device(mc, state, stats_ptr, diag_ptr, stream_ptr):
     """lp of the current walkers from the statistics of one run of all W rows; asynchronous on ``stream_ptr``."""
     lib = require_device()
     _check(lib.simplyp_mcmc_init_device(C.byref(mc), C.byref(state), stats_ptr, diag_ptr, stream_ptr))
+
+
+def predictive_draws_device(dims, out_ptr, member_ptr, sc_ptr, diag_ptr, series_desc_ptr, n_series, draws_ptr,
+                            n_members_total, member_offset, obs_error, seed, stream_ptr):
+    """Draws of the simulated series of one full-output chunk into its columns of draws [V][D][M_total];
+    asynchronous on ``stream_ptr``."""
+    lib = require_device()
+    _check(lib.simplyp_predictive_draws_device(C.byref(dims), out_ptr, member_ptr, sc_ptr, diag_ptr, series_desc_ptr,
+                                               int(n_series), draws_ptr, int(n_members_total), int(member_offset),
+                                               1 if obs_error else 0, int(seed) & 0xFFFFFFFFFFFFFFFF, stream_ptr))
+
+
+def nanquantile_workspace_bytes(n_rows, n_cols):
+    n = load().simplyp_nanquantile_workspace_bytes(int(n_rows), int(n_cols))
+    if n < 0:
+        _check(int(n))
+    return int(n)
+
+
+def nanquantile_device(x_ptr, n_rows, n_cols, q, quant_ptr, mean_ptr, count_ptr, ws_ptr, ws_bytes, stream_ptr):
+    """np.nanquantile of every row of x [n_rows][n_cols] (``q`` a host sequence) into quantiles [n_q][n_rows], the
+    mean and the count of the non-NaN entries; asynchronous on ``stream_ptr``."""
+    lib = require_device()
+    qa = (C.c_double * max(len(q), 1))(*[float(v) for v in q])
+    _check(lib.simplyp_nanquantile_device(x_ptr, int(n_rows), int(n_cols), qa, len(q), quant_ptr, mean_ptr, count_ptr,
+                                          ws_ptr, int(ws_bytes), stream_ptr))
 
 
 def workspace_bytes(dims, calibrate, rank_stats=False):

@@ -15,6 +15,8 @@
 //   fp64_peak_kernel, fp64_latency_kernel  DFMA throughput / latency probes for the roofline denominator
 //   mcmc_propose_kernel, mcmc_accept_kernel, mcmc_advance_kernel, mcmc_init_kernel  ensemble sampler (stretch move,
 //                                   arithmetic in simplyp_mcmc.cuh) over the fused log-likelihood
+//   predictive_draws_kernel         posterior predictive draws of the simulated series (simplyp_bands.cuh)
+//   nanquantile_kernel, nq_prepare_kernel, nq_hist_kernel, nq_pick_kernel  np.nanquantile of the rows of a matrix
 //
 // There is deliberately no host implementation of the integration in this library.
 #include <cuda_runtime.h>
@@ -32,6 +34,7 @@
 #include "simplyp_quad.cuh"
 #include "simplyp_plan.cuh"
 #include "simplyp_mcmc.cuh"
+#include "simplyp_bands.cuh"
 
 using namespace simplyp;
 
@@ -389,9 +392,10 @@ struct CalIO : IOBase<ROUTED> {
       double* row = a.flux + (((size_t)m * a.S + s) * a.D + day) * 4;
       row[0] = acc[0]; row[1] = acc[1]; row[2] = acc[2]; row[3] = acc[3];
     }
-    // simulated counterparts of the observed series in the reference's own order of operations (model.py:784-793,
-    // :840-845): Q_cumecs = Qr*A*1000/86400, concentrations (flux/Qr)/A_catch.  The quotients are formed by sp_div
-    // (reciprocal, product, one fma of the exact remainder: the IEEE quotient in all but rare last-bit cases) because
+    // simulated counterparts of the observed series (sim_series_value, simplyp_bands.cuh) in the reference's own order
+    // of operations (model.py:784-793, :840-845): Q_cumecs = Qr*A*1000/86400, concentrations (flux/Qr)/A_catch.
+    // The quotients are formed by sp_div (reciprocal, product, one fma of the exact remainder: the IEEE quotient in
+    // all but rare last-bit cases) because
     // Spearman's r is sensitive to the last bit wherever simulated values tie (recession days at the groundwater floor:
     // 2e-6 on 13,700 pairs between two orders of evaluation).  A true IEEE division would bring its slow-path
     // subroutine into the kernel: its mere presence, never executed, cost 2-3 % of the run time (A/B on one box).
@@ -404,15 +408,7 @@ struct CalIO : IOBase<ROUTED> {
       const double o = __ldg(a.obs + (size_t)v * a.D + day);
       if (o != o) continue;  // no observation that day
       const int kind = __ldg(a.obs_desc + 2 * v + 1);
-      double sim;
-      switch (kind) {
-        case SIMPLYP_V_Q:   sim = sp_div(acc[0] * A * 1000.0, 86400.0, 1.0 / 86400.0); break;
-        case SIMPLYP_V_SS:  sim = sp_div(sp_div(acc[1], acc[0], rQ), A, rA); break;
-        case SIMPLYP_V_TDP: sim = sp_div(sp_div(acc[2], acc[0], rQ), A, rA); break;
-        case SIMPLYP_V_PP:  sim = sp_div(sp_div(acc[3], acc[0], rQ), A, rA); break;
-        case SIMPLYP_V_TP:  sim = sp_div(sp_div(acc[2], acc[0], rQ), A, rA) + sp_div(sp_div(acc[3], acc[0], rQ), A, rA); break;
-        default:            sim = sp_div(sp_div(acc[2], acc[0], rQ), A, rA) * f_TDP; break;
-      }
+      const double sim = sim_series_value(kind, acc[0], acc[1], acc[2], acc[3], A, rQ, rA, f_TDP);   // (predictive_draws_kernel too)
       if (a.sim_obs != nullptr) a.sim_obs[((size_t)m * a.V + v) * a.D + day] = sim;
       const double* oc = a.obs_const + 8 * v;
       const double mo = __ldg(oc + OC_MEAN);
@@ -1664,6 +1660,246 @@ int check_mcmc(const SimplypMcmc* mc, const SimplypMcmcState* st) {
   return SIMPLYP_OK;
 }
 
+// ------------------------------------------------------------------------------------------ predictive bands
+// Draws of V simulated series (sim_series_value, the values the fused statistics see) from the full output of a chunk
+// of Mc members, optionally through the likelihood's error model (band_draw / band_epsilon): one block per
+// (32 days, 32 members, series), 32 x 8 threads.  The out rows are read with the lane over days (consecutive rows of
+// one member), the tile is transposed in shared memory and written with the lane over members, since
+// draws[v][d][member_offset + m] is member-contiguous for the selection.  A member with a non-zero status word at any
+// reach draws NaN everywhere (the sampler gives it -inf).
+constexpr int DRAW_TILE = 32;
+__global__ void __launch_bounds__(256) predictive_draws_kernel(const double* out, const double* member_params,
+                                                               const double* sc_params, const int64_t* diag,
+                                                               const int32_t* series_desc, int Mc, int S, int D,
+                                                               int Msc, long long M_total, long long member_offset,
+                                                               int obs_error, uint64_t seed, double* draws) {
+  __shared__ double tile[DRAW_TILE][DRAW_TILE + 1];
+  __shared__ int failed[DRAW_TILE];
+  const int v = blockIdx.z, d0 = blockIdx.x * DRAW_TILE, m0 = blockIdx.y * DRAW_TILE;
+  const int tx = threadIdx.x, ty = threadIdx.y;
+  const int s = series_desc[2 * v], kind = series_desc[2 * v + 1];
+  if (ty == 0) {
+    int f = 0;
+    if (m0 + tx < Mc)
+      for (int r = 0; r < S; ++r) f |= diag[((size_t)(m0 + tx) * S + r) * SIMPLYP_NDIAG + SIMPLYP_DG_STATUS] != 0;
+    failed[tx] = f;
+  }
+  __syncthreads();
+  const int d = d0 + tx;
+  for (int j = ty; j < DRAW_TILE; j += blockDim.y) {
+    const int m = m0 + j;
+    if (m >= Mc || d >= D) continue;
+    double y = NAN;
+    if (!failed[j]) {
+      const double* row = out + (((size_t)m * S + s) * D + d) * SIMPLYP_NOUT;
+      const double* mp = member_params + (size_t)m * SIMPLYP_NP_MEMBER;
+      const double A = sc_params[((size_t)(Msc > 1 ? m : 0) * S + s) * SIMPLYP_NP_SC + SIMPLYP_SC_A_CATCH];
+      const double Qr = row[SIMPLYP_O_QR];
+      y = sim_series_value(kind, Qr, row[SIMPLYP_O_MSUS_FLUX], row[SIMPLYP_O_TDP_FLUX], row[SIMPLYP_O_PP_FLUX], A,
+                           sp_rcp(Qr), sp_rcp(A), mp[SIMPLYP_P_F_TDP]);
+      if (obs_error)
+        y = band_draw(y, mp[SIMPLYP_P_ERR_M0 + kind], band_epsilon(seed, (int)(member_offset + m), d, v));
+    }
+    tile[j][tx] = y;
+  }
+  __syncthreads();
+  const int m = m0 + tx;
+  for (int j = ty; j < DRAW_TILE; j += blockDim.y) {
+    const int dd = d0 + j;
+    if (m < Mc && dd < D) draws[((size_t)v * D + dd) * M_total + member_offset + m] = tile[tx][j];
+  }
+}
+
+// np.nanquantile(x, q, axis=-1) of every row of x[R][N], with the mean and the count of the non-NaN entries.  The
+// quantile values travel by value in the launch (a captured launch replays them).  Order statistics are exact: the
+// entries are turned into order-preserving keys (nq_key, NaN last) and either sorted in shared memory
+// (nanquantile_kernel, one block a row) or selected digit by digit in global memory (nq_*_kernel, longer rows).
+struct NqArgs {
+  int n_q;
+  double q[SIMPLYP_NQ_MAX];
+};
+constexpr int NQ_THREADS = 1024;
+constexpr int NQ_RANKS = 2 * SIMPLYP_NQ_MAX;     // two neighbours a quantile
+constexpr int NQ_BINS = 256;                      // 8-bit digits, 8 passes
+// Global-path workspace of one row: histograms [NQ_RANKS][NQ_BINS], then rank left / key prefix per neighbour, the
+// weights g and the count.
+struct NqRow {
+  unsigned hist[NQ_RANKS][NQ_BINS];
+  unsigned long long k[NQ_RANKS];
+  unsigned long long prefix[NQ_RANKS];
+  double g[SIMPLYP_NQ_MAX];
+  long long n;
+};
+
+// Count and sum of the non-NaN entries of one row, reduced in a fixed order (the result does not depend on timing).
+// Every thread returns the block's totals.
+__device__ void nq_count_sum(const double* row, long long N, uint64_t* keys, long long* n_out, double* sum_out) {
+  __shared__ double red_s[NQ_THREADS / 32];
+  __shared__ long long red_n[NQ_THREADS / 32];
+  double sum = 0.0;
+  long long n = 0;
+  for (long long i = threadIdx.x; i < N; i += blockDim.x) {
+    const double v = row[i];
+    if (keys) keys[i] = nq_key(v);
+    if (v == v) { sum += v; ++n; }
+  }
+  for (int o = 16; o > 0; o >>= 1) {
+    sum += __shfl_down_sync(0xffffffffu, sum, o);
+    n += __shfl_down_sync(0xffffffffu, n, o);
+  }
+  const int w = threadIdx.x >> 5, nw = blockDim.x >> 5;
+  if ((threadIdx.x & 31) == 0) { red_s[w] = sum; red_n[w] = n; }
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    sum = threadIdx.x < nw ? red_s[threadIdx.x] : 0.0;
+    n = threadIdx.x < nw ? red_n[threadIdx.x] : 0;
+    for (int o = 16; o > 0; o >>= 1) {
+      sum += __shfl_down_sync(0xffffffffu, sum, o);
+      n += __shfl_down_sync(0xffffffffu, n, o);
+    }
+    if (threadIdx.x == 0) { red_s[0] = sum; red_n[0] = n; }
+  }
+  __syncthreads();
+  *sum_out = red_s[0];
+  *n_out = red_n[0];
+}
+
+// Rows of N <= the shared-memory capacity: keys[N] in dynamic shared memory, sorted by a bitonic network on the next
+// power of two.  The comparators all put the smaller key first (the first step of every merge compares mirrored
+// positions), so the virtual padding of largest keys never moves and every comparator that reaches it is skipped.
+__global__ void __launch_bounds__(NQ_THREADS) nanquantile_kernel(const double* x, long long R, long long N,
+                                                                 const NqArgs qa, double* quant, double* mean,
+                                                                 int64_t* count) {
+  extern __shared__ uint64_t keys[];
+  const long long r = blockIdx.x;
+  long long n;
+  double sum;
+  nq_count_sum(x + r * N, N, keys, &n, &sum);
+  long long P = 1;
+  while (P < N) P <<= 1;
+  for (long long k = 2; k <= P; k <<= 1) {
+    for (long long j = k >> 1; j > 0; j >>= 1) {
+      for (long long t = threadIdx.x; t < P / 2; t += blockDim.x) {
+        const long long i = 2 * j * (t / j) + (t % j);
+        const long long p = (j == (k >> 1)) ? (i ^ (k - 1)) : (i + j);
+        if (p < N) {
+          const uint64_t a = keys[i], b = keys[p];
+          if (b < a) { keys[i] = b; keys[p] = a; }
+        }
+      }
+      __syncthreads();
+    }
+  }
+  if (threadIdx.x < qa.n_q) {
+    double res = NAN;
+    if (n > 0) {
+      long long lo, hi;
+      double g;
+      nq_index(n, qa.q[threadIdx.x], &lo, &hi, &g);
+      res = nq_lerp(nq_value(keys[lo]), nq_value(keys[hi]), g);
+    }
+    quant[(size_t)threadIdx.x * R + r] = res;
+  }
+  if (threadIdx.x == 0) {
+    mean[r] = n > 0 ? sum / (double)n : NAN;
+    count[r] = n;
+  }
+}
+
+// Longer rows, 1: count, mean and the ranks of the neighbours of every quantile; histograms zeroed.
+__global__ void __launch_bounds__(NQ_THREADS) nq_prepare_kernel(const double* x, long long N, const NqArgs qa,
+                                                                NqRow* ws, double* mean, int64_t* count) {
+  const long long r = blockIdx.x;
+  NqRow& w = ws[r];
+  long long n;
+  double sum;
+  nq_count_sum(x + r * N, N, nullptr, &n, &sum);
+  for (int i = threadIdx.x; i < NQ_RANKS * NQ_BINS; i += blockDim.x) (&w.hist[0][0])[i] = 0u;
+  if (threadIdx.x < qa.n_q && n > 0) {
+    long long lo, hi;
+    double g;
+    nq_index(n, qa.q[threadIdx.x], &lo, &hi, &g);
+    w.k[2 * threadIdx.x] = (unsigned long long)lo;
+    w.k[2 * threadIdx.x + 1] = (unsigned long long)hi;
+    w.prefix[2 * threadIdx.x] = w.prefix[2 * threadIdx.x + 1] = 0ull;
+    w.g[threadIdx.x] = g;
+  }
+  if (threadIdx.x == 0) {
+    w.n = n;
+    mean[r] = n > 0 ? sum / (double)n : NAN;
+    count[r] = n;
+  }
+}
+
+// 2: the histogram of digit `pass` (from the top) of the keys that share each neighbour's prefix so far; blocks of
+// 256 threads over a slice (blockIdx.y) of one row (blockIdx.x), counted in shared memory first.
+constexpr int NQ_HIST_THREADS = 256, NQ_HIST_PER_THREAD = 16;
+__global__ void __launch_bounds__(NQ_HIST_THREADS) nq_hist_kernel(const double* x, long long N, int n_q, int pass,
+                                                                  NqRow* ws) {
+  __shared__ unsigned h[NQ_RANKS][NQ_BINS];
+  __shared__ unsigned long long pre[NQ_RANKS];
+  const long long r = blockIdx.x;
+  NqRow& w = ws[r];
+  const int nr = 2 * n_q;
+  for (int i = threadIdx.x; i < NQ_RANKS * NQ_BINS; i += blockDim.x) (&h[0][0])[i] = 0u;
+  if (threadIdx.x < nr) pre[threadIdx.x] = w.prefix[threadIdx.x];
+  __syncthreads();
+  if (w.n == 0) return;
+  const int shift = 56 - 8 * pass;
+  const unsigned long long mask = pass == 0 ? 0ull : (~0ull << (shift + 8));
+  const long long base = (long long)blockIdx.y * NQ_HIST_THREADS * NQ_HIST_PER_THREAD;
+  const double* row = x + r * N;
+  for (int e = 0; e < NQ_HIST_PER_THREAD; ++e) {
+    const long long i = base + (long long)e * NQ_HIST_THREADS + threadIdx.x;
+    if (i >= N) break;
+    const uint64_t key = nq_key(row[i]);
+    const unsigned digit = (unsigned)(key >> shift) & 0xFFu;
+    for (int j = 0; j < nr; ++j)
+      if (((key ^ pre[j]) & mask) == 0) atomicAdd(&h[j][digit], 1u);
+  }
+  __syncthreads();
+  for (int i = threadIdx.x; i < nr * NQ_BINS; i += blockDim.x) {
+    const unsigned c = (&h[0][0])[i];
+    if (c) atomicAdd(&(&w.hist[0][0])[i], c);
+  }
+}
+
+// 3: every neighbour takes the digit whose cumulative count passes its rank; the histograms are zeroed for the next
+// pass.  After the last pass the prefixes are the keys of the neighbours and the quantiles are interpolated.
+__global__ void nq_pick_kernel(long long R, const NqArgs qa, int pass, NqRow* ws, double* quant) {
+  const long long r = blockIdx.x;
+  NqRow& w = ws[r];
+  const int j = threadIdx.x, nr = 2 * qa.n_q;
+  if (j < nr && w.n > 0) {
+    const int shift = 56 - 8 * pass;
+    unsigned long long k = w.k[j], below = 0;
+    int b = 0;
+    for (; b < NQ_BINS - 1; ++b) {
+      const unsigned long long c = w.hist[j][b];
+      if (below + c > k) break;
+      below += c;
+    }
+    w.k[j] = k - below;
+    w.prefix[j] |= (unsigned long long)b << shift;
+    for (int i = 0; i < NQ_BINS; ++i) w.hist[j][i] = 0u;
+  }
+  if (pass == 7) {
+    __syncthreads();
+    if (j < qa.n_q)
+      quant[(size_t)j * R + r] =
+          w.n > 0 ? nq_lerp(nq_value(w.prefix[2 * j]), nq_value(w.prefix[2 * j + 1]), w.g[j]) : NAN;
+  }
+}
+
+// Rows up to this many entries take the shared-memory path on the current device.
+long long nq_shared_cap() {
+  int dev = 0, optin = 0;
+  if (cudaGetDevice(&dev) != cudaSuccess ||
+      cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
+    return 0;
+  return (optin - 1024) / (long long)sizeof(uint64_t);   // (1 KB for the reductions' static shared memory)
+}
+
 }  // namespace
 
 // ============================================================================================ C-ABI
@@ -2063,6 +2299,80 @@ int simplyp_mcmc_init_device(const SimplypMcmc* mc, const SimplypMcmcState* stat
                                                                                                diag);
   g_launches.fetch_add(1);
   SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
+int simplyp_predictive_draws_device(const SimplypDims* dims, const double* out, const double* member_params,
+                                    const double* sc_params, const int64_t* diag, const int32_t* series_desc,
+                                    int32_t n_series, double* draws, int64_t n_members_total, int64_t member_offset,
+                                    int32_t obs_error, uint64_t seed, void* stream) {
+  if (!dims || !out || !member_params || !sc_params || !diag || !series_desc || !draws)
+    return fail(SIMPLYP_EINVAL, "predictive draws: null argument%s");
+  const int M = dims->n_members, S = dims->n_sc, D = dims->n_days, Msc = dims->n_sc_param_sets;
+  if (M < 1 || M > 65535 * DRAW_TILE || S < 1 || D < 0 || (Msc != 1 && Msc != M) || n_series < 1 || n_series > 65535)
+    return fail(SIMPLYP_EINVAL, "predictive draws: bad dims (1 <= M <= 2097120 a chunk, S >= 1, D >= 0, Msc = 1 or M, "
+                                "1..65535 series)%s");
+  if (member_offset < 0 || n_members_total > INT32_MAX || member_offset + M > n_members_total)
+    return fail(SIMPLYP_EINVAL, "predictive draws: members outside 0..n_members_total - 1 (at most 2^31 - 1)%s");
+  if (obs_error != 0 && obs_error != 1) return fail(SIMPLYP_EINVAL, "predictive draws: obs_error must be 0 or 1%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  if (D == 0) return SIMPLYP_OK;
+  const dim3 grid((unsigned)((D + DRAW_TILE - 1) / DRAW_TILE), (unsigned)((M + DRAW_TILE - 1) / DRAW_TILE),
+                  (unsigned)n_series);
+  predictive_draws_kernel<<<grid, dim3(DRAW_TILE, 8), 0, static_cast<cudaStream_t>(stream)>>>(
+      out, member_params, sc_params, diag, series_desc, M, S, D, Msc, n_members_total, member_offset, obs_error, seed,
+      draws);
+  g_launches.fetch_add(1);
+  SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
+int64_t simplyp_nanquantile_workspace_bytes(int64_t n_rows, int64_t n_cols) {
+  if (n_rows < 0 || n_cols < 0) return fail(SIMPLYP_EINVAL, "nanquantile: negative dims%s");
+  if (n_cols <= nq_shared_cap()) return 0;
+  return n_rows * (int64_t)sizeof(NqRow);
+}
+
+int simplyp_nanquantile_device(const double* x, int64_t n_rows, int64_t n_cols, const double* q, int32_t n_q,
+                               double* quantiles, double* mean, int64_t* count, void* workspace,
+                               int64_t workspace_bytes, void* stream) {
+  if (!x || !q || !quantiles || !mean || !count) return fail(SIMPLYP_EINVAL, "nanquantile: null argument%s");
+  if (n_rows < 0 || n_rows > INT32_MAX || n_cols < 1 || n_q < 1 || n_q > SIMPLYP_NQ_MAX)
+    return fail(SIMPLYP_EINVAL, "nanquantile: bad dims (0..2^31 - 1 rows, n_cols >= 1, 1..SIMPLYP_NQ_MAX quantiles)%s");
+  NqArgs qa;
+  qa.n_q = n_q;
+  for (int i = 0; i < SIMPLYP_NQ_MAX; ++i) qa.q[i] = i < n_q ? q[i] : 0.0;
+  for (int i = 0; i < n_q; ++i)
+    if (!(qa.q[i] >= 0.0 && qa.q[i] <= 1.0)) return fail(SIMPLYP_EINVAL, "nanquantile: quantiles must lie in [0, 1]%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  const int64_t need = simplyp_nanquantile_workspace_bytes(n_rows, n_cols);
+  if (need > 0 && (!workspace || workspace_bytes < need))
+    return fail(SIMPLYP_EINVAL, "nanquantile: workspace smaller than simplyp_nanquantile_workspace_bytes%s");
+  if (n_rows == 0) return SIMPLYP_OK;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  if (need == 0) {
+    const size_t smem = (size_t)n_cols * sizeof(uint64_t);
+    if (smem > 48 * 1024)
+      SP_CUDA(cudaFuncSetAttribute(nanquantile_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    nanquantile_kernel<<<(unsigned)n_rows, NQ_THREADS, smem, st>>>(x, n_rows, n_cols, qa, quantiles, mean, count);
+    g_launches.fetch_add(1);
+    SP_CUDA(cudaGetLastError());
+    return SIMPLYP_OK;
+  }
+  const long long per_block = (long long)NQ_HIST_THREADS * NQ_HIST_PER_THREAD;
+  const long long slices = (n_cols + per_block - 1) / per_block;
+  if (slices > 65535) return fail(SIMPLYP_EINVAL, "nanquantile: rows of at most 65535 * 4096 entries%s");
+  NqRow* ws = static_cast<NqRow*>(workspace);
+  nq_prepare_kernel<<<(unsigned)n_rows, NQ_THREADS, 0, st>>>(x, n_cols, qa, ws, mean, count);
+  g_launches.fetch_add(1);
+  SP_CUDA(cudaGetLastError());
+  const dim3 hgrid((unsigned)n_rows, (unsigned)slices);
+  for (int pass = 0; pass < 8; ++pass) {
+    nq_hist_kernel<<<hgrid, NQ_HIST_THREADS, 0, st>>>(x, n_cols, n_q, pass, ws);
+    nq_pick_kernel<<<(unsigned)n_rows, NQ_RANKS, 0, st>>>(n_rows, qa, pass, ws, quantiles);
+    g_launches.fetch_add(2);
+    SP_CUDA(cudaGetLastError());
+  }
   return SIMPLYP_OK;
 }
 

@@ -151,6 +151,47 @@ class Engine:
                                           r.data_ptr(), int(r.numel()), wb.data_ptr(), stream)
         return wb
 
+    # ------------------------------------------------------------------ posterior predictive bands
+    def predictive_draws(self, out, member_params, sc_params, diag, series_desc, draws, member_offset=0,
+                         obs_error=False, seed=0):
+        """Simulated series of a full-output chunk (``out`` [Mc][S][D][25], ``diag`` [Mc][S][4] from :meth:`run`)
+        written into columns ``member_offset .. member_offset + Mc`` of ``draws`` [V][D][M_total] for the series
+        ``series_desc`` [V][2] int32 (run-order reach, ``packing.VAR_KINDS`` index), optionally through the
+        likelihood's error model (``simplyp_predictive_draws_device``).  Returns ``draws``; asynchronous."""
+        torch = _torch()
+        Mc, S, D = out.shape[0], out.shape[1], out.shape[2]
+        if sc_params.dim() == 2:
+            sc_params = sc_params.unsqueeze(0)
+        dims = _cabi.make_dims(Mc, S, D, sc_params.shape[0], 0, 0)
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            _cabi.predictive_draws_device(dims, out.data_ptr(), member_params.data_ptr(), sc_params.data_ptr(),
+                                          diag.data_ptr(), series_desc.data_ptr(), series_desc.shape[0],
+                                          draws.data_ptr(), draws.shape[2], member_offset, obs_error, seed, stream)
+        return draws
+
+    def nanquantile(self, x, q, quantiles=None, mean=None, count=None):
+        """``np.nanquantile(x, q, axis=-1)`` of a [R][N] fp64 matrix, bitwise, with the mean and the count of the
+        non-NaN entries of every row (``simplyp_nanquantile_device``).  Returns (quantiles [n_q][R], mean [R],
+        count [R] int64); asynchronous.  Rows longer than shared memory holds use this engine's workspace."""
+        torch = _torch()
+        if x.dim() != 2 or x.dtype != torch.float64 or not x.is_contiguous():
+            raise ValueError("nanquantile takes a contiguous [R][N] float64 matrix")
+        R, N = x.shape
+        if quantiles is None:
+            quantiles = torch.empty((len(q), R), dtype=torch.float64, device=self.device)
+        if mean is None:
+            mean = torch.empty(R, dtype=torch.float64, device=self.device)
+        if count is None:
+            count = torch.empty(R, dtype=torch.int64, device=self.device)
+        need = _cabi.nanquantile_workspace_bytes(R, N)
+        ws = self._workspace(need) if need > 0 else None
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            _cabi.nanquantile_device(x.data_ptr(), R, N, q, quantiles.data_ptr(), mean.data_ptr(), count.data_ptr(),
+                                     ws.data_ptr() if ws is not None else None, need, stream)
+        return quantiles, mean, count
+
     # ------------------------------------------------------------------ Thornthwaite PET
     def thornthwaite_pet(self, t_air, month_start, year_is_leap, latitude_deg, out=None, out_stride=1):
         """Reference ``daily_PET`` (``inputs.py:232-312``) on the device: ``t_air`` [D] (device or host),

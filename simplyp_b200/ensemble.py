@@ -9,6 +9,8 @@ collective is one all-gather of the per-member fit statistics.
 """
 from __future__ import annotations
 
+from dataclasses import dataclass
+
 import numpy as np
 
 from . import packing as pk
@@ -435,3 +437,140 @@ def run_ensemble_to_dir(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, s
         with open(os.path.join(out_dir, "manifest.json"), "w") as f:
             json.dump(manifest, f, indent=1)
     return manifest
+
+
+# --------------------------------------------------------------------------- posterior predictive bands
+DEFAULT_BAND_SEED = 20260102
+
+
+@dataclass
+class PredictiveBands:
+    """What :func:`predictive_bands` returns.  ``quantiles`` [n_q][V][D] is the layout of
+    ``np.nanquantile(draws, q, axis=-1)``; ``mean`` [V][D] and ``count`` [V][D] are the mean and the number of the
+    members that entered every (series, day) — all members but the ``n_failed`` whose integration raised a status bit.
+    ``labels`` [(sc_id, variable)] name the series, ``dates`` the days."""
+    q: np.ndarray
+    quantiles: np.ndarray
+    mean: np.ndarray
+    count: np.ndarray
+    n_failed: int
+    labels: list
+    dates: object
+
+    def band(self, q):
+        """The band [V][D] of quantile value ``q`` (one of ``self.q``)."""
+        hits = np.flatnonzero(self.q == float(q))
+        if hits.size == 0:
+            raise ValueError("%r is not one of the computed quantiles %s" % (q, list(self.q)))
+        return self.quantiles[hits[0]]
+
+    def coverage(self, obs_dict, lo, hi):
+        """Per series label: ``(observed days, fraction of them with band_lo <= obs <= band_hi)`` for the bands of
+        the quantile values ``lo`` and ``hi``; ``obs_dict`` as ``calibrate_ensemble`` takes it."""
+        b_lo, b_hi = self.band(lo), self.band(hi)
+        out = {}
+        for v, (sc_id, var) in enumerate(self.labels):
+            df = obs_dict.get(sc_id)
+            if df is None or var not in df.columns:
+                out[(sc_id, var)] = (0, float("nan"))
+                continue
+            ser = df[var]
+            o = ser[~ser.index.duplicated()].reindex(self.dates).to_numpy(dtype="float64")
+            seen = ~np.isnan(o)
+            n = int(seen.sum())
+            inside = int(np.sum((b_lo[v][seen] <= o[seen]) & (o[seen] <= b_hi[v][seen])))
+            out[(sc_id, var)] = (n, inside / n if n else float("nan"))
+        return out
+
+
+def _check_band_quantiles(quantiles):
+    q = np.asarray(quantiles, dtype=np.float64).reshape(-1)
+    if q.size == 0 or q.size > 16:
+        raise ValueError("1..16 quantile values, got %d" % q.size)
+    if not np.all(np.isfinite(q)) or np.any(q < 0.0) or np.any(q > 1.0):
+        raise ValueError("quantile values must be finite and lie in [0, 1], got %s" % list(q))
+    return q
+
+
+def _band_series(series, topo):
+    series = list(series)
+    if not series:
+        raise ValueError("no series: give a list of (sc_id, variable)")
+    pos = {s: i for i, s in enumerate(topo.sc_ids)}
+    desc = []
+    for sc_id, var in series:
+        if var not in pk.VAR_INDEX:
+            raise ValueError("unknown variable %r: one of %s" % (var, pk.VAR_KINDS))
+        try:
+            sc_key = int(sc_id)
+        except (TypeError, ValueError):
+            sc_key = None
+        if sc_key not in pos:
+            raise ValueError("reach %r is not in SC_list" % (sc_id,))
+        desc.append((pos[sc_key], pk.VAR_INDEX[var]))
+    return np.asarray(desc, dtype=np.int32).reshape(-1, 2), [(int(s), v) for s, v in series]
+
+
+def predictive_bands(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, samples, series,
+                     quantiles=(0.025, 0.25, 0.5, 0.75, 0.975), obs_error=False, seed=DEFAULT_BAND_SEED,
+                     members_per_chunk=None, step_len=1.0, rtol=None, atol=None, snow_on_device=False, engine=None):
+    """Posterior predictive bands: quantiles over the members of ``samples`` (e.g. ``McmcResult.flat_samples``) of
+    the simulated series ``series`` [(sc_id, variable)], variable in ``packing.VAR_KINDS`` — Q_cumecs or a
+    concentration in mg/l, the values the fused statistics compare with the observations.
+
+    The members are integrated in full-output chunks of ``members_per_chunk`` (default: about 1 GiB of output a
+    chunk); each chunk is turned on the device into its columns of a [V][D][M] matrix of draws, and one selection
+    launch gives ``np.nanquantile`` of every (series, day) over the members, bitwise.  With ``obs_error`` every draw
+    also carries the likelihood's error model, y = s + m s eps with eps ~ N(0, 1) and m the member's ``err_m:<var>``,
+    keyed by ``seed``: a draw depends on (seed, member, day, series) only, not on the chunking.  A member whose
+    integration raised a status bit enters no band (``n_failed``).  ``snow_on_device`` as in
+    ``calibrate_ensemble``.
+
+    Raises ``ValueError`` before any device work for an unknown variable, a reach not in ``SC_list``, an empty
+    ``series``, quantile values that are not finite, lie outside [0, 1] or number more than 16, and a matrix of
+    draws (8 V D M bytes) larger than half of the free device memory.
+    """
+    import torch
+
+    from .engine import Engine
+    from .model import make_options
+
+    q = _check_band_quantiles(quantiles)
+    topo = pk.build_topology(p_struc, p["SC_list"])
+    desc, labels = _band_series(series, topo)
+    p_LU, p_SC = p_LU.copy(deep=True), p_SC.copy(deep=True)
+    pk.validate_land_use(p_SC, p["SC_list"])
+    pk.check_erosion_windows(p)
+    opt = make_options(p_SU, p, dynamic_options, topo, step_len, rtol, atol)
+    opt.snow_on_device = 1 if snow_on_device else 0
+    member, sc = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, topo.sc_ids), samples)
+    M, S, D, V = member.shape[0], topo.n_sc, len(met_df), desc.shape[0]
+    eng = engine or Engine()
+    draw_bytes = 8 * V * D * M
+    if draw_bytes > eng.free_bytes() // 2:
+        raise ValueError("the draws need %.1f GB, more than half of the free device memory: thin the samples "
+                         "(e.g. flat_samples(burn, thin=n))" % (draw_bytes / 1e9))
+    row_bytes = S * D * pk.NOUT * 8
+    if members_per_chunk is None:
+        members_per_chunk = max(1, (1 << 30) // max(row_bytes, 1))
+    chunk = int(max(1, min(int(members_per_chunk), M)))
+    dev = eng.device
+    d_forc = eng.to_device(pk.forcing_matrix(met_df, raw_snow=bool(snow_on_device)))
+    d_mem, d_sc, d_desc = eng.to_device(member), eng.to_device(sc), eng.to_device(desc)
+    draws = torch.empty((V, D, M), dtype=torch.float64, device=dev)
+    out = torch.empty((chunk, S, D, pk.NOUT), dtype=torch.float64, device=dev)
+    diag = torch.zeros((M, S, pk.NDIAG), dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        for m0 in range(0, M, chunk):
+            n = min(chunk, M - m0)
+            scp = d_sc if d_sc.shape[0] == 1 else d_sc[m0:m0 + n]
+            eng.run(d_forc, d_mem[m0:m0 + n], scp, topo.parent_offsets, topo.parent_ids, opt, out=out[:n],
+                    diag=diag[m0:m0 + n])
+            eng.predictive_draws(out[:n], d_mem[m0:m0 + n], scp, diag[m0:m0 + n], d_desc, draws, m0, obs_error, seed)
+        del out
+        quant, mean, count = eng.nanquantile(draws.view(V * D, M), q)
+    torch.cuda.synchronize(dev)
+    n_failed = int(np.any(diag.cpu().numpy()[:, :, 3] != 0, axis=1).sum())
+    return PredictiveBands(q=q, quantiles=quant.cpu().numpy().reshape(len(q), V, D),
+                           mean=mean.cpu().numpy().reshape(V, D), count=count.cpu().numpy().reshape(V, D),
+                           n_failed=n_failed, labels=labels, dates=met_df.index)
