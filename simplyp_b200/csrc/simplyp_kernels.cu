@@ -122,7 +122,6 @@ struct KArgs {
 constexpr int COST_BUCKETS = 4096;
 
 // Placement plan (simplyp_plan.cuh): device-side bookkeeping of the claims, an int array in the workspace.
-constexpr int PLAN_MAX_SM = 1024;                  // %smid is folded into this range
 constexpr int PLAN_FIRST_NEXT = 0;
 constexpr int PLAN_SKIPS = 1;                      // blocks that left without a list (launches with more blocks than lists)
 constexpr int PLAN_SM_ARR = 16;                    // [PLAN_MAX_SM] blocks that have arrived on the SM
@@ -144,8 +143,7 @@ enum { OC_N = 0, OC_MEAN, OC_SS, OC_MEAN_LOG, OC_SS_LOG, OC_SUM, OC_STD, OC_SS_R
 // There is no producer warp: threads walk through the days at their own pace, and the LAST thread of the
 // block to leave tile k re-arms the slot and issues the copy of tile k+FORC_SLOTS into it.  A thread that
 // runs ahead of the ring polls (mbarrier.test_wait) once per loop iteration instead of blocking, so the
-// slowest thread — which is always inside a resident tile — is never held up.
-constexpr int FORC_TILE = 128;    // days per tile (4 KB)
+// slowest thread — which is always inside a resident tile — is never held up.  FORC_TILE: simplyp_plan.cuh.
 constexpr int FORC_SLOTS = 4;     // ring depth (16 KB per block)
 
 struct ForcingRing {
@@ -478,10 +476,9 @@ struct CalIO : IOBase<ROUTED> {
 // ------------------------------------------------------------------------------------------ K1 (quad form)
 // One QUAD of lanes per (member, sub-catchment) item, 8 items per warp in day lock-step (simplyp_quad.cuh).
 // Shared memory: one QuadMem per quad, then the forcing ring.
-// MINB = resident blocks per SM the register allocation is made for (quad_minblocks): 2 (186 registers) for ensembles
-// of at most 2 blocks per SM, 3 (164 registers, no spills either) up to 9 blocks per SM — with the placement plan
-// below 3 blocks per SM — and 4 (128 registers, 16 warps per SM, ~150 B of spills) when the ensemble fills the machine
-// several times over.  Networks (STIFF): 2 (226 registers) or 3 (168 registers, 40 B of spills), see launch_levels.
+// MINB = resident blocks per SM the register allocation is made for, chosen by launch_config (simplyp_plan.cuh): 2 (186
+// registers), 3 (164 registers, no spills either) or 4 (128 registers, 16 warps per SM, ~150 B of spills); networks
+// (STIFF) 2 (226 registers) or 3 (168 registers, 40 B of spills).
 // A launch is either an ensemble of one sub-catchment (optionally the pilot or the continuation of one, optionally
 // planned) or a network (tickets in dispatch order, optionally swept in epochs: KArgs::epoch_days).
 enum { MODE_RUN = 0, MODE_CAL = 1 };
@@ -1240,78 +1237,43 @@ ThreadOptions make_topt(const SimplypOptions& o) {
   return t;
 }
 
-// Shared launcher: one launch; the reach DAG is swept as a day-skewed wavefront inside the kernel.
-// Register budget of the quad kernel for a grid of `grid` blocks (see the kernel's comment).
-int quad_minblocks(long long grid) {
-  if (const char* e = getenv("SIMPLYP_QUAD_MINBLOCKS")) { const int v = atoi(e); if (v >= 2 && v <= 4) return v; }
-  int dev = 0, n_sm = 148;
-  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-  if (grid <= 2ll * n_sm) return 2;                 // every block resident at 2 per SM (184 registers)
-  // Beyond that the 168-register build (3 blocks per SM, no spills) up to about 4x10^4 members; the 128-register
-  // build (4 blocks per SM, 136 B of spills in the step loop) only where the machine is several waves deep.  Round 2,
-  // B200, 3 vs 4 blocks: 2x10^4 members 19.6 vs 20.9 ms, 4x10^4 35.1 vs 35.3, 1.6x10^5 131.7-132.0 vs 130.3-131.1.
-  if (grid <= 9ll * n_sm) return 3;
-  return 4;
+// The quad kernel in the register variant `minb` (launch_config).  Networks (STIFF) have no 4-blocks build.
+template <int MODE, bool STIFF>
+void launch_quad(int minb, long long grid, size_t smem, cudaStream_t st, const KArgs& a) {
+  const unsigned g = (unsigned)grid, block = 128;
+  if (minb == 2) simplyp_quad_kernel<MODE, 2, STIFF><<<g, block, smem, st>>>(a);
+  else if (minb == 3 || STIFF) simplyp_quad_kernel<MODE, 3, STIFF><<<g, block, smem, st>>>(a);
+  else if constexpr (!STIFF) simplyp_quad_kernel<MODE, 4, false><<<g, block, smem, st>>>(a);
 }
 
 // Pilot + counting sort: fills a.perm (one sub-catchment, quad kernel).  3 small launches + the pilot.
 template <int MODE>
-int order_members_by_cost(const SimplypDims& dims, const SimplypOptions& opt, KArgs& a, const WsLayout& L, char* ws,
-                          cudaStream_t st) {
-  const int days = opt.pilot_days > 0 ? opt.pilot_days : 8;
-  if (opt.pilot_days < 0 || !ws || dims.n_sc != 1 || dims.n_members < 512 || dims.n_days < 8 * days) return SIMPLYP_OK;
-  // the pilot is the run's own first `days` days (same kernel, member order): it leaves every member's midnight
+int order_members_by_cost(const SimplypDims& dims, const LaunchConfig& c, KArgs& a, const WsLayout& L, char* ws,
+                          size_t smem, cudaStream_t st) {
+  if (c.pilot_days == 0) return SIMPLYP_OK;
+  // the pilot is the run's own first `pilot_days` days (same kernel, member order): it leaves every member's midnight
   // state in the carry area, and the main launch continues from there in cost order
   a.carry = reinterpret_cast<QuadCarry*>(ws + L.off_carry);
   a.carry_stats = reinterpret_cast<double*>(ws + L.off_carry_stats);
   KArgs p = a;
-  p.day_end = days;
+  p.day_end = c.pilot_days;
   p.diag = nullptr;
   p.perm = nullptr;
   p.pilot_pass = 1;
   p.cost = reinterpret_cast<unsigned*>(ws + L.off_cost);
   p.hist = reinterpret_cast<unsigned*>(ws + L.off_hist);
-  a.day_begin = days;
+  a.day_begin = c.pilot_days;
   int* perm = reinterpret_cast<int*>(ws + L.off_perm);
   SP_CUDA(cudaMemsetAsync(p.hist, 0, sizeof(unsigned) * COST_BUCKETS, st));
-  const int block = 128, qpb = block / 4;
-  const long long grid = ((long long)dims.n_members + qpb - 1) / qpb;
-  const size_t smem = (size_t)qpb * sizeof(QuadMem) + sizeof(ForcingRing) +
-                      (MODE == MODE_CAL ? (size_t)qpb * STAT_STRIDE * sizeof(double) : 0);
-  // register variant of the pilot pass (the variants give the same bits): when the 2-blocks-per-SM build would leave
-  // a few blocks queued behind the resident ones, the 3-blocks build runs them all at once
-  int pilot_minb = quad_minblocks(grid);
-  {
-    int dev0 = 0, nsm0 = 0;
-    if (cudaGetDevice(&dev0) == cudaSuccess) cudaDeviceGetAttribute(&nsm0, cudaDevAttrMultiProcessorCount, dev0);
-    if (pilot_minb == 2 && nsm0 > 0 && grid > 2ll * nsm0) pilot_minb = 3;
-    if (const char* e = getenv("SIMPLYP_PILOT_MINBLOCKS")) { const int v = atoi(e); if (v >= 2 && v <= 4) pilot_minb = v; }
-  }
-  if (pilot_minb == 2) simplyp_quad_kernel<MODE, 2, false><<<(unsigned)grid, block, smem, st>>>(p);
-  else if (pilot_minb == 3) simplyp_quad_kernel<MODE, 3, false><<<(unsigned)grid, block, smem, st>>>(p);
-  else simplyp_quad_kernel<MODE, 4, false><<<(unsigned)grid, block, smem, st>>>(p);
+  launch_quad<MODE, false>(c.pilot_minb, (dims.n_members + 31ll) / 32, smem, st, p);
   cost_scan_kernel<<<1, 1024, 0, st>>>(p.hist);
-  // latency-bound regime (every block resident at once: 2 per SM, or 3 on some SMs with the 168-register build):
-  // planned placement, see PLAN_*.  B200, round 2, planned / unplanned 3-blocks launch: 10^4 members 9.4 / 11.6 ms,
-  // 1.2x10^4 11.0 / 12.0, 1.4x10^4 12.0 / 12.5 (the chained 2-blocks plan of round 1: 10.8 / 12.5 / 13.4).
   MemberLayout lay = {0, 0, 0, 0};
-  int dev = 0, n_sm = 0;
-  if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-  const char* e_plan = getenv("SIMPLYP_SM_PLAN");
-  PlanShape shape;
-  const int minb = quad_minblocks(grid);
-  int q_max = n_sm - 1;
-  if (const char* e = getenv("SIMPLYP_PLAN_QMAX")) q_max = atoi(e);       // A/B runs
-  if ((minb == 2 || (minb == 3 && grid <= 2ll * n_sm + q_max)) && n_sm <= PLAN_MAX_SM && dims.n_members >= 2048 &&
-      !(e_plan && atoi(e_plan) == 0) && plan_shape(grid, n_sm, shape, minb)) {
-    int solo = dims.n_members / 100 / 4 * 4;         // about one warp in five of the heavy blocks (10^4 members:
-                                                     // 0 / 24 / 96 / 240 led warps 9.55 / 9.42 / 9.35 / 9.51 ms)
-    if (const char* e = getenv("SIMPLYP_SOLO_WARPS")) { const int v = atoi(e); if (v >= 0) solo = v; }
-    lay = member_layout(shape, dims.n_members, solo);
+  if (c.plan) {                                      // see PLAN_*
+    lay = member_layout(c.shape, dims.n_members, c.solo);
     int* plan = reinterpret_cast<int*>(ws + L.off_plan);
     SP_CUDA(cudaMemsetAsync(plan, 0, sizeof(int) * PLAN_INTS, st));
     a.plan = plan;
-    a.shape = shape;
+    a.shape = c.shape;
   }
   cost_scatter_kernel<<<(dims.n_members + 255) / 256, 256, 0, st>>>(p.cost, p.hist, perm, dims.n_members, lay);
   g_launches.fetch_add(3);
@@ -1395,25 +1357,25 @@ int launch_levels(const SimplypDims& dims, const SimplypOptions& opt, KArgs a, c
   const int E = po_host[S];
   const WsLayout L = ws_layout(dims, E, CAL);
   constexpr int MODE = CAL ? MODE_CAL : MODE_RUN;
-  const int block = 128, qpb = block / 4;
+  const int qpb = 32;                        // items per block of 128 threads
   const size_t smem = (size_t)qpb * sizeof(QuadMem) + sizeof(ForcingRing) +
                       (CAL ? (size_t)qpb * STAT_STRIDE * sizeof(double) : 0);
   a.n_work = S;
+  int dev = 0, n_sm = 0;
+  SP_CUDA(cudaGetDevice(&dev));
+  SP_CUDA(cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev));
+  const LaunchOverrides ov = read_launch_overrides();
 
   if (S == 1 && E == 0) {                    // an ensemble of one sub-catchment: items are the members
     int* zp = nullptr;
     SP_CUDA(cudaGetSymbolAddress((void**)&zp, g_zero_offsets));
     a.parent_offsets = zp;   // {0, 0}: no parents
     a.parent_ids = zp;
-    const long long grid = (((long long)dims.n_members + 7) / 8 * 8 + qpb - 1) / qpb;
-    const int rc = order_members_by_cost<MODE>(dims, opt, a, L, ws, st);
+    const LaunchConfig c =
+        launch_config({dims.n_members, dims.n_days, false, 0, 0, opt.pilot_days, ws != nullptr, n_sm}, ov);
+    const int rc = order_members_by_cost<MODE>(dims, c, a, L, ws, smem, st);
     if (rc) return rc;
-    const int minb = quad_minblocks(grid);
-    // planned placement: the launch fills the resident slots (one block per list at 2 per SM, 3 n_sm blocks at 3 per SM)
-    const unsigned g = a.plan ? (unsigned)a.shape.n_launch() : (unsigned)grid;
-    if (minb == 2) simplyp_quad_kernel<MODE, 2, false><<<g, block, smem, st>>>(a);
-    else if (minb == 3) simplyp_quad_kernel<MODE, 3, false><<<g, block, smem, st>>>(a);
-    else simplyp_quad_kernel<MODE, 4, false><<<(unsigned)grid, block, smem, st>>>(a);
+    launch_quad<MODE, false>(c.minb, c.grid, smem, st, a);
     g_launches.fetch_add(1);
     SP_CUDA(cudaGetLastError());
     return SIMPLYP_OK;
@@ -1461,32 +1423,14 @@ int launch_levels(const SimplypDims& dims, const SimplypOptions& opt, KArgs a, c
     const long long n = (long long)(i_ls[l + 1] - i_ls[l]) * dims.n_members;
     bound += (n + 7) / 8 * 8 + ((dims.n_members % 8 != 0 && i_ls[l + 1] - i_ls[l] > 1) ? 8 : 0);
   }
-  long long grid = (bound + qpb - 1) / qpb;
-  const long long grid_one_epoch = grid;
-  // Epoch sweep (KArgs::epoch_days): a whole number of forcing tiles per epoch.  Without it the launch is the bulk of
-  // the headwaters followed by the chains of the main-stem reaches at low occupancy.  An epoch should be long against
-  // the depth of the network (the wavefront needs one day-time per level to reach the outlet): four days per level,
-  // at least 256.  B200, round 2, one piece / 256 / 512 / 1024 / 2048 days per epoch: config 3 (32 levels) at 64
-  // members 767 / 555 / 564 / 567 / 583 ms, at 256 members 2185 / 1922 / 1920 / 1932 / 1929; config 5 (487 levels) at
-  // 8 members 2565 / 2788 / 2550 / 2411 / 2348 ms, at 1 member 1339 / 1297 / 1244 / 1253 / 1279.
-  int epoch_days = (4 * nl + FORC_TILE - 1) / FORC_TILE * FORC_TILE;
-  if (epoch_days < 2 * FORC_TILE) epoch_days = 2 * FORC_TILE;
-  {
-    // a launch of at most one block per SM has no bulk phase to overlap with, and its chain warps have their SMs to
-    // themselves: swept in epochs they would only get neighbours (config 3 at 1 / 8 members, 15 / 72 blocks: 549 / 548
-    // ms in one piece, 590 / 573 in epochs; config 5 at 1 member, 227 blocks, still gains: 1394 -> 1307 ms)
-    int dev = 0, n_sm = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-    if (grid <= (long long)n_sm) epoch_days = 0;
-  }
-  if (const char* e = getenv("SIMPLYP_EPOCH_DAYS")) epoch_days = atoi(e) / FORC_TILE * FORC_TILE;   // 0: off (A/B runs)
-  if (epoch_days > 0 && dims.n_days > epoch_days && grid * ((dims.n_days + epoch_days - 1) / epoch_days) < (1ll << 30)) {
-    a.epoch_days = epoch_days;
-    a.n_epochs = (dims.n_days + epoch_days - 1) / epoch_days;
+  const LaunchConfig c = launch_config(
+      {dims.n_members, dims.n_days, true, nl, (bound + qpb - 1) / qpb, opt.pilot_days, ws != nullptr, n_sm}, ov);
+  if (c.n_epochs > 0) {
+    a.epoch_days = c.epoch_days;
+    a.n_epochs = c.n_epochs;
     a.epoch_done = reinterpret_cast<int*>(ws + L.off_epoch_done);
     a.carry = reinterpret_cast<QuadCarry*>(ws + L.off_carry);
     a.carry_stats = reinterpret_cast<double*>(ws + L.off_carry_stats);
-    grid *= a.n_epochs;
     if (es != nullptr && es->flags_dev != nullptr && a.n_epochs <= es->capacity) {
       a.epoch_count = reinterpret_cast<unsigned*>(ws + L.off_epoch_count);
       a.epoch_flags_host = es->flags_dev;
@@ -1494,20 +1438,7 @@ int launch_levels(const SimplypDims& dims, const SimplypOptions& opt, KArgs a, c
       es->epoch_days = a.epoch_days;
     }
   }
-  // Networks get the build with the Rosenbrock path for stiff (main-stem) reaches.  Its 2-blocks-per-SM variant (226
-  // registers) serves launches that the chains of the main stem bound; when the items of one epoch fill the machine
-  // several times over, the 3-blocks variant (168 registers, 40 B of spills) is faster.  B200, round 2, 2 / 3 blocks:
-  // config 3 at 64 members (512 blocks per epoch) 557 / 666 ms, at 256 members (2048) 1921 / 1739; config 5 at 8
-  // members (1024) 2346 / 2166, at 1 member (128) 1266 / 1583.
-  int net_minb = 2;
-  {
-    int dev = 0, n_sm = 148;
-    if (cudaGetDevice(&dev) == cudaSuccess) cudaDeviceGetAttribute(&n_sm, cudaDevAttrMultiProcessorCount, dev);
-    if (grid_one_epoch >= 6ll * n_sm) net_minb = 3;
-  }
-  if (const char* e = getenv("SIMPLYP_NET_MINBLOCKS")) { const int v = atoi(e); if (v == 2 || v == 3) net_minb = v; }
-  if (net_minb == 3) simplyp_quad_kernel<MODE, 3, true><<<(unsigned)grid, block, smem, st>>>(a);
-  else simplyp_quad_kernel<MODE, 2, true><<<(unsigned)grid, block, smem, st>>>(a);
+  launch_quad<MODE, true>(c.minb, c.grid, smem, st, a);
   g_launches.fetch_add(2);
   SP_CUDA(cudaGetLastError());
   return SIMPLYP_OK;

@@ -110,6 +110,21 @@ def run_quad_split(forcing, member_params, sc_params, parent_offsets, parent_ids
     return out, diag
 
 
+LAUNCH_CONFIG_FIELDS = ("grid", "minb", "pilot_days", "pilot_minb", "plan", "nY", "nP", "Q", "resident", "solo",
+                        "epoch_days", "n_epochs")
+
+
+def launch_config(M, D, n_sm, network=False, n_levels=0, grid_one_epoch=0, pilot_days=0, workspace=True):
+    """launch_config() of simplyp_plan.cuh under the SIMPLYP_* overrides in os.environ, as a dict of
+    LAUNCH_CONFIG_FIELDS."""
+    lib = load()
+    out = np.zeros(len(LAUNCH_CONFIG_FIELDS), dtype=np.int64)
+    lib.hostemu_launch_config(C.c_int(M), C.c_int(D), C.c_int(int(network)), C.c_int(n_levels),
+                              C.c_longlong(grid_one_epoch), C.c_int(pilot_days), C.c_int(int(workspace)), C.c_int(n_sm),
+                              out.ctypes.data_as(C.c_void_p))
+    return dict(zip(LAUNCH_CONFIG_FIELDS, (int(x) for x in out)))
+
+
 def plan(M, n_sm, solo, resident=2):
     """Placement plan arithmetic: (index_of_rank [M], list_of_block [B], pos_in_list [B],
     (nY, nP, Q, n_lists, n_launch, resident)) or None."""

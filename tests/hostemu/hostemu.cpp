@@ -178,6 +178,17 @@ extern "C" int hostemu_plan(int M, int n_sm, int solo, int resident, int* index_
   return 1;
 }
 
+// Launch policy of the quad kernel (simplyp_plan.cuh) under the overrides in the environment.  out[12]: grid, minb,
+// pilot_days, pilot_minb, plan, nY, nP, Q, resident, solo, epoch_days, n_epochs.
+extern "C" void hostemu_launch_config(int M, int D, int network, int n_levels, long long grid_one_epoch, int pilot_days,
+                                      int workspace, int n_sm, long long* out) {
+  const LaunchInputs in = {M, D, network != 0, n_levels, grid_one_epoch, pilot_days, workspace != 0, n_sm};
+  const LaunchConfig c = launch_config(in, read_launch_overrides());
+  const long long v[12] = {c.grid, c.minb, c.pilot_days, c.pilot_minb, c.plan, c.shape.nY, c.shape.nP, c.shape.Q,
+                           c.shape.resident, c.solo, c.epoch_days, c.n_epochs};
+  memcpy(out, v, sizeof(v));
+}
+
 // The quad formulation of ode_f against the scalar rhs() at one state: returns the largest relative
 // difference over the 12 derivatives (dQr/dt and dVr/dt are recovered from du/dt and the quad's slot B).
 extern "C" double hostemu_quad_rhs_check(const double* mp, const double* sp, double P, double E, double doy,
