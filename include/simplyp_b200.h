@@ -386,6 +386,51 @@ int simplyp_nanquantile_device(const double* x, int64_t n_rows, int64_t n_cols, 
                                double* quantiles, double* mean, int64_t* count, void* workspace,
                                int64_t workspace_bytes, void* stream);
 
+/* ---- Sobol' sensitivity indices over a Saltelli design ------------------------------------------------------------
+ * SALib's sobol.sample / sobol.analyze on the device.  K free parameters (the sampler's targets and boxes,
+ * SimplypMcmcParam), N = n_base samples, P = K + 2 design members a sample (2K + 2 with second order).
+ *
+ * simplyp_sobol_design_device: overwrites the target columns of the design members [member_offset, member_offset + n)
+ *   of member_params [N P][NP_MEMBER] and sc_params [N P][S][NP_SC] (or [1][S][NP_SC] without SC targets); the other
+ *   columns keep what the caller put there (the base vectors).  Member m = i P + slot takes Sobol' point skip + i of
+ *   the unscrambled 2K-dimensional sequence (Joe-Kuo new-joe-kuo-6.21201, SciPy's qmc.Sobol(scramble=False, bits=32)):
+ *   slot 0 = A (coordinates 0..K-1), slot 1+j = AB_j (A with column j from B = coordinates K..2K-1), slot K+1+j =
+ *   BA_j (second order: B with column j from A), slot P-1 = B.  Value = lo + (hi - lo) u, each operation rounded.
+ * simplyp_sobol_outputs_device: Y[n_rows][M] from the fused statistics of the design (stats [M][V][NSTAT], diag
+ *   [M][S][NDIAG]); row r is stats[.][rows[r][0]][rows[r][1]], or the sampler's member lp when rows[r][1] = -1
+ *   (rows[n_rows][2] int32 on the device).  A member with a non-zero status word gives NaN in every row.
+ * simplyp_sobol_indices_device: per row of Y[n_rows][N P] (member-major, as the design), with sample i used when its
+ *   P values are all finite (n used; n < 2 or a zero variance gives NaN indices), c the mean of the used values,
+ *   a = A - c etc. and V the population variance of {a_i} u {b_i}:
+ *     S1_j = mean(b (ab_j - a)) / V,  ST_j = mean((a - ab_j)^2) / (2 V),
+ *     S2_jk = mean(ba_j ab_k - a b) / V - S1_j - S1_k  (j < k, second order; NaN elsewhere).
+ *   Bootstrap: resample t < n_boot draws n used samples with replacement, draw k at position (w n) >> 32 with w word
+ *   k mod 4 of Philox4x32-10 keyed by `seed`, counter (t, k / 4, 0, 3); c stays, V is recomputed;
+ *   *_conf = conf_z * std(ddof 1) over the resamples (NaN with n_boot < 2).  Outputs: S1, ST, S1_conf, ST_conf
+ *   [n_rows][K]; S2, S2_conf [n_rows][K][K] (second order only, else may be NULL); mean (c), var (V) [n_rows];
+ *   n_used [n_rows].  Sums run in a fixed order: results are bitwise reproducible.  Needs
+ *   simplyp_sobol_workspace_bytes(sb, n_rows) bytes of device workspace.
+ * All three only enqueue work on `stream` (no allocation, no synchronisation), so they can be captured into a graph. */
+typedef struct {
+  int32_t n_free;           /* K: 1..SIMPLYP_MCMC_MAX_FREE */
+  int32_t n_sc;             /* S of the design's runs */
+  int32_t sc_per_member;    /* sc_params is [N P][S][NP_SC] (required by the SC targets) */
+  int32_t second_order;     /* 0 or 1 */
+  int64_t n_base;           /* N: a power of two >= 2 */
+  int64_t skip;             /* first Sobol' point; skip + N <= 2^32 */
+  SimplypMcmcParam param[SIMPLYP_MCMC_MAX_FREE];
+} SimplypSobol;
+
+int simplyp_sobol_design_device(const SimplypSobol* sb, int64_t member_offset, int64_t n_members,
+                                double* member_params, double* sc_params, void* stream);
+int simplyp_sobol_outputs_device(const double* stats, const int64_t* diag, int64_t n_members, int32_t n_obs_series,
+                                 int32_t n_sc, const int32_t* rows, int32_t n_rows, double* y, void* stream);
+int64_t simplyp_sobol_workspace_bytes(const SimplypSobol* sb, int64_t n_rows);
+int simplyp_sobol_indices_device(const SimplypSobol* sb, const double* y, int64_t n_rows, int32_t n_boot,
+                                 double conf_z, uint64_t seed, double* S1, double* ST, double* S1_conf,
+                                 double* ST_conf, double* S2, double* S2_conf, double* mean, double* var,
+                                 int64_t* n_used, void* workspace, int64_t workspace_bytes, void* stream);
+
 /* Host-buffer forms: same arguments as HOST pointers; the library stages them through its own
  * (cached) device buffers on `device`, runs and copies the result back before returning. */
 int simplyp_run_host(int device, const SimplypDims* dims, const SimplypOptions* opt,

@@ -26,7 +26,8 @@ EXPORTS = [
     "simplyp_calibrate_gather_device", "simplyp_peer_alloc", "simplyp_peer_free", "simplyp_ipc_export",
     "simplyp_ipc_import", "simplyp_ipc_close", "simplyp_mcmc_propose_device", "simplyp_mcmc_accept_device",
     "simplyp_mcmc_init_device", "simplyp_predictive_draws_device", "simplyp_nanquantile_workspace_bytes",
-    "simplyp_nanquantile_device",
+    "simplyp_nanquantile_device", "simplyp_sobol_design_device", "simplyp_sobol_outputs_device",
+    "simplyp_sobol_workspace_bytes", "simplyp_sobol_indices_device",
 ]
 MAX_RANKS = 8
 
@@ -70,6 +71,11 @@ class SimplypMcmcState(C.Structure):
     _fields_ = [("walkers", C.c_void_p), ("lp", C.c_void_p), ("proposals", C.c_void_p), ("log_z", C.c_void_p),
                 ("out_of_box", C.c_void_p), ("iteration", C.c_void_p), ("accepted", C.c_void_p),
                 ("chain", C.c_void_p), ("chain_lp", C.c_void_p), ("n_saved", C.c_int64), ("chain_base", C.c_int64)]
+
+
+class SimplypSobol(C.Structure):
+    _fields_ = [("n_free", C.c_int32), ("n_sc", C.c_int32), ("sc_per_member", C.c_int32), ("second_order", C.c_int32),
+                ("n_base", C.c_int64), ("skip", C.c_int64), ("param", SimplypMcmcParam * MCMC_MAX_FREE)]
 
 
 class SimplypError(RuntimeError):
@@ -149,6 +155,16 @@ def load():
     lib.simplyp_nanquantile_workspace_bytes.restype = C.c_int64
     lib.simplyp_nanquantile_device.argtypes = [vp, C.c_int64, C.c_int64, dp, C.c_int32, vp, vp, vp, vp, C.c_int64, vp]
     lib.simplyp_nanquantile_device.restype = C.c_int
+    sbp = C.POINTER(SimplypSobol)
+    lib.simplyp_sobol_design_device.argtypes = [sbp, C.c_int64, C.c_int64, vp, vp, vp]
+    lib.simplyp_sobol_design_device.restype = C.c_int
+    lib.simplyp_sobol_outputs_device.argtypes = [vp, vp, C.c_int64, C.c_int32, C.c_int32, vp, C.c_int32, vp, vp]
+    lib.simplyp_sobol_outputs_device.restype = C.c_int
+    lib.simplyp_sobol_workspace_bytes.argtypes = [sbp, C.c_int64]
+    lib.simplyp_sobol_workspace_bytes.restype = C.c_int64
+    lib.simplyp_sobol_indices_device.argtypes = [sbp, vp, C.c_int64, C.c_int32, C.c_double, C.c_uint64, vp, vp, vp,
+                                                 vp, vp, vp, vp, vp, vp, vp, C.c_int64, vp]
+    lib.simplyp_sobol_indices_device.restype = C.c_int
     if lib.simplyp_abi_version() != 4:
         raise SimplypError("ABI version mismatch")
     _lib = lib
@@ -412,6 +428,50 @@ def nanquantile_device(x_ptr, n_rows, n_cols, q, quant_ptr, mean_ptr, count_ptr,
     qa = (C.c_double * max(len(q), 1))(*[float(v) for v in q])
     _check(lib.simplyp_nanquantile_device(x_ptr, int(n_rows), int(n_cols), qa, len(q), quant_ptr, mean_ptr, count_ptr,
                                           ws_ptr, int(ws_bytes), stream_ptr))
+
+
+def make_sobol(targets, lo, hi, n_sc, n_base, skip=0, sc_per_member=False, second_order=False):
+    """SimplypSobol for ``targets`` [(kind, index, pos)] (as :func:`make_mcmc`) with the boxes ``[lo[k], hi[k]]``."""
+    if not 1 <= len(targets) <= MCMC_MAX_FREE:
+        raise ValueError("1..%d free parameters" % MCMC_MAX_FREE)
+    sb = SimplypSobol()
+    sb.n_free, sb.n_sc = len(targets), int(n_sc)
+    sb.sc_per_member, sb.second_order = 1 if sc_per_member else 0, 1 if second_order else 0
+    sb.n_base, sb.skip = int(n_base), int(skip)
+    for k, (kind, index, pos) in enumerate(targets):
+        p = sb.param[k]
+        p.kind, p.index, p.pos, p.lo, p.hi = int(kind), int(index), int(pos), float(lo[k]), float(hi[k])
+    return sb
+
+
+def sobol_design_device(sb, member_offset, n_members, member_ptr, sc_ptr, stream_ptr):
+    """Target columns of design members [member_offset, member_offset + n_members); asynchronous on ``stream_ptr``."""
+    lib = require_device()
+    _check(lib.simplyp_sobol_design_device(C.byref(sb), int(member_offset), int(n_members), member_ptr, sc_ptr,
+                                           stream_ptr))
+
+
+def sobol_outputs_device(stats_ptr, diag_ptr, n_members, n_obs_series, n_sc, rows_ptr, n_rows, y_ptr, stream_ptr):
+    """Objective rows Y [n_rows][M] from the fused statistics; asynchronous on ``stream_ptr``."""
+    lib = require_device()
+    _check(lib.simplyp_sobol_outputs_device(stats_ptr, diag_ptr, int(n_members), int(n_obs_series), int(n_sc),
+                                            rows_ptr, int(n_rows), y_ptr, stream_ptr))
+
+
+def sobol_workspace_bytes(sb, n_rows):
+    n = load().simplyp_sobol_workspace_bytes(C.byref(sb), int(n_rows))
+    if n < 0:
+        _check(int(n))
+    return int(n)
+
+
+def sobol_indices_device(sb, y_ptr, n_rows, n_boot, conf_z, seed, S1, ST, S1_conf, ST_conf, S2, S2_conf, mean, var,
+                         n_used, ws_ptr, ws_bytes, stream_ptr):
+    """Sobol' indices and bootstrap confidences of every row of Y [n_rows][N P]; asynchronous on ``stream_ptr``."""
+    lib = require_device()
+    _check(lib.simplyp_sobol_indices_device(C.byref(sb), y_ptr, int(n_rows), int(n_boot), float(conf_z),
+                                            int(seed) & 0xFFFFFFFFFFFFFFFF, S1, ST, S1_conf, ST_conf, S2, S2_conf,
+                                            mean, var, n_used, ws_ptr, int(ws_bytes), stream_ptr))
 
 
 def workspace_bytes(dims, calibrate, rank_stats=False):

@@ -35,6 +35,7 @@
 #include "simplyp_plan.cuh"
 #include "simplyp_mcmc.cuh"
 #include "simplyp_bands.cuh"
+#include "simplyp_sobol.cuh"
 
 using namespace simplyp;
 
@@ -1564,6 +1565,24 @@ __global__ void mcmc_init_kernel(const SimplypMcmc mc, const SimplypMcmcState st
                             diag + (size_t)w * mc.n_sc * SIMPLYP_NDIAG, mc.n_sc);
 }
 
+// The targets and boxes of K free parameters (the sampler's and the sensitivity design's); `what` prefixes the message.
+int check_targets(const SimplypMcmcParam* param, int K, int n_sc, int sc_per_member, const char* what) {
+  for (int i = 0; i < K; ++i) {
+    const SimplypMcmcParam& p = param[i];
+    if (!(p.lo < p.hi) || !std::isfinite(p.lo) || !std::isfinite(p.hi)) return fail(SIMPLYP_EINVAL, "%s: need finite lo < hi", what);
+    if (p.kind == SIMPLYP_MCMC_MEMBER) {
+      if (p.index < 0 || p.index >= SIMPLYP_NP_MEMBER) return fail(SIMPLYP_EINVAL, "%s: member column out of range", what);
+    } else if (p.kind == SIMPLYP_MCMC_SC_ALL || p.kind == SIMPLYP_MCMC_SC_AT) {
+      if (p.index < 0 || p.index >= SIMPLYP_NP_SC) return fail(SIMPLYP_EINVAL, "%s: SC row out of range", what);
+      if (p.kind == SIMPLYP_MCMC_SC_AT && (p.pos < 0 || p.pos >= n_sc)) return fail(SIMPLYP_EINVAL, "%s: SC position out of range", what);
+      if (!sc_per_member) return fail(SIMPLYP_EINVAL, "%s: SC targets need per-member sc_params", what);
+    } else {
+      return fail(SIMPLYP_EINVAL, "%s: unknown target kind", what);
+    }
+  }
+  return SIMPLYP_OK;
+}
+
 int check_mcmc(const SimplypMcmc* mc, const SimplypMcmcState* st) {
   if (!mc || !st) return fail(SIMPLYP_EINVAL, "mcmc: null argument%s");
   const int K = mc->n_free;
@@ -1571,19 +1590,8 @@ int check_mcmc(const SimplypMcmc* mc, const SimplypMcmcState* st) {
   if (mc->n_walkers < 2 * K || mc->n_walkers % 2 != 0) return fail(SIMPLYP_EINVAL, "mcmc: an even number of walkers >= 2 K%s");
   if (mc->n_sc < 1 || mc->n_obs_series < 0 || mc->thin < 1) return fail(SIMPLYP_EINVAL, "mcmc: bad n_sc / n_obs_series / thin%s");
   if (!(mc->stretch > 1.0 && mc->stretch < INFINITY)) return fail(SIMPLYP_EINVAL, "mcmc: stretch scale must be > 1%s");
-  for (int i = 0; i < K; ++i) {
-    const SimplypMcmcParam& p = mc->param[i];
-    if (!(p.lo < p.hi) || !std::isfinite(p.lo) || !std::isfinite(p.hi)) return fail(SIMPLYP_EINVAL, "mcmc: need finite lo < hi%s");
-    if (p.kind == SIMPLYP_MCMC_MEMBER) {
-      if (p.index < 0 || p.index >= SIMPLYP_NP_MEMBER) return fail(SIMPLYP_EINVAL, "mcmc: member column out of range%s");
-    } else if (p.kind == SIMPLYP_MCMC_SC_ALL || p.kind == SIMPLYP_MCMC_SC_AT) {
-      if (p.index < 0 || p.index >= SIMPLYP_NP_SC) return fail(SIMPLYP_EINVAL, "mcmc: SC row out of range%s");
-      if (p.kind == SIMPLYP_MCMC_SC_AT && (p.pos < 0 || p.pos >= mc->n_sc)) return fail(SIMPLYP_EINVAL, "mcmc: SC position out of range%s");
-      if (!mc->sc_per_member) return fail(SIMPLYP_EINVAL, "mcmc: SC targets need per-member sc_params%s");
-    } else {
-      return fail(SIMPLYP_EINVAL, "mcmc: unknown target kind%s");
-    }
-  }
+  const int rc = check_targets(mc->param, K, mc->n_sc, mc->sc_per_member, "mcmc");
+  if (rc) return rc;
   if (!st->walkers || !st->lp || !st->proposals || !st->log_z || !st->out_of_box || !st->iteration || !st->accepted)
     return fail(SIMPLYP_EINVAL, "mcmc: null state pointer%s");
   if (st->n_saved < 0 || (st->n_saved > 0 && (!st->chain || !st->chain_lp))) return fail(SIMPLYP_EINVAL, "mcmc: null chain%s");
@@ -1829,6 +1837,376 @@ long long nq_shared_cap() {
       cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev) != cudaSuccess)
     return 0;
   return (optin - 1024) / (long long)sizeof(uint64_t);   // (1 KB for the reductions' static shared memory)
+}
+
+// ------------------------------------------------------------------------------------------ Sobol' sensitivity
+// Design: one thread per member row (simplyp_sobol.cuh holds the point and value arithmetic).
+__global__ void sobol_design_kernel(const SimplypSobol sb, long long member_offset, long long n, double* member_params,
+                                    double* sc_params) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n) return;
+  const long long m = member_offset + idx;
+  const int S = sb.n_sc;
+  double* mrow = member_params + (size_t)m * SIMPLYP_NP_MEMBER;
+  double* srow = sc_params + (sb.sc_per_member ? (size_t)m * S * SIMPLYP_NP_SC : 0);
+  for (int j = 0; j < sb.n_free; ++j) {
+    const SimplypMcmcParam& p = sb.param[j];
+    const double v = sobol_design_value(sb, m, j);
+    if (p.kind == SIMPLYP_MCMC_MEMBER) {
+      mrow[p.index] = v;
+    } else if (p.kind == SIMPLYP_MCMC_SC_AT) {
+      srow[(size_t)p.pos * SIMPLYP_NP_SC + p.index] = v;
+    } else {
+      for (int s = 0; s < S; ++s) srow[(size_t)s * SIMPLYP_NP_SC + p.index] = v;
+    }
+  }
+}
+
+// Objective rows Y[r][m] from the fused statistics: one thread per (member, row).
+__global__ void sobol_outputs_kernel(const double* stats, const int64_t* diag, long long M, int V, int S,
+                                     const int32_t* rows, double* y) {
+  const long long m = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (m >= M) return;
+  const int r = blockIdx.y, v = rows[2 * r], slot = rows[2 * r + 1];
+  const int64_t* dg = diag + (size_t)m * S * SIMPLYP_NDIAG;
+  int failed = 0;
+  for (int s = 0; s < S; ++s) failed |= dg[(size_t)s * SIMPLYP_NDIAG + SIMPLYP_DG_STATUS] != 0;
+  const double* st = stats + (size_t)m * V * SIMPLYP_NSTAT;
+  y[(size_t)r * M + m] = failed ? NAN : (slot < 0 ? mcmc_member_lp(st, V, dg, S) : st[(size_t)v * SIMPLYP_NSTAT + slot]);
+}
+
+// Estimators.  A warp walks a list of draws of one row; lane l owns the parameters l and l + 32 (first-order sums in
+// registers, its rows of the second-order triangle in shared memory).  Each draw's P centred values are staged in the
+// warp's shared memory, so every lane sees a, b, AB_k and BA_j.  The point estimates split the used samples over the
+// 8 warps of one block a row; the bootstrap spreads the resamples of a row over SB_SLOTS warps (resample t goes to warp
+// slot t mod SB_SLOTS), each keeping sums of (resampled index - point estimate) and its square, which one thread per
+// output adds up over the slots in order.  Every sum has a fixed order, so nothing depends on scheduling.
+constexpr int SB_WARPS = 8;
+constexpr int SB_GROUPS = 8;                        // bootstrap blocks a row
+constexpr int SB_SLOTS = SB_WARPS * SB_GROUPS;
+constexpr long long SB_PASS_BYTES = 256ll << 20;    // workspace of one pass of rows
+
+struct SbAcc {
+  double s1[2], st[2];        // sum b (ab_j - a), sum (a - ab_j)^2 for j = lane, lane + 32
+  double sa, sb, saa, sbb;    // sum a, sum b, sum a^2, sum b^2
+};
+
+__device__ void sb_process(const double* yr, int P, int K, int so, double c, long long i, double* rec, double* acc2,
+                           SbAcc& w) {
+  const int lane = threadIdx.x & 31;
+  for (int e = lane; e < P; e += 32) rec[e] = yr[(size_t)i * P + e] - c;
+  __syncwarp();
+  const double a = rec[0], b = rec[P - 1];
+  w.sa += a;
+  w.sb += b;
+  w.saa += a * a;
+  w.sbb += b * b;
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const int j = lane + 32 * h;
+    if (j >= K) continue;
+    const double ab = rec[1 + j], d = a - ab;
+    w.s1[h] += b * (ab - a);
+    w.st[h] += d * d;
+    if (so) {
+      const double ba = rec[K + 1 + j], a_b = a * b;
+      double* row = acc2 + sobol_pair(K, j, j + 1) - (j + 1);
+      for (int k = j + 1; k < K; ++k) row[k] += ba * rec[1 + k] - a_b;
+    }
+  }
+  __syncwarp();
+}
+
+// Draws k in [k0, k1) of one row: sample used[pos(k)], pos(k) = k (BOOT = false) or the bootstrap pick of resample t
+// (BOOT = true, k0 = 0).  Positions come 128 at a time, four a lane, and are broadcast in draw order.
+template <bool BOOT>
+__device__ void sb_accumulate(const double* yr, int P, int K, int so, double c, const int* used, uint32_t n,
+                              long long k0, long long k1, uint64_t seed, uint32_t t, double* rec, double* acc2,
+                              SbAcc& w) {
+  const int lane = threadIdx.x & 31;
+  for (long long base = k0; base < k1; base += 128) {
+    uint32_t pos[4];
+    if (BOOT) {
+      uint32_t r[4];
+      sobol_boot_words(seed, t, (uint32_t)(base >> 2) + lane, r);
+#pragma unroll
+      for (int q = 0; q < 4; ++q) pos[q] = sobol_boot_pick(r[q], n);
+    } else {
+#pragma unroll
+      for (int q = 0; q < 4; ++q) pos[q] = (uint32_t)(base + 4 * lane + q);
+    }
+    const int cnt = (int)(k1 - base < 128 ? k1 - base : 128);
+    for (int src = 0; src * 4 < cnt; ++src) {
+#pragma unroll
+      for (int q = 0; q < 4; ++q) {
+        const uint32_t p = __shfl_sync(0xffffffffu, pos[q], src);
+        if (src * 4 + q < cnt) sb_process(yr, P, K, so, c, used[p], rec, acc2, w);
+      }
+    }
+  }
+}
+
+__device__ void sb_zero(SbAcc& w) {
+  w.s1[0] = w.s1[1] = w.st[0] = w.st[1] = 0.0;
+  w.sa = w.sb = w.saa = w.sbb = 0.0;
+}
+
+// Zero lane j's rows of a warp's second-order triangle.
+__device__ void sb_zero_rows(double* acc2, int K, int so) {
+  if (!so) return;
+  const int lane = threadIdx.x & 31;
+  for (int j = lane; j < K; j += 32)
+    for (int k = j + 1; k < K; ++k) acc2[sobol_pair(K, j, k)] = 0.0;
+  __syncwarp();
+}
+
+// Fixed-order sum of one value a thread over the block (lanes by xor tree, then the warps in order).
+__device__ double sb_block_sum(double v, double* scratch) {
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  __syncthreads();
+  if (lane == 0) scratch[warp] = v;
+  __syncthreads();
+  double s = 0.0;
+  for (int w = 0; w < SB_WARPS; ++w) s += scratch[w];
+  return s;
+}
+
+// Shared memory of one warp: P staged values, the second-order triangle, the K first-order indices of a resample.
+__host__ __device__ inline int sb_warp_doubles(int K, int so) {
+  return sobol_slots(K, so) + (so ? K * (K - 1) / 2 : 0) + K;
+}
+
+// One block a row: used samples (in order) into used_ws, c, V, and the point estimates.
+__global__ void __launch_bounds__(SB_WARPS * 32) sobol_point_kernel(const SimplypSobol sb, const double* y,
+                                                                    long long row0, int* used_ws, double* S1,
+                                                                    double* ST, double* S2, double* mean, double* var,
+                                                                    int64_t* n_used) {
+  extern __shared__ double sb_smem[];
+  __shared__ double part[SB_WARPS][2 * SIMPLYP_MCMC_MAX_FREE];
+  __shared__ double s1v[SIMPLYP_MCMC_MAX_FREE];
+  __shared__ double scratch[SB_WARPS];
+  __shared__ int wcount[SB_WARPS];
+  const int K = sb.n_free, so = sb.second_order, P = sobol_slots(K, so);
+  const long long N = sb.n_base, r = row0 + blockIdx.x;
+  const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const double* yr = y + (size_t)r * N * P;
+  int* used = used_ws + (size_t)blockIdx.x * N;
+
+  long long n = 0;
+  for (long long i0 = 0; i0 < N; i0 += SB_WARPS * 32) {
+    const long long i = i0 + tid;
+    bool ok = i < N;
+    for (int e = 0; ok && e < P; ++e) ok = isfinite(yr[(size_t)i * P + e]);
+    const unsigned mask = __ballot_sync(0xffffffffu, ok);
+    if (lane == 0) wcount[warp] = __popc(mask);
+    __syncthreads();
+    long long off = n;
+    int total = 0;
+    for (int w = 0; w < SB_WARPS; ++w) {
+      if (w < warp) off += wcount[w];
+      total += wcount[w];
+    }
+    if (ok) used[off + __popc(mask & ((1u << lane) - 1u))] = (int)i;
+    n += total;
+    __syncthreads();
+  }
+
+  double s = 0.0;
+  for (long long q = tid; q < n; q += SB_WARPS * 32)
+    for (int e = 0; e < P; ++e) s += yr[(size_t)used[q] * P + e];
+  const double c = n > 0 ? sb_block_sum(s, scratch) / ((double)n * P) : NAN;
+  s = 0.0;
+  for (long long q = tid; q < n; q += SB_WARPS * 32) {
+    const double* x = yr + (size_t)used[q] * P;
+    s += x[0] - c;
+    s += x[P - 1] - c;
+  }
+  const double mu = sb_block_sum(s, scratch) / (2.0 * n);
+  s = 0.0;
+  for (long long q = tid; q < n; q += SB_WARPS * 32) {
+    const double* x = yr + (size_t)used[q] * P;
+    const double da = (x[0] - c) - mu, db = (x[P - 1] - c) - mu;
+    s += da * da;
+    s += db * db;
+  }
+  const double V = n >= 2 ? sb_block_sum(s, scratch) / (2.0 * n) : NAN;
+  const bool ok = n >= 2 && V > 0.0;
+
+  double* rec = sb_smem + (size_t)warp * sb_warp_doubles(K, so);
+  double* acc2 = rec + P;
+  sb_zero_rows(acc2, K, so);
+  SbAcc w;
+  sb_zero(w);
+  if (ok) sb_accumulate<false>(yr, P, K, so, c, used, (uint32_t)n, n * warp / SB_WARPS, n * (warp + 1) / SB_WARPS, 0,
+                               0, rec, acc2, w);
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const int j = lane + 32 * h;
+    if (j < K) {
+      part[warp][j] = w.s1[h];
+      part[warp][SIMPLYP_MCMC_MAX_FREE + j] = w.st[h];
+    }
+  }
+  __syncthreads();
+  for (int j = tid; j < K; j += SB_WARPS * 32) {
+    double a1 = 0.0, aT = 0.0;
+    for (int v = 0; v < SB_WARPS; ++v) {
+      a1 += part[v][j];
+      aT += part[v][SIMPLYP_MCMC_MAX_FREE + j];
+    }
+    const double s1 = ok ? (a1 / n) / V : NAN;
+    s1v[j] = s1;
+    S1[(size_t)r * K + j] = s1;
+    ST[(size_t)r * K + j] = ok ? 0.5 * (aT / n) / V : NAN;
+  }
+  if (so) {
+    __syncthreads();
+    for (int q = tid; q < K * K; q += SB_WARPS * 32) {
+      const int j = q / K, k = q % K;
+      double v2 = NAN;
+      if (j < k && ok) {
+        const int pr = sobol_pair(K, j, k);
+        double a2 = 0.0;
+        for (int v = 0; v < SB_WARPS; ++v) a2 += sb_smem[(size_t)v * sb_warp_doubles(K, so) + P + pr];
+        v2 = (a2 / n) / V - s1v[j] - s1v[k];
+      }
+      S2[(size_t)r * K * K + q] = v2;
+    }
+  }
+  if (tid == 0) {
+    mean[r] = c;
+    var[r] = V;
+    n_used[r] = n;
+  }
+}
+
+// Grid (SB_GROUPS, rows of the pass): warp slot u = blockIdx.x * SB_WARPS + warp takes resamples u, u + SB_SLOTS, ...
+// part1[row][u][4][K]: sums of d and d^2 for S1 and ST (d = resampled - point estimate); part2[row][u][pair][2]
+// likewise for S2.
+__global__ void __launch_bounds__(SB_WARPS * 32) sobol_boot_kernel(const SimplypSobol sb, const double* y,
+                                                                   long long row0, const int* used_ws, int n_boot,
+                                                                   uint64_t seed, const double* S1, const double* ST,
+                                                                   const double* S2, const double* mean,
+                                                                   const int64_t* n_used, double* part1,
+                                                                   double* part2) {
+  extern __shared__ double sb_smem[];
+  const int K = sb.n_free, so = sb.second_order, P = sobol_slots(K, so), np2 = so ? K * (K - 1) / 2 : 0;
+  const long long N = sb.n_base, rl = blockIdx.y, r = row0 + rl;
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, u = blockIdx.x * SB_WARPS + warp;
+  const double* yr = y + (size_t)r * N * P;
+  const int* used = used_ws + (size_t)rl * N;
+  const long long n = n_used[r];
+  const double c = mean[r];
+  double* rec = sb_smem + (size_t)warp * sb_warp_doubles(K, so);
+  double* acc2 = rec + P;
+  double* s1t = acc2 + np2;
+  double* p1 = part1 + ((size_t)rl * SB_SLOTS + u) * 4 * K;
+  double* p2 = part2 + ((size_t)rl * SB_SLOTS + u) * 2 * np2;
+  double d1[2] = {0.0, 0.0}, q1[2] = {0.0, 0.0}, dT[2] = {0.0, 0.0}, qT[2] = {0.0, 0.0};
+  if (so)
+    for (int j = lane; j < K; j += 32)
+      for (int k = j + 1; k < K; ++k) p2[2 * sobol_pair(K, j, k)] = p2[2 * sobol_pair(K, j, k) + 1] = 0.0;
+  for (int t = u; n >= 2 && t < n_boot; t += SB_SLOTS) {
+    SbAcc w;
+    sb_zero(w);
+    sb_zero_rows(acc2, K, so);
+    sb_accumulate<true>(yr, P, K, so, c, used, (uint32_t)n, 0, n, seed, (uint32_t)t, rec, acc2, w);
+    const double two = 2.0 * n, mu = (w.sa + w.sb) / two, Vt = (w.saa + w.sbb) / two - mu * mu;
+    const bool ok = Vt > 0.0;
+#pragma unroll
+    for (int h = 0; h < 2; ++h) {
+      const int j = lane + 32 * h;
+      if (j >= K) continue;
+      const double s1 = ok ? (w.s1[h] / n) / Vt : NAN, st = ok ? 0.5 * (w.st[h] / n) / Vt : NAN;
+      s1t[j] = s1;
+      const double e1 = s1 - S1[(size_t)r * K + j], eT = st - ST[(size_t)r * K + j];
+      d1[h] += e1;
+      q1[h] += e1 * e1;
+      dT[h] += eT;
+      qT[h] += eT * eT;
+    }
+    __syncwarp();
+    if (so)
+      for (int j = lane; j < K; j += 32)
+        for (int k = j + 1; k < K; ++k) {
+          const int pr = sobol_pair(K, j, k);
+          const double s2 = ok ? (acc2[pr] / n) / Vt - s1t[j] - s1t[k] : NAN;
+          const double e2 = s2 - S2[((size_t)r * K + j) * K + k];
+          p2[2 * pr] += e2;
+          p2[2 * pr + 1] += e2 * e2;
+        }
+    __syncwarp();
+  }
+#pragma unroll
+  for (int h = 0; h < 2; ++h) {
+    const int j = lane + 32 * h;
+    if (j >= K) continue;
+    p1[j] = d1[h];
+    p1[K + j] = q1[h];
+    p1[2 * K + j] = dT[h];
+    p1[3 * K + j] = qT[h];
+  }
+}
+
+// conf = z std(ddof 1) over the resamples, from the per-slot sums, added in slot order.
+__global__ void sobol_conf_kernel(const SimplypSobol sb, long long row0, int n_boot, double z, const int64_t* n_used,
+                                  const double* part1, const double* part2, double* S1_conf, double* ST_conf,
+                                  double* S2_conf) {
+  const int K = sb.n_free, so = sb.second_order, np2 = so ? K * (K - 1) / 2 : 0;
+  const long long rl = blockIdx.x, r = row0 + rl;
+  const bool ok = n_boot >= 2 && n_used[r] >= 2;
+  const int n_out = 2 * K + (so ? K * K : 0);
+  for (int q = threadIdx.x; q < n_out; q += blockDim.x) {
+    double d = 0.0, dd = 0.0;
+    bool pair = true;
+    if (q < 2 * K) {
+      const int which = q / K, j = q % K;
+      for (int u = 0; u < SB_SLOTS; ++u) {
+        const double* p1 = part1 + ((size_t)rl * SB_SLOTS + u) * 4 * K;
+        d += p1[2 * K * which + j];
+        dd += p1[2 * K * which + K + j];
+      }
+    } else {
+      const int j = (q - 2 * K) / K, k = (q - 2 * K) % K;
+      pair = j < k;
+      if (pair)
+        for (int u = 0; u < SB_SLOTS; ++u) {
+          const double* p2 = part2 + ((size_t)rl * SB_SLOTS + u) * 2 * np2 + 2 * sobol_pair(K, j, k);
+          d += p2[0];
+          dd += p2[1];
+        }
+    }
+    const double nb = (double)n_boot, v = (dd - d * d / nb) / (nb - 1.0);
+    const double conf = (ok && pair) ? z * sqrt(v > 0.0 ? v : 0.0) : NAN;
+    if (q < K) S1_conf[(size_t)r * K + q] = conf;
+    else if (q < 2 * K) ST_conf[(size_t)r * K + q - K] = conf;
+    else S2_conf[(size_t)r * K * K + q - 2 * K] = conf;
+  }
+}
+
+int check_sobol(const SimplypSobol* sb) {
+  if (!sb) return fail(SIMPLYP_EINVAL, "sobol: null argument%s");
+  const int K = sb->n_free;
+  if (K < 1 || K > SIMPLYP_MCMC_MAX_FREE) return fail(SIMPLYP_EINVAL, "sobol: 1..SIMPLYP_MCMC_MAX_FREE free parameters%s");
+  if (sb->n_sc < 1 || (sb->second_order != 0 && sb->second_order != 1))
+    return fail(SIMPLYP_EINVAL, "sobol: bad n_sc / second_order%s");
+  const int64_t N = sb->n_base;
+  if (N < 2 || N > (1ll << 31) || (N & (N - 1)) != 0) return fail(SIMPLYP_EINVAL, "sobol: n_base must be a power of two in 2..2^31%s");
+  if (sb->skip < 0 || sb->skip + N > (1ll << 32)) return fail(SIMPLYP_EINVAL, "sobol: need skip >= 0 and skip + n_base <= 2^32%s");
+  return check_targets(sb->param, K, sb->n_sc, sb->sc_per_member, "sobol");
+}
+
+// Rows a pass of the estimators handles, and the workspace of one row.
+int64_t sobol_row_bytes(const SimplypSobol& sb) {
+  const int K = sb.n_free, np2 = sb.second_order ? K * (K - 1) / 2 : 0;
+  return ((4 * sb.n_base + 7) & ~7ll) + (int64_t)SB_SLOTS * 8 * (4 * K + 2 * np2);
+}
+int64_t sobol_pass_rows(const SimplypSobol& sb, int64_t n_rows) {
+  int64_t rows = SB_PASS_BYTES / sobol_row_bytes(sb);
+  if (rows < 1) rows = 1;
+  if (rows > 65535) rows = 65535;
+  return rows < n_rows ? rows : n_rows;
 }
 
 }  // namespace
@@ -2302,6 +2680,86 @@ int simplyp_nanquantile_device(const double* x, int64_t n_rows, int64_t n_cols, 
     nq_hist_kernel<<<hgrid, NQ_HIST_THREADS, 0, st>>>(x, n_cols, n_q, pass, ws);
     nq_pick_kernel<<<(unsigned)n_rows, NQ_RANKS, 0, st>>>(n_rows, qa, pass, ws, quantiles);
     g_launches.fetch_add(2);
+    SP_CUDA(cudaGetLastError());
+  }
+  return SIMPLYP_OK;
+}
+
+int simplyp_sobol_design_device(const SimplypSobol* sb, int64_t member_offset, int64_t n_members,
+                                double* member_params, double* sc_params, void* stream) {
+  const int rc = check_sobol(sb);
+  if (rc) return rc;
+  if (!member_params || !sc_params) return fail(SIMPLYP_EINVAL, "sobol design: null parameter rows%s");
+  const int64_t total = sb->n_base * sobol_slots(sb->n_free, sb->second_order);
+  if (member_offset < 0 || n_members < 0 || member_offset + n_members > total)
+    return fail(SIMPLYP_EINVAL, "sobol design: members outside 0 .. n_base * P - 1%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  if (n_members == 0) return SIMPLYP_OK;
+  sobol_design_kernel<<<(unsigned)((n_members + 127) / 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
+      *sb, member_offset, n_members, member_params, sc_params);
+  g_launches.fetch_add(1);
+  SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
+int simplyp_sobol_outputs_device(const double* stats, const int64_t* diag, int64_t n_members, int32_t n_obs_series,
+                                 int32_t n_sc, const int32_t* rows, int32_t n_rows, double* y, void* stream) {
+  if (!diag || !rows || !y || (n_obs_series > 0 && !stats)) return fail(SIMPLYP_EINVAL, "sobol outputs: null argument%s");
+  if (n_members < 0 || n_members > (int64_t)INT32_MAX * 128 || n_obs_series < 0 || n_sc < 1 || n_rows < 1 ||
+      n_rows > 65535)
+    return fail(SIMPLYP_EINVAL, "sobol outputs: bad dims (M >= 0, V >= 0, S >= 1, 1..65535 rows)%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  if (n_members == 0) return SIMPLYP_OK;
+  const dim3 grid((unsigned)((n_members + 255) / 256), (unsigned)n_rows);
+  sobol_outputs_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(stats, diag, n_members, n_obs_series,
+                                                                           n_sc, rows, y);
+  g_launches.fetch_add(1);
+  SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
+int64_t simplyp_sobol_workspace_bytes(const SimplypSobol* sb, int64_t n_rows) {
+  const int rc = check_sobol(sb);
+  if (rc) return rc;
+  if (n_rows < 0) return fail(SIMPLYP_EINVAL, "sobol: negative row count%s");
+  return sobol_pass_rows(*sb, n_rows) * sobol_row_bytes(*sb);
+}
+
+int simplyp_sobol_indices_device(const SimplypSobol* sb, const double* y, int64_t n_rows, int32_t n_boot,
+                                 double conf_z, uint64_t seed, double* S1, double* ST, double* S1_conf,
+                                 double* ST_conf, double* S2, double* S2_conf, double* mean, double* var,
+                                 int64_t* n_used, void* workspace, int64_t workspace_bytes, void* stream) {
+  const int rc = check_sobol(sb);
+  if (rc) return rc;
+  if (!y || !S1 || !ST || !S1_conf || !ST_conf || !mean || !var || !n_used || (sb->second_order && (!S2 || !S2_conf)))
+    return fail(SIMPLYP_EINVAL, "sobol indices: null argument%s");
+  if (n_rows < 0 || n_boot < 0 || n_boot > 10000 || !(conf_z >= 0.0 && conf_z < INFINITY))
+    return fail(SIMPLYP_EINVAL, "sobol indices: need n_rows >= 0, n_boot in 0..10^4 and a finite conf_z >= 0%s");
+  const int64_t need = simplyp_sobol_workspace_bytes(sb, n_rows);
+  if (!workspace || workspace_bytes < need)
+    return fail(SIMPLYP_EINVAL, "sobol indices: workspace smaller than simplyp_sobol_workspace_bytes%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  if (n_rows == 0) return SIMPLYP_OK;
+  const int K = sb->n_free, so = sb->second_order;
+  const size_t smem = (size_t)SB_WARPS * sb_warp_doubles(K, so) * sizeof(double);
+  if (smem > 48 * 1024) {
+    SP_CUDA(cudaFuncSetAttribute(sobol_point_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+    SP_CUDA(cudaFuncSetAttribute(sobol_boot_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  }
+  const int64_t rows = sobol_pass_rows(*sb, n_rows);
+  char* ws = static_cast<char*>(workspace);
+  int* used = reinterpret_cast<int*>(ws);
+  double* part1 = reinterpret_cast<double*>(ws + rows * ((4 * sb->n_base + 7) & ~7ll));
+  double* part2 = part1 + (size_t)rows * SB_SLOTS * 4 * K;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  for (int64_t r0 = 0; r0 < n_rows; r0 += rows) {
+    const int64_t nr = n_rows - r0 < rows ? n_rows - r0 : rows;
+    sobol_point_kernel<<<(unsigned)nr, SB_WARPS * 32, smem, st>>>(*sb, y, r0, used, S1, ST, S2, mean, var, n_used);
+    sobol_boot_kernel<<<dim3(SB_GROUPS, (unsigned)nr), SB_WARPS * 32, smem, st>>>(
+        *sb, y, r0, used, n_boot, seed, S1, ST, S2, mean, n_used, part1, part2);
+    sobol_conf_kernel<<<(unsigned)nr, 256, 0, st>>>(*sb, r0, n_boot, conf_z, n_used, part1, part2, S1_conf, ST_conf,
+                                                    S2_conf);
+    g_launches.fetch_add(3);
     SP_CUDA(cudaGetLastError());
   }
   return SIMPLYP_OK;

@@ -192,6 +192,58 @@ class Engine:
                                      ws.data_ptr() if ws is not None else None, need, stream)
         return quantiles, mean, count
 
+    # ------------------------------------------------------------------ Sobol' sensitivity
+    def sobol_design(self, sb, member_params, sc_params, member_offset=0, n_members=None):
+        """Write the target columns of design members ``member_offset .. member_offset + n_members`` (default: to
+        the end) of ``member_params`` [N P][NP_MEMBER] and ``sc_params`` ([N P] or [1])[S][NP_SC] for the
+        :class:`_cabi.SimplypSobol` ``sb`` (``simplyp_sobol_design_device``).  Asynchronous."""
+        torch = _torch()
+        if n_members is None:
+            n_members = member_params.shape[0] - member_offset
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            _cabi.sobol_design_device(sb, member_offset, n_members, member_params.data_ptr(), sc_params.data_ptr(),
+                                      stream)
+        return member_params, sc_params
+
+    def sobol_outputs(self, stats, diag, rows, y):
+        """Objective rows ``y`` [R][M] from the fused statistics ``stats`` [M][V][10] and ``diag`` [M][S][4];
+        ``rows`` [R][2] int32 on the device = (series, ``packing.STAT_NAMES`` slot, or -1 for the sampler's lp)
+        (``simplyp_sobol_outputs_device``).  Asynchronous."""
+        torch = _torch()
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            _cabi.sobol_outputs_device(stats.data_ptr(), diag.data_ptr(), stats.shape[0], stats.shape[1],
+                                       diag.shape[1], rows.data_ptr(), rows.shape[0], y.data_ptr(), stream)
+        return y
+
+    def sobol_indices(self, sb, y, n_boot, conf_z, seed, out=None):
+        """Sobol' indices of every row of ``y`` [R][N P] with bootstrap confidences (``simplyp_sobol_indices_device``).
+        Returns a dict of device tensors S1, ST, S1_conf, ST_conf [R][K], S2, S2_conf [R][K][K] (second order
+        only), mean, var [R] and n_used [R]; ``out`` may give them preallocated.  Asynchronous."""
+        torch = _torch()
+        if y.dim() != 2 or y.dtype != torch.float64 or not y.is_contiguous():
+            raise ValueError("sobol_indices takes a contiguous [R][N P] float64 matrix")
+        R, K = y.shape[0], sb.n_free
+        f64 = dict(dtype=torch.float64, device=self.device)
+        if out is None:
+            out = {k: torch.empty((R, K), **f64) for k in ("S1", "ST", "S1_conf", "ST_conf")}
+            if sb.second_order:
+                out.update({k: torch.empty((R, K, K), **f64) for k in ("S2", "S2_conf")})
+            out.update(mean=torch.empty(R, **f64), var=torch.empty(R, **f64),
+                       n_used=torch.empty(R, dtype=torch.int64, device=self.device))
+        need = _cabi.sobol_workspace_bytes(sb, R)
+        ws = self._workspace(need)
+
+        def ptr(k):
+            return out[k].data_ptr() if k in out else None
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            _cabi.sobol_indices_device(sb, y.data_ptr(), R, n_boot, conf_z, seed, ptr("S1"), ptr("ST"),
+                                       ptr("S1_conf"), ptr("ST_conf"), ptr("S2"), ptr("S2_conf"), ptr("mean"),
+                                       ptr("var"), ptr("n_used"), ws.data_ptr(), need, stream)
+        return out
+
     # ------------------------------------------------------------------ Thornthwaite PET
     def thornthwaite_pet(self, t_air, month_start, year_is_leap, latitude_deg, out=None, out_stride=1):
         """Reference ``daily_PET`` (``inputs.py:232-312``) on the device: ``t_air`` [D] (device or host),
