@@ -431,6 +431,71 @@ int simplyp_sobol_indices_device(const SimplypSobol* sb, const double* y, int64_
                                  double* ST_conf, double* S2, double* S2_conf, double* mean, double* var,
                                  int64_t* n_used, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- differential evolution ---------------------------------------------------------------------------------------
+ * scipy.optimize.differential_evolution(updating='deferred', polish=False) over the fit statistics: the best parameter
+ * set of K free parameters (the sampler's targets and boxes, SimplypMcmcParam) in a population of N members.  The
+ * population lives in the unit cube; member rows get lo/hi-clamped values arg1 + (u - 0.5) arg2.  One generation is:
+ *   simplyp_de_trial_device   -> trial[N][K] and the target columns of member_params (and sc_params) rows;
+ *   zero diag, simplyp_calibrate_device on all N rows, simplyp_sobol_outputs_device -> y[R][N];
+ *   simplyp_de_select_device  -> E = -sum_r weights[r] y[r][m] (+inf for a non-zero status word or a NaN), a trial
+ *                                replaces its target when E_trial <= E_target; then one block reduces, in a fixed
+ *                                order, the best index (lowest among the minimal energies), the mean and population
+ *                                std of the finite energies and the counts; writes history row g + 1 - history_base =
+ *                                (-E_best, -mean, std, replaced); adds the failed evaluations (E = +inf) to n_failed;
+ *                                increments the generation g; sets converged = 1 and converged_at = g + 1 when every
+ *                                energy is finite and std <= tol_abs + tol |mean|.
+ * Once converged is set, trial and select return at once: replays queued after convergence change nothing.
+ * simplyp_de_init_device: energies, best, history row 0 and n_failed from the evaluation of the population (the
+ *   caller wrote its rows), converged = 0.
+ * Random words: Philox4x32-10 keyed by the seed; member i at generation g takes group q of four words from counter
+ * (i, g lo, g hi, 4 + 256 q), the generation's mutation factor F ~ U(mutation_lo, mutation_hi) from counter
+ * (0xFFFFFFFF, g lo, g hi, 4); the word assignment is documented in csrc/simplyp_de.cuh.
+ * All three only enqueue work on `stream` (no allocation, no synchronisation), so they can be captured into a graph. */
+enum {
+  SIMPLYP_DE_BEST1BIN = 0,  /* b' = x_best + F (x_r0 - x_r1) */
+  SIMPLYP_DE_RAND1BIN       /* b' = x_r0 + F (x_r1 - x_r2)   */
+};
+
+typedef struct {
+  int32_t n_population;     /* N: >= 3 (best1bin) or >= 4 (rand1bin), < 2^31 */
+  int32_t n_free;           /* K: 1..SIMPLYP_MCMC_MAX_FREE */
+  int32_t n_sc;             /* S of the calibration runs */
+  int32_t sc_per_member;    /* sc_params is [N][S][NP_SC] (required by the SC targets) */
+  int32_t strategy;         /* SIMPLYP_DE_BEST1BIN or SIMPLYP_DE_RAND1BIN */
+  int32_t n_rows;           /* R objective rows of y, 1..65535 */
+  uint64_t seed;            /* Philox key: (low word, high word) */
+  double  mutation_lo, mutation_hi;   /* 0 <= lo <= hi < 2 */
+  double  recombination;    /* CR in [0, 1] */
+  double  tol, tol_abs;     /* finite, >= 0 */
+  SimplypMcmcParam param[SIMPLYP_MCMC_MAX_FREE];
+} SimplypDe;
+
+typedef struct {            /* device pointers */
+  double*  population;      /* [N][K] unit cube */
+  double*  energy;          /* [N] */
+  double*  trial;           /* [N][K] unit cube */
+  int32_t* flags;           /* [N] bit 0: trial accepted, bit 1: evaluation failed */
+  const double* weights;    /* [R] */
+  int64_t* generation;      /* [1] g, generations completed */
+  int64_t* best;            /* [1] index of the best member */
+  int64_t* converged;       /* [1] 0 or 1 */
+  int64_t* converged_at;    /* [1] generation at which converged was set */
+  int64_t* n_failed;        /* [1] evaluations with E = +inf */
+  double*  history;         /* [n_history][4] */
+  int64_t  n_history;
+  int64_t  history_base;    /* generation g + 1 ends in row g + 1 - history_base; the init writes row 0 */
+} SimplypDeState;
+
+/* member_params [N][NP_MEMBER], sc_params [1 or N][S][NP_SC]: the population's rows. */
+int simplyp_de_trial_device(const SimplypDe* de, const SimplypDeState* state, double* member_params,
+                            double* sc_params, void* stream);
+/* y [R][N] (simplyp_sobol_outputs_device) and diag [N][S][NDIAG] of the evaluation of the trials. */
+int simplyp_de_select_device(const SimplypDe* de, const SimplypDeState* state, const double* y, const int64_t* diag,
+                             void* stream);
+/* y [R][N] and diag [N][S][NDIAG] of the evaluation of the population. */
+int simplyp_de_init_device(const SimplypDe* de, const SimplypDeState* state, const double* y, const int64_t* diag,
+                           void* stream);
+
 /* Host-buffer forms: same arguments as HOST pointers; the library stages them through its own
  * (cached) device buffers on `device`, runs and copies the result back before returning. */
 int simplyp_run_host(int device, const SimplypDims* dims, const SimplypOptions* opt,

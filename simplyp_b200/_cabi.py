@@ -27,7 +27,8 @@ EXPORTS = [
     "simplyp_ipc_import", "simplyp_ipc_close", "simplyp_mcmc_propose_device", "simplyp_mcmc_accept_device",
     "simplyp_mcmc_init_device", "simplyp_predictive_draws_device", "simplyp_nanquantile_workspace_bytes",
     "simplyp_nanquantile_device", "simplyp_sobol_design_device", "simplyp_sobol_outputs_device",
-    "simplyp_sobol_workspace_bytes", "simplyp_sobol_indices_device",
+    "simplyp_sobol_workspace_bytes", "simplyp_sobol_indices_device", "simplyp_de_trial_device",
+    "simplyp_de_select_device", "simplyp_de_init_device",
 ]
 MAX_RANKS = 8
 
@@ -54,6 +55,7 @@ class SimplypPeerGather(C.Structure):
 MCMC_MAX_FREE = 64
 NQ_MAX = 16
 MCMC_MEMBER, MCMC_SC_ALL, MCMC_SC_AT = 0, 1, 2
+DE_STRATEGIES = {"best1bin": 0, "rand1bin": 1}
 
 
 class SimplypMcmcParam(C.Structure):
@@ -76,6 +78,20 @@ class SimplypMcmcState(C.Structure):
 class SimplypSobol(C.Structure):
     _fields_ = [("n_free", C.c_int32), ("n_sc", C.c_int32), ("sc_per_member", C.c_int32), ("second_order", C.c_int32),
                 ("n_base", C.c_int64), ("skip", C.c_int64), ("param", SimplypMcmcParam * MCMC_MAX_FREE)]
+
+
+class SimplypDe(C.Structure):
+    _fields_ = [("n_population", C.c_int32), ("n_free", C.c_int32), ("n_sc", C.c_int32), ("sc_per_member", C.c_int32),
+                ("strategy", C.c_int32), ("n_rows", C.c_int32), ("seed", C.c_uint64), ("mutation_lo", C.c_double),
+                ("mutation_hi", C.c_double), ("recombination", C.c_double), ("tol", C.c_double),
+                ("tol_abs", C.c_double), ("param", SimplypMcmcParam * MCMC_MAX_FREE)]
+
+
+class SimplypDeState(C.Structure):
+    _fields_ = [("population", C.c_void_p), ("energy", C.c_void_p), ("trial", C.c_void_p), ("flags", C.c_void_p),
+                ("weights", C.c_void_p), ("generation", C.c_void_p), ("best", C.c_void_p), ("converged", C.c_void_p),
+                ("converged_at", C.c_void_p), ("n_failed", C.c_void_p), ("history", C.c_void_p),
+                ("n_history", C.c_int64), ("history_base", C.c_int64)]
 
 
 class SimplypError(RuntimeError):
@@ -165,6 +181,13 @@ def load():
     lib.simplyp_sobol_indices_device.argtypes = [sbp, vp, C.c_int64, C.c_int32, C.c_double, C.c_uint64, vp, vp, vp,
                                                  vp, vp, vp, vp, vp, vp, vp, C.c_int64, vp]
     lib.simplyp_sobol_indices_device.restype = C.c_int
+    dep, dsp = C.POINTER(SimplypDe), C.POINTER(SimplypDeState)
+    lib.simplyp_de_trial_device.argtypes = [dep, dsp, vp, vp, vp]
+    lib.simplyp_de_trial_device.restype = C.c_int
+    lib.simplyp_de_select_device.argtypes = [dep, dsp, vp, vp, vp]
+    lib.simplyp_de_select_device.restype = C.c_int
+    lib.simplyp_de_init_device.argtypes = [dep, dsp, vp, vp, vp]
+    lib.simplyp_de_init_device.restype = C.c_int
     if lib.simplyp_abi_version() != 4:
         raise SimplypError("ABI version mismatch")
     _lib = lib
@@ -472,6 +495,50 @@ def sobol_indices_device(sb, y_ptr, n_rows, n_boot, conf_z, seed, S1, ST, S1_con
     _check(lib.simplyp_sobol_indices_device(C.byref(sb), y_ptr, int(n_rows), int(n_boot), float(conf_z),
                                             int(seed) & 0xFFFFFFFFFFFFFFFF, S1, ST, S1_conf, ST_conf, S2, S2_conf,
                                             mean, var, n_used, ws_ptr, int(ws_bytes), stream_ptr))
+
+
+def make_de(n_population, targets, lo, hi, n_sc, n_rows, sc_per_member=False, strategy="best1bin",
+            mutation=(0.5, 1.0), recombination=0.7, tol=0.01, tol_abs=0.0, seed=0):
+    """SimplypDe for ``targets`` [(kind, index, pos)] (as :func:`make_mcmc`) with the boxes ``[lo[k], hi[k]]``."""
+    if not 1 <= len(targets) <= MCMC_MAX_FREE:
+        raise ValueError("1..%d free parameters" % MCMC_MAX_FREE)
+    de = SimplypDe()
+    de.n_population, de.n_free, de.n_sc, de.n_rows = int(n_population), len(targets), int(n_sc), int(n_rows)
+    de.sc_per_member, de.strategy = 1 if sc_per_member else 0, DE_STRATEGIES[strategy]
+    de.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+    de.mutation_lo, de.mutation_hi = float(mutation[0]), float(mutation[1])
+    de.recombination, de.tol, de.tol_abs = float(recombination), float(tol), float(tol_abs)
+    for k, (kind, index, pos) in enumerate(targets):
+        p = de.param[k]
+        p.kind, p.index, p.pos, p.lo, p.hi = int(kind), int(index), int(pos), float(lo[k]), float(hi[k])
+    return de
+
+
+def make_de_state(population, energy, trial, flags, weights, generation, best, converged, converged_at, n_failed,
+                  history, n_history, history_base=0):
+    """SimplypDeState from device pointers (torch ``.data_ptr()`` integers)."""
+    st = SimplypDeState()
+    st.population, st.energy, st.trial, st.flags, st.weights = population, energy, trial, flags, weights
+    st.generation, st.best, st.converged, st.converged_at = generation, best, converged, converged_at
+    st.n_failed, st.history, st.n_history, st.history_base = n_failed, history, int(n_history), int(history_base)
+    return st
+
+
+def de_trial_device(de, state, member_ptr, sc_ptr, stream_ptr):
+    """Trials of every member into ``trial`` and the target columns of its rows; asynchronous on ``stream_ptr``."""
+    _check(require_device().simplyp_de_trial_device(C.byref(de), C.byref(state), member_ptr, sc_ptr, stream_ptr))
+
+
+def de_select_device(de, state, y_ptr, diag_ptr, stream_ptr):
+    """Selection, reduction and history row of one generation from the trials' objective rows y [R][N] and diag;
+    asynchronous on ``stream_ptr``."""
+    _check(require_device().simplyp_de_select_device(C.byref(de), C.byref(state), y_ptr, diag_ptr, stream_ptr))
+
+
+def de_init_device(de, state, y_ptr, diag_ptr, stream_ptr):
+    """Energies, best member and history row 0 from the population's objective rows y [R][N] and diag; asynchronous
+    on ``stream_ptr``."""
+    _check(require_device().simplyp_de_init_device(C.byref(de), C.byref(state), y_ptr, diag_ptr, stream_ptr))
 
 
 def workspace_bytes(dims, calibrate, rank_stats=False):

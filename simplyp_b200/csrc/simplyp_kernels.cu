@@ -17,6 +17,7 @@
 //                                   arithmetic in simplyp_mcmc.cuh) over the fused log-likelihood
 //   predictive_draws_kernel         posterior predictive draws of the simulated series (simplyp_bands.cuh)
 //   nanquantile_kernel, nq_prepare_kernel, nq_hist_kernel, nq_pick_kernel  np.nanquantile of the rows of a matrix
+//   de_trial_kernel, de_select_kernel, de_init_kernel, de_reduce_kernel  differential evolution (simplyp_de.cuh)
 //
 // There is deliberately no host implementation of the integration in this library.
 #include <cuda_runtime.h>
@@ -36,6 +37,7 @@
 #include "simplyp_mcmc.cuh"
 #include "simplyp_bands.cuh"
 #include "simplyp_sobol.cuh"
+#include "simplyp_de.cuh"
 
 using namespace simplyp;
 
@@ -2209,6 +2211,134 @@ int64_t sobol_pass_rows(const SimplypSobol& sb, int64_t n_rows) {
   return rows < n_rows ? rows : n_rows;
 }
 
+// ------------------------------------------------------------------------------------------ differential evolution
+// One thread per member (simplyp_de.cuh holds the arithmetic); once converged is set every kernel returns at once.
+__global__ void de_trial_kernel(const SimplypDe de, const SimplypDeState st, double* member_params, double* sc_params) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= de.n_population || *st.converged) return;
+  const long long g = *st.generation;
+  const int K = de.n_free, S = de.n_sc;
+  double* tr = st.trial + (size_t)i * K;
+  de_trial_member(de, st.population, *st.best, g, i, de_dither(de, g), tr);
+  double* mrow = member_params + (size_t)i * SIMPLYP_NP_MEMBER;
+  double* srow = sc_params + (de.sc_per_member ? (size_t)i * S * SIMPLYP_NP_SC : 0);
+  for (int j = 0; j < K; ++j) {
+    const SimplypMcmcParam& p = de.param[j];
+    const double v = de_scale(p, tr[j]);
+    if (p.kind == SIMPLYP_MCMC_MEMBER) {
+      mrow[p.index] = v;
+    } else if (p.kind == SIMPLYP_MCMC_SC_AT) {
+      srow[(size_t)p.pos * SIMPLYP_NP_SC + p.index] = v;
+    } else {
+      for (int s = 0; s < S; ++s) srow[(size_t)s * SIMPLYP_NP_SC + p.index] = v;
+    }
+  }
+}
+
+__global__ void de_select_kernel(const SimplypDe de, const SimplypDeState st, const double* y, const int64_t* diag) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= de.n_population || *st.converged) return;
+  const double e = de_energy(y, de.n_population, de.n_rows, st.weights, i,
+                             diag + (size_t)i * de.n_sc * SIMPLYP_NDIAG, de.n_sc);
+  const int acc = de_select_member(de.n_free, i, e, st.trial + (size_t)i * de.n_free, st.population, st.energy);
+  st.flags[i] = acc | (e == INFINITY ? 2 : 0);
+}
+
+__global__ void de_init_kernel(const SimplypDe de, const SimplypDeState st, const double* y, const int64_t* diag) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= de.n_population) return;
+  const double e = de_energy(y, de.n_population, de.n_rows, st.weights, i,
+                             diag + (size_t)i * de.n_sc * SIMPLYP_NDIAG, de.n_sc);
+  st.energy[i] = e;
+  st.flags[i] = e == INFINITY ? 2 : 0;
+}
+
+// One block.  Thread t walks members t, t + DE_THREADS, ... in order, then a tree halves the partials in order: the
+// result does not depend on scheduling (tests/de_reference.py restates the order).  Sums run over the finite energies.
+constexpr int DE_THREADS = 256;
+__global__ void de_reduce_kernel(const SimplypDe de, const SimplypDeState st, int init) {
+  __shared__ double s_e[DE_THREADS], s_sum[DE_THREADS];
+  __shared__ long long s_i[DE_THREADS], s_fin[DE_THREADS], s_acc[DE_THREADS], s_fail[DE_THREADS];
+  if (!init && *st.converged) return;
+  const int t = threadIdx.x, N = de.n_population;
+  double be = INFINITY, sum = 0.0;
+  long long bi = N, fin = 0, acc = 0, nfail = 0;
+  for (int i = t; i < N; i += DE_THREADS) {
+    const double e = st.energy[i];
+    if (e < be || (e == be && i < bi)) { be = e; bi = i; }
+    const int finite = fabs(e) < INFINITY;
+    sum = mc_add(sum, finite ? e : 0.0);
+    fin += finite;
+    acc += st.flags[i] & 1;
+    nfail += (st.flags[i] >> 1) & 1;
+  }
+  s_e[t] = be; s_i[t] = bi; s_sum[t] = sum; s_fin[t] = fin; s_acc[t] = acc; s_fail[t] = nfail;
+  __syncthreads();
+  for (int s = DE_THREADS / 2; s > 0; s >>= 1) {
+    if (t < s) {
+      if (s_e[t + s] < s_e[t] || (s_e[t + s] == s_e[t] && s_i[t + s] < s_i[t])) { s_e[t] = s_e[t + s]; s_i[t] = s_i[t + s]; }
+      s_sum[t] = mc_add(s_sum[t], s_sum[t + s]);
+      s_fin[t] += s_fin[t + s]; s_acc[t] += s_acc[t + s]; s_fail[t] += s_fail[t + s];
+    }
+    __syncthreads();
+  }
+  const long long n_fin = s_fin[0];
+  const double mean = n_fin ? mc_div(s_sum[0], (double)n_fin) : NAN;
+  double ss = 0.0;
+  for (int i = t; i < N; i += DE_THREADS) {
+    const double e = st.energy[i];
+    const double d = fabs(e) < INFINITY ? mc_sub(e, mean) : 0.0;
+    ss = mc_add(ss, mc_mul(d, d));
+  }
+  __syncthreads();
+  s_sum[t] = ss;
+  __syncthreads();
+  for (int s = DE_THREADS / 2; s > 0; s >>= 1) {
+    if (t < s) s_sum[t] = mc_add(s_sum[t], s_sum[t + s]);
+    __syncthreads();
+  }
+  if (t != 0) return;
+  const double sd = n_fin ? sqrt(mc_div(s_sum[0], (double)n_fin)) : NAN;
+  const long long g = *st.generation;
+  const long long row = init ? 0 : g + 1 - st.history_base;
+  if (row >= 0 && row < st.n_history) {
+    double* h = st.history + (size_t)row * 4;
+    h[0] = -s_e[0]; h[1] = -mean; h[2] = sd; h[3] = (double)s_acc[0];
+  }
+  *st.best = s_i[0];
+  *st.n_failed += s_fail[0];
+  if (init) {
+    *st.converged = 0;
+    return;
+  }
+  *st.generation = g + 1;
+  if (n_fin == N && sd <= mc_add(de.tol_abs, mc_mul(de.tol, fabs(mean)))) {
+    *st.converged = 1;
+    *st.converged_at = g + 1;
+  }
+}
+
+int check_de(const SimplypDe* de, const SimplypDeState* st) {
+  if (!de || !st) return fail(SIMPLYP_EINVAL, "de: null argument%s");
+  const int K = de->n_free, N = de->n_population;
+  if (K < 1 || K > SIMPLYP_MCMC_MAX_FREE) return fail(SIMPLYP_EINVAL, "de: 1..SIMPLYP_MCMC_MAX_FREE free parameters%s");
+  if (de->strategy != SIMPLYP_DE_BEST1BIN && de->strategy != SIMPLYP_DE_RAND1BIN) return fail(SIMPLYP_EINVAL, "de: unknown strategy%s");
+  if (N < (de->strategy == SIMPLYP_DE_RAND1BIN ? 4 : 3) || N == INT32_MAX)
+    return fail(SIMPLYP_EINVAL, "de: n_population below what the strategy needs (3 for best1bin, 4 for rand1bin)%s");
+  if (de->n_sc < 1 || de->n_rows < 1 || de->n_rows > 65535) return fail(SIMPLYP_EINVAL, "de: bad n_sc / n_rows%s");
+  if (!(de->mutation_lo >= 0.0 && de->mutation_lo <= de->mutation_hi && de->mutation_hi < 2.0))
+    return fail(SIMPLYP_EINVAL, "de: need 0 <= mutation_lo <= mutation_hi < 2%s");
+  if (!(de->recombination >= 0.0 && de->recombination <= 1.0)) return fail(SIMPLYP_EINVAL, "de: recombination outside [0, 1]%s");
+  if (!(de->tol >= 0.0 && de->tol < INFINITY && de->tol_abs >= 0.0 && de->tol_abs < INFINITY))
+    return fail(SIMPLYP_EINVAL, "de: tol and tol_abs must be finite and >= 0%s");
+  const int rc = check_targets(de->param, K, de->n_sc, de->sc_per_member, "de");
+  if (rc) return rc;
+  if (!st->population || !st->energy || !st->trial || !st->flags || !st->weights || !st->generation || !st->best ||
+      !st->converged || !st->converged_at || !st->n_failed || (st->n_history > 0 && !st->history) || st->n_history < 0)
+    return fail(SIMPLYP_EINVAL, "de: null state pointer%s");
+  return SIMPLYP_OK;
+}
+
 }  // namespace
 
 // ============================================================================================ C-ABI
@@ -2762,6 +2892,50 @@ int simplyp_sobol_indices_device(const SimplypSobol* sb, const double* y, int64_
     g_launches.fetch_add(3);
     SP_CUDA(cudaGetLastError());
   }
+  return SIMPLYP_OK;
+}
+
+int simplyp_de_trial_device(const SimplypDe* de, const SimplypDeState* state, double* member_params,
+                            double* sc_params, void* stream) {
+  const int rc = check_de(de, state);
+  if (rc) return rc;
+  if (!member_params || !sc_params) return fail(SIMPLYP_EINVAL, "de: null parameter rows%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  const int N = de->n_population;
+  de_trial_kernel<<<(N + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(*de, *state, member_params,
+                                                                                  sc_params);
+  g_launches.fetch_add(1);
+  SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
+int simplyp_de_select_device(const SimplypDe* de, const SimplypDeState* state, const double* y, const int64_t* diag,
+                             void* stream) {
+  const int rc = check_de(de, state);
+  if (rc) return rc;
+  if (!y || !diag) return fail(SIMPLYP_EINVAL, "de: null objective rows or diag%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  const int N = de->n_population;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  de_select_kernel<<<(N + 127) / 128, 128, 0, st>>>(*de, *state, y, diag);
+  de_reduce_kernel<<<1, DE_THREADS, 0, st>>>(*de, *state, 0);
+  g_launches.fetch_add(2);
+  SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
+int simplyp_de_init_device(const SimplypDe* de, const SimplypDeState* state, const double* y, const int64_t* diag,
+                           void* stream) {
+  const int rc = check_de(de, state);
+  if (rc) return rc;
+  if (!y || !diag) return fail(SIMPLYP_EINVAL, "de: null objective rows or diag%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  const int N = de->n_population;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  de_init_kernel<<<(N + 127) / 128, 128, 0, st>>>(*de, *state, y, diag);
+  de_reduce_kernel<<<1, DE_THREADS, 0, st>>>(*de, *state, 1);
+  g_launches.fetch_add(2);
+  SP_CUDA(cudaGetLastError());
   return SIMPLYP_OK;
 }
 

@@ -244,6 +244,28 @@ class Engine:
                                        ptr("var"), ptr("n_used"), ws.data_ptr(), need, stream)
         return out
 
+    # ------------------------------------------------------------------ differential evolution
+    def _de_call(self, fn, *args):
+        torch = _torch()
+        with torch.cuda.device(self.device):
+            fn(*args, torch.cuda.current_stream().cuda_stream)
+
+    def de_trial(self, de, state, member_params, sc_params):
+        """Trials of the :class:`_cabi.SimplypDe` population ``state`` into its trial buffer and the target columns of
+        ``member_params`` [N][NP_MEMBER] / ``sc_params`` ([N] or [1])[S][NP_SC] (``simplyp_de_trial_device``).
+        Asynchronous."""
+        self._de_call(_cabi.de_trial_device, de, state, member_params.data_ptr(), sc_params.data_ptr())
+
+    def de_select(self, de, state, y, diag):
+        """Selection of one generation from the trials' objective rows ``y`` [R][N] (:meth:`sobol_outputs`) and
+        ``diag`` [N][S][4] (``simplyp_de_select_device``).  Asynchronous."""
+        self._de_call(_cabi.de_select_device, de, state, y.data_ptr(), diag.data_ptr())
+
+    def de_init(self, de, state, y, diag):
+        """Energies, best member and history row 0 from the population's objective rows ``y`` [R][N] and ``diag``
+        (``simplyp_de_init_device``).  Asynchronous."""
+        self._de_call(_cabi.de_init_device, de, state, y.data_ptr(), diag.data_ptr())
+
     # ------------------------------------------------------------------ Thornthwaite PET
     def thornthwaite_pet(self, t_air, month_start, year_is_leap, latitude_deg, out=None, out_stride=1):
         """Reference ``daily_PET`` (``inputs.py:232-312``) on the device: ``t_air`` [D] (device or host),

@@ -53,6 +53,22 @@ class SobolResult:
                              "ST_conf": self.ST_conf[r]}, index=list(self.names))
 
 
+def objective_rows(obs_labels, objectives):
+    """Rows of ``simplyp_sobol_outputs_device`` for the statistics ``objectives`` (names of ``OBJECTIVES``) of the
+    observed series ``obs_labels`` [(sc_id, variable)]: (rows [R][2] int32 = (series, ``packing.STAT_NAMES`` slot, or
+    -1 for lp), labels [(sc_id, variable, statistic)], ``(None, None, "lp")`` for lp, last)."""
+    rows, labels = [], []
+    for v, (sc, var) in enumerate(obs_labels):
+        for o in objectives:
+            if o != "lp":
+                rows.append((v, pk.STAT_NAMES.index(o)))
+                labels.append((sc, var, o))
+    if "lp" in objectives:
+        rows.append((0, -1))
+        labels.append((None, None, "lp"))
+    return np.asarray(rows, dtype=np.int32).reshape(-1, 2), labels
+
+
 def _check_request(n_base, skip, objectives, series, obs_dict, n_boot, conf_level):
     n_base, skip = int(n_base), int(skip)
     if n_base < 2 or n_base & (n_base - 1):
@@ -117,16 +133,7 @@ def sobol_indices(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, ranges,
     else:
         obs, obs_desc, obs_labels = pk.obs_arrays(obs_dict, topo, met_df.index, variables)
         V = obs.shape[0]
-        rows, labels = [], []
-        for v, (sc, var) in enumerate(obs_labels):
-            for o in objectives:
-                if o != "lp":
-                    rows.append((v, pk.STAT_NAMES.index(o)))
-                    labels.append((sc, var, o))
-        if "lp" in objectives:
-            rows.append((0, -1))
-            labels.append((None, None, "lp"))
-        rows = np.asarray(rows, dtype=np.int32).reshape(-1, 2)
+        rows, labels = objective_rows(obs_labels, objectives)
     R = len(labels)
     p_LU, p_SC = p_LU.copy(deep=True), p_SC.copy(deep=True)
     pk.validate_land_use(p_SC, p["SC_list"])
