@@ -386,6 +386,35 @@ int simplyp_nanquantile_device(const double* x, int64_t n_rows, int64_t n_cols, 
                                double* quantiles, double* mean, int64_t* count, void* workspace,
                                int64_t workspace_bytes, void* stream);
 
+/* ---- period aggregates ---------------------------------------------------------------------------------------------
+ * Period means, loads and flow-weighted mean concentrations of an ensemble, per reach and into the receiving water
+ * body (simplyp_periods.cuh).  For a chunk of M members (dims: M, S, D, Msc = 1 or M) of a full-output run,
+ * out[M][S][D][25], member_params[M][NP_MEMBER], sc_params[Msc][S][NP_SC] and diag[M][S][NDIAG] on the device, writes
+ * values[n_series * n_periods][n_members_total] (row v * n_periods + p) at columns member_offset .. member_offset +
+ * M - 1.
+ * HOST arrays, passed to the kernel by value:
+ *   series_desc[n_series][3] = (target, kind, statistic): target a run-order reach 0..S-1 or SIMPLYP_PERIOD_WATERBODY
+ *     (the reaches waterbody_reaches[n_waterbody_reaches], run order, summed as simplyp_sum_to_waterbody_device sums
+ *     them), kind SIMPLYP_V_*, statistic
+ *       SIMPLYP_PERIOD_MEAN  mean over the period's days of the daily value (a reach: the value the fit statistics see;
+ *                            the water body: its Q_cumecs or concentration column),
+ *       SIMPLYP_PERIOD_LOAD  sum of the daily flux in kg (Q: volume in m3 = sum of Q_cumecs * 86400),
+ *       SIMPLYP_PERIOD_FWMC  sum of the flux / sum of Q_cumecs * 1000/86400 in mg/l (not for Q);
+ *   period_bounds[n_periods][2] = first and last day (inclusive) of each period, 0 <= first <= last < D.
+ * Every sum runs over the days in ascending order, one rounding per addition, so a value depends on neither the
+ * chunking nor the launch.  A member with a non-zero SIMPLYP_DG_STATUS word at any reach gives NaN in every row.
+ * Only enqueues work on `stream`, so it can be captured into a graph. */
+#define SIMPLYP_PERIOD_MAX_SERIES 64
+#define SIMPLYP_PERIOD_MAX_PERIODS 2048
+#define SIMPLYP_PERIOD_MAX_REACHES 256
+#define SIMPLYP_PERIOD_WATERBODY (-1)
+enum { SIMPLYP_PERIOD_MEAN = 0, SIMPLYP_PERIOD_LOAD = 1, SIMPLYP_PERIOD_FWMC = 2 };
+int simplyp_period_aggregates_device(const SimplypDims* dims, const double* out, const double* member_params,
+                                     const double* sc_params, const int64_t* diag, const int32_t* series_desc,
+                                     int32_t n_series, const int32_t* period_bounds, int32_t n_periods,
+                                     const int32_t* waterbody_reaches, int32_t n_waterbody_reaches, double* values,
+                                     int64_t n_members_total, int64_t member_offset, void* stream);
+
 /* ---- Sobol' sensitivity indices over a Saltelli design ------------------------------------------------------------
  * SALib's sobol.sample / sobol.analyze on the device.  K free parameters (the sampler's targets and boxes,
  * SimplypMcmcParam), N = n_base samples, P = K + 2 design members a sample (2K + 2 with second order).

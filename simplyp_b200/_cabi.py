@@ -28,7 +28,7 @@ EXPORTS = [
     "simplyp_mcmc_init_device", "simplyp_predictive_draws_device", "simplyp_nanquantile_workspace_bytes",
     "simplyp_nanquantile_device", "simplyp_sobol_design_device", "simplyp_sobol_outputs_device",
     "simplyp_sobol_workspace_bytes", "simplyp_sobol_indices_device", "simplyp_de_trial_device",
-    "simplyp_de_select_device", "simplyp_de_init_device",
+    "simplyp_de_select_device", "simplyp_de_init_device", "simplyp_period_aggregates_device",
 ]
 MAX_RANKS = 8
 
@@ -54,6 +54,9 @@ class SimplypPeerGather(C.Structure):
 
 MCMC_MAX_FREE = 64
 NQ_MAX = 16
+PERIOD_MAX_SERIES, PERIOD_MAX_PERIODS, PERIOD_MAX_REACHES = 64, 2048, 256
+PERIOD_WATERBODY = -1
+PERIOD_STATS = {"mean": 0, "load": 1, "fwmc": 2}
 MCMC_MEMBER, MCMC_SC_ALL, MCMC_SC_AT = 0, 1, 2
 DE_STRATEGIES = {"best1bin": 0, "rand1bin": 1}
 
@@ -167,6 +170,9 @@ def load():
     lib.simplyp_predictive_draws_device.argtypes = [C.POINTER(SimplypDims), vp, vp, vp, vp, vp, C.c_int32, vp,
                                                     C.c_int64, C.c_int64, C.c_int32, C.c_uint64, vp]
     lib.simplyp_predictive_draws_device.restype = C.c_int
+    lib.simplyp_period_aggregates_device.argtypes = [C.POINTER(SimplypDims), vp, vp, vp, vp, ip, C.c_int32, ip,
+                                                     C.c_int32, ip, C.c_int32, vp, C.c_int64, C.c_int64, vp]
+    lib.simplyp_period_aggregates_device.restype = C.c_int
     lib.simplyp_nanquantile_workspace_bytes.argtypes = [C.c_int64, C.c_int64]
     lib.simplyp_nanquantile_workspace_bytes.restype = C.c_int64
     lib.simplyp_nanquantile_device.argtypes = [vp, C.c_int64, C.c_int64, dp, C.c_int32, vp, vp, vp, vp, C.c_int64, vp]
@@ -435,6 +441,22 @@ def predictive_draws_device(dims, out_ptr, member_ptr, sc_ptr, diag_ptr, series_
     _check(lib.simplyp_predictive_draws_device(C.byref(dims), out_ptr, member_ptr, sc_ptr, diag_ptr, series_desc_ptr,
                                                int(n_series), draws_ptr, int(n_members_total), int(member_offset),
                                                1 if obs_error else 0, int(seed) & 0xFFFFFFFFFFFFFFFF, stream_ptr))
+
+
+def period_aggregates_device(dims, out_ptr, member_ptr, sc_ptr, diag_ptr, series_desc, period_bounds, wb_reaches,
+                             values_ptr, n_members_total, member_offset, stream_ptr):
+    """Period aggregates of one full-output chunk into its columns of values [V P][M_total]; ``series_desc`` [V][3],
+    ``period_bounds`` [P][2] and ``wb_reaches`` [n] are host int32 arrays, passed to the kernel by value.
+    Asynchronous on ``stream_ptr``."""
+    lib = require_device()
+    desc = np.ascontiguousarray(series_desc, dtype=np.int32).reshape(-1, 3)
+    bounds = np.ascontiguousarray(period_bounds, dtype=np.int32).reshape(-1, 2)
+    wb = np.ascontiguousarray(wb_reaches, dtype=np.int32).reshape(-1)
+    ip = C.POINTER(C.c_int32)
+    _check(lib.simplyp_period_aggregates_device(C.byref(dims), out_ptr, member_ptr, sc_ptr, diag_ptr,
+                                                desc.ctypes.data_as(ip), desc.shape[0], bounds.ctypes.data_as(ip),
+                                                bounds.shape[0], wb.ctypes.data_as(ip) if wb.size else None, wb.size,
+                                                values_ptr, int(n_members_total), int(member_offset), stream_ptr))
 
 
 def nanquantile_workspace_bytes(n_rows, n_cols):

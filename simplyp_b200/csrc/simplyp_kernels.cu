@@ -17,6 +17,8 @@
 //                                   arithmetic in simplyp_mcmc.cuh) over the fused log-likelihood
 //   predictive_draws_kernel         posterior predictive draws of the simulated series (simplyp_bands.cuh)
 //   nanquantile_kernel, nq_prepare_kernel, nq_hist_kernel, nq_pick_kernel  np.nanquantile of the rows of a matrix
+//   period_aggregate_kernel         period means, loads and flow-weighted concentrations of an ensemble
+//                                   (simplyp_periods.cuh)
 //   de_trial_kernel, de_select_kernel, de_init_kernel, de_reduce_kernel  differential evolution (simplyp_de.cuh)
 //
 // There is deliberately no host implementation of the integration in this library.
@@ -36,6 +38,7 @@
 #include "simplyp_plan.cuh"
 #include "simplyp_mcmc.cuh"
 #include "simplyp_bands.cuh"
+#include "simplyp_periods.cuh"
 #include "simplyp_sobol.cuh"
 #include "simplyp_de.cuh"
 
@@ -902,8 +905,9 @@ __global__ void spearman_long_kernel(const double* sim_obs, const double* obs_ra
 // ------------------------------------------------------------------------------------------ waterbody sums
 // sum_to_waterbody (model.py:851-900) on the raw output: for every (member, day) the reaches flagged
 // In_final_flux? == 1 are summed — Q_cumecs (= Qr*A_catch*1000/86400, :784), Msus/TDP/PP daily fluxes — and the
-// concentrations (:889-892) and derived species (derived_P_species, :831-847) follow.  One thread per (member, day);
-// consecutive threads take consecutive days, so the strided row reads of a warp fall in neighbouring rows.
+// concentrations (:889-892) and derived species (derived_P_species, :831-847) follow (simplyp_periods.cuh).  One
+// thread per (member, day); consecutive threads take consecutive days, so the strided row reads of a warp fall in
+// neighbouring rows.
 // wb[m][d][SIMPLYP_NWB] = Q_cumecs, Msus_kg/day, TDP_kg/day, PP_kg/day, SS_mgl, TDP_mgl, PP_mgl, TP_mgl,
 //                          TP_kg/day, SRP_mgl, SRP_kg/day
 __global__ void waterbody_kernel(const double* out, const double* sc_params, const double* member_params,
@@ -915,21 +919,11 @@ __global__ void waterbody_kernel(const double* out, const double* sc_params, con
   double q = 0.0, ms = 0.0, td = 0.0, pp = 0.0;
   for (int k = 0; k < n_reaches; ++k) {
     const int s = reaches[k];
-    const double* row = out + (((size_t)m * S + s) * D + d) * SIMPLYP_NOUT;
-    q += row[SIMPLYP_O_QR] * scp[(size_t)s * SIMPLYP_NP_SC + SIMPLYP_SC_A_CATCH] * 1000.0 / 86400.0;
-    ms += row[SIMPLYP_O_MSUS_FLUX];
-    td += row[SIMPLYP_O_TDP_FLUX];
-    pp += row[SIMPLYP_O_PP_FLUX];
+    wb_add_reach<WbPlain>(out + (((size_t)m * S + s) * D + d) * SIMPLYP_NOUT, scp + (size_t)s * SIMPLYP_NP_SC, q, ms,
+                          td, pp);
   }
   const double f_TDP = member_params[(size_t)m * SIMPLYP_NP_MEMBER + SIMPLYP_P_F_TDP];
-  const double c = 1000.0 / 86400.0;
-  double* w = wb + (size_t)idx * SIMPLYP_NWB;
-  const double ss_mgl = (ms / q) * c, tdp_mgl = (td / q) * c, pp_mgl = (pp / q) * c;
-  w[0] = q; w[1] = ms; w[2] = td; w[3] = pp; w[4] = ss_mgl; w[5] = tdp_mgl; w[6] = pp_mgl;
-  w[7] = tdp_mgl + pp_mgl;        // TP_mgl   (:842)
-  w[8] = td + pp;                 // TP_kg/day (:843)
-  w[9] = tdp_mgl * f_TDP;         // SRP_mgl  (:844)
-  w[10] = td * f_TDP;             // SRP_kg/day (:845)
+  wb_columns<WbPlain>(q, ms, td, pp, f_TDP, wb + (size_t)idx * SIMPLYP_NWB);
 }
 
 // ------------------------------------------------------------------------------------------ Thornthwaite PET
@@ -1649,6 +1643,65 @@ __global__ void __launch_bounds__(256) predictive_draws_kernel(const double* out
     const int dd = d0 + j;
     if (m < Mc && dd < D) draws[((size_t)v * D + dd) * M_total + member_offset + m] = tile[tx][j];
   }
+}
+
+// ------------------------------------------------------------------------------------------ period aggregates
+// values[v * n_periods + p][member_offset + m] = the aggregate of series v over period p (simplyp_periods.cuh) for the
+// members m of a full-output chunk of Mc members.  One block per (32 members, period, series), 32 x 8 threads: the out
+// rows are read with the lane over days (consecutive rows of one member) into a tile of 32 days x 32 members in shared
+// memory; lane tx of the first warp then adds its member's days in ascending order, carrying its sums from tile to
+// tile, and stores the result with the lane over members.  The series, the period bounds and the water-body reaches
+// travel by value in the launch (a captured launch replays them).  A member with a non-zero status word at any reach
+// gives NaN.
+struct PeriodArgs {
+  int n_series, n_periods, n_wb;
+  int series[SIMPLYP_PERIOD_MAX_SERIES][3];     // (target, kind, statistic)
+  int bounds[SIMPLYP_PERIOD_MAX_PERIODS][2];    // first and last day, inclusive
+  int wb[SIMPLYP_PERIOD_MAX_REACHES];           // run-order reaches of the water body
+};
+constexpr int PERIOD_TILE = 32;
+__global__ void __launch_bounds__(256) period_aggregate_kernel(const double* out, const double* member_params,
+                                                               const double* sc_params, const int64_t* diag,
+                                                               const __grid_constant__ PeriodArgs pa, int Mc, int S,
+                                                               int D, int Msc, long long M_total,
+                                                               long long member_offset, double* values) {
+  __shared__ double tile_x[PERIOD_TILE][PERIOD_TILE + 1], tile_q[PERIOD_TILE][PERIOD_TILE + 1];
+  __shared__ int skip[PERIOD_TILE];
+  const int v = blockIdx.z, p = blockIdx.y, m0 = blockIdx.x * PERIOD_TILE;
+  const int tx = threadIdx.x, ty = threadIdx.y;
+  const int target = pa.series[v][0], kind = pa.series[v][1], stat = pa.series[v][2];
+  const int first = pa.bounds[p][0], last = pa.bounds[p][1];
+  if (ty == 0) {
+    int f = m0 + tx >= Mc;
+    if (!f)
+      for (int r = 0; r < S; ++r) f |= diag[((size_t)(m0 + tx) * S + r) * SIMPLYP_NDIAG + SIMPLYP_DG_STATUS] != 0;
+    skip[tx] = f;
+  }
+  __syncthreads();
+  double sx = 0.0, sq = 0.0;
+  for (int d0 = first; d0 <= last; d0 += PERIOD_TILE) {
+    const int d = d0 + tx;
+    if (d <= last)
+      for (int j = ty; j < PERIOD_TILE; j += blockDim.y) {
+        const int m = m0 + j;
+        if (skip[j]) continue;
+        period_day(out + (size_t)m * S * D * SIMPLYP_NOUT, sc_params + (size_t)(Msc > 1 ? m : 0) * S * SIMPLYP_NP_SC,
+                   member_params[(size_t)m * SIMPLYP_NP_MEMBER + SIMPLYP_P_F_TDP], D, d, target, kind, stat, pa.wb,
+                   pa.n_wb, &tile_x[j][tx], &tile_q[j][tx]);
+      }
+    __syncthreads();
+    if (ty == 0) {
+      const int n = min(PERIOD_TILE, last - d0 + 1);
+      for (int k = 0; k < n; ++k) {
+        sx = mc_add(sx, tile_x[tx][k]);
+        sq = mc_add(sq, tile_q[tx][k]);
+      }
+    }
+    __syncthreads();
+  }
+  if (ty == 0 && m0 + tx < Mc)
+    values[((size_t)v * pa.n_periods + p) * M_total + member_offset + m0 + tx] =
+        skip[tx] ? NAN : period_result(stat, sx, sq, last - first + 1);
 }
 
 // np.nanquantile(x, q, axis=-1) of every row of x[R][N], with the mean and the count of the non-NaN entries.  The
@@ -2761,6 +2814,62 @@ int simplyp_predictive_draws_device(const SimplypDims* dims, const double* out, 
   predictive_draws_kernel<<<grid, dim3(DRAW_TILE, 8), 0, static_cast<cudaStream_t>(stream)>>>(
       out, member_params, sc_params, diag, series_desc, M, S, D, Msc, n_members_total, member_offset, obs_error, seed,
       draws);
+  g_launches.fetch_add(1);
+  SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
+int simplyp_period_aggregates_device(const SimplypDims* dims, const double* out, const double* member_params,
+                                     const double* sc_params, const int64_t* diag, const int32_t* series_desc,
+                                     int32_t n_series, const int32_t* period_bounds, int32_t n_periods,
+                                     const int32_t* waterbody_reaches, int32_t n_waterbody_reaches, double* values,
+                                     int64_t n_members_total, int64_t member_offset, void* stream) {
+  if (!dims || !out || !member_params || !sc_params || !diag || !series_desc || !period_bounds || !values ||
+      (n_waterbody_reaches > 0 && !waterbody_reaches))
+    return fail(SIMPLYP_EINVAL, "period aggregates: null argument%s");
+  const int M = dims->n_members, S = dims->n_sc, D = dims->n_days, Msc = dims->n_sc_param_sets;
+  if (M < 1 || S < 1 || D < 1 || (Msc != 1 && Msc != M) || n_series < 1 || n_series > SIMPLYP_PERIOD_MAX_SERIES ||
+      n_periods < 1 || n_periods > SIMPLYP_PERIOD_MAX_PERIODS || n_waterbody_reaches < 0 ||
+      n_waterbody_reaches > SIMPLYP_PERIOD_MAX_REACHES)
+    return fail(SIMPLYP_EINVAL, "period aggregates: bad dims (M, S, D >= 1, Msc = 1 or M, "
+                                "1..SIMPLYP_PERIOD_MAX_SERIES series, 1..SIMPLYP_PERIOD_MAX_PERIODS periods, "
+                                "0..SIMPLYP_PERIOD_MAX_REACHES reaches)%s");
+  if (member_offset < 0 || n_members_total > INT32_MAX || member_offset + M > n_members_total)
+    return fail(SIMPLYP_EINVAL, "period aggregates: members outside 0..n_members_total - 1 (at most 2^31 - 1)%s");
+  PeriodArgs pa;
+  pa.n_series = n_series;
+  pa.n_periods = n_periods;
+  pa.n_wb = n_waterbody_reaches;
+  for (int k = 0; k < n_waterbody_reaches; ++k) {
+    pa.wb[k] = waterbody_reaches[k];
+    if (pa.wb[k] < 0 || pa.wb[k] >= S)
+      return fail(SIMPLYP_EINVAL, "period aggregates: water-body reach outside 0..S-1%s");
+  }
+  for (int v = 0; v < n_series; ++v) {
+    const int target = series_desc[3 * v], kind = series_desc[3 * v + 1], stat = series_desc[3 * v + 2];
+    if (target != SIMPLYP_PERIOD_WATERBODY && (target < 0 || target >= S))
+      return fail(SIMPLYP_EINVAL, "period aggregates: reach outside 0..S-1%s");
+    if (target == SIMPLYP_PERIOD_WATERBODY && n_waterbody_reaches == 0)
+      return fail(SIMPLYP_EINVAL, "period aggregates: a water-body series without water-body reaches%s");
+    if (kind < SIMPLYP_V_Q || kind > SIMPLYP_V_SRP)
+      return fail(SIMPLYP_EINVAL, "period aggregates: bad variable kind%s");
+    if (stat < SIMPLYP_PERIOD_MEAN || stat > SIMPLYP_PERIOD_FWMC ||
+        (stat == SIMPLYP_PERIOD_FWMC && kind == SIMPLYP_V_Q))
+      return fail(SIMPLYP_EINVAL, "period aggregates: bad statistic (fwmc of Q is undefined)%s");
+    pa.series[v][0] = target;
+    pa.series[v][1] = kind;
+    pa.series[v][2] = stat;
+  }
+  for (int p = 0; p < n_periods; ++p) {
+    pa.bounds[p][0] = period_bounds[2 * p];
+    pa.bounds[p][1] = period_bounds[2 * p + 1];
+    if (pa.bounds[p][0] < 0 || pa.bounds[p][0] > pa.bounds[p][1] || pa.bounds[p][1] >= D)
+      return fail(SIMPLYP_EINVAL, "period aggregates: period outside the record or reversed%s");
+  }
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  const dim3 grid((unsigned)((M + PERIOD_TILE - 1) / PERIOD_TILE), (unsigned)n_periods, (unsigned)n_series);
+  period_aggregate_kernel<<<grid, dim3(PERIOD_TILE, 8), 0, static_cast<cudaStream_t>(stream)>>>(
+      out, member_params, sc_params, diag, pa, M, S, D, Msc, n_members_total, member_offset, values);
   g_launches.fetch_add(1);
   SP_CUDA(cudaGetLastError());
   return SIMPLYP_OK;

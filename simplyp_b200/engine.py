@@ -170,6 +170,26 @@ class Engine:
                                           draws.data_ptr(), draws.shape[2], member_offset, obs_error, seed, stream)
         return draws
 
+    def period_aggregates(self, out, member_params, sc_params, diag, series_desc, period_bounds, wb_reaches, values,
+                          member_offset=0):
+        """Period means, loads and flow-weighted concentrations of a full-output chunk (``out`` [Mc][S][D][25],
+        ``diag`` [Mc][S][4] from :meth:`run`) written into columns ``member_offset .. member_offset + Mc`` of
+        ``values`` [V P][M_total], row v P + p (``simplyp_period_aggregates_device``).  ``series_desc`` [V][3] =
+        (run-order reach or ``_cabi.PERIOD_WATERBODY``, ``packing.VAR_KINDS`` index, ``_cabi.PERIOD_STATS`` code),
+        ``period_bounds`` [P][2] (first and last day) and ``wb_reaches`` (run-order reaches of the water body) are
+        host arrays.  Returns ``values``; asynchronous."""
+        torch = _torch()
+        Mc, S, D = out.shape[0], out.shape[1], out.shape[2]
+        if sc_params.dim() == 2:
+            sc_params = sc_params.unsqueeze(0)
+        dims = _cabi.make_dims(Mc, S, D, sc_params.shape[0], 0, 0)
+        with torch.cuda.device(self.device):
+            stream = torch.cuda.current_stream().cuda_stream
+            _cabi.period_aggregates_device(dims, out.data_ptr(), member_params.data_ptr(), sc_params.data_ptr(),
+                                           diag.data_ptr(), series_desc, period_bounds, wb_reaches, values.data_ptr(),
+                                           values.shape[1], member_offset, stream)
+        return values
+
     def nanquantile(self, x, q, quantiles=None, mean=None, count=None):
         """``np.nanquantile(x, q, axis=-1)`` of a [R][N] fp64 matrix, bitwise, with the mean and the count of the
         non-NaN entries of every row (``simplyp_nanquantile_device``).  Returns (quantiles [n_q][R], mean [R],

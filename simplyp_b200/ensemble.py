@@ -511,6 +511,39 @@ def _band_series(series, topo):
     return np.asarray(desc, dtype=np.int32).reshape(-1, 2), [(int(s), v) for s, v in series]
 
 
+def _integrate_in_chunks(eng, met_df, topo, opt, member, sc, members_per_chunk, snow_on_device, consume):
+    """Integrate the members of ``member`` / ``sc`` (``pack_members``) in full-output chunks of ``members_per_chunk``
+    (default: about 1 GiB of output a chunk) into one reused device buffer, and after each chunk enqueue
+    ``consume(out [n][S][D][25], member rows [n], sc rows [1 or n], diag rows [n], first member)``, which reads the
+    chunk's output in place before the next chunk overwrites it.  Returns the per-member diagnostics [M][S][4] on the
+    device; asynchronous."""
+    import torch
+
+    M, S, D = member.shape[0], topo.n_sc, len(met_df)
+    row_bytes = S * D * pk.NOUT * 8
+    if members_per_chunk is None:
+        members_per_chunk = max(1, (1 << 30) // max(row_bytes, 1))
+    chunk = int(max(1, min(int(members_per_chunk), M)))
+    dev = eng.device
+    d_forc = eng.to_device(pk.forcing_matrix(met_df, raw_snow=bool(snow_on_device)))
+    d_mem, d_sc = eng.to_device(member), eng.to_device(sc)
+    out = torch.empty((chunk, S, D, pk.NOUT), dtype=torch.float64, device=dev)
+    diag = torch.zeros((M, S, pk.NDIAG), dtype=torch.int64, device=dev)
+    with torch.cuda.device(dev):
+        for m0 in range(0, M, chunk):
+            n = min(chunk, M - m0)
+            scp = d_sc if d_sc.shape[0] == 1 else d_sc[m0:m0 + n]
+            eng.run(d_forc, d_mem[m0:m0 + n], scp, topo.parent_offsets, topo.parent_ids, opt, out=out[:n],
+                    diag=diag[m0:m0 + n])
+            consume(out[:n], d_mem[m0:m0 + n], scp, diag[m0:m0 + n], m0)
+    return diag
+
+
+def _n_failed(diag):
+    """Members whose integration raised a status bit at any reach (diag after a synchronise)."""
+    return int(np.any(diag.cpu().numpy()[:, :, 3] != 0, axis=1).sum())
+
+
 def predictive_bands(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, samples, series,
                      quantiles=(0.025, 0.25, 0.5, 0.75, 0.975), obs_error=False, seed=DEFAULT_BAND_SEED,
                      members_per_chunk=None, step_len=1.0, rtol=None, atol=None, snow_on_device=False, engine=None):
@@ -544,33 +577,258 @@ def predictive_bands(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, samp
     opt = make_options(p_SU, p, dynamic_options, topo, step_len, rtol, atol)
     opt.snow_on_device = 1 if snow_on_device else 0
     member, sc = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, topo.sc_ids), samples)
-    M, S, D, V = member.shape[0], topo.n_sc, len(met_df), desc.shape[0]
+    M, D, V = member.shape[0], len(met_df), desc.shape[0]
     eng = engine or Engine()
     draw_bytes = 8 * V * D * M
     if draw_bytes > eng.free_bytes() // 2:
         raise ValueError("the draws need %.1f GB, more than half of the free device memory: thin the samples "
                          "(e.g. flat_samples(burn, thin=n))" % (draw_bytes / 1e9))
-    row_bytes = S * D * pk.NOUT * 8
-    if members_per_chunk is None:
-        members_per_chunk = max(1, (1 << 30) // max(row_bytes, 1))
-    chunk = int(max(1, min(int(members_per_chunk), M)))
     dev = eng.device
-    d_forc = eng.to_device(pk.forcing_matrix(met_df, raw_snow=bool(snow_on_device)))
-    d_mem, d_sc, d_desc = eng.to_device(member), eng.to_device(sc), eng.to_device(desc)
+    d_desc = eng.to_device(desc)
     draws = torch.empty((V, D, M), dtype=torch.float64, device=dev)
-    out = torch.empty((chunk, S, D, pk.NOUT), dtype=torch.float64, device=dev)
-    diag = torch.zeros((M, S, pk.NDIAG), dtype=torch.int64, device=dev)
+
+    def draw(out, d_mem, scp, diag, m0):
+        eng.predictive_draws(out, d_mem, scp, diag, d_desc, draws, m0, obs_error, seed)
+    diag = _integrate_in_chunks(eng, met_df, topo, opt, member, sc, members_per_chunk, snow_on_device, draw)
     with torch.cuda.device(dev):
-        for m0 in range(0, M, chunk):
-            n = min(chunk, M - m0)
-            scp = d_sc if d_sc.shape[0] == 1 else d_sc[m0:m0 + n]
-            eng.run(d_forc, d_mem[m0:m0 + n], scp, topo.parent_offsets, topo.parent_ids, opt, out=out[:n],
-                    diag=diag[m0:m0 + n])
-            eng.predictive_draws(out[:n], d_mem[m0:m0 + n], scp, diag[m0:m0 + n], d_desc, draws, m0, obs_error, seed)
-        del out
         quant, mean, count = eng.nanquantile(draws.view(V * D, M), q)
     torch.cuda.synchronize(dev)
-    n_failed = int(np.any(diag.cpu().numpy()[:, :, 3] != 0, axis=1).sum())
+    n_failed = _n_failed(diag)
     return PredictiveBands(q=q, quantiles=quant.cpu().numpy().reshape(len(q), V, D),
                            mean=mean.cpu().numpy().reshape(V, D), count=count.cpu().numpy().reshape(V, D),
                            n_failed=n_failed, labels=labels, dates=met_df.index)
+
+
+# --------------------------------------------------------------------------- period loads and concentrations
+PERIOD_STATISTICS = ("mean", "load", "fwmc")
+
+
+def period_bounds(dates, periods):
+    """``periods`` as (bounds [P][2] int32 = first and last day index of each period, inclusive, labels [P] str).
+
+    ``"year"``: calendar years (labels ``"2004"``), ``"month"``: calendar months (``"2004-01"``), ``"all"``: the whole
+    record, or a list of ``(start, end)`` dates, inclusive (labels ``"start/end"``), which may overlap.  A partial
+    first or last year or month is kept."""
+    import pandas as pd
+
+    idx = pd.DatetimeIndex(dates)
+    D = len(idx)
+    if D == 0:
+        raise ValueError("an empty record has no periods")
+    if isinstance(periods, str):
+        if periods == "all":
+            keys = np.zeros(D, dtype=np.int64)
+            names = ["%s/%s" % (idx[0].date(), idx[-1].date())]
+        elif periods == "year":
+            keys = idx.year.to_numpy()
+            names = None
+        elif periods == "month":
+            keys = idx.year.to_numpy() * 12 + (idx.month.to_numpy() - 1)
+            names = None
+        else:
+            raise ValueError("unknown periods %r: 'year', 'month', 'all' or a list of (start, end) dates" % periods)
+        change = np.flatnonzero(np.diff(keys)) + 1
+        first = np.concatenate([[0], change])
+        last = np.concatenate([change - 1, [D - 1]])
+        if names is None:
+            names = [str(idx[i].year) if periods == "year" else "%04d-%02d" % (idx[i].year, idx[i].month)
+                     for i in first]
+        return np.stack([first, last], axis=1).astype(np.int32), names
+    ranges = list(periods)
+    if not ranges:
+        raise ValueError("no periods: give 'year', 'month', 'all' or a list of (start, end) dates")
+    bounds, names = [], []
+    for rng in ranges:
+        try:
+            start, end = (pd.Timestamp(t) for t in rng)
+        except (TypeError, ValueError):
+            raise ValueError("a period is a (start, end) pair of dates, got %r" % (rng,))
+        if start > end:
+            raise ValueError("period %s/%s is reversed" % (start.date(), end.date()))
+        if start < idx[0] or end > idx[-1]:
+            raise ValueError("period %s/%s is not inside the record %s/%s"
+                             % (start.date(), end.date(), idx[0].date(), idx[-1].date()))
+        lo, hi = int(idx.searchsorted(start, "left")), int(idx.searchsorted(end, "right")) - 1
+        if hi < lo:
+            raise ValueError("period %s/%s holds no day of the record" % (start.date(), end.date()))
+        bounds.append((lo, hi))
+        names.append("%s/%s" % (start.date(), end.date()))
+    return np.asarray(bounds, dtype=np.int32).reshape(-1, 2), names
+
+
+def _period_series(series, topo, p_struc):
+    """(desc [V][3] int32 for ``simplyp_period_aggregates_device``, labels [(target, variable, statistic)],
+    run-order water-body reaches)."""
+    from . import _cabi
+
+    series = list(series)
+    if not series:
+        raise ValueError("no series: give a list of (target, variable, statistic)")
+    pos = {s: i for i, s in enumerate(topo.sc_ids)}
+    desc, labels, wb = [], [], None
+    for item in series:
+        try:
+            target, var, stat = item
+        except (TypeError, ValueError):
+            raise ValueError("a series is (target, variable, statistic), got %r" % (item,))
+        if var not in pk.VAR_INDEX:
+            raise ValueError("unknown variable %r: one of %s" % (var, pk.VAR_KINDS))
+        if stat not in PERIOD_STATISTICS:
+            raise ValueError("unknown statistic %r: one of %s" % (stat, list(PERIOD_STATISTICS)))
+        if stat == "fwmc" and var == "Q":
+            raise ValueError("the flow-weighted mean concentration of Q is undefined")
+        if isinstance(target, str) and target == "waterbody":
+            if wb is None:
+                flag = p_struc["In_final_flux?"]
+                wb = [pos[int(r)] for r in flag[flag == 1].index.values if int(r) in pos]
+                if not wb:
+                    raise ValueError("'waterbody' needs at least one reach flagged In_final_flux? == 1")
+            code, label = _cabi.PERIOD_WATERBODY, "waterbody"
+        else:
+            try:
+                key = int(target)
+            except (TypeError, ValueError):
+                key = None
+            if key not in pos:
+                raise ValueError("reach %r is not in SC_list" % (target,))
+            code, label = pos[key], key
+        desc.append((code, pk.VAR_INDEX[var], _cabi.PERIOD_STATS[stat]))
+        labels.append((label, var, stat))
+    if len(desc) > _cabi.PERIOD_MAX_SERIES:
+        raise ValueError("at most %d series, got %d" % (_cabi.PERIOD_MAX_SERIES, len(desc)))
+    if wb is not None and len(wb) > _cabi.PERIOD_MAX_REACHES:
+        raise ValueError("at most %d reaches in the water body" % _cabi.PERIOD_MAX_REACHES)
+    return np.asarray(desc, dtype=np.int32).reshape(-1, 3), labels, np.asarray(wb or [], dtype=np.int32)
+
+
+@dataclass
+class PeriodStatistics:
+    """What :func:`period_statistics` returns.  Row r = v * n_periods + p is series v (``series[v]``, a
+    (target, variable, statistic)) over period p (``periods[p]``).  ``values`` [R][M] holds every member's aggregate
+    (NaN for the ``n_failed`` members whose integration raised a status bit), ``quantiles`` [n_q][R] is
+    ``np.nanquantile(values, q, axis=-1)``, ``mean`` [R] and ``count`` [R] are the mean and the number of the non-NaN
+    entries of a row.  ``bounds`` [P][2] are the first and last day index of each period, ``n_days`` [P] its days."""
+    q: np.ndarray
+    quantiles: np.ndarray
+    values: np.ndarray
+    mean: np.ndarray
+    count: np.ndarray
+    n_failed: int
+    series: list
+    periods: list
+    bounds: np.ndarray
+    n_days: np.ndarray
+    dates: object
+
+    @property
+    def labels(self):
+        """Row labels: (target, variable, statistic, period), series-major."""
+        return [s + (p,) for s in self.series for p in self.periods]
+
+    def row(self, row_or_label):
+        """The row index of an int or of a label (target, variable, statistic, period); the period may be given as
+        its label or, for a year, as the int year."""
+        if isinstance(row_or_label, (int, np.integer)):
+            r = int(row_or_label)
+            if not 0 <= r < self.values.shape[0]:
+                raise ValueError("row %d outside 0..%d" % (r, self.values.shape[0] - 1))
+            return r
+        lab = tuple(row_or_label)
+        if len(lab) != 4:
+            raise ValueError("a row label is (target, variable, statistic, period), got %r" % (row_or_label,))
+        key = (lab[0], lab[1], lab[2], str(lab[3]))
+        for r, l in enumerate(self.labels):
+            if l == key:
+                return r
+        raise ValueError("no row %r" % (row_or_label,))
+
+    def exceedance(self, row_or_label, threshold):
+        """Fraction of the finite entries of a row of ``values`` greater than ``threshold`` (NaN if none)."""
+        v = self.values[self.row(row_or_label)]
+        v = v[np.isfinite(v)]
+        return float(np.count_nonzero(v > threshold)) / v.size if v.size else float("nan")
+
+    def table(self):
+        """A DataFrame with one row per (target, variable, statistic, period): the period's first and last date and
+        number of days, the quantiles (columns ``q<value>``), the mean and the count."""
+        import pandas as pd
+
+        P = len(self.periods)
+        rows = []
+        for r, (target, var, stat, period) in enumerate(self.labels):
+            p = r % P
+            row = {"target": target, "variable": var, "statistic": stat, "period": period,
+                   "start": self.dates[self.bounds[p, 0]], "end": self.dates[self.bounds[p, 1]],
+                   "n_days": int(self.n_days[p])}
+            for k, qv in enumerate(self.q):
+                row["q%g" % qv] = self.quantiles[k, r]
+            row["mean"] = self.mean[r]
+            row["count"] = int(self.count[r])
+            rows.append(row)
+        return pd.DataFrame(rows)
+
+
+def period_statistics(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, samples, series, periods="year",
+                      quantiles=(0.025, 0.5, 0.975), members_per_chunk=None, step_len=1.0, rtol=None, atol=None,
+                      snow_on_device=False, engine=None):
+    """Period loads, flow-weighted mean concentrations and means over the members of ``samples`` (e.g.
+    ``McmcResult.flat_samples``), with their quantiles: what a catchment delivers per year, month or any set of date
+    ranges, per reach and into the receiving water body, with its uncertainty.
+
+    ``series`` [(target, variable, statistic)]: target a reach id of ``SC_list`` or ``"waterbody"`` (the reaches flagged
+    ``In_final_flux? == 1``, summed as ``sum_to_waterbody`` sums them), variable in ``packing.VAR_KINDS``, statistic
+      ``"mean"``  mean over the period's days of the daily value (Q_cumecs, or a concentration in mg/l); for a reach the
+                  value the fit statistics and ``predictive_bands`` see;
+      ``"load"``  sum of the daily flux in kg (for Q the volume in m3, the sum of Q_cumecs * 86400);
+      ``"fwmc"``  flow-weighted mean concentration in mg/l, sum of the flux / sum of Q_cumecs * 1000/86400 (not Q).
+    ``periods``: ``"year"``, ``"month"``, ``"all"`` or a list of (start, end) dates, inclusive (:func:`period_bounds`).
+
+    The members are integrated in full-output chunks as in :func:`predictive_bands`; each chunk is reduced on the
+    device over the days of every period in ascending order (one rounding per addition, so every value is bitwise
+    independent of the chunking) into its columns of a [R][M] matrix, R = len(series) * n_periods, series-major, and
+    one selection launch gives ``np.nanquantile`` of every row, bitwise.  A member whose integration raised a status
+    bit gives NaN in every row (``n_failed``).
+
+    Raises ``ValueError`` before any device work for an unknown variable or statistic, ``"fwmc"`` of Q, a reach not in
+    ``SC_list``, ``"waterbody"`` with no flagged reach, an empty ``series``, unknown ``periods``, an explicit range
+    that is reversed, not inside the record or holds no day of it, bad quantile values, more series, periods or
+    water-body reaches than ``simplyp_period_aggregates_device`` takes, and a values matrix (8 R M bytes) larger than
+    half of the free device memory.
+    """
+    import torch
+
+    from . import _cabi
+    from .engine import Engine
+    from .model import make_options
+
+    q = _check_band_quantiles(quantiles)
+    topo = pk.build_topology(p_struc, p["SC_list"])
+    desc, labels, wb = _period_series(series, topo, p_struc)
+    bounds, names = period_bounds(met_df.index, periods)
+    if bounds.shape[0] > _cabi.PERIOD_MAX_PERIODS:
+        raise ValueError("at most %d periods, got %d" % (_cabi.PERIOD_MAX_PERIODS, bounds.shape[0]))
+    p_LU, p_SC = p_LU.copy(deep=True), p_SC.copy(deep=True)
+    pk.validate_land_use(p_SC, p["SC_list"])
+    pk.check_erosion_windows(p)
+    opt = make_options(p_SU, p, dynamic_options, topo, step_len, rtol, atol)
+    opt.snow_on_device = 1 if snow_on_device else 0
+    member, sc = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, topo.sc_ids), samples)
+    M, R = member.shape[0], desc.shape[0] * bounds.shape[0]
+    eng = engine or Engine()
+    value_bytes = 8 * R * M
+    if value_bytes > eng.free_bytes() // 2:
+        raise ValueError("the values need %.1f GB, more than half of the free device memory: thin the samples "
+                         "(e.g. flat_samples(burn, thin=n)) or ask for fewer series or periods" % (value_bytes / 1e9))
+    dev = eng.device
+    values = torch.empty((R, M), dtype=torch.float64, device=dev)
+
+    def aggregate(out, d_mem, scp, diag, m0):
+        eng.period_aggregates(out, d_mem, scp, diag, desc, bounds, wb, values, m0)
+    diag = _integrate_in_chunks(eng, met_df, topo, opt, member, sc, members_per_chunk, snow_on_device, aggregate)
+    with torch.cuda.device(dev):
+        quant, mean, count = eng.nanquantile(values, q)
+    torch.cuda.synchronize(dev)
+    return PeriodStatistics(q=q, quantiles=quant.cpu().numpy(), values=values.cpu().numpy(),
+                            mean=mean.cpu().numpy(), count=count.cpu().numpy(), n_failed=_n_failed(diag),
+                            series=labels, periods=names, bounds=bounds,
+                            n_days=(bounds[:, 1] - bounds[:, 0] + 1).astype(np.int64), dates=met_df.index)
