@@ -211,7 +211,7 @@ int simplyp_topology_levels(int32_t n_sc, const int32_t* parent_offsets, const i
 
 /* Bytes of device workspace simplyp_*_device needs for these dims (flux exchange, flags, cost ordering).
  * `calibrate`: 0 = simplyp_run_device, 1 = simplyp_calibrate_device, 3 = simplyp_calibrate_device with
- * SimplypOptions.rank_stats set.  dims->reserved[0] must hold the number of edges of the reach topology. */
+ * SimplypOptions.rank_stats set, and simplyp_calibrate_ar1_device.  dims->reserved[0] must hold the number of edges of the reach topology. */
 int64_t simplyp_workspace_bytes(const SimplypDims* dims, int calibrate);
 
 /* Full-output integration (replaces model.py:365-724 for every member):
@@ -267,6 +267,33 @@ int simplyp_calibrate_gather_device(const SimplypDims* dims, const SimplypOption
                                     const double* obs, const int32_t* obs_desc,
                                     const SimplypPeerGather* gather, int64_t* diag, void* workspace, void* stream);
 
+/* Calibration mode with an autocorrelated (AR(1)) error model in the log-likelihood (simplyp_ar1.cuh): for a series v
+ * with observed days t_1 < ... < t_n, eta_i = (o_i - s_i) / sigma_i with sigma_i = m s_i as in SIMPLYP_ST_LOGLIK,
+ * rho_1 = 0, rho_i = phi^(t_i - t_{i-1}), and
+ *   LOGLIK = sum_i [ -1/2 ln 2pi - ln sigma_i - 1/2 ln(1 - rho_i^2) - (eta_i - rho_i eta_{i-1})^2 / (2 (1 - rho_i^2)) ],
+ * the exact log-density of N(s, Sigma), Sigma_ij = sigma_i sigma_j phi^|t_i - t_j| (Schoups & Vrugt 2010, Gaussian
+ * case).  phi = 0 gives the iid value; a series with no observed day gives 0; |phi| >= 1, s <= 0, sigma <= 0 or a
+ * non-finite term give -inf.
+ * Runs simplyp_calibrate_device with the simulated value of every observed day kept in the workspace (Spearman's r is
+ * still computed only with SimplypOptions.rank_stats), then one kernel overwrites stats[m][v][SIMPLYP_ST_LOGLIK] of
+ * every series v with col[v] >= 0 by the value above, with phi of member m = phi[m * row_stride + col[v]] (device
+ * memory: a column of the caller's parameter rows, e.g. the sampler's proposals).  Nothing else in stats changes, and
+ * series with col[v] < 0 keep the iid value.  The value of a row is bitwise independent of M and of the member order.
+ * Workspace: simplyp_workspace_bytes(dims, 3).  Needs n_obs_series <= SIMPLYP_AR1_MAX_SERIES.  The peer-gather entry
+ * point (simplyp_calibrate_gather_device) has no AR(1) form. */
+#define SIMPLYP_AR1_MAX_SERIES 64
+typedef struct {
+  const double* phi;        /* device */
+  int64_t row_stride;       /* >= 0 (0: every member reads row 0) */
+  int32_t col[SIMPLYP_AR1_MAX_SERIES];
+} SimplypAr1;
+
+int simplyp_calibrate_ar1_device(const SimplypDims* dims, const SimplypOptions* opt,
+                                 const double* forcing, const double* member_params, const double* sc_params,
+                                 const int32_t* parent_offsets, const int32_t* parent_ids,
+                                 const double* obs, const int32_t* obs_desc, const SimplypAr1* ar1,
+                                 double* stats, int64_t* diag, void* workspace, void* stream);
+
 /* Peer-visible device memory for the buffers above: a zeroed cudaMalloc allocation of its own (an IPC handle maps a
  * whole allocation), its 64-byte CUDA IPC handle, and the mapping of another process's handle into this one. */
 int simplyp_peer_alloc(int64_t bytes, void** dptr);
@@ -313,7 +340,10 @@ int simplyp_thornthwaite_pet_device(int32_t n_days, int32_t n_months, const doub
 enum {
   SIMPLYP_MCMC_MEMBER = 0,  /* member_params[.][index]                                   */
   SIMPLYP_MCMC_SC_ALL,      /* sc_params[.][s][index] for every sub-catchment s          */
-  SIMPLYP_MCMC_SC_AT        /* sc_params[.][pos][index], pos = position in the run order */
+  SIMPLYP_MCMC_SC_AT,       /* sc_params[.][pos][index], pos = position in the run order */
+  SIMPLYP_MCMC_ERROR_MODEL  /* written into no parameter row: an error-model parameter (the AR(1) phi of series kind
+                               `index`) that simplyp_calibrate_ar1_device reads from the proposals / walkers / scaled
+                               trials themselves */
 };
 
 typedef struct {
@@ -524,6 +554,9 @@ int simplyp_de_select_device(const SimplypDe* de, const SimplypDeState* state, c
 /* y [R][N] and diag [N][S][NDIAG] of the evaluation of the population. */
 int simplyp_de_init_device(const SimplypDe* de, const SimplypDeState* state, const double* y, const int64_t* diag,
                            void* stream);
+/* Parameter values out[n][K] of unit-cube rows unit[n][K] (the population or the trials), the value the member rows get:
+ * how the error-model targets (SIMPLYP_MCMC_ERROR_MODEL), which no row holds, reach simplyp_calibrate_ar1_device. */
+int simplyp_de_scale_device(const SimplypDe* de, const double* unit, int64_t n, double* out, void* stream);
 
 /* Host-buffer forms: same arguments as HOST pointers; the library stages them through its own
  * (cached) device buffers on `device`, runs and copies the result back before returning. */

@@ -29,6 +29,7 @@ EXPORTS = [
     "simplyp_nanquantile_device", "simplyp_sobol_design_device", "simplyp_sobol_outputs_device",
     "simplyp_sobol_workspace_bytes", "simplyp_sobol_indices_device", "simplyp_de_trial_device",
     "simplyp_de_select_device", "simplyp_de_init_device", "simplyp_period_aggregates_device",
+    "simplyp_calibrate_ar1_device", "simplyp_de_scale_device",
 ]
 MAX_RANKS = 8
 
@@ -57,7 +58,8 @@ NQ_MAX = 16
 PERIOD_MAX_SERIES, PERIOD_MAX_PERIODS, PERIOD_MAX_REACHES = 64, 2048, 256
 PERIOD_WATERBODY = -1
 PERIOD_STATS = {"mean": 0, "load": 1, "fwmc": 2}
-MCMC_MEMBER, MCMC_SC_ALL, MCMC_SC_AT = 0, 1, 2
+MCMC_MEMBER, MCMC_SC_ALL, MCMC_SC_AT, MCMC_ERROR_MODEL = 0, 1, 2, 3
+AR1_MAX_SERIES = 64
 DE_STRATEGIES = {"best1bin": 0, "rand1bin": 1}
 
 
@@ -95,6 +97,10 @@ class SimplypDeState(C.Structure):
                 ("weights", C.c_void_p), ("generation", C.c_void_p), ("best", C.c_void_p), ("converged", C.c_void_p),
                 ("converged_at", C.c_void_p), ("n_failed", C.c_void_p), ("history", C.c_void_p),
                 ("n_history", C.c_int64), ("history_base", C.c_int64)]
+
+
+class SimplypAr1(C.Structure):
+    _fields_ = [("phi", C.c_void_p), ("row_stride", C.c_int64), ("col", C.c_int32 * AR1_MAX_SERIES)]
 
 
 class SimplypError(RuntimeError):
@@ -150,6 +156,9 @@ def load():
     lib.simplyp_calibrate_gather_device.argtypes = [C.POINTER(SimplypDims), C.POINTER(SimplypOptions), vp, vp, vp, ip,
                                                     ip, vp, vp, C.POINTER(SimplypPeerGather), vp, vp, vp]
     lib.simplyp_calibrate_gather_device.restype = C.c_int
+    lib.simplyp_calibrate_ar1_device.argtypes = [C.POINTER(SimplypDims), C.POINTER(SimplypOptions), vp, vp, vp, ip, ip,
+                                                 vp, vp, C.POINTER(SimplypAr1), vp, vp, vp, vp]
+    lib.simplyp_calibrate_ar1_device.restype = C.c_int
     lib.simplyp_peer_alloc.argtypes = [C.c_int64, C.POINTER(C.c_void_p)]
     lib.simplyp_peer_alloc.restype = C.c_int
     lib.simplyp_peer_free.argtypes = [vp]
@@ -194,6 +203,8 @@ def load():
     lib.simplyp_de_select_device.restype = C.c_int
     lib.simplyp_de_init_device.argtypes = [dep, dsp, vp, vp, vp]
     lib.simplyp_de_init_device.restype = C.c_int
+    lib.simplyp_de_scale_device.argtypes = [dep, vp, C.c_int64, vp, vp]
+    lib.simplyp_de_scale_device.restype = C.c_int
     if lib.simplyp_abi_version() != 4:
         raise SimplypError("ABI version mismatch")
     _lib = lib
@@ -347,6 +358,29 @@ def calibrate_gather_device(dims, opt, forcing_ptr, member_ptr, sc_ptr, parent_o
     _check(lib.simplyp_calibrate_gather_device(C.byref(dims), C.byref(opt), forcing_ptr, member_ptr, sc_ptr, _iptr(po),
                                                _iptr(pid), obs_ptr, desc_ptr, C.byref(gather), diag_ptr, ws_ptr,
                                                stream_ptr))
+
+
+def make_ar1(phi_ptr, row_stride, col):
+    """SimplypAr1: phi of member m, series v at ``phi_ptr`` (device) + (m * row_stride + col[v]) doubles; col[v] < 0
+    keeps the iid likelihood of series v."""
+    col = [int(c) for c in col]
+    if len(col) > AR1_MAX_SERIES:
+        raise ValueError("at most %d series with an AR(1) error model" % AR1_MAX_SERIES)
+    ar = SimplypAr1()
+    ar.phi, ar.row_stride = phi_ptr, int(row_stride)
+    for v in range(AR1_MAX_SERIES):
+        ar.col[v] = col[v] if v < len(col) else -1
+    return ar
+
+
+def calibrate_ar1_device(dims, opt, forcing_ptr, member_ptr, sc_ptr, parent_offsets, parent_ids, obs_ptr, desc_ptr,
+                         ar1, stats_ptr, diag_ptr, ws_ptr, stream_ptr):
+    """Calibration with the AR(1) error model of ``ar1`` (:func:`make_ar1`) in the log-likelihood."""
+    lib = require_device()
+    po, pid = _topology_arrays(parent_offsets, parent_ids)
+    _check(lib.simplyp_calibrate_ar1_device(C.byref(dims), C.byref(opt), forcing_ptr, member_ptr, sc_ptr, _iptr(po),
+                                            _iptr(pid), obs_ptr, desc_ptr, C.byref(ar1), stats_ptr, diag_ptr, ws_ptr,
+                                            stream_ptr))
 
 
 def peer_alloc(n_bytes):
@@ -561,6 +595,11 @@ def de_init_device(de, state, y_ptr, diag_ptr, stream_ptr):
     """Energies, best member and history row 0 from the population's objective rows y [R][N] and diag; asynchronous
     on ``stream_ptr``."""
     _check(require_device().simplyp_de_init_device(C.byref(de), C.byref(state), y_ptr, diag_ptr, stream_ptr))
+
+
+def de_scale_device(de, unit_ptr, n, out_ptr, stream_ptr):
+    """Parameter values out [n][K] of unit-cube rows unit [n][K]; asynchronous on ``stream_ptr``."""
+    _check(require_device().simplyp_de_scale_device(C.byref(de), unit_ptr, int(n), out_ptr, stream_ptr))
 
 
 def workspace_bytes(dims, calibrate, rank_stats=False):

@@ -41,6 +41,7 @@
 #include "simplyp_periods.cuh"
 #include "simplyp_sobol.cuh"
 #include "simplyp_de.cuh"
+#include "simplyp_ar1.cuh"
 
 using namespace simplyp;
 
@@ -1516,16 +1517,7 @@ __global__ void mcmc_propose_kernel(const SimplypMcmc mc, const SimplypMcmcState
   const double* src = out ? st.walkers + (size_t)w * K : prop;
   double* mrow = member_params + (size_t)w * SIMPLYP_NP_MEMBER;
   double* srow = sc_params + (mc.sc_per_member ? (size_t)w * S * SIMPLYP_NP_SC : 0);
-  for (int i = 0; i < K; ++i) {
-    const SimplypMcmcParam& p = mc.param[i];
-    if (p.kind == SIMPLYP_MCMC_MEMBER) {
-      mrow[p.index] = src[i];
-    } else if (p.kind == SIMPLYP_MCMC_SC_AT) {
-      srow[(size_t)p.pos * SIMPLYP_NP_SC + p.index] = src[i];
-    } else {
-      for (int s = 0; s < S; ++s) srow[(size_t)s * SIMPLYP_NP_SC + p.index] = src[i];
-    }
-  }
+  for (int i = 0; i < K; ++i) mcmc_write_target(mc.param[i], S, src[i], mrow, srow);
 }
 
 // Half 1 also stores the chain slot of the iteration: thread k writes walker k (half 0, final since the half-0
@@ -1572,6 +1564,8 @@ int check_targets(const SimplypMcmcParam* param, int K, int n_sc, int sc_per_mem
       if (p.index < 0 || p.index >= SIMPLYP_NP_SC) return fail(SIMPLYP_EINVAL, "%s: SC row out of range", what);
       if (p.kind == SIMPLYP_MCMC_SC_AT && (p.pos < 0 || p.pos >= n_sc)) return fail(SIMPLYP_EINVAL, "%s: SC position out of range", what);
       if (!sc_per_member) return fail(SIMPLYP_EINVAL, "%s: SC targets need per-member sc_params", what);
+    } else if (p.kind == SIMPLYP_MCMC_ERROR_MODEL) {
+      if (p.index < 0 || p.index >= SIMPLYP_NVARKIND) return fail(SIMPLYP_EINVAL, "%s: error-model kind out of range", what);
     } else {
       return fail(SIMPLYP_EINVAL, "%s: unknown target kind", what);
     }
@@ -1904,17 +1898,7 @@ __global__ void sobol_design_kernel(const SimplypSobol sb, long long member_offs
   const int S = sb.n_sc;
   double* mrow = member_params + (size_t)m * SIMPLYP_NP_MEMBER;
   double* srow = sc_params + (sb.sc_per_member ? (size_t)m * S * SIMPLYP_NP_SC : 0);
-  for (int j = 0; j < sb.n_free; ++j) {
-    const SimplypMcmcParam& p = sb.param[j];
-    const double v = sobol_design_value(sb, m, j);
-    if (p.kind == SIMPLYP_MCMC_MEMBER) {
-      mrow[p.index] = v;
-    } else if (p.kind == SIMPLYP_MCMC_SC_AT) {
-      srow[(size_t)p.pos * SIMPLYP_NP_SC + p.index] = v;
-    } else {
-      for (int s = 0; s < S; ++s) srow[(size_t)s * SIMPLYP_NP_SC + p.index] = v;
-    }
-  }
+  for (int j = 0; j < sb.n_free; ++j) mcmc_write_target(sb.param[j], S, sobol_design_value(sb, m, j), mrow, srow);
 }
 
 // Objective rows Y[r][m] from the fused statistics: one thread per (member, row).
@@ -2275,17 +2259,15 @@ __global__ void de_trial_kernel(const SimplypDe de, const SimplypDeState st, dou
   de_trial_member(de, st.population, *st.best, g, i, de_dither(de, g), tr);
   double* mrow = member_params + (size_t)i * SIMPLYP_NP_MEMBER;
   double* srow = sc_params + (de.sc_per_member ? (size_t)i * S * SIMPLYP_NP_SC : 0);
-  for (int j = 0; j < K; ++j) {
-    const SimplypMcmcParam& p = de.param[j];
-    const double v = de_scale(p, tr[j]);
-    if (p.kind == SIMPLYP_MCMC_MEMBER) {
-      mrow[p.index] = v;
-    } else if (p.kind == SIMPLYP_MCMC_SC_AT) {
-      srow[(size_t)p.pos * SIMPLYP_NP_SC + p.index] = v;
-    } else {
-      for (int s = 0; s < S; ++s) srow[(size_t)s * SIMPLYP_NP_SC + p.index] = v;
-    }
-  }
+  for (int j = 0; j < K; ++j) mcmc_write_target(de.param[j], S, de_scale(de.param[j], tr[j]), mrow, srow);
+}
+
+// Parameter values of unit-cube rows: one thread per (row, parameter).
+__global__ void de_scale_kernel(const SimplypDe de, const double* unit, long long n, double* out) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  const int K = de.n_free;
+  if (idx >= n * K) return;
+  out[idx] = de_scale(de.param[idx % K], unit[idx]);
 }
 
 __global__ void de_select_kernel(const SimplypDe de, const SimplypDeState st, const double* y, const int64_t* diag) {
@@ -2461,7 +2443,7 @@ static int calibrate_device_impl(const SimplypDims* dims, const SimplypOptions* 
                                  const double* member_params, const double* sc_params,
                                  const int32_t* parent_offsets, const int32_t* parent_ids, const double* obs,
                                  const int32_t* obs_desc, double* stats, int64_t* diag, void* workspace,
-                                 void* stream, const SimplypPeerGather* pg) {
+                                 void* stream, const SimplypPeerGather* pg, const SimplypAr1* ar1) {
   int rc = check_common(dims, opt, forcing, member_params, sc_params, parent_offsets);
   if (rc) return rc;
   if (dims->n_obs_series < 0 || (dims->n_obs_series > 0 && (!obs || !obs_desc || !stats)))
@@ -2471,7 +2453,9 @@ static int calibrate_device_impl(const SimplypDims* dims, const SimplypOptions* 
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const int V = dims->n_obs_series;
   const bool ranks = opt->rank_stats != 0 && V > 0 && dims->n_days > 0;
-  const WsLayout L = ws_layout(*dims, parent_offsets[dims->n_sc], true, ranks);
+  // the simulated value of every observed day, for Spearman's r and for the AR(1) likelihood
+  const bool keep_sim = (ranks || ar1 != nullptr) && V > 0 && dims->n_days > 0;
+  const WsLayout L = ws_layout(*dims, parent_offsets[dims->n_sc], true, keep_sim);
   char* ws = static_cast<char*>(workspace);
   KArgs a = base_args(*dims, *opt, forcing, member_params, sc_params);
   a.diag = reinterpret_cast<long long*>(diag);
@@ -2496,6 +2480,8 @@ static int calibrate_device_impl(const SimplypDims* dims, const SimplypOptions* 
       if (ranks) {
         obs_rank_kernel<<<V, 256, 0, st>>>(obs, dims->n_days, obs_rank, reinterpret_cast<double*>(ws + L.off_oc));
         g_launches.fetch_add(1);
+      }
+      if (keep_sim) {
         a.sim_obs = reinterpret_cast<double*>(ws + L.off_sim_obs);
         // a day without a finite simulated value must read as NaN (dropped pair)
         SP_CUDA(cudaMemsetAsync(a.sim_obs, 0xff, sizeof(double) * (size_t)dims->n_members * V * dims->n_days, st));
@@ -2524,6 +2510,13 @@ static int calibrate_device_impl(const SimplypDims* dims, const SimplypOptions* 
     g_launches.fetch_add(1);
     SP_CUDA(cudaGetLastError());
   }
+  if (keep_sim && ar1 != nullptr) {
+    const long long rows = (long long)dims->n_members * V;
+    ar1_loglik_kernel<<<(unsigned)((rows + AR1_WARPS - 1) / AR1_WARPS), AR1_WARPS * 32, 0, st>>>(
+        a.sim_obs, obs, obs_desc, member_params, *ar1, dims->n_members, V, dims->n_days, stats);
+    g_launches.fetch_add(1);
+    SP_CUDA(cudaGetLastError());
+  }
   if (pg != nullptr && pg->n_ranks > 1) {
     PeerFlags f;
     for (int r = 0; r < SIMPLYP_MAX_RANKS; ++r) f.bufs[r] = r < pg->n_ranks ? pg->flag_bufs[r] : nullptr;
@@ -2541,7 +2534,21 @@ int simplyp_calibrate_device(const SimplypDims* dims, const SimplypOptions* opt,
                              const int32_t* obs_desc, double* stats, int64_t* diag, void* workspace,
                              void* stream) {
   return calibrate_device_impl(dims, opt, forcing, member_params, sc_params, parent_offsets, parent_ids, obs, obs_desc,
-                               stats, diag, workspace, stream, nullptr);
+                               stats, diag, workspace, stream, nullptr, nullptr);
+}
+
+int simplyp_calibrate_ar1_device(const SimplypDims* dims, const SimplypOptions* opt, const double* forcing,
+                                 const double* member_params, const double* sc_params,
+                                 const int32_t* parent_offsets, const int32_t* parent_ids, const double* obs,
+                                 const int32_t* obs_desc, const SimplypAr1* ar1, double* stats, int64_t* diag,
+                                 void* workspace, void* stream) {
+  if (!ar1 || !dims) return fail(SIMPLYP_EINVAL, "ar1: null argument%s");
+  if (dims->n_obs_series > SIMPLYP_AR1_MAX_SERIES) return fail(SIMPLYP_EINVAL, "ar1: at most SIMPLYP_AR1_MAX_SERIES series%s");
+  if (ar1->row_stride < 0) return fail(SIMPLYP_EINVAL, "ar1: negative row stride%s");
+  for (int v = 0; v < dims->n_obs_series; ++v)
+    if (ar1->col[v] >= 0 && !ar1->phi) return fail(SIMPLYP_EINVAL, "ar1: null phi%s");
+  return calibrate_device_impl(dims, opt, forcing, member_params, sc_params, parent_offsets, parent_ids, obs, obs_desc,
+                               stats, diag, workspace, stream, nullptr, ar1);
 }
 
 int simplyp_calibrate_gather_device(const SimplypDims* dims, const SimplypOptions* opt, const double* forcing,
@@ -2560,7 +2567,7 @@ int simplyp_calibrate_gather_device(const SimplypDims* dims, const SimplypOption
   double* stats = gather->stats_bufs[gather->rank] +
                   (size_t)gather->member_offset * (dims->n_obs_series > 0 ? dims->n_obs_series : 0) * SIMPLYP_NSTAT;
   return calibrate_device_impl(dims, opt, forcing, member_params, sc_params, parent_offsets, parent_ids, obs, obs_desc,
-                               stats, diag, workspace, stream, gather);
+                               stats, diag, workspace, stream, gather, nullptr);
 }
 
 int simplyp_peer_alloc(int64_t bytes, void** dptr) {
@@ -3044,6 +3051,21 @@ int simplyp_de_init_device(const SimplypDe* de, const SimplypDeState* state, con
   de_init_kernel<<<(N + 127) / 128, 128, 0, st>>>(*de, *state, y, diag);
   de_reduce_kernel<<<1, DE_THREADS, 0, st>>>(*de, *state, 1);
   g_launches.fetch_add(2);
+  SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
+int simplyp_de_scale_device(const SimplypDe* de, const double* unit, int64_t n, double* out, void* stream) {
+  if (!de || !unit || !out || n < 0) return fail(SIMPLYP_EINVAL, "de_scale: null argument or negative count%s");
+  const int K = de->n_free;
+  if (K < 1 || K > SIMPLYP_MCMC_MAX_FREE) return fail(SIMPLYP_EINVAL, "de_scale: 1..SIMPLYP_MCMC_MAX_FREE free parameters%s");
+  const int rc = check_targets(de->param, K, de->n_sc, de->sc_per_member, "de_scale");
+  if (rc) return rc;
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  if (n == 0) return SIMPLYP_OK;
+  const long long total = (long long)n * K;
+  de_scale_kernel<<<(unsigned)((total + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(*de, unit, n, out);
+  g_launches.fetch_add(1);
   SP_CUDA(cudaGetLastError());
   return SIMPLYP_OK;
 }

@@ -111,6 +111,19 @@ SP_HD int mcmc_propose_walker(const SimplypMcmc& mc, const double* walkers, long
   return out;
 }
 
+// Writes value v of free parameter p into the member's parameter row mrow[NP_MEMBER] or its sub-catchment rows
+// srow[S][NP_SC] (the sampler's proposals, the DE trials and the Sobol' design all place their values this way).  An
+// error-model parameter (SIMPLYP_MCMC_ERROR_MODEL) is in no row: simplyp_calibrate_ar1_device reads it where it is.
+SP_HD void mcmc_write_target(const SimplypMcmcParam& p, int S, double v, double* mrow, double* srow) {
+  if (p.kind == SIMPLYP_MCMC_MEMBER) {
+    mrow[p.index] = v;
+  } else if (p.kind == SIMPLYP_MCMC_SC_AT) {
+    srow[(size_t)p.pos * SIMPLYP_NP_SC + p.index] = v;
+  } else if (p.kind == SIMPLYP_MCMC_SC_ALL) {
+    for (int s = 0; s < S; ++s) srow[(size_t)s * SIMPLYP_NP_SC + p.index] = v;
+  }
+}
+
 // Log-probability of one member from its fused statistics: the sum of the Gaussian log-likelihoods of its V series
 // (stats row [V][SIMPLYP_NSTAT]), or -inf if the integration of any of its S sub-catchments raised a status bit
 // (diag row [S][SIMPLYP_NDIAG]) or the sum is not a number.  The uniform prior adds 0 inside the box.

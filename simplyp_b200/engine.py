@@ -81,33 +81,42 @@ class Engine:
 
     # ------------------------------------------------------------------ fused statistics
     def calibrate(self, forcing, member_params, sc_params, parent_offsets, parent_ids, obs, obs_desc, opt,
-                  stats=None, diag=None, max_workspace_bytes=None, peer_gather=None):
+                  stats=None, diag=None, max_workspace_bytes=None, peer_gather=None, phi=None, phi_col=None):
         """Returns (stats [M][V][10], diag [M][S][4]); asynchronous on the current stream.
+
+        With ``phi`` (a contiguous [M][P] fp64 device tensor) and ``phi_col`` ([V] ints) the log-likelihood of series v
+        has the AR(1) error model with phi = ``phi[m][phi_col[v]]`` (``simplyp_calibrate_ar1_device``); series with
+        ``phi_col[v] < 0`` keep the iid value.
 
         With ``peer_gather`` (an :class:`ensemble.PeerGather`; the members given here are this rank's shard) the
         statistics of ALL ranks come back, [M_total][V][10]: the kernel stores them into every rank's buffer and a flag
         exchange ends the call on the stream — no collective follows.
 
         The workspace grows with the members: M*S*D*32 bytes of flux exchange for networks (S > 1) and M*V*D*8
-        bytes of simulated values with ``opt.rank_stats``; members are processed in chunks that keep it under
+        bytes of simulated values with ``opt.rank_stats`` or ``phi``; members are processed in chunks that keep it under
         ``max_workspace_bytes`` (default: half of the free HBM).
         """
         torch = _torch()
         D, M, Msc, S, sc_params = self._shapes(forcing, member_params, sc_params)
         V = obs.shape[0]
         n_edges = int(parent_offsets[-1])
+        if phi is not None and (phi.dim() != 2 or phi.shape[0] != M or phi.dtype != torch.float64
+                                or not phi.is_contiguous() or phi_col is None or len(phi_col) != V):
+            raise ValueError("phi must be a contiguous [M][P] float64 tensor and phi_col hold one column per series")
         if stats is None and peer_gather is None:
             stats = torch.empty((M, V, pk.NSTAT), dtype=torch.float64, device=self.device)
         if diag is None:
             diag = torch.zeros((M, S, pk.NDIAG), dtype=torch.int64, device=self.device)
         chunk = M
-        per_member = (32 * S * D if S > 1 else 0) + (8 * V * D if opt.rank_stats else 0)
+        keep_sim = bool(opt.rank_stats) or phi is not None
+        per_member = (32 * S * D if S > 1 else 0) + (8 * V * D if keep_sim else 0)
         if per_member > 0:
             budget = max_workspace_bytes if max_workspace_bytes is not None else self.free_bytes() // 2
             chunk = max(1, min(M, int(budget // per_member)))
         if peer_gather is not None:
-            if chunk < M or opt.rank_stats or M != peer_gather.hi - peer_gather.lo:
-                raise _cabi.SimplypError("peer_gather: one launch of this rank's whole shard, without rank statistics")
+            if chunk < M or keep_sim or M != peer_gather.hi - peer_gather.lo:
+                raise _cabi.SimplypError("peer_gather: one launch of this rank's whole shard, without rank statistics "
+                                         "or an AR(1) error model")
             with torch.cuda.device(self.device):
                 stream = torch.cuda.current_stream().cuda_stream
                 dims = _cabi.make_dims(M, S, D, 1 if Msc == 1 else M, V, n_edges)
@@ -122,12 +131,16 @@ class Engine:
             for m0 in range(0, M, chunk):
                 m1 = min(M, m0 + chunk)
                 dims = _cabi.make_dims(m1 - m0, S, D, 1 if Msc == 1 else (m1 - m0), V, n_edges)
-                ws = self._workspace(_cabi.workspace_bytes(dims, True, bool(opt.rank_stats)))
+                ws = self._workspace(_cabi.workspace_bytes(dims, True, keep_sim))
                 scp = sc_params if Msc == 1 else sc_params[m0:m1]
-                _cabi.calibrate_device(dims, opt, forcing.data_ptr(), member_params[m0:m1].data_ptr(),
-                                       scp.data_ptr(), parent_offsets, parent_ids, obs.data_ptr(),
-                                       obs_desc.data_ptr(), stats[m0:m1].data_ptr(), diag[m0:m1].data_ptr(),
-                                       ws.data_ptr(), stream)
+                args = (dims, opt, forcing.data_ptr(), member_params[m0:m1].data_ptr(), scp.data_ptr(), parent_offsets,
+                        parent_ids, obs.data_ptr(), obs_desc.data_ptr())
+                tail = (stats[m0:m1].data_ptr(), diag[m0:m1].data_ptr(), ws.data_ptr(), stream)
+                if phi is None:
+                    _cabi.calibrate_device(*args, *tail)
+                else:
+                    ar1 = _cabi.make_ar1(phi[m0:m1].data_ptr(), phi.shape[1], phi_col)
+                    _cabi.calibrate_ar1_device(*args, ar1, *tail)
         return stats, diag
 
     # ------------------------------------------------------------------ receiving water body
@@ -280,6 +293,11 @@ class Engine:
         """Selection of one generation from the trials' objective rows ``y`` [R][N] (:meth:`sobol_outputs`) and
         ``diag`` [N][S][4] (``simplyp_de_select_device``).  Asynchronous."""
         self._de_call(_cabi.de_select_device, de, state, y.data_ptr(), diag.data_ptr())
+
+    def de_scale(self, de, unit, out):
+        """Parameter values ``out`` [n][K] of unit-cube rows ``unit`` [n][K] (``simplyp_de_scale_device``).
+        Asynchronous."""
+        self._de_call(_cabi.de_scale_device, de, unit.data_ptr(), unit.shape[0], out.data_ptr())
 
     def de_init(self, de, state, y, diag):
         """Energies, best member and history row 0 from the population's objective rows ``y`` [R][N] and ``diag``

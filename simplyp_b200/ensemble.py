@@ -37,11 +37,13 @@ def latin_hypercube(n, ranges=None, seed=20260101):
     return out
 
 
-def pack_members(base_member, base_sc, samples):
+def pack_members(base_member, base_sc, samples, return_phi=False):
     """Broadcast the base parameter vectors over the ensemble and apply the sampled columns.
 
     base_member [NP_MEMBER], base_sc [S][NP_SC], samples: dict name -> [M].
-    Returns (member_params [M][NP_MEMBER], sc_params [1 or M][S][NP_SC]).
+    Returns (member_params [M][NP_MEMBER], sc_params [1 or M][S][NP_SC]).  The AR(1) error-model parameters
+    ``err_phi:<kind>`` are in neither: with ``return_phi`` they come back separately as a third item, a dict
+    name -> [M] in the order of ``samples``.
     """
     M = len(next(iter(samples.values()))) if samples else 1
     member = np.repeat(np.asarray(base_member, dtype=np.float64)[None, :], M, axis=0)
@@ -49,9 +51,12 @@ def pack_members(base_member, base_sc, samples):
     per_member_sc = any(k.startswith("sc:") for k in samples)
     if per_member_sc:
         sc = np.repeat(sc, M, axis=0)
+    phi = {}
     for name, vals in samples.items():
         vals = np.asarray(vals, dtype=np.float64)
-        if name.startswith("sc:"):
+        if name.startswith(pk.ERR_PHI):
+            phi[name] = vals
+        elif name.startswith("sc:"):
             row = name[3:]
             if "@" in row:                       # sc:<row>@<position in run order>
                 row, at = row.split("@")
@@ -60,6 +65,8 @@ def pack_members(base_member, base_sc, samples):
                 sc[:, :, pk.SC_INDEX[row]] = vals[:, None]
         else:
             member[:, pk.MEMBER_INDEX[name]] = vals
+    if return_phi:
+        return np.ascontiguousarray(member), np.ascontiguousarray(sc), phi
     return np.ascontiguousarray(member), np.ascontiguousarray(sc)
 
 
@@ -69,7 +76,7 @@ def apply_member_to_pandas(samples, i, p, p_LU, p_SC):
     p, p_LU, p_SC = p.copy(deep=True), p_LU.copy(deep=True), p_SC.copy(deep=True)
     for name, vals in samples.items():
         v = float(vals[i])
-        if name.startswith("err_m:"):
+        if name.startswith("err_m:") or name.startswith(pk.ERR_PHI):
             continue
         if name.startswith("sc:"):
             row = name[3:]
@@ -284,6 +291,10 @@ def calibrate_ensemble(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, ob
     ``snow_on_device``: ``met_df`` carries the raw ``Precipitation`` and ``T_air``; the degree-day snow module
     (reference ``inputs.py:159-210``) runs per member on the device, so ``D_snow_0`` and ``f_DDSM`` may be sampled.
     ``rank_stats``: also reduce Spearman's r (the whole table of ``goodness_of_fit_stats``).
+    ``err_phi:<variable>`` in ``samples`` gives the log-likelihood of that variable's series the AR(1) error model with
+    that lag-one autocorrelation (``simplyp_calibrate_ar1_device``); the other statistics do not change.  An
+    ``err_phi`` name of an unknown variable or of one not among ``variables`` raises ``ValueError`` before any device
+    work.
 
     Returns ``(stats [M][V][10] torch tensor on the device, labels [(reach, variable)], diag)``.
     """
@@ -300,18 +311,22 @@ def calibrate_ensemble(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, ob
     opt = make_options(p_SU, p, dynamic_options, topo, step_len, rtol, atol)
     opt.snow_on_device = 1 if snow_on_device else 0
     opt.rank_stats = 1 if rank_stats else 0
-    member, sc = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, topo.sc_ids), samples)
+    member, sc, phi = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, topo.sc_ids), samples,
+                                   return_phi=True)
     M = member.shape[0]
     rank, world = (dist.get_rank(), dist.get_world_size()) if (dist.is_available() and dist.is_initialized()) else (0, 1)
     lo, hi = shard_bounds(M, world, rank)
     obs, desc, labels = pk.obs_arrays(obs_dict, topo, met_df.index, variables)
+    phi_col = pk.ar1_columns(list(phi), labels, variables)
     eng = engine or Engine()
     d_forc = eng.to_device(pk.forcing_matrix(met_df, raw_snow=bool(snow_on_device)))
     d_mem = eng.to_device(member[lo:hi])
     d_sc = eng.to_device(sc if sc.shape[0] == 1 else sc[lo:hi])
     d_obs = eng.to_device(obs)
     d_desc = eng.to_device(desc)
-    stats, diag = eng.calibrate(d_forc, d_mem, d_sc, topo.parent_offsets, topo.parent_ids, d_obs, d_desc, opt)
+    d_phi = eng.to_device(np.stack(list(phi.values()), axis=1)[lo:hi]) if phi else None
+    stats, diag = eng.calibrate(d_forc, d_mem, d_sc, topo.parent_offsets, topo.parent_ids, d_obs, d_desc, opt,
+                                phi=d_phi, phi_col=phi_col if phi else None)
     if gather and world > 1:
         stats = all_gather_stats(stats, M)
     torch.cuda.synchronize(eng.device)
@@ -557,7 +572,9 @@ def predictive_bands(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, samp
     also carries the likelihood's error model, y = s + m s eps with eps ~ N(0, 1) and m the member's ``err_m:<var>``,
     keyed by ``seed``: a draw depends on (seed, member, day, series) only, not on the chunking.  A member whose
     integration raised a status bit enters no band (``n_failed``).  ``snow_on_device`` as in
-    ``calibrate_ensemble``.
+    ``calibrate_ensemble``.  AR(1) error-model columns ``err_phi:<var>`` of ``samples`` (a posterior sampled with
+    them) are accepted and ignored: the AR(1) process has unit variance, so each day's marginal N(s, (m s)^2) does not
+    depend on phi, and neither does a daily quantile.
 
     Raises ``ValueError`` before any device work for an unknown variable, a reach not in ``SC_list``, an empty
     ``series``, quantile values that are not finite, lie outside [0, 1] or number more than 16, and a matrix of
@@ -787,7 +804,8 @@ def period_statistics(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, sam
     device over the days of every period in ascending order (one rounding per addition, so every value is bitwise
     independent of the chunking) into its columns of a [R][M] matrix, R = len(series) * n_periods, series-major, and
     one selection launch gives ``np.nanquantile`` of every row, bitwise.  A member whose integration raised a status
-    bit gives NaN in every row (``n_failed``).
+    bit gives NaN in every row (``n_failed``).  AR(1) error-model columns ``err_phi:<var>`` of ``samples`` are accepted
+    and ignored: the aggregates are of the simulated series, which do not depend on phi.
 
     Raises ``ValueError`` before any device work for an unknown variable or statistic, ``"fwmc"`` of Q, a reach not in
     ``SC_list``, ``"waterbody"`` with no flagged reach, an empty ``series``, unknown ``periods``, an explicit range

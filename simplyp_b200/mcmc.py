@@ -12,6 +12,8 @@ at the start and at the end.
 The log-probability of a parameter set is the sum of the Gaussian log-likelihoods of the observed series
 (``SIMPLYP_ST_LOGLIK``, ``MCMC.ipynb:213-242``; the error scales ``err_m:<var>`` may be sampled) plus the log of the
 unnormalised box prior (0 inside, -inf outside).  A parameter set whose integration raised a status bit gets -inf.
+Sampling ``err_phi:<var>`` gives the series of that variable the AR(1) error model of ``simplyp_calibrate_ar1_device``
+(autocorrelated residuals, Schoups & Vrugt 2010) with phi sampled alongside the model parameters.
 """
 from __future__ import annotations
 
@@ -34,6 +36,11 @@ _SNOW = ("D_snow_0", "f_DDSM")
 def _target(name, n_sc, snow_on_device):
     """(kind, index, pos) of the C-ABI for a parameter name of ``ensemble.pack_members``; ValueError if it cannot be
     sampled."""
+    if name.startswith(pk.ERR_PHI):
+        kind = name[len(pk.ERR_PHI):]
+        if kind not in pk.VAR_INDEX:
+            raise ValueError("unknown series kind in %r: one of %s" % (name, pk.VAR_KINDS))
+        return (_cabi.MCMC_ERROR_MODEL, pk.VAR_INDEX[kind], 0)
     if name.startswith("sc:"):
         row, at = name[3:], None
         if "@" in row:
@@ -147,6 +154,9 @@ class _Sampler:
         member, sc = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, self.topo.sc_ids),
                                   {n: x0[:, k] for k, n in enumerate(self.names)})
         obs, desc, self.labels = pk.obs_arrays(obs_dict, self.topo, met_df.index, variables)
+        # the AR(1) phi of series v is column phi_col[v] of the walkers (initial evaluation) and of the proposals
+        col = pk.ar1_columns(self.names, self.labels, variables)
+        self.phi_col = col if any(c >= 0 for c in col) else None
         self.W, self.H, self.K, self.V, self.S = W, W // 2, K, obs.shape[0], n_sc
         self.n_steps, self.thin, self.start = int(n_steps), int(thin), int(start_iteration)
         self.n_saved = (self.start + self.n_steps) // self.thin - self.start // self.thin
@@ -175,6 +185,7 @@ class _Sampler:
         self.accepted = torch.zeros(W, dtype=i64, device=dev)
         self.chain = torch.zeros((self.n_saved, W, K), dtype=f64, device=dev)
         self.chain_lp = torch.zeros((self.n_saved, W), dtype=f64, device=dev)
+        self.ws_budget = eng.free_bytes() // 2 if self.phi_col is not None else None
         self.mc = _cabi.make_mcmc(W, targets, self.bounds[:, 0], self.bounds[:, 1], n_sc, self.V,
                                   sc_per_member=sc.shape[0] > 1, thin=self.thin, seed=seed, stretch=stretch)
         self.state = _cabi.make_mcmc_state(
@@ -195,7 +206,7 @@ class _Sampler:
         with self._device():
             self.diag.zero_()
             self.eng.calibrate(self.d_forc, mem, sc, self.topo.parent_offsets, self.topo.parent_ids, self.d_obs,
-                               self.d_desc, self.opt, stats=self.stats, diag=self.diag)
+                               self.d_desc, self.opt, stats=self.stats, diag=self.diag, **self._phi(self.walkers))
             _cabi.mcmc_init_device(self.mc, self.state, self.stats.data_ptr(), self.diag.data_ptr(), self._stream())
         lp = self.lp.cpu().numpy()
         bad = np.flatnonzero(~np.isfinite(lp))
@@ -213,7 +224,13 @@ class _Sampler:
         with self._device():
             self.diag[lo:hi].zero_()
             self.eng.calibrate(self.d_forc, mem, sc, self.topo.parent_offsets, self.topo.parent_ids, self.d_obs,
-                               self.d_desc, self.opt, stats=self.stats[lo:hi], diag=self.diag[lo:hi])
+                               self.d_desc, self.opt, stats=self.stats[lo:hi], diag=self.diag[lo:hi],
+                               **self._phi(self.proposals))
+
+    def _phi(self, rows):
+        # the workspace budget is fixed up front: no memory query while an iteration is being captured
+        return {} if self.phi_col is None else {"phi": rows, "phi_col": self.phi_col,
+                                                "max_workspace_bytes": self.ws_budget}
 
     def accept(self, half):
         lo = half * self.H
@@ -267,14 +284,16 @@ def sample(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, obs_dict, prio
 
     Inputs are those of ``ensemble.calibrate_ensemble``; ``priors`` maps parameter names of
     ``ensemble.pack_members`` (member fields, ``sc:<row>``, ``sc:<row>@<run-order position>``) to the bounds
-    ``(lo, hi)`` of a uniform prior (``ensemble.TARLAND_RANGES`` works as it is).  The other parameters keep the
+    ``(lo, hi)`` of a uniform prior (``ensemble.TARLAND_RANGES`` works as it is), and ``err_phi:<var>`` to the box of
+    the AR(1) autocorrelation of the residuals of ``var`` (e.g. (0, 0.99)).  The other parameters keep the
     values of ``p`` / ``p_LU`` / ``p_SC``.  ``initial``: walkers [W][K] (or a dict name -> [W], or an
     :class:`McmcResult` to continue, with ``start_iteration=result.iterations``); default: a Latin hypercube over the
     prior box drawn with ``seed``, which also keys the sampler's random numbers.  ``thin``: every ``thin``-th
     iteration is stored.  ``stretch``: the scale a of the stretch move.
 
     Raises ``ValueError`` before any device work for a name that cannot be sampled — unknown, the integer-valued
-    ``d_maxE_*``, the land-use fractions ``sc:f_*``, ``D_snow_0`` / ``f_DDSM`` without ``snow_on_device`` — for bounds
+    ``d_maxE_*``, the land-use fractions ``sc:f_*``, ``D_snow_0`` / ``f_DDSM`` without ``snow_on_device``, ``err_phi``
+    of an unknown variable or of one not among ``variables`` — for bounds
     that are not finite with lo < hi, and for an odd ``n_walkers`` or fewer than twice the free parameters; after the
     initial evaluation, if an initial walker's log-probability is not finite.
     """

@@ -152,6 +152,8 @@ class _Optimizer:
         topo = pk.build_topology(p_struc, p["SC_list"])
         obs, desc, obs_labels = pk.obs_arrays(obs_dict, topo, met_df.index, variables)
         rows, self.labels, self.weights = _objective_weights(objective, obs_labels)
+        col = pk.ar1_columns(self.names, obs_labels, variables)
+        self.phi_col = col if any(c >= 0 for c in col) else None
         if initial is None:
             u0 = latin_hypercube_unit(N, K, seed)
         elif isinstance(initial, DeResult):
@@ -201,6 +203,9 @@ class _Optimizer:
         self.stats = torch.zeros((N, self.V, pk.NSTAT), dtype=f64, device=dev)
         self.diag = torch.zeros((N, n_sc, pk.NDIAG), dtype=i64, device=dev)
         self.y = torch.zeros((self.R, N), dtype=f64, device=dev)
+        # parameter values of the rows being evaluated: where the AR(1) phi, which no member row holds, is read
+        self.values = torch.zeros((N, K), dtype=f64, device=dev) if self.phi_col is not None else None
+        self.ws_budget = eng.free_bytes() // 2 if self.phi_col is not None else None
         self.population = eng.to_device(u0)
         self.energy = torch.zeros(N, dtype=f64, device=dev)
         self.trial = torch.zeros((N, K), dtype=f64, device=dev)
@@ -220,16 +225,23 @@ class _Optimizer:
         import torch
         return torch.cuda.device(self.eng.device)
 
-    def evaluate(self):
-        """Zero the status words, integrate all N rows with the fused statistics, take the objective rows."""
+    def evaluate(self, unit=None):
+        """Zero the status words, integrate all N rows with the fused statistics, take the objective rows.  ``unit``:
+        the unit-cube rows the member rows hold (default: the trials), where an AR(1) phi is read."""
+        unit = self.trial if unit is None else unit
         with self._device():
             self.diag.zero_()
+            phi = {}
+            if self.phi_col is not None:
+                self.eng.de_scale(self.de, unit, self.values)
+                # (a fixed workspace budget: no memory query while a generation is being captured)
+                phi = {"phi": self.values, "phi_col": self.phi_col, "max_workspace_bytes": self.ws_budget}
             self.eng.calibrate(self.d_forc, self.d_mem, self.d_sc, self.topo.parent_offsets, self.topo.parent_ids,
-                               self.d_obs, self.d_desc, self.opt, stats=self.stats, diag=self.diag)
+                               self.d_obs, self.d_desc, self.opt, stats=self.stats, diag=self.diag, **phi)
             self.eng.sobol_outputs(self.stats, self.diag, self.d_rows, self.y)
 
     def evaluate_initial(self):
-        self.evaluate()
+        self.evaluate(self.population)
         self.eng.de_init(self.de, self.state, self.y, self.diag)
 
     def trial_step(self):
@@ -298,8 +310,9 @@ def differential_evolution(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options
     ``n_population`` members over at most ``max_generations`` generations.
 
     Inputs are those of ``ensemble.calibrate_ensemble``; ``ranges`` maps parameter names of ``ensemble.pack_members``
-    to boxes ``(lo, hi)``, as ``mcmc.sample`` takes them (``ensemble.TARLAND_RANGES`` works as it is).  The other
-    parameters keep the values of ``p`` / ``p_LU`` / ``p_SC``.
+    to boxes ``(lo, hi)``, as ``mcmc.sample`` takes them (``ensemble.TARLAND_RANGES`` works as it is), including the
+    AR(1) autocorrelations ``err_phi:<var>`` of the likelihood's residuals.  The other parameters keep the values of
+    ``p`` / ``p_LU`` / ``p_SC``.
 
     ``objective``: a statistic of ``DE_OBJECTIVES`` (weight 1 on every observed series of ``variables``; ``"lp"`` is the
     sampler's log-probability, so the default finds the maximum likelihood), or a dict of weights ``{stat: w}`` (every

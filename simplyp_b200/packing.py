@@ -48,6 +48,10 @@ STAT_NAMES = ["n", "NSE", "log_NSE", "loglik", "r2", "pbias", "nRMSD", "SSE", "s
 
 DEFAULT_ERR_M = 0.5   # likelihood error scale when the ensemble does not sample it
 
+# ``err_phi:<kind>``: the lag-one autocorrelation phi of the AR(1) error model of the series of that kind
+# (simplyp_calibrate_ar1_device).  Not a column of the member vector: it is passed to the likelihood on its own.
+ERR_PHI = "err_phi:"
+
 
 def _f(x):
     try:
@@ -202,3 +206,20 @@ def obs_arrays(obs_dict, topology, date_index, variables=None, min_obs=10):
     D = len(date_index)
     obs = np.asarray(rows, dtype=np.float64).reshape(len(rows), D) if rows else np.zeros((0, D))
     return obs, np.asarray(desc, dtype=np.int32).reshape(len(desc), 2), labels
+
+
+def ar1_columns(names, labels, variables):
+    """``SimplypAr1.col`` of the observed series ``labels`` [(sc_id, variable)]: the position in ``names`` of
+    ``err_phi:<variable>``, or -1 (iid likelihood).  Raises ``ValueError`` for an ``err_phi`` name of an unknown kind
+    or of a kind not among ``variables`` (None: every kind)."""
+    pos = {}
+    for j, name in enumerate(names):
+        if not name.startswith(ERR_PHI):
+            continue
+        kind = name[len(ERR_PHI):]
+        if kind not in VAR_INDEX:
+            raise ValueError("unknown series kind in %r: one of %s" % (name, VAR_KINDS))
+        if variables is not None and kind not in variables:
+            raise ValueError("%r: %s is not among the calibrated variables %s" % (name, kind, list(variables)))
+        pos[kind] = j
+    return [pos.get(var, -1) for _sc, var in labels]

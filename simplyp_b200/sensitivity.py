@@ -110,7 +110,8 @@ def sobol_indices(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, ranges,
     integration failed removes its sample.  Confidences are ``z(conf_level)`` times the standard deviation over
     ``n_boot`` bootstrap resamples drawn with ``seed``.
 
-    Raises ``ValueError`` before any device work for everything ``mcmc.sample`` refuses in ``ranges``, an
+    Raises ``ValueError`` before any device work for everything ``mcmc.sample`` refuses in ``ranges``, the AR(1)
+    error-model parameters ``err_phi:*``, an
     ``n_base`` that is not a power of two >= 2, skip + n_base > 2^32, both or neither of ``objectives`` and
     ``series``, objectives without ``obs_dict`` or unknown, a bad series, ``n_boot`` outside 0..10^4, ``conf_level``
     outside (0, 1), and outputs plus design rows needing more than half of the free device memory.
@@ -120,6 +121,9 @@ def sobol_indices(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, ranges,
     from .model import make_options
 
     n_sc = len(p["SC_list"])
+    phi = [n for n in ranges if str(n).startswith(pk.ERR_PHI)]
+    if phi:
+        raise ValueError("%s: the AR(1) error model is not part of the fit statistics a Sobol' design evaluates" % phi)
     names, targets, bounds = _check_priors(ranges, n_sc, snow_on_device)
     n_base, skip, objectives = _check_request(n_base, skip, objectives, series, obs_dict, n_boot, conf_level)
     topo = pk.build_topology(p_struc, p["SC_list"])
