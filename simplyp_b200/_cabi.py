@@ -424,18 +424,31 @@ def thornthwaite_pet_device(n_days, n_months, t_air_ptr, t_stride, month_start_p
                                                   C.c_void_p(stream_ptr)))
 
 
+def _u64(seed):
+    """A seed as the uint64 the C-ABI takes (Python ints of any sign or size, modulo 2^64)."""
+    return int(seed) & 0xFFFFFFFFFFFFFFFF
+
+
+def _free_params(spec, targets, lo, hi):
+    """``spec`` (SimplypMcmc, SimplypSobol or SimplypDe) with ``n_free`` and ``param`` set to the free parameters
+    ``targets`` [(kind, index, pos)] (``MCMC_MEMBER`` / ``MCMC_SC_ALL`` / ``MCMC_SC_AT`` / ``MCMC_ERROR_MODEL``) and
+    their boxes ``[lo[k], hi[k]]``."""
+    if not 1 <= len(targets) <= MCMC_MAX_FREE:
+        raise ValueError("1..%d free parameters" % MCMC_MAX_FREE)
+    spec.n_free = len(targets)
+    for k, (kind, index, pos) in enumerate(targets):
+        p = spec.param[k]
+        p.kind, p.index, p.pos, p.lo, p.hi = int(kind), int(index), int(pos), float(lo[k]), float(hi[k])
+    return spec
+
+
 def make_mcmc(n_walkers, targets, lo, hi, n_sc, n_obs_series, sc_per_member=False, thin=1, seed=0, stretch=2.0):
     """SimplypMcmc for ``targets`` [(kind, index, pos)] (``MCMC_MEMBER`` / ``MCMC_SC_ALL`` / ``MCMC_SC_AT``) with the
     prior box ``[lo[k], hi[k]]``."""
-    if not 1 <= len(targets) <= MCMC_MAX_FREE:
-        raise ValueError("1..%d free parameters" % MCMC_MAX_FREE)
-    mc = SimplypMcmc()
-    mc.n_walkers, mc.n_free, mc.n_sc, mc.n_obs_series = int(n_walkers), len(targets), int(n_sc), int(n_obs_series)
+    mc = _free_params(SimplypMcmc(), targets, lo, hi)
+    mc.n_walkers, mc.n_sc, mc.n_obs_series = int(n_walkers), int(n_sc), int(n_obs_series)
     mc.sc_per_member, mc.thin = 1 if sc_per_member else 0, int(thin)
-    mc.seed, mc.stretch = int(seed) & 0xFFFFFFFFFFFFFFFF, float(stretch)
-    for k, (kind, index, pos) in enumerate(targets):
-        p = mc.param[k]
-        p.kind, p.index, p.pos, p.lo, p.hi = int(kind), int(index), int(pos), float(lo[k]), float(hi[k])
+    mc.seed, mc.stretch = _u64(seed), float(stretch)
     return mc
 
 
@@ -474,7 +487,7 @@ def predictive_draws_device(dims, out_ptr, member_ptr, sc_ptr, diag_ptr, series_
     lib = require_device()
     _check(lib.simplyp_predictive_draws_device(C.byref(dims), out_ptr, member_ptr, sc_ptr, diag_ptr, series_desc_ptr,
                                                int(n_series), draws_ptr, int(n_members_total), int(member_offset),
-                                               1 if obs_error else 0, int(seed) & 0xFFFFFFFFFFFFFFFF, stream_ptr))
+                                               1 if obs_error else 0, _u64(seed), stream_ptr))
 
 
 def period_aggregates_device(dims, out_ptr, member_ptr, sc_ptr, diag_ptr, series_desc, period_bounds, wb_reaches,
@@ -511,15 +524,10 @@ def nanquantile_device(x_ptr, n_rows, n_cols, q, quant_ptr, mean_ptr, count_ptr,
 
 def make_sobol(targets, lo, hi, n_sc, n_base, skip=0, sc_per_member=False, second_order=False):
     """SimplypSobol for ``targets`` [(kind, index, pos)] (as :func:`make_mcmc`) with the boxes ``[lo[k], hi[k]]``."""
-    if not 1 <= len(targets) <= MCMC_MAX_FREE:
-        raise ValueError("1..%d free parameters" % MCMC_MAX_FREE)
-    sb = SimplypSobol()
-    sb.n_free, sb.n_sc = len(targets), int(n_sc)
+    sb = _free_params(SimplypSobol(), targets, lo, hi)
+    sb.n_sc = int(n_sc)
     sb.sc_per_member, sb.second_order = 1 if sc_per_member else 0, 1 if second_order else 0
     sb.n_base, sb.skip = int(n_base), int(skip)
-    for k, (kind, index, pos) in enumerate(targets):
-        p = sb.param[k]
-        p.kind, p.index, p.pos, p.lo, p.hi = int(kind), int(index), int(pos), float(lo[k]), float(hi[k])
     return sb
 
 
@@ -549,24 +557,19 @@ def sobol_indices_device(sb, y_ptr, n_rows, n_boot, conf_z, seed, S1, ST, S1_con
     """Sobol' indices and bootstrap confidences of every row of Y [n_rows][N P]; asynchronous on ``stream_ptr``."""
     lib = require_device()
     _check(lib.simplyp_sobol_indices_device(C.byref(sb), y_ptr, int(n_rows), int(n_boot), float(conf_z),
-                                            int(seed) & 0xFFFFFFFFFFFFFFFF, S1, ST, S1_conf, ST_conf, S2, S2_conf,
+                                            _u64(seed), S1, ST, S1_conf, ST_conf, S2, S2_conf,
                                             mean, var, n_used, ws_ptr, int(ws_bytes), stream_ptr))
 
 
 def make_de(n_population, targets, lo, hi, n_sc, n_rows, sc_per_member=False, strategy="best1bin",
             mutation=(0.5, 1.0), recombination=0.7, tol=0.01, tol_abs=0.0, seed=0):
     """SimplypDe for ``targets`` [(kind, index, pos)] (as :func:`make_mcmc`) with the boxes ``[lo[k], hi[k]]``."""
-    if not 1 <= len(targets) <= MCMC_MAX_FREE:
-        raise ValueError("1..%d free parameters" % MCMC_MAX_FREE)
-    de = SimplypDe()
-    de.n_population, de.n_free, de.n_sc, de.n_rows = int(n_population), len(targets), int(n_sc), int(n_rows)
+    de = _free_params(SimplypDe(), targets, lo, hi)
+    de.n_population, de.n_sc, de.n_rows = int(n_population), int(n_sc), int(n_rows)
     de.sc_per_member, de.strategy = 1 if sc_per_member else 0, DE_STRATEGIES[strategy]
-    de.seed = int(seed) & 0xFFFFFFFFFFFFFFFF
+    de.seed = _u64(seed)
     de.mutation_lo, de.mutation_hi = float(mutation[0]), float(mutation[1])
     de.recombination, de.tol, de.tol_abs = float(recombination), float(tol), float(tol_abs)
-    for k, (kind, index, pos) in enumerate(targets):
-        p = de.param[k]
-        p.kind, p.index, p.pos, p.lo, p.hi = int(kind), int(index), int(pos), float(lo[k]), float(hi[k])
     return de
 
 

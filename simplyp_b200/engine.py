@@ -20,6 +20,21 @@ def _torch():
     return torch
 
 
+def half_free_bytes(eng):
+    """Half of the free memory of ``eng``'s device: the most the buffers of an ensemble driver may take, and the default
+    workspace budget of :meth:`Engine.calibrate`.  A driver that captures CUDA graphs takes its budget up front, so
+    that nothing queries memory during a capture."""
+    return eng.free_bytes() // 2
+
+
+def check_device_memory(eng, nbytes, what, hint):
+    """``ValueError`` "<what> <GB>, more than half of the free device memory: <hint>" if ``nbytes`` exceed
+    :func:`half_free_bytes`; asks ``eng`` for nothing but ``free_bytes()``, so a driver calls it before any device
+    work."""
+    if nbytes > half_free_bytes(eng):
+        raise ValueError("%s %.1f GB, more than half of the free device memory: %s" % (what, nbytes / 1e9, hint))
+
+
 class Engine:
     """One engine per process / GPU."""
 
@@ -51,15 +66,42 @@ class Engine:
         free, _total = torch.cuda.mem_get_info(self.device)
         return int(free)
 
+    def context(self):
+        """This engine's device as torch's current device."""
+        return _torch().cuda.device(self.device)
+
+    def _call(self, fn, *args):
+        """``fn(*args, stream)`` on this device, ``stream`` being torch's current stream."""
+        with self.context():
+            fn(*args, _torch().cuda.current_stream().cuda_stream)
+
+    def capture(self, step):
+        """``step()``, which only enqueues work, captured into a CUDA graph on this device."""
+        torch = _torch()
+        g = torch.cuda.CUDAGraph()
+        with self.context(), torch.cuda.graph(g):
+            step()
+        return g
+
     @staticmethod
-    def _shapes(forcing, member_params, sc_params):
+    def _sc_sets(sc_params):
+        """SC parameters as [Msc][S][NP_SC]: a [S][NP_SC] matrix is the one set of every member."""
+        return sc_params.unsqueeze(0) if sc_params.dim() == 2 else sc_params
+
+    @classmethod
+    def _shapes(cls, forcing, member_params, sc_params):
         D = forcing.shape[0]
         M = member_params.shape[0]
-        if sc_params.dim() == 2:
-            sc_params = sc_params.unsqueeze(0)
+        sc_params = cls._sc_sets(sc_params)
         Msc, S = sc_params.shape[0], sc_params.shape[1]
         assert forcing.shape[1] == pk.NF and member_params.shape[1] == pk.NP_MEMBER and sc_params.shape[2] == pk.NP_SC
         return D, M, Msc, S, sc_params
+
+    @classmethod
+    def _output_dims(cls, out, sc_params):
+        """(SimplypDims, SC parameter sets) of a full-output chunk ``out`` [M][S][D][25]."""
+        sc_params = cls._sc_sets(sc_params)
+        return _cabi.make_dims(out.shape[0], out.shape[1], out.shape[2], sc_params.shape[0], 0, 0), sc_params
 
     # ------------------------------------------------------------------ full output
     def run(self, forcing, member_params, sc_params, parent_offsets, parent_ids, opt, out=None, diag=None):
@@ -73,10 +115,8 @@ class Engine:
         if diag is None:
             diag = torch.zeros((M, S, pk.NDIAG), dtype=torch.int64, device=self.device)
         ws = self._workspace(_cabi.workspace_bytes(dims, False))
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            _cabi.run_device(dims, opt, forcing.data_ptr(), member_params.data_ptr(), sc_params.data_ptr(),
-                             parent_offsets, parent_ids, out.data_ptr(), diag.data_ptr(), ws.data_ptr(), stream)
+        self._call(_cabi.run_device, dims, opt, forcing.data_ptr(), member_params.data_ptr(), sc_params.data_ptr(),
+                   parent_offsets, parent_ids, out.data_ptr(), diag.data_ptr(), ws.data_ptr())
         return out, diag
 
     # ------------------------------------------------------------------ fused statistics
@@ -111,36 +151,32 @@ class Engine:
         keep_sim = bool(opt.rank_stats) or phi is not None
         per_member = (32 * S * D if S > 1 else 0) + (8 * V * D if keep_sim else 0)
         if per_member > 0:
-            budget = max_workspace_bytes if max_workspace_bytes is not None else self.free_bytes() // 2
+            budget = max_workspace_bytes if max_workspace_bytes is not None else half_free_bytes(self)
             chunk = max(1, min(M, int(budget // per_member)))
         if peer_gather is not None:
             if chunk < M or keep_sim or M != peer_gather.hi - peer_gather.lo:
                 raise _cabi.SimplypError("peer_gather: one launch of this rank's whole shard, without rank statistics "
                                          "or an AR(1) error model")
-            with torch.cuda.device(self.device):
-                stream = torch.cuda.current_stream().cuda_stream
-                dims = _cabi.make_dims(M, S, D, 1 if Msc == 1 else M, V, n_edges)
-                ws = self._workspace(_cabi.workspace_bytes(dims, True, False))
-                desc, gathered = peer_gather.descriptor()
-                _cabi.calibrate_gather_device(dims, opt, forcing.data_ptr(), member_params.data_ptr(),
-                                              sc_params.data_ptr(), parent_offsets, parent_ids, obs.data_ptr(),
-                                              obs_desc.data_ptr(), desc, diag.data_ptr(), ws.data_ptr(), stream)
+            dims = _cabi.make_dims(M, S, D, 1 if Msc == 1 else M, V, n_edges)
+            ws = self._workspace(_cabi.workspace_bytes(dims, True, False))
+            desc, gathered = peer_gather.descriptor()
+            self._call(_cabi.calibrate_gather_device, dims, opt, forcing.data_ptr(), member_params.data_ptr(),
+                       sc_params.data_ptr(), parent_offsets, parent_ids, obs.data_ptr(), obs_desc.data_ptr(), desc,
+                       diag.data_ptr(), ws.data_ptr())
             return gathered, diag
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            for m0 in range(0, M, chunk):
-                m1 = min(M, m0 + chunk)
-                dims = _cabi.make_dims(m1 - m0, S, D, 1 if Msc == 1 else (m1 - m0), V, n_edges)
-                ws = self._workspace(_cabi.workspace_bytes(dims, True, keep_sim))
-                scp = sc_params if Msc == 1 else sc_params[m0:m1]
-                args = (dims, opt, forcing.data_ptr(), member_params[m0:m1].data_ptr(), scp.data_ptr(), parent_offsets,
-                        parent_ids, obs.data_ptr(), obs_desc.data_ptr())
-                tail = (stats[m0:m1].data_ptr(), diag[m0:m1].data_ptr(), ws.data_ptr(), stream)
-                if phi is None:
-                    _cabi.calibrate_device(*args, *tail)
-                else:
-                    ar1 = _cabi.make_ar1(phi[m0:m1].data_ptr(), phi.shape[1], phi_col)
-                    _cabi.calibrate_ar1_device(*args, ar1, *tail)
+        for m0 in range(0, M, chunk):
+            m1 = min(M, m0 + chunk)
+            dims = _cabi.make_dims(m1 - m0, S, D, 1 if Msc == 1 else (m1 - m0), V, n_edges)
+            ws = self._workspace(_cabi.workspace_bytes(dims, True, keep_sim))
+            scp = sc_params if Msc == 1 else sc_params[m0:m1]
+            args = (dims, opt, forcing.data_ptr(), member_params[m0:m1].data_ptr(), scp.data_ptr(), parent_offsets,
+                    parent_ids, obs.data_ptr(), obs_desc.data_ptr())
+            tail = (stats[m0:m1].data_ptr(), diag[m0:m1].data_ptr(), ws.data_ptr())
+            if phi is None:
+                self._call(_cabi.calibrate_device, *args, *tail)
+            else:
+                ar1 = _cabi.make_ar1(phi[m0:m1].data_ptr(), phi.shape[1], phi_col)
+                self._call(_cabi.calibrate_ar1_device, *args, ar1, *tail)
         return stats, diag
 
     # ------------------------------------------------------------------ receiving water body
@@ -152,16 +188,12 @@ class Engine:
         device: ``out`` [M][S][D][25] from :meth:`run`, ``reaches`` = run-order indices of the reaches flagged
         ``In_final_flux? == 1``.  Returns [M][D][11] (columns ``WATERBODY_COLUMNS``); asynchronous."""
         torch = _torch()
-        M, S, D = out.shape[0], out.shape[1], out.shape[2]
-        if sc_params.dim() == 2:
-            sc_params = sc_params.unsqueeze(0)
-        dims = _cabi.make_dims(M, S, D, sc_params.shape[0], 0, 0)
+        dims, sc_params = self._output_dims(out, sc_params)
         r = torch.as_tensor(np.asarray(reaches, dtype=np.int32), device=self.device)
-        wb = torch.empty((M, D, len(self.WATERBODY_COLUMNS)), dtype=torch.float64, device=self.device)
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            _cabi.sum_to_waterbody_device(dims, out.data_ptr(), sc_params.data_ptr(), member_params.data_ptr(),
-                                          r.data_ptr(), int(r.numel()), wb.data_ptr(), stream)
+        wb = torch.empty((out.shape[0], out.shape[2], len(self.WATERBODY_COLUMNS)), dtype=torch.float64,
+                         device=self.device)
+        self._call(_cabi.sum_to_waterbody_device, dims, out.data_ptr(), sc_params.data_ptr(), member_params.data_ptr(),
+                   r.data_ptr(), int(r.numel()), wb.data_ptr())
         return wb
 
     # ------------------------------------------------------------------ posterior predictive bands
@@ -171,16 +203,10 @@ class Engine:
         written into columns ``member_offset .. member_offset + Mc`` of ``draws`` [V][D][M_total] for the series
         ``series_desc`` [V][2] int32 (run-order reach, ``packing.VAR_KINDS`` index), optionally through the
         likelihood's error model (``simplyp_predictive_draws_device``).  Returns ``draws``; asynchronous."""
-        torch = _torch()
-        Mc, S, D = out.shape[0], out.shape[1], out.shape[2]
-        if sc_params.dim() == 2:
-            sc_params = sc_params.unsqueeze(0)
-        dims = _cabi.make_dims(Mc, S, D, sc_params.shape[0], 0, 0)
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            _cabi.predictive_draws_device(dims, out.data_ptr(), member_params.data_ptr(), sc_params.data_ptr(),
-                                          diag.data_ptr(), series_desc.data_ptr(), series_desc.shape[0],
-                                          draws.data_ptr(), draws.shape[2], member_offset, obs_error, seed, stream)
+        dims, sc_params = self._output_dims(out, sc_params)
+        self._call(_cabi.predictive_draws_device, dims, out.data_ptr(), member_params.data_ptr(), sc_params.data_ptr(),
+                   diag.data_ptr(), series_desc.data_ptr(), series_desc.shape[0], draws.data_ptr(), draws.shape[2],
+                   member_offset, obs_error, seed)
         return draws
 
     def period_aggregates(self, out, member_params, sc_params, diag, series_desc, period_bounds, wb_reaches, values,
@@ -191,16 +217,10 @@ class Engine:
         (run-order reach or ``_cabi.PERIOD_WATERBODY``, ``packing.VAR_KINDS`` index, ``_cabi.PERIOD_STATS`` code),
         ``period_bounds`` [P][2] (first and last day) and ``wb_reaches`` (run-order reaches of the water body) are
         host arrays.  Returns ``values``; asynchronous."""
-        torch = _torch()
-        Mc, S, D = out.shape[0], out.shape[1], out.shape[2]
-        if sc_params.dim() == 2:
-            sc_params = sc_params.unsqueeze(0)
-        dims = _cabi.make_dims(Mc, S, D, sc_params.shape[0], 0, 0)
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            _cabi.period_aggregates_device(dims, out.data_ptr(), member_params.data_ptr(), sc_params.data_ptr(),
-                                           diag.data_ptr(), series_desc, period_bounds, wb_reaches, values.data_ptr(),
-                                           values.shape[1], member_offset, stream)
+        dims, sc_params = self._output_dims(out, sc_params)
+        self._call(_cabi.period_aggregates_device, dims, out.data_ptr(), member_params.data_ptr(), sc_params.data_ptr(),
+                   diag.data_ptr(), series_desc, period_bounds, wb_reaches, values.data_ptr(), values.shape[1],
+                   member_offset)
         return values
 
     def nanquantile(self, x, q, quantiles=None, mean=None, count=None):
@@ -219,10 +239,8 @@ class Engine:
             count = torch.empty(R, dtype=torch.int64, device=self.device)
         need = _cabi.nanquantile_workspace_bytes(R, N)
         ws = self._workspace(need) if need > 0 else None
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            _cabi.nanquantile_device(x.data_ptr(), R, N, q, quantiles.data_ptr(), mean.data_ptr(), count.data_ptr(),
-                                     ws.data_ptr() if ws is not None else None, need, stream)
+        self._call(_cabi.nanquantile_device, x.data_ptr(), R, N, q, quantiles.data_ptr(), mean.data_ptr(),
+                   count.data_ptr(), ws.data_ptr() if ws is not None else None, need)
         return quantiles, mean, count
 
     # ------------------------------------------------------------------ Sobol' sensitivity
@@ -230,24 +248,18 @@ class Engine:
         """Write the target columns of design members ``member_offset .. member_offset + n_members`` (default: to
         the end) of ``member_params`` [N P][NP_MEMBER] and ``sc_params`` ([N P] or [1])[S][NP_SC] for the
         :class:`_cabi.SimplypSobol` ``sb`` (``simplyp_sobol_design_device``).  Asynchronous."""
-        torch = _torch()
         if n_members is None:
             n_members = member_params.shape[0] - member_offset
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            _cabi.sobol_design_device(sb, member_offset, n_members, member_params.data_ptr(), sc_params.data_ptr(),
-                                      stream)
+        self._call(_cabi.sobol_design_device, sb, member_offset, n_members, member_params.data_ptr(),
+                   sc_params.data_ptr())
         return member_params, sc_params
 
     def sobol_outputs(self, stats, diag, rows, y):
         """Objective rows ``y`` [R][M] from the fused statistics ``stats`` [M][V][10] and ``diag`` [M][S][4];
         ``rows`` [R][2] int32 on the device = (series, ``packing.STAT_NAMES`` slot, or -1 for the sampler's lp)
         (``simplyp_sobol_outputs_device``).  Asynchronous."""
-        torch = _torch()
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            _cabi.sobol_outputs_device(stats.data_ptr(), diag.data_ptr(), stats.shape[0], stats.shape[1],
-                                       diag.shape[1], rows.data_ptr(), rows.shape[0], y.data_ptr(), stream)
+        self._call(_cabi.sobol_outputs_device, stats.data_ptr(), diag.data_ptr(), stats.shape[0], stats.shape[1],
+                   diag.shape[1], rows.data_ptr(), rows.shape[0], y.data_ptr())
         return y
 
     def sobol_indices(self, sb, y, n_boot, conf_z, seed, out=None):
@@ -270,39 +282,32 @@ class Engine:
 
         def ptr(k):
             return out[k].data_ptr() if k in out else None
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            _cabi.sobol_indices_device(sb, y.data_ptr(), R, n_boot, conf_z, seed, ptr("S1"), ptr("ST"),
-                                       ptr("S1_conf"), ptr("ST_conf"), ptr("S2"), ptr("S2_conf"), ptr("mean"),
-                                       ptr("var"), ptr("n_used"), ws.data_ptr(), need, stream)
+        self._call(_cabi.sobol_indices_device, sb, y.data_ptr(), R, n_boot, conf_z, seed, ptr("S1"), ptr("ST"),
+                   ptr("S1_conf"), ptr("ST_conf"), ptr("S2"), ptr("S2_conf"), ptr("mean"), ptr("var"), ptr("n_used"),
+                   ws.data_ptr(), need)
         return out
 
     # ------------------------------------------------------------------ differential evolution
-    def _de_call(self, fn, *args):
-        torch = _torch()
-        with torch.cuda.device(self.device):
-            fn(*args, torch.cuda.current_stream().cuda_stream)
-
     def de_trial(self, de, state, member_params, sc_params):
         """Trials of the :class:`_cabi.SimplypDe` population ``state`` into its trial buffer and the target columns of
         ``member_params`` [N][NP_MEMBER] / ``sc_params`` ([N] or [1])[S][NP_SC] (``simplyp_de_trial_device``).
         Asynchronous."""
-        self._de_call(_cabi.de_trial_device, de, state, member_params.data_ptr(), sc_params.data_ptr())
+        self._call(_cabi.de_trial_device, de, state, member_params.data_ptr(), sc_params.data_ptr())
 
     def de_select(self, de, state, y, diag):
         """Selection of one generation from the trials' objective rows ``y`` [R][N] (:meth:`sobol_outputs`) and
         ``diag`` [N][S][4] (``simplyp_de_select_device``).  Asynchronous."""
-        self._de_call(_cabi.de_select_device, de, state, y.data_ptr(), diag.data_ptr())
+        self._call(_cabi.de_select_device, de, state, y.data_ptr(), diag.data_ptr())
 
     def de_scale(self, de, unit, out):
         """Parameter values ``out`` [n][K] of unit-cube rows ``unit`` [n][K] (``simplyp_de_scale_device``).
         Asynchronous."""
-        self._de_call(_cabi.de_scale_device, de, unit.data_ptr(), unit.shape[0], out.data_ptr())
+        self._call(_cabi.de_scale_device, de, unit.data_ptr(), unit.shape[0], out.data_ptr())
 
     def de_init(self, de, state, y, diag):
         """Energies, best member and history row 0 from the population's objective rows ``y`` [R][N] and ``diag``
         (``simplyp_de_init_device``).  Asynchronous."""
-        self._de_call(_cabi.de_init_device, de, state, y.data_ptr(), diag.data_ptr())
+        self._call(_cabi.de_init_device, de, state, y.data_ptr(), diag.data_ptr())
 
     # ------------------------------------------------------------------ Thornthwaite PET
     def thornthwaite_pet(self, t_air, month_start, year_is_leap, latitude_deg, out=None, out_stride=1):
@@ -318,8 +323,6 @@ class Engine:
         if out is None:
             out = torch.empty(D, dtype=torch.float64, device=self.device)
             out_stride = 1
-        with torch.cuda.device(self.device):
-            stream = torch.cuda.current_stream().cuda_stream
-            _cabi.thornthwaite_pet_device(D, NM, t.data_ptr(), 1, ms.data_ptr(), lp.data_ptr(), latitude_deg,
-                                          out.data_ptr(), out_stride, stream)
+        self._call(_cabi.thornthwaite_pet_device, D, NM, t.data_ptr(), 1, ms.data_ptr(), lp.data_ptr(), latitude_deg,
+                   out.data_ptr(), out_stride)
         return out

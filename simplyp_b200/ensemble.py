@@ -70,6 +70,34 @@ def pack_members(base_member, base_sc, samples, return_phi=False):
     return np.ascontiguousarray(member), np.ascontiguousarray(sc)
 
 
+@dataclass
+class _ModelInputs:
+    """What :func:`_model_inputs` returns: the host inputs every ensemble driver starts from."""
+    topo: pk.Topology
+    opt: object                 # SimplypOptions
+    member: np.ndarray          # base member vector [NP_MEMBER]
+    sc: np.ndarray              # base SC matrix [S][NP_SC]
+    forcing: np.ndarray         # [D][NF]
+
+
+def _model_inputs(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, step_len=1.0, rtol=None, atol=None,
+                  snow_on_device=False):
+    """The reference's checks of the land use and the erosion windows, the topology, the options (with
+    ``snow_on_device``), the base parameter vectors :func:`pack_members` broadcasts and the forcing matrix (raw
+    precipitation with ``snow_on_device``).  Host work only, on copies of the frames: a driver calls it before any
+    device work."""
+    from .model import make_options
+
+    p_LU, p_SC = p_LU.copy(deep=True), p_SC.copy(deep=True)
+    pk.validate_land_use(p_SC, p["SC_list"])
+    pk.check_erosion_windows(p)
+    topo = pk.build_topology(p_struc, p["SC_list"])
+    opt = make_options(p_SU, p, dynamic_options, topo, step_len, rtol, atol)
+    opt.snow_on_device = 1 if snow_on_device else 0
+    return _ModelInputs(topo, opt, pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, topo.sc_ids),
+                        pk.forcing_matrix(met_df, raw_snow=bool(snow_on_device)))
+
+
 def apply_member_to_pandas(samples, i, p, p_LU, p_SC):
     """Copies of the reference's pandas objects with member ``i``'s sampled values written in — this is how
     the oracle / the reference is run on the same member."""
@@ -302,24 +330,18 @@ def calibrate_ensemble(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, ob
     import torch.distributed as dist
 
     from .engine import Engine
-    from .model import make_options
 
-    p_LU, p_SC = p_LU.copy(deep=True), p_SC.copy(deep=True)
-    pk.validate_land_use(p_SC, p["SC_list"])
-    pk.check_erosion_windows(p)
-    topo = pk.build_topology(p_struc, p["SC_list"])
-    opt = make_options(p_SU, p, dynamic_options, topo, step_len, rtol, atol)
-    opt.snow_on_device = 1 if snow_on_device else 0
+    inp = _model_inputs(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, step_len, rtol, atol, snow_on_device)
+    topo, opt = inp.topo, inp.opt
     opt.rank_stats = 1 if rank_stats else 0
-    member, sc, phi = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, topo.sc_ids), samples,
-                                   return_phi=True)
+    member, sc, phi = pack_members(inp.member, inp.sc, samples, return_phi=True)
     M = member.shape[0]
     rank, world = (dist.get_rank(), dist.get_world_size()) if (dist.is_available() and dist.is_initialized()) else (0, 1)
     lo, hi = shard_bounds(M, world, rank)
     obs, desc, labels = pk.obs_arrays(obs_dict, topo, met_df.index, variables)
     phi_col = pk.ar1_columns(list(phi), labels, variables)
     eng = engine or Engine()
-    d_forc = eng.to_device(pk.forcing_matrix(met_df, raw_snow=bool(snow_on_device)))
+    d_forc = eng.to_device(inp.forcing)
     d_mem = eng.to_device(member[lo:hi])
     d_sc = eng.to_device(sc if sc.shape[0] == 1 else sc[lo:hi])
     d_obs = eng.to_device(obs)
@@ -359,14 +381,10 @@ def run_ensemble_to_dir(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, s
     import torch.distributed as dist
 
     from .engine import Engine
-    from .model import make_options
 
-    p_LU, p_SC = p_LU.copy(deep=True), p_SC.copy(deep=True)
-    pk.validate_land_use(p_SC, p["SC_list"])
-    pk.check_erosion_windows(p)
-    topo = pk.build_topology(p_struc, p["SC_list"])
-    opt = make_options(p_SU, p, dynamic_options, topo, step_len, rtol, atol)
-    member, sc = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, topo.sc_ids), samples)
+    inp = _model_inputs(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, step_len, rtol, atol)
+    topo, opt = inp.topo, inp.opt
+    member, sc = pack_members(inp.member, inp.sc, samples)
     M, S, D = member.shape[0], len(topo.sc_ids), len(met_df)
     cols = list(pk.RAW_COLS) if columns is None else list(columns)
     col_idx = [pk.RAW_COLS.index(c) for c in cols]
@@ -391,7 +409,7 @@ def run_ensemble_to_dir(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, s
     if members_per_chunk is None:
         members_per_chunk = max(1, (1 << 30) // max(row_bytes, 1))
     chunk = int(max(1, min(members_per_chunk, hi - lo))) if hi > lo else 1
-    d_forc = eng.to_device(pk.forcing_matrix(met_df))
+    d_forc = eng.to_device(inp.forcing)
     d_mem = eng.to_device(member[lo:hi]) if hi > lo else None
     d_sc = eng.to_device(sc if sc.shape[0] == 1 else sc[lo:hi]) if hi > lo else None
     dev_buf = [torch.empty((chunk, S, D, pk.NOUT), dtype=torch.float64, device=eng.device) for _ in range(2)]
@@ -526,31 +544,27 @@ def _band_series(series, topo):
     return np.asarray(desc, dtype=np.int32).reshape(-1, 2), [(int(s), v) for s, v in series]
 
 
-def _integrate_in_chunks(eng, met_df, topo, opt, member, sc, members_per_chunk, snow_on_device, consume):
-    """Integrate the members of ``member`` / ``sc`` (``pack_members``) in full-output chunks of ``members_per_chunk``
-    (default: about 1 GiB of output a chunk) into one reused device buffer, and after each chunk enqueue
-    ``consume(out [n][S][D][25], member rows [n], sc rows [1 or n], diag rows [n], first member)``, which reads the
-    chunk's output in place before the next chunk overwrites it.  Returns the per-member diagnostics [M][S][4] on the
-    device; asynchronous."""
+def _integrate_in_chunks(eng, d_forc, d_mem, d_sc, topo, opt, members_per_chunk, consume):
+    """Integrate the member rows ``d_mem`` [M][NP_MEMBER] / ``d_sc`` [1 or M][S][NP_SC] with the forcing ``d_forc``
+    (all on the device) in full-output chunks of ``members_per_chunk`` (default: about 1 GiB of output a chunk) into
+    one reused device buffer, and after each chunk enqueue ``consume(out [n][S][D][25], member rows [n], sc rows
+    [1 or n], diag rows [n], first member)``, which reads the chunk's output in place before the next chunk overwrites
+    it.  Returns the per-member diagnostics [M][S][4] on the device; asynchronous."""
     import torch
 
-    M, S, D = member.shape[0], topo.n_sc, len(met_df)
+    M, S, D = d_mem.shape[0], topo.n_sc, d_forc.shape[0]
     row_bytes = S * D * pk.NOUT * 8
     if members_per_chunk is None:
         members_per_chunk = max(1, (1 << 30) // max(row_bytes, 1))
     chunk = int(max(1, min(int(members_per_chunk), M)))
-    dev = eng.device
-    d_forc = eng.to_device(pk.forcing_matrix(met_df, raw_snow=bool(snow_on_device)))
-    d_mem, d_sc = eng.to_device(member), eng.to_device(sc)
-    out = torch.empty((chunk, S, D, pk.NOUT), dtype=torch.float64, device=dev)
-    diag = torch.zeros((M, S, pk.NDIAG), dtype=torch.int64, device=dev)
-    with torch.cuda.device(dev):
-        for m0 in range(0, M, chunk):
-            n = min(chunk, M - m0)
-            scp = d_sc if d_sc.shape[0] == 1 else d_sc[m0:m0 + n]
-            eng.run(d_forc, d_mem[m0:m0 + n], scp, topo.parent_offsets, topo.parent_ids, opt, out=out[:n],
-                    diag=diag[m0:m0 + n])
-            consume(out[:n], d_mem[m0:m0 + n], scp, diag[m0:m0 + n], m0)
+    out = torch.empty((chunk, S, D, pk.NOUT), dtype=torch.float64, device=eng.device)
+    diag = torch.zeros((M, S, pk.NDIAG), dtype=torch.int64, device=eng.device)
+    for m0 in range(0, M, chunk):
+        n = min(chunk, M - m0)
+        scp = d_sc if d_sc.shape[0] == 1 else d_sc[m0:m0 + n]
+        eng.run(d_forc, d_mem[m0:m0 + n], scp, topo.parent_offsets, topo.parent_ids, opt, out=out[:n],
+                diag=diag[m0:m0 + n])
+        consume(out[:n], d_mem[m0:m0 + n], scp, diag[m0:m0 + n], m0)
     return diag
 
 
@@ -582,31 +596,23 @@ def predictive_bands(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, samp
     """
     import torch
 
-    from .engine import Engine
-    from .model import make_options
+    from .engine import Engine, check_device_memory
 
     q = _check_band_quantiles(quantiles)
-    topo = pk.build_topology(p_struc, p["SC_list"])
-    desc, labels = _band_series(series, topo)
-    p_LU, p_SC = p_LU.copy(deep=True), p_SC.copy(deep=True)
-    pk.validate_land_use(p_SC, p["SC_list"])
-    pk.check_erosion_windows(p)
-    opt = make_options(p_SU, p, dynamic_options, topo, step_len, rtol, atol)
-    opt.snow_on_device = 1 if snow_on_device else 0
-    member, sc = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, topo.sc_ids), samples)
+    inp = _model_inputs(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, step_len, rtol, atol, snow_on_device)
+    desc, labels = _band_series(series, inp.topo)
+    member, sc = pack_members(inp.member, inp.sc, samples)
     M, D, V = member.shape[0], len(met_df), desc.shape[0]
     eng = engine or Engine()
-    draw_bytes = 8 * V * D * M
-    if draw_bytes > eng.free_bytes() // 2:
-        raise ValueError("the draws need %.1f GB, more than half of the free device memory: thin the samples "
-                         "(e.g. flat_samples(burn, thin=n))" % (draw_bytes / 1e9))
+    check_device_memory(eng, 8 * V * D * M, "the draws need", "thin the samples (e.g. flat_samples(burn, thin=n))")
     dev = eng.device
     d_desc = eng.to_device(desc)
     draws = torch.empty((V, D, M), dtype=torch.float64, device=dev)
 
     def draw(out, d_mem, scp, diag, m0):
         eng.predictive_draws(out, d_mem, scp, diag, d_desc, draws, m0, obs_error, seed)
-    diag = _integrate_in_chunks(eng, met_df, topo, opt, member, sc, members_per_chunk, snow_on_device, draw)
+    diag = _integrate_in_chunks(eng, eng.to_device(inp.forcing), eng.to_device(member), eng.to_device(sc), inp.topo,
+                                inp.opt, members_per_chunk, draw)
     with torch.cuda.device(dev):
         quant, mean, count = eng.nanquantile(draws.view(V * D, M), q)
     torch.cuda.synchronize(dev)
@@ -816,33 +822,26 @@ def period_statistics(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, sam
     import torch
 
     from . import _cabi
-    from .engine import Engine
-    from .model import make_options
+    from .engine import Engine, check_device_memory
 
     q = _check_band_quantiles(quantiles)
-    topo = pk.build_topology(p_struc, p["SC_list"])
-    desc, labels, wb = _period_series(series, topo, p_struc)
+    inp = _model_inputs(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, step_len, rtol, atol, snow_on_device)
+    desc, labels, wb = _period_series(series, inp.topo, p_struc)
     bounds, names = period_bounds(met_df.index, periods)
     if bounds.shape[0] > _cabi.PERIOD_MAX_PERIODS:
         raise ValueError("at most %d periods, got %d" % (_cabi.PERIOD_MAX_PERIODS, bounds.shape[0]))
-    p_LU, p_SC = p_LU.copy(deep=True), p_SC.copy(deep=True)
-    pk.validate_land_use(p_SC, p["SC_list"])
-    pk.check_erosion_windows(p)
-    opt = make_options(p_SU, p, dynamic_options, topo, step_len, rtol, atol)
-    opt.snow_on_device = 1 if snow_on_device else 0
-    member, sc = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, topo.sc_ids), samples)
+    member, sc = pack_members(inp.member, inp.sc, samples)
     M, R = member.shape[0], desc.shape[0] * bounds.shape[0]
     eng = engine or Engine()
-    value_bytes = 8 * R * M
-    if value_bytes > eng.free_bytes() // 2:
-        raise ValueError("the values need %.1f GB, more than half of the free device memory: thin the samples "
-                         "(e.g. flat_samples(burn, thin=n)) or ask for fewer series or periods" % (value_bytes / 1e9))
+    check_device_memory(eng, 8 * R * M, "the values need", "thin the samples (e.g. flat_samples(burn, thin=n)) or ask "
+                        "for fewer series or periods")
     dev = eng.device
     values = torch.empty((R, M), dtype=torch.float64, device=dev)
 
     def aggregate(out, d_mem, scp, diag, m0):
         eng.period_aggregates(out, d_mem, scp, diag, desc, bounds, wb, values, m0)
-    diag = _integrate_in_chunks(eng, met_df, topo, opt, member, sc, members_per_chunk, snow_on_device, aggregate)
+    diag = _integrate_in_chunks(eng, eng.to_device(inp.forcing), eng.to_device(member), eng.to_device(sc), inp.topo,
+                                inp.opt, members_per_chunk, aggregate)
     with torch.cuda.device(dev):
         quant, mean, count = eng.nanquantile(values, q)
     torch.cuda.synchronize(dev)

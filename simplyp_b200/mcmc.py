@@ -116,8 +116,7 @@ class _Sampler:
     def __init__(self, met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, obs_dict, priors, n_walkers, n_steps, *,
                  variables=("Q", "TDP"), seed=DEFAULT_SEED, initial=None, start_iteration=0, thin=1, stretch=2.0,
                  step_len=1.0, rtol=None, atol=None, snow_on_device=False, engine=None):
-        from .ensemble import latin_hypercube, pack_members
-        from .model import make_options
+        from .ensemble import _model_inputs, latin_hypercube, pack_members
 
         # ---- host-side validation, before any device work
         n_sc = len(p["SC_list"])
@@ -145,14 +144,10 @@ class _Sampler:
             raise ValueError("initial walkers must have shape (%d, %d), got %s" % (W, K, x0.shape))
         if not np.all((x0 >= self.bounds[:, 0]) & (x0 <= self.bounds[:, 1])):
             raise ValueError("initial walkers must lie inside the prior box")
-        p_LU, p_SC = p_LU.copy(deep=True), p_SC.copy(deep=True)
-        pk.validate_land_use(p_SC, p["SC_list"])
-        pk.check_erosion_windows(p)
-        self.topo = pk.build_topology(p_struc, p["SC_list"])
-        self.opt = make_options(p_SU, p, dynamic_options, self.topo, step_len, rtol, atol)
-        self.opt.snow_on_device = 1 if snow_on_device else 0
-        member, sc = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, self.topo.sc_ids),
-                                  {n: x0[:, k] for k, n in enumerate(self.names)})
+        inp = _model_inputs(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, step_len, rtol, atol,
+                            snow_on_device)
+        self.topo, self.opt = inp.topo, inp.opt
+        member, sc = pack_members(inp.member, inp.sc, {n: x0[:, k] for k, n in enumerate(self.names)})
         obs, desc, self.labels = pk.obs_arrays(obs_dict, self.topo, met_df.index, variables)
         # the AR(1) phi of series v is column phi_col[v] of the walkers (initial evaluation) and of the proposals
         col = pk.ar1_columns(self.names, self.labels, variables)
@@ -163,15 +158,13 @@ class _Sampler:
 
         # ---- device state
         import torch
-        from .engine import Engine
+        from .engine import Engine, check_device_memory, half_free_bytes
 
         self.eng = eng = engine or Engine()
-        chain_bytes = 8 * self.n_saved * W * (K + 1)
-        if chain_bytes > eng.free_bytes() // 2:
-            raise ValueError("the chain needs %.1f GB, more than half of the free device memory: store every n-th "
-                             "iteration with thin=n" % (chain_bytes / 1e9))
+        check_device_memory(eng, 8 * self.n_saved * W * (K + 1), "the chain needs",
+                            "store every n-th iteration with thin=n")
         dev, f64, i64 = eng.device, torch.float64, torch.int64
-        self.d_forc = eng.to_device(pk.forcing_matrix(met_df, raw_snow=bool(snow_on_device)))
+        self.d_forc = eng.to_device(inp.forcing)
         self.d_mem, self.d_sc = eng.to_device(member), eng.to_device(sc)
         self.d_obs, self.d_desc = eng.to_device(obs), eng.to_device(desc)
         self.stats = torch.zeros((W, self.V, pk.NSTAT), dtype=f64, device=dev)
@@ -185,17 +178,13 @@ class _Sampler:
         self.accepted = torch.zeros(W, dtype=i64, device=dev)
         self.chain = torch.zeros((self.n_saved, W, K), dtype=f64, device=dev)
         self.chain_lp = torch.zeros((self.n_saved, W), dtype=f64, device=dev)
-        self.ws_budget = eng.free_bytes() // 2 if self.phi_col is not None else None
+        self.ws_budget = half_free_bytes(eng) if self.phi_col is not None else None
         self.mc = _cabi.make_mcmc(W, targets, self.bounds[:, 0], self.bounds[:, 1], n_sc, self.V,
                                   sc_per_member=sc.shape[0] > 1, thin=self.thin, seed=seed, stretch=stretch)
         self.state = _cabi.make_mcmc_state(
             self.walkers.data_ptr(), self.lp.data_ptr(), self.proposals.data_ptr(), self.log_z.data_ptr(),
             self.out_of_box.data_ptr(), self.iteration.data_ptr(), self.accepted.data_ptr(), self.chain.data_ptr(),
             self.chain_lp.data_ptr(), self.n_saved, self.start // self.thin)
-
-    def _stream(self):
-        import torch
-        return torch.cuda.current_stream(self.eng.device).cuda_stream
 
     def _rows(self, lo, hi):
         return self.d_mem[lo:hi], (self.d_sc if self.d_sc.shape[0] == 1 else self.d_sc[lo:hi])
@@ -207,16 +196,14 @@ class _Sampler:
             self.diag.zero_()
             self.eng.calibrate(self.d_forc, mem, sc, self.topo.parent_offsets, self.topo.parent_ids, self.d_obs,
                                self.d_desc, self.opt, stats=self.stats, diag=self.diag, **self._phi(self.walkers))
-            _cabi.mcmc_init_device(self.mc, self.state, self.stats.data_ptr(), self.diag.data_ptr(), self._stream())
+            self.eng._call(_cabi.mcmc_init_device, self.mc, self.state, self.stats.data_ptr(), self.diag.data_ptr())
         lp = self.lp.cpu().numpy()
         bad = np.flatnonzero(~np.isfinite(lp))
         if bad.size:
             raise ValueError("the log-probability of initial walker %d is not finite" % bad[0])
 
     def propose(self, half):
-        with self._device():
-            _cabi.mcmc_propose_device(self.mc, self.state, half, self.d_mem.data_ptr(), self.d_sc.data_ptr(),
-                                      self._stream())
+        self.eng._call(_cabi.mcmc_propose_device, self.mc, self.state, half, self.d_mem.data_ptr(), self.d_sc.data_ptr())
 
     def evaluate(self, half):
         lo, hi = half * self.H, (half + 1) * self.H
@@ -234,9 +221,8 @@ class _Sampler:
 
     def accept(self, half):
         lo = half * self.H
-        with self._device():
-            _cabi.mcmc_accept_device(self.mc, self.state, half, self.stats[lo].data_ptr(), self.diag[lo].data_ptr(),
-                                     self._stream())
+        self.eng._call(_cabi.mcmc_accept_device, self.mc, self.state, half, self.stats[lo].data_ptr(),
+                       self.diag[lo].data_ptr())
 
     def iteration_step(self):
         """Enqueue one iteration: propose, evaluate, accept for half 0, then for half 1."""
@@ -246,17 +232,11 @@ class _Sampler:
             self.accept(half)
 
     def _device(self):
-        import torch
-        return torch.cuda.device(self.eng.device)
+        return self.eng.context()
 
     def capture(self):
         """One iteration captured into a CUDA graph (the iteration counter lives on the device)."""
-        import torch
-        g = torch.cuda.CUDAGraph()
-        with self._device():
-            with torch.cuda.graph(g):
-                self.iteration_step()
-        return g
+        return self.eng.capture(self.iteration_step)
 
     def run(self):
         """The first iteration directly (it also loads every kernel), the others as replays of a captured one."""

@@ -126,9 +126,8 @@ class _Optimizer:
                  max_generations, *, objective="lp", variables=("Q", "TDP"), strategy="best1bin", mutation=(0.5, 1.0),
                  recombination=0.7, tol=0.01, tol_abs=0.0, seed=DEFAULT_DE_SEED, initial=None, start_generation=0,
                  check_every=10, step_len=1.0, rtol=None, atol=None, snow_on_device=False, engine=None):
-        from .ensemble import pack_members
+        from .ensemble import _model_inputs, pack_members
         from .mcmc import _check_priors
-        from .model import make_options
 
         # ---- host-side validation, before any device work
         n_sc = len(p["SC_list"])
@@ -149,8 +148,10 @@ class _Optimizer:
         for name, v in (("tol", tol), ("tol_abs", tol_abs)):
             if not (np.isfinite(float(v)) and float(v) >= 0.0):
                 raise ValueError("%s must be finite and >= 0, got %r" % (name, v))
-        topo = pk.build_topology(p_struc, p["SC_list"])
-        obs, desc, obs_labels = pk.obs_arrays(obs_dict, topo, met_df.index, variables)
+        inp = _model_inputs(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, step_len, rtol, atol,
+                            snow_on_device)
+        self.topo, self.opt = inp.topo, inp.opt
+        obs, desc, obs_labels = pk.obs_arrays(obs_dict, self.topo, met_df.index, variables)
         rows, self.labels, self.weights = _objective_weights(objective, obs_labels)
         col = pk.ar1_columns(self.names, obs_labels, variables)
         self.phi_col = col if any(c >= 0 for c in col) else None
@@ -173,13 +174,7 @@ class _Optimizer:
         u0 = np.ascontiguousarray(u0, dtype=np.float64)
         if u0.shape != (N, K):
             raise ValueError("initial population must have shape (%d, %d), got %s" % (N, K, u0.shape))
-        p_LU, p_SC = p_LU.copy(deep=True), p_SC.copy(deep=True)
-        pk.validate_land_use(p_SC, p["SC_list"])
-        pk.check_erosion_windows(p)
-        self.topo = topo
-        self.opt = make_options(p_SU, p, dynamic_options, topo, step_len, rtol, atol)
-        self.opt.snow_on_device = 1 if snow_on_device else 0
-        member, sc = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, topo.sc_ids),
+        member, sc = pack_members(inp.member, inp.sc,
                                   {n: scale(u0, self.bounds)[:, k] for k, n in enumerate(self.names)})
         self.N, self.K, self.V, self.S, self.R = N, K, obs.shape[0], n_sc, rows.shape[0]
         self.max_generations, self.start = int(max_generations), int(start_generation)
@@ -187,16 +182,14 @@ class _Optimizer:
 
         # ---- device state
         import torch
-        from .engine import Engine
+        from .engine import Engine, check_device_memory, half_free_bytes
 
         self.eng = eng = engine or Engine()
         need = 8 * N * (self.V * pk.NSTAT + n_sc * pk.NDIAG + pk.NP_MEMBER + (sc.shape[0] > 1) * n_sc * pk.NP_SC
                         + 2 * K + self.R + 2) + 32 * (self.max_generations + 1)
-        if need > eng.free_bytes() // 2:
-            raise ValueError("the population needs %.1f GB, more than half of the free device memory: use a smaller "
-                             "n_population" % (need / 1e9))
+        check_device_memory(eng, need, "the population needs", "use a smaller n_population")
         dev, f64, i64 = eng.device, torch.float64, torch.int64
-        self.d_forc = eng.to_device(pk.forcing_matrix(met_df, raw_snow=bool(snow_on_device)))
+        self.d_forc = eng.to_device(inp.forcing)
         self.d_mem, self.d_sc = eng.to_device(member), eng.to_device(sc)
         self.d_obs, self.d_desc = eng.to_device(obs), eng.to_device(desc)
         self.d_rows, self.d_weights = eng.to_device(rows), eng.to_device(self.weights)
@@ -205,7 +198,7 @@ class _Optimizer:
         self.y = torch.zeros((self.R, N), dtype=f64, device=dev)
         # parameter values of the rows being evaluated: where the AR(1) phi, which no member row holds, is read
         self.values = torch.zeros((N, K), dtype=f64, device=dev) if self.phi_col is not None else None
-        self.ws_budget = eng.free_bytes() // 2 if self.phi_col is not None else None
+        self.ws_budget = half_free_bytes(eng) if self.phi_col is not None else None
         self.population = eng.to_device(u0)
         self.energy = torch.zeros(N, dtype=f64, device=dev)
         self.trial = torch.zeros((N, K), dtype=f64, device=dev)
@@ -222,8 +215,7 @@ class _Optimizer:
                                          self.history.data_ptr(), self.max_generations + 1, self.start)
 
     def _device(self):
-        import torch
-        return torch.cuda.device(self.eng.device)
+        return self.eng.context()
 
     def evaluate(self, unit=None):
         """Zero the status words, integrate all N rows with the fused statistics, take the objective rows.  ``unit``:
@@ -258,12 +250,7 @@ class _Optimizer:
 
     def capture(self):
         """One generation captured into a CUDA graph (the generation counter lives on the device)."""
-        import torch
-        g = torch.cuda.CUDAGraph()
-        with self._device():
-            with torch.cuda.graph(g):
-                self.generation_step()
-        return g
+        return self.eng.capture(self.generation_step)
 
     def converged(self):
         return bool(self.counters[2].item())

@@ -116,9 +116,8 @@ def sobol_indices(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, ranges,
     ``series``, objectives without ``obs_dict`` or unknown, a bad series, ``n_boot`` outside 0..10^4, ``conf_level``
     outside (0, 1), and outputs plus design rows needing more than half of the free device memory.
     """
-    from .ensemble import _band_series, pack_members
+    from .ensemble import _band_series, _integrate_in_chunks, _model_inputs, _n_failed, pack_members
     from .mcmc import _check_priors
-    from .model import make_options
 
     n_sc = len(p["SC_list"])
     phi = [n for n in ranges if str(n).startswith(pk.ERR_PHI)]
@@ -126,7 +125,8 @@ def sobol_indices(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, ranges,
         raise ValueError("%s: the AR(1) error model is not part of the fit statistics a Sobol' design evaluates" % phi)
     names, targets, bounds = _check_priors(ranges, n_sc, snow_on_device)
     n_base, skip, objectives = _check_request(n_base, skip, objectives, series, obs_dict, n_boot, conf_level)
-    topo = pk.build_topology(p_struc, p["SC_list"])
+    inp = _model_inputs(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, step_len, rtol, atol, snow_on_device)
+    topo, opt = inp.topo, inp.opt
     K, S, D = len(names), topo.n_sc, len(met_df)
     P = 2 * K + 2 if second_order else K + 2
     M = n_base * P
@@ -139,32 +139,25 @@ def sobol_indices(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, ranges,
         V = obs.shape[0]
         rows, labels = objective_rows(obs_labels, objectives)
     R = len(labels)
-    p_LU, p_SC = p_LU.copy(deep=True), p_SC.copy(deep=True)
-    pk.validate_land_use(p_SC, p["SC_list"])
-    pk.check_erosion_windows(p)
-    opt = make_options(p_SU, p, dynamic_options, topo, step_len, rtol, atol)
-    opt.snow_on_device = 1 if snow_on_device else 0
     z = statistics.NormalDist().inv_cdf(0.5 + float(conf_level) / 2.0)
 
     import torch
 
-    from .engine import Engine
+    from .engine import Engine, check_device_memory
 
     eng = engine or Engine()
     sc_per_member = any(t[0] != _cabi.MCMC_MEMBER for t in targets)
     design_bytes = 8 * M * (pk.NP_MEMBER + (S * pk.NP_SC if sc_per_member else 0))
-    need = 8 * R * M + design_bytes
-    if need > eng.free_bytes() // 2:
-        raise ValueError("the outputs and the design need %.1f GB, more than half of the free device memory: use a "
-                         "smaller n_base or fewer rows" % (need / 1e9))
-    base_m, base_sc = pack_members(pk.member_vector(p, p_LU), pk.sc_matrix(p_SC, topo.sc_ids), {})
+    check_device_memory(eng, 8 * R * M + design_bytes, "the outputs and the design need",
+                        "use a smaller n_base or fewer rows")
+    base_m, base_sc = pack_members(inp.member, inp.sc, {})
     dev = eng.device
     d_mem = eng.to_device(base_m).expand(M, pk.NP_MEMBER).contiguous()
     d_sc = eng.to_device(base_sc)
     if sc_per_member:
         d_sc = d_sc.expand(M, S, pk.NP_SC).contiguous()
     sb = _cabi.make_sobol(targets, bounds[:, 0], bounds[:, 1], S, n_base, skip, sc_per_member, second_order)
-    d_forc = eng.to_device(pk.forcing_matrix(met_df, raw_snow=bool(snow_on_device)))
+    d_forc = eng.to_device(inp.forcing)
     y = torch.empty((R, M), dtype=torch.float64, device=dev)
     with torch.cuda.device(dev):
         eng.sobol_design(sb, d_mem, d_sc)
@@ -174,24 +167,15 @@ def sobol_indices(met_df, p_struc, p_SU, p_LU, p_SC, p, dynamic_options, ranges,
             eng.sobol_outputs(stats, diag, d_rows, y)
             del stats
         else:
-            d_desc = eng.to_device(desc)
-            row_bytes = S * D * pk.NOUT * 8
-            if members_per_chunk is None:
-                members_per_chunk = max(1, (1 << 30) // max(row_bytes, 1))
-            chunk = int(max(1, min(int(members_per_chunk), M)))
-            out = torch.empty((chunk, S, D, pk.NOUT), dtype=torch.float64, device=dev)
-            diag = torch.zeros((M, S, pk.NDIAG), dtype=torch.int64, device=dev)
-            for m0 in range(0, M, chunk):
-                n = min(chunk, M - m0)
-                scp = d_sc if d_sc.shape[0] == 1 else d_sc[m0:m0 + n]
-                eng.run(d_forc, d_mem[m0:m0 + n], scp, topo.parent_offsets, topo.parent_ids, opt, out=out[:n],
-                        diag=diag[m0:m0 + n])
-                eng.predictive_draws(out[:n], d_mem[m0:m0 + n], scp, diag[m0:m0 + n], d_desc, y.view(V, D, M), m0)
-            del out
+            d_desc, draws = eng.to_device(desc), y.view(V, D, M)
+
+            def draw(out, mem, scp, diag, m0):
+                eng.predictive_draws(out, mem, scp, diag, d_desc, draws, m0)
+            diag = _integrate_in_chunks(eng, d_forc, d_mem, d_sc, topo, opt, members_per_chunk, draw)
         del d_mem, d_sc
         res = eng.sobol_indices(sb, y, int(n_boot), z, seed)
     torch.cuda.synchronize(dev)
-    n_failed = int(np.any(diag.cpu().numpy()[:, :, 3] != 0, axis=1).sum())
+    n_failed = _n_failed(diag)
     host = {k: v.cpu().numpy() for k, v in res.items()}
     return SobolResult(names=list(names), bounds=bounds, labels=labels, S1=host["S1"], ST=host["ST"],
                        S1_conf=host["S1_conf"], ST_conf=host["ST_conf"], S2=host.get("S2"),
