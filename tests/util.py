@@ -16,6 +16,17 @@ def max_rel(a, b):
     return float(np.nanmax(out)) if out.size else 0.0
 
 
+def max_rel_floored(a, b, floor):
+    """max |a-b| / (|b| + floor): the relative error where |b| >> floor, the absolute error in units of the floor
+    where |b| << floor (``floor`` broadcasts against ``b``, e.g. one value per day).  With floor = atol/rtol it is the
+    error in units of an integrator's error weight atol + rtol |b|, over rtol."""
+    a = np.asarray(a, dtype=float)
+    b = np.asarray(b, dtype=float)
+    if not b.size:
+        return 0.0
+    return float(np.max(np.abs(a - b) / (np.abs(b) + floor)))     # a NaN in ``a`` is returned, not skipped
+
+
 def max_mixed(a, b, rtol, atol_frac=1e-6):
     """max |a-b| / (rtol*|b| + rtol*atol_frac*max|b|): <= 1 means within a mixed abs/rel tolerance.
 
