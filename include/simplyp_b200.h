@@ -558,6 +558,74 @@ int simplyp_de_init_device(const SimplypDe* de, const SimplypDeState* state, con
  * how the error-model targets (SIMPLYP_MCMC_ERROR_MODEL), which no row holds, reach simplyp_calibrate_ar1_device. */
 int simplyp_de_scale_device(const SimplypDe* de, const double* unit, int64_t n, double* out, void* stream);
 
+/* ---- NSGA-II ------------------------------------------------------------------------------------------------------
+ * Deb et al.'s (2002) NSGA-II over M fit statistics (the reference C code v1.1.6): the Pareto front of K free
+ * parameters (the sampler's targets and boxes, SimplypMcmcParam) in a population of N members living in the unit cube.
+ * Member rows get the lo/hi-clamped values of simplyp_de_scale_device.  Objectives are oriented f = sense * y, larger
+ * is better; a member is infeasible when a status word of its integration is set or one of its M objectives is not a
+ * finite number, and then holds NaN in every objective.  One generation is:
+ *   simplyp_nsga2_offspring_device -> N/2 pairs: two binary tournaments, SBX, polynomial mutation; offspring[N][K] and
+ *                                     the target columns of member_params (and sc_params) rows 0..N-1;
+ *   zero diag, simplyp_calibrate_device on the N offspring rows, simplyp_sobol_outputs_device -> y[M][N];
+ *   simplyp_nsga2_survive_device   -> over the 2N points (parents 0..N-1, offspring N..2N-1): non-dominated ranks
+ *                                     (infeasible points form the last rank; ranking stops once >= N points are
+ *                                     ranked), crowding distances within each front, the N survivors in the order
+ *                                     (rank asc, crowding desc, index asc) kept in ascending index; history row
+ *                                     g + 1 - history_base = (first-front size among the survivors, fronts ranked,
+ *                                     best y of each objective over the feasible survivors); n_failed += infeasible
+ *                                     offspring; generation g += 1.
+ * simplyp_nsga2_init_device: objectives, ranks, crowding, history row 0 and n_failed of the population from its own
+ *   evaluation (the caller wrote its rows); the generation counter is left alone.
+ * Selection: each parent of a pair is the better of two distinct members drawn uniformly (lower rank, then larger
+ * crowding, then lower index).  Random words: Philox4x32-10 keyed by the seed, pair p at generation g takes group q of
+ * four words from counter (p, g lo, g hi, 5 + 256 q); the word assignment is documented in csrc/simplyp_nsga2.cuh.
+ * Ranking runs as one cooperative launch (cudaLaunchCooperativeKernel) with a grid barrier between fronts, so the
+ * number of fronts never changes the enqueued work.  The survival needs simplyp_nsga2_workspace_bytes(ns) bytes of
+ * device workspace.  All three only enqueue work on `stream` (no allocation, no synchronisation), so they can be
+ * captured into a graph. */
+#define SIMPLYP_NSGA2_MAX_OBJECTIVES 16
+
+typedef struct {
+  int32_t n_population;     /* N: even, 4..2^29 */
+  int32_t n_free;           /* K: 1..SIMPLYP_MCMC_MAX_FREE */
+  int32_t n_objectives;     /* M: 2..SIMPLYP_NSGA2_MAX_OBJECTIVES */
+  int32_t n_sc;             /* S of the calibration runs */
+  int32_t sc_per_member;    /* sc_params is [N][S][NP_SC] (required by the SC targets) */
+  int32_t reserved;
+  uint64_t seed;            /* Philox key: (low word, high word) */
+  double  crossover;        /* SBX probability of a pair, [0, 1] */
+  double  mutation;         /* polynomial mutation probability of a variable, [0, 1] */
+  double  eta_c, eta_m;     /* distribution indices, finite, >= 0 */
+  double  sense[SIMPLYP_NSGA2_MAX_OBJECTIVES];   /* +1: maximised, -1: minimised */
+  SimplypMcmcParam param[SIMPLYP_MCMC_MAX_FREE];
+} SimplypNsga2;
+
+typedef struct {            /* device pointers */
+  double*  population;      /* [N][K] unit cube */
+  double*  objectives;      /* [N][M] y of the population (NaN rows: infeasible) */
+  int32_t* rank;            /* [N] 0 = first front */
+  double*  crowding;        /* [N] */
+  double*  offspring;       /* [N][K] unit cube */
+  int64_t* generation;      /* [1] g, generations completed */
+  int64_t* n_failed;        /* [1] infeasible evaluations */
+  double*  history;         /* [n_history][2 + M] */
+  int64_t  n_history;
+  int64_t  history_base;    /* generation g + 1 ends in row g + 1 - history_base; the init writes row 0 */
+  void*    workspace;       /* simplyp_nsga2_workspace_bytes(ns) bytes */
+  int64_t  workspace_bytes;
+} SimplypNsga2State;
+
+int64_t simplyp_nsga2_workspace_bytes(const SimplypNsga2* ns);
+/* y [M][N] (simplyp_sobol_outputs_device) and diag [N][S][NDIAG] of the evaluation of the population. */
+int simplyp_nsga2_init_device(const SimplypNsga2* ns, const SimplypNsga2State* state, const double* y,
+                              const int64_t* diag, void* stream);
+/* member_params [N][NP_MEMBER], sc_params [1 or N][S][NP_SC]: the offspring's rows. */
+int simplyp_nsga2_offspring_device(const SimplypNsga2* ns, const SimplypNsga2State* state, double* member_params,
+                                   double* sc_params, void* stream);
+/* y [M][N] and diag [N][S][NDIAG] of the evaluation of the offspring. */
+int simplyp_nsga2_survive_device(const SimplypNsga2* ns, const SimplypNsga2State* state, const double* y,
+                                 const int64_t* diag, void* stream);
+
 /* Host-buffer forms: same arguments as HOST pointers; the library stages them through its own
  * (cached) device buffers on `device`, runs and copies the result back before returning. */
 int simplyp_run_host(int device, const SimplypDims* dims, const SimplypOptions* opt,

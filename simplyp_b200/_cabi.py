@@ -29,7 +29,8 @@ EXPORTS = [
     "simplyp_nanquantile_device", "simplyp_sobol_design_device", "simplyp_sobol_outputs_device",
     "simplyp_sobol_workspace_bytes", "simplyp_sobol_indices_device", "simplyp_de_trial_device",
     "simplyp_de_select_device", "simplyp_de_init_device", "simplyp_period_aggregates_device",
-    "simplyp_calibrate_ar1_device", "simplyp_de_scale_device",
+    "simplyp_calibrate_ar1_device", "simplyp_de_scale_device", "simplyp_nsga2_workspace_bytes",
+    "simplyp_nsga2_init_device", "simplyp_nsga2_offspring_device", "simplyp_nsga2_survive_device",
 ]
 MAX_RANKS = 8
 
@@ -61,6 +62,7 @@ PERIOD_STATS = {"mean": 0, "load": 1, "fwmc": 2}
 MCMC_MEMBER, MCMC_SC_ALL, MCMC_SC_AT, MCMC_ERROR_MODEL = 0, 1, 2, 3
 AR1_MAX_SERIES = 64
 DE_STRATEGIES = {"best1bin": 0, "rand1bin": 1}
+NSGA2_MAX_OBJECTIVES = 16
 
 
 class SimplypMcmcParam(C.Structure):
@@ -97,6 +99,20 @@ class SimplypDeState(C.Structure):
                 ("weights", C.c_void_p), ("generation", C.c_void_p), ("best", C.c_void_p), ("converged", C.c_void_p),
                 ("converged_at", C.c_void_p), ("n_failed", C.c_void_p), ("history", C.c_void_p),
                 ("n_history", C.c_int64), ("history_base", C.c_int64)]
+
+
+class SimplypNsga2(C.Structure):
+    _fields_ = [("n_population", C.c_int32), ("n_free", C.c_int32), ("n_objectives", C.c_int32), ("n_sc", C.c_int32),
+                ("sc_per_member", C.c_int32), ("reserved", C.c_int32), ("seed", C.c_uint64), ("crossover", C.c_double),
+                ("mutation", C.c_double), ("eta_c", C.c_double), ("eta_m", C.c_double),
+                ("sense", C.c_double * NSGA2_MAX_OBJECTIVES), ("param", SimplypMcmcParam * MCMC_MAX_FREE)]
+
+
+class SimplypNsga2State(C.Structure):
+    _fields_ = [("population", C.c_void_p), ("objectives", C.c_void_p), ("rank", C.c_void_p), ("crowding", C.c_void_p),
+                ("offspring", C.c_void_p), ("generation", C.c_void_p), ("n_failed", C.c_void_p),
+                ("history", C.c_void_p), ("n_history", C.c_int64), ("history_base", C.c_int64),
+                ("workspace", C.c_void_p), ("workspace_bytes", C.c_int64)]
 
 
 class SimplypAr1(C.Structure):
@@ -205,6 +221,12 @@ def load():
     lib.simplyp_de_init_device.restype = C.c_int
     lib.simplyp_de_scale_device.argtypes = [dep, vp, C.c_int64, vp, vp]
     lib.simplyp_de_scale_device.restype = C.c_int
+    nsp, nssp = C.POINTER(SimplypNsga2), C.POINTER(SimplypNsga2State)
+    lib.simplyp_nsga2_workspace_bytes.argtypes = [nsp]
+    lib.simplyp_nsga2_workspace_bytes.restype = C.c_int64
+    for name in ("simplyp_nsga2_init_device", "simplyp_nsga2_offspring_device", "simplyp_nsga2_survive_device"):
+        getattr(lib, name).argtypes = [nsp, nssp, vp, vp, vp]
+        getattr(lib, name).restype = C.c_int
     if lib.simplyp_abi_version() != 4:
         raise SimplypError("ABI version mismatch")
     _lib = lib
@@ -430,9 +452,9 @@ def _u64(seed):
 
 
 def _free_params(spec, targets, lo, hi):
-    """``spec`` (SimplypMcmc, SimplypSobol or SimplypDe) with ``n_free`` and ``param`` set to the free parameters
-    ``targets`` [(kind, index, pos)] (``MCMC_MEMBER`` / ``MCMC_SC_ALL`` / ``MCMC_SC_AT`` / ``MCMC_ERROR_MODEL``) and
-    their boxes ``[lo[k], hi[k]]``."""
+    """``spec`` (SimplypMcmc, SimplypSobol, SimplypDe or SimplypNsga2) with ``n_free`` and ``param`` set to the free
+    parameters ``targets`` [(kind, index, pos)] (``MCMC_MEMBER`` / ``MCMC_SC_ALL`` / ``MCMC_SC_AT`` /
+    ``MCMC_ERROR_MODEL``) and their boxes ``[lo[k], hi[k]]``."""
     if not 1 <= len(targets) <= MCMC_MAX_FREE:
         raise ValueError("1..%d free parameters" % MCMC_MAX_FREE)
     spec.n_free = len(targets)
@@ -603,6 +625,59 @@ def de_init_device(de, state, y_ptr, diag_ptr, stream_ptr):
 def de_scale_device(de, unit_ptr, n, out_ptr, stream_ptr):
     """Parameter values out [n][K] of unit-cube rows unit [n][K]; asynchronous on ``stream_ptr``."""
     _check(require_device().simplyp_de_scale_device(C.byref(de), unit_ptr, int(n), out_ptr, stream_ptr))
+
+
+def make_nsga2(n_population, targets, lo, hi, n_sc, sense, sc_per_member=False, crossover=0.9, mutation=None,
+               eta_c=15.0, eta_m=20.0, seed=0):
+    """SimplypNsga2 for ``targets`` [(kind, index, pos)] (as :func:`make_mcmc`) with the boxes ``[lo[k], hi[k]]`` and
+    the objective senses ``sense`` [M] (+1 maximised, -1 minimised); ``mutation`` None is 1/K."""
+    ns = _free_params(SimplypNsga2(), targets, lo, hi)
+    ns.n_population, ns.n_sc, ns.n_objectives = int(n_population), int(n_sc), len(sense)
+    ns.sc_per_member = 1 if sc_per_member else 0
+    for m, v in enumerate(sense):
+        ns.sense[m] = float(v)
+    ns.seed = _u64(seed)
+    ns.crossover = float(crossover)
+    ns.mutation = 1.0 / ns.n_free if mutation is None else float(mutation)
+    ns.eta_c, ns.eta_m = float(eta_c), float(eta_m)
+    return ns
+
+
+def make_nsga2_state(population, objectives, rank, crowding, offspring, generation, n_failed, history, n_history,
+                     workspace, workspace_bytes, history_base=0):
+    """SimplypNsga2State from device pointers (torch ``.data_ptr()`` integers)."""
+    st = SimplypNsga2State()
+    st.population, st.objectives, st.rank, st.crowding = population, objectives, rank, crowding
+    st.offspring, st.generation, st.n_failed = offspring, generation, n_failed
+    st.history, st.n_history, st.history_base = history, int(n_history), int(history_base)
+    st.workspace, st.workspace_bytes = workspace, int(workspace_bytes)
+    return st
+
+
+def nsga2_workspace_bytes(ns):
+    n = load().simplyp_nsga2_workspace_bytes(C.byref(ns))
+    if n < 0:
+        _check(int(n))
+    return int(n)
+
+
+def nsga2_init_device(ns, state, y_ptr, diag_ptr, stream_ptr):
+    """Objectives, ranks, crowding and history row 0 of the population from its objective rows y [M][N] and diag;
+    asynchronous on ``stream_ptr``."""
+    _check(require_device().simplyp_nsga2_init_device(C.byref(ns), C.byref(state), y_ptr, diag_ptr, stream_ptr))
+
+
+def nsga2_offspring_device(ns, state, member_ptr, sc_ptr, stream_ptr):
+    """Offspring of every pair into ``offspring`` and the target columns of their rows; asynchronous on
+    ``stream_ptr``."""
+    _check(require_device().simplyp_nsga2_offspring_device(C.byref(ns), C.byref(state), member_ptr, sc_ptr,
+                                                           stream_ptr))
+
+
+def nsga2_survive_device(ns, state, y_ptr, diag_ptr, stream_ptr):
+    """Ranking, crowding, survival and history row of one generation from the offspring's objective rows y [M][N] and
+    diag; asynchronous on ``stream_ptr``."""
+    _check(require_device().simplyp_nsga2_survive_device(C.byref(ns), C.byref(state), y_ptr, diag_ptr, stream_ptr))
 
 
 def workspace_bytes(dims, calibrate, rank_stats=False):

@@ -20,8 +20,11 @@
 //   period_aggregate_kernel         period means, loads and flow-weighted concentrations of an ensemble
 //                                   (simplyp_periods.cuh)
 //   de_trial_kernel, de_select_kernel, de_init_kernel, de_reduce_kernel  differential evolution (simplyp_de.cuh)
+//   nsga2_offspring_kernel, nsga2_load_kernel, nsga2_rank_kernel (cooperative), nsga2_crowd_kernel,
+//   nsga2_select_kernel, nsga2_compact_kernel, nsga2_scatter_kernel, nsga2_commit_kernel  NSGA-II (simplyp_nsga2.cuh)
 //
 // There is deliberately no host implementation of the integration in this library.
+#include <cooperative_groups.h>
 #include <cuda_runtime.h>
 
 #include <atomic>
@@ -41,6 +44,7 @@
 #include "simplyp_periods.cuh"
 #include "simplyp_sobol.cuh"
 #include "simplyp_de.cuh"
+#include "simplyp_nsga2.cuh"
 #include "simplyp_ar1.cuh"
 
 using namespace simplyp;
@@ -2374,6 +2378,393 @@ int check_de(const SimplypDe* de, const SimplypDeState* st) {
   return SIMPLYP_OK;
 }
 
+// ------------------------------------------------------------------------------------------ NSGA-II
+// Survival over n points (2N in a generation, the N members of the population at the init): load (oriented
+// objectives), rank (cooperative: dominator counts, then peeling front by front with a grid barrier in between), crowd,
+// select, compact (one block: survivor positions, history row, generation counter), scatter into scratch rows, commit.
+// The pairwise passes tile the other points through shared memory; no pass keeps more than O(n (K + M)) state.
+constexpr int NS_THREADS = 256, NS_TILE = 256, NS_SCAN = 1024;
+constexpr int NS_NCTL = 8;   // ctl: front sizes [3], fronts ranked, last rank, points ranked before the last rank
+
+// Workspace of the survival (simplyp_nsga2_workspace_bytes): doubles first, then int32 arrays.
+struct Nsga2Ws {
+  double *f, *crowd, *su, *so, *sc;
+  int32_t *rank, *count, *fronts, *dest, *sr, *ctl;
+  SP_HD Nsga2Ws(const SimplypNsga2& ns, void* base) {
+    const size_t N = (size_t)ns.n_population, n = 2 * N, K = ns.n_free, M = ns.n_objectives;
+    f = static_cast<double*>(base);   // [2N][M] oriented objectives, NaN rows for infeasible points
+    crowd = f + n * M;                // [2N]
+    su = crowd + n;                   // [N][K] survivors' unit rows
+    so = su + N * K;                  // [N][M] survivors' objectives
+    sc = so + N * M;                  // [N] survivors' crowding
+    rank = reinterpret_cast<int32_t*>(sc + N);   // [2N] -1: not ranked
+    count = rank + n;                 // [2N] dominators not yet peeled
+    fronts = count + n;               // [3][2N] member lists of the current and next fronts
+    dest = fronts + 3 * n;            // [2N] 1/0 survives, then position among the survivors or -1
+    sr = dest + n;                    // [N] survivors' ranks
+    ctl = sr + N;                     // [NS_NCTL]
+  }
+  static int64_t bytes(const SimplypNsga2& ns) {
+    const int64_t N = ns.n_population, n = 2 * N, K = ns.n_free, M = ns.n_objectives;
+    return 8 * (n * M + n + N * K + N * M + N) + 4 * (n + n + 3 * n + n + N + NS_NCTL);
+  }
+};
+
+__global__ void nsga2_offspring_kernel(const SimplypNsga2 ns, const SimplypNsga2State st, double* member_params,
+                                       double* sc_params) {
+  const int p = blockIdx.x * blockDim.x + threadIdx.x;
+  if (p >= ns.n_population / 2) return;
+  const int K = ns.n_free, S = ns.n_sc;
+  double* c1 = st.offspring + (size_t)(2 * p) * K;
+  double* c2 = c1 + K;
+  nsga2_offspring_pair(ns, st.population, st.rank, st.crowding, *st.generation, p, c1, c2, nullptr);
+  for (int c = 0; c < 2; ++c) {
+    const int m = 2 * p + c;
+    const double* u = c ? c2 : c1;
+    double* mrow = member_params + (size_t)m * SIMPLYP_NP_MEMBER;
+    double* srow = sc_params + (ns.sc_per_member ? (size_t)m * S * SIMPLYP_NP_SC : 0);
+    for (int j = 0; j < K; ++j) mcmc_write_target(ns.param[j], S, de_scale(ns.param[j], u[j]), mrow, srow);
+  }
+}
+
+// Oriented objectives of the n points: the population's stored rows, and the evaluated members' y[M][N] with their
+// status words (the init evaluates the population itself and stores its objectives).
+__global__ void nsga2_load_kernel(const SimplypNsga2 ns, const SimplypNsga2State st, const double* y,
+                                  const int64_t* diag, int init) {
+  const int N = ns.n_population, M = ns.n_objectives, n = init ? N : 2 * N;
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  Nsga2Ws ws(ns, st.workspace);
+  if (i == 0)
+    for (int c = 0; c < NS_NCTL; ++c) ws.ctl[c] = 0;
+  if (i >= n) return;
+  double* f = ws.f + (size_t)i * M;
+  if (!init && i < N) {
+    nsga2_orient(ns, st.objectives + (size_t)i * M, 1, 0, f);
+  } else {
+    const int e = init ? i : i - N;
+    int status = 0;
+    for (int s = 0; s < ns.n_sc; ++s) status |= diag[((size_t)e * ns.n_sc + s) * SIMPLYP_NDIAG + SIMPLYP_DG_STATUS] != 0;
+    if (!nsga2_orient(ns, y + e, N, status, f)) atomicAdd(reinterpret_cast<unsigned long long*>(st.n_failed), 1ull);
+  }
+  ws.rank[i] = -1;
+  ws.crowd[i] = 0.0;
+}
+
+// Loads the oriented rows of points idx(t0 .. t0 + nt - 1) into s_f[nt][M].
+template <typename Idx>
+__device__ void nsga2_tile(const double* f, int M, int t0, int nt, Idx idx, double* s_f) {
+  for (int k = threadIdx.x; k < nt * M; k += blockDim.x) {
+    const int jj = k / M;
+    s_f[k] = f[(size_t)idx(t0 + jj) * M + (k - jj * M)];
+  }
+}
+
+// Number of rows of s_f[nt][M] that dominate fq.
+__device__ int nsga2_count_dominators(const double* s_f, int nt, const double (&fq)[SIMPLYP_NSGA2_MAX_OBJECTIVES],
+                                      int M) {
+  int d = 0;
+  for (int jj = 0; jj < nt; ++jj) d += nsga2_dominates(s_f + jj * M, fq, M);
+  return d;
+}
+
+// Non-dominated ranks of the n points until at least N are ranked.  Cooperative launch: every block takes the points
+// base + threadIdx.x of the same grid-stride loop in every pass, so a point's count and rank stay with one thread.
+__global__ void __launch_bounds__(NS_THREADS) nsga2_rank_kernel(const SimplypNsga2 ns, const SimplypNsga2State st,
+                                                                int n) {
+  namespace cg = cooperative_groups;
+  cg::grid_group grid = cg::this_grid();
+  __shared__ double s_f[NS_TILE * SIMPLYP_NSGA2_MAX_OBJECTIVES];
+  Nsga2Ws ws(ns, st.workspace);
+  const int M = ns.n_objectives, target = ns.n_population, stride = gridDim.x * blockDim.x;
+  double fq[SIMPLYP_NSGA2_MAX_OBJECTIVES];
+  // dominator counts over all points; front 0 = the feasible points nobody dominates
+  for (int base = blockIdx.x * blockDim.x; base < n; base += stride) {
+    const int q = base + threadIdx.x;
+#pragma unroll
+    for (int m = 0; m < SIMPLYP_NSGA2_MAX_OBJECTIVES; ++m) fq[m] = q < n && m < M ? ws.f[(size_t)q * M + m] : NAN;
+    const int ok = q < n && fq[0] == fq[0];
+    int cnt = 0;
+    for (int t0 = 0; t0 < n; t0 += NS_TILE) {
+      const int nt = n - t0 < NS_TILE ? n - t0 : NS_TILE;
+      __syncthreads();
+      nsga2_tile(ws.f, M, t0, nt, [](int j) { return j; }, s_f);
+      __syncthreads();
+      if (ok) cnt += nsga2_count_dominators(s_f, nt, fq, M);
+    }
+    if (ok) {
+      ws.count[q] = cnt;
+      if (cnt == 0) {
+        ws.rank[q] = 0;
+        ws.fronts[atomicAdd(&ws.ctl[0], 1)] = q;
+      }
+    }
+  }
+  grid.sync();
+  // peel: the members of front k take themselves off the counts of the points they dominate
+  int k = 0, cur = ws.ctl[0], ranked = cur;
+  while (ranked < target && cur > 0) {
+    const int* list = ws.fronts + (size_t)(k % 3) * n;
+    int* next = ws.fronts + (size_t)((k + 1) % 3) * n;
+    if (blockIdx.x == 0 && threadIdx.x == 0) ws.ctl[(k + 2) % 3] = 0;   // read before the last barrier, next written after the coming one
+    for (int base = blockIdx.x * blockDim.x; base < n; base += stride) {
+      const int q = base + threadIdx.x;
+      const int ok = q < n && ws.rank[q] < 0 && ws.f[(size_t)q * M] == ws.f[(size_t)q * M];
+      if (!__syncthreads_or(ok)) continue;
+#pragma unroll
+      for (int m = 0; m < SIMPLYP_NSGA2_MAX_OBJECTIVES; ++m) fq[m] = ok && m < M ? ws.f[(size_t)q * M + m] : NAN;
+      int d = 0;
+      for (int t0 = 0; t0 < cur; t0 += NS_TILE) {
+        const int nt = cur - t0 < NS_TILE ? cur - t0 : NS_TILE;
+        __syncthreads();
+        nsga2_tile(ws.f, M, t0, nt, [list](int j) { return list[j]; }, s_f);
+        __syncthreads();
+        if (ok) d += nsga2_count_dominators(s_f, nt, fq, M);
+      }
+      if (ok && d) {
+        const int c = ws.count[q] - d;
+        ws.count[q] = c;
+        if (c == 0) {
+          ws.rank[q] = k + 1;
+          next[atomicAdd(&ws.ctl[(k + 1) % 3], 1)] = q;
+        }
+      }
+    }
+    grid.sync();
+    cur = ws.ctl[(k + 1) % 3];
+    ranked += cur;
+    ++k;
+  }
+  // front k holds cur points; with cur == 0 every feasible point is ranked and the infeasible ones form rank k
+  const int infeasible_rank = cur == 0 && ranked < target;
+  if (infeasible_rank)
+    for (int q = blockIdx.x * blockDim.x + threadIdx.x; q < n; q += stride)
+      if (ws.rank[q] < 0) ws.rank[q] = k;
+  if (blockIdx.x == 0 && threadIdx.x == 0) {
+    ws.ctl[3] = k + 1;
+    ws.ctl[4] = k;
+    ws.ctl[5] = infeasible_rank ? ranked : ranked - cur;
+  }
+}
+
+// Crowding distance of every ranked feasible point within its front (infeasible and unranked points: 0).  Per
+// objective, the neighbours in the front's order by (f_m, index) are the nearest values above and below.
+__global__ void __launch_bounds__(NS_THREADS) nsga2_crowd_kernel(const SimplypNsga2 ns, const SimplypNsga2State st,
+                                                                 int n) {
+  __shared__ double s_v[NS_TILE];
+  __shared__ int32_t s_r[NS_TILE];
+  Nsga2Ws ws(ns, st.workspace);
+  const int M = ns.n_objectives, i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int ri = i < n ? ws.rank[i] : -1;
+  const int act = ri >= 0 && ws.f[(size_t)i * M] == ws.f[(size_t)i * M];
+  if (!__syncthreads_or(act)) return;
+  double crowd = 0.0;
+  for (int m = 0; m < M; ++m) {
+    const double fi = act ? ws.f[(size_t)i * M + m] : 0.0;
+    double next = INFINITY, prev = -INFINITY, mx = fi, mn = fi;
+    int has_next = 0, has_prev = 0;
+    for (int t0 = 0; t0 < n; t0 += NS_TILE) {
+      const int nt = n - t0 < NS_TILE ? n - t0 : NS_TILE;
+      __syncthreads();
+      for (int jj = threadIdx.x; jj < nt; jj += blockDim.x) {
+        s_v[jj] = ws.f[(size_t)(t0 + jj) * M + m];
+        s_r[jj] = ws.rank[t0 + jj];
+      }
+      __syncthreads();
+      if (!act) continue;
+      for (int jj = 0; jj < nt; ++jj) {
+        const int j = t0 + jj;
+        if (s_r[jj] != ri || j == i) continue;
+        const double v = s_v[jj];
+        mx = v > mx ? v : mx;
+        mn = v < mn ? v : mn;
+        if (v > fi || (v == fi && j > i)) {
+          has_next = 1;
+          next = v < next ? v : next;
+        } else {
+          has_prev = 1;
+          prev = v > prev ? v : prev;
+        }
+      }
+    }
+    crowd = mc_add(crowd, nsga2_crowd_term(!has_next || !has_prev, next, prev, mx, mn));
+  }
+  if (act) ws.crowd[i] = crowd;
+}
+
+// Survivors: every point of a rank below the last; of the last rank, the need = N - (points before it) first in the
+// order (crowding desc, index asc).  dest[i] = 1 / 0.
+__global__ void __launch_bounds__(NS_THREADS) nsga2_select_kernel(const SimplypNsga2 ns, const SimplypNsga2State st,
+                                                                  int n) {
+  __shared__ double s_c[NS_TILE];
+  __shared__ int32_t s_r[NS_TILE];
+  Nsga2Ws ws(ns, st.workspace);
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  const int last = ws.ctl[4], need = ns.n_population - ws.ctl[5];
+  const int ri = i < n ? ws.rank[i] : -1;
+  const int act = ri == last;
+  const double ci = i < n ? ws.crowd[i] : 0.0;
+  int before = 0;
+  if (__syncthreads_or(act)) {
+    for (int t0 = 0; t0 < n; t0 += NS_TILE) {
+      const int nt = n - t0 < NS_TILE ? n - t0 : NS_TILE;
+      __syncthreads();
+      for (int jj = threadIdx.x; jj < nt; jj += blockDim.x) {
+        s_c[jj] = ws.crowd[t0 + jj];
+        s_r[jj] = ws.rank[t0 + jj];
+      }
+      __syncthreads();
+      if (!act) continue;
+      for (int jj = 0; jj < nt; ++jj)
+        before += s_r[jj] == last && (s_c[jj] > ci || (s_c[jj] == ci && t0 + jj < i));
+    }
+  }
+  if (i < n) ws.dest[i] = (ri >= 0 && ri < last) || (act && before < need);
+}
+
+// One block: survivor positions in ascending index (dest[i] = position or -1), the history row and the counters.
+__global__ void __launch_bounds__(NS_SCAN) nsga2_compact_kernel(const SimplypNsga2 ns, const SimplypNsga2State st,
+                                                                int n, int init) {
+  __shared__ int32_t s_warp[NS_SCAN / 32];
+  __shared__ double s_red[NS_SCAN];
+  __shared__ int32_t s_cnt[NS_SCAN];
+  Nsga2Ws ws(ns, st.workspace);
+  const int t = threadIdx.x, lane = t & 31, warp = t >> 5, M = ns.n_objectives;
+  int base = 0;
+  for (int c0 = 0; c0 < n; c0 += NS_SCAN) {
+    const int i = c0 + t;
+    const int s = i < n ? ws.dest[i] : 0;
+    const unsigned b = __ballot_sync(0xFFFFFFFFu, s);
+    if (lane == 0) s_warp[warp] = __popc(b);
+    __syncthreads();
+    int off = base;
+    for (int w = 0; w < warp; ++w) off += s_warp[w];
+    int total = 0;
+    for (int w = 0; w < NS_SCAN / 32; ++w) total += s_warp[w];
+    if (i < n) ws.dest[i] = s ? off + __popc(b & ((1u << lane) - 1u)) : -1;
+    __syncthreads();
+    base += total;
+  }
+  __syncthreads();
+  // first-front size among the survivors
+  int n0 = 0;
+  for (int i = t; i < n; i += NS_SCAN) n0 += ws.dest[i] >= 0 && ws.rank[i] == 0;
+  s_cnt[t] = n0;
+  __syncthreads();
+  for (int s = NS_SCAN / 2; s > 0; s >>= 1) {
+    if (t < s) s_cnt[t] += s_cnt[t + s];
+    __syncthreads();
+  }
+  n0 = s_cnt[0];
+  const long long g = *st.generation;
+  const long long row = init ? 0 : g + 1 - st.history_base;
+  double* h = row >= 0 && row < st.n_history ? st.history + (size_t)row * (2 + M) : nullptr;
+  // best of each objective over the feasible survivors (a maximum of oriented values: exact in any order)
+  for (int m = 0; m < M; ++m) {
+    double best = -INFINITY;
+    for (int i = t; i < n; i += NS_SCAN) {
+      const double v = ws.f[(size_t)i * M + m];
+      if (ws.dest[i] >= 0 && v == v && v > best) best = v;
+    }
+    __syncthreads();
+    s_red[t] = best;
+    __syncthreads();
+    for (int s = NS_SCAN / 2; s > 0; s >>= 1) {
+      if (t < s && s_red[t + s] > s_red[t]) s_red[t] = s_red[t + s];
+      __syncthreads();
+    }
+    if (t == 0 && h) h[2 + m] = s_red[0] == -INFINITY ? NAN : mc_mul(ns.sense[m], s_red[0]);
+  }
+  if (t != 0) return;
+  if (h) {
+    h[0] = (double)n0;
+    h[1] = (double)ws.ctl[3];
+  }
+  if (!init) *st.generation = g + 1;
+}
+
+// Survivors into the scratch rows at their positions.
+__global__ void nsga2_scatter_kernel(const SimplypNsga2 ns, const SimplypNsga2State st, int n) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  Nsga2Ws ws(ns, st.workspace);
+  const int d = ws.dest[i];
+  if (d < 0) return;
+  const int N = ns.n_population, K = ns.n_free, M = ns.n_objectives;
+  const double* u = i < N ? st.population + (size_t)i * K : st.offspring + (size_t)(i - N) * K;
+  for (int j = 0; j < K; ++j) ws.su[(size_t)d * K + j] = u[j];
+  for (int m = 0; m < M; ++m) ws.so[(size_t)d * M + m] = mc_mul(ns.sense[m], ws.f[(size_t)i * M + m]);
+  ws.sr[d] = ws.rank[i];
+  ws.sc[d] = ws.crowd[i];
+}
+
+// Scratch rows into the population.
+__global__ void nsga2_commit_kernel(const SimplypNsga2 ns, const SimplypNsga2State st) {
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= ns.n_population) return;
+  Nsga2Ws ws(ns, st.workspace);
+  const int K = ns.n_free, M = ns.n_objectives;
+  for (int j = 0; j < K; ++j) st.population[(size_t)i * K + j] = ws.su[(size_t)i * K + j];
+  for (int m = 0; m < M; ++m) st.objectives[(size_t)i * M + m] = ws.so[(size_t)i * M + m];
+  st.rank[i] = ws.sr[i];
+  st.crowding[i] = ws.sc[i];
+}
+
+int check_nsga2(const SimplypNsga2* ns, const SimplypNsga2State* st) {
+  if (!ns || !st) return fail(SIMPLYP_EINVAL, "nsga2: null argument%s");
+  const int K = ns->n_free, N = ns->n_population, M = ns->n_objectives;
+  if (K < 1 || K > SIMPLYP_MCMC_MAX_FREE) return fail(SIMPLYP_EINVAL, "nsga2: 1..SIMPLYP_MCMC_MAX_FREE free parameters%s");
+  if (N < 4 || N % 2 != 0 || N > (1 << 29)) return fail(SIMPLYP_EINVAL, "nsga2: n_population must be even, 4..2^29%s");
+  if (M < 2 || M > SIMPLYP_NSGA2_MAX_OBJECTIVES) return fail(SIMPLYP_EINVAL, "nsga2: 2..SIMPLYP_NSGA2_MAX_OBJECTIVES objectives%s");
+  if (ns->n_sc < 1) return fail(SIMPLYP_EINVAL, "nsga2: bad n_sc%s");
+  if (!(ns->crossover >= 0.0 && ns->crossover <= 1.0 && ns->mutation >= 0.0 && ns->mutation <= 1.0))
+    return fail(SIMPLYP_EINVAL, "nsga2: crossover and mutation must lie in [0, 1]%s");
+  if (!(ns->eta_c >= 0.0 && ns->eta_c < INFINITY && ns->eta_m >= 0.0 && ns->eta_m < INFINITY))
+    return fail(SIMPLYP_EINVAL, "nsga2: eta_c and eta_m must be finite and >= 0%s");
+  for (int m = 0; m < M; ++m)
+    if (ns->sense[m] != 1.0 && ns->sense[m] != -1.0) return fail(SIMPLYP_EINVAL, "nsga2: sense must be +1 or -1%s");
+  const int rc = check_targets(ns->param, K, ns->n_sc, ns->sc_per_member, "nsga2");
+  if (rc) return rc;
+  if (!st->population || !st->objectives || !st->rank || !st->crowding || !st->offspring || !st->generation ||
+      !st->n_failed || (st->n_history > 0 && !st->history) || st->n_history < 0 || !st->workspace)
+    return fail(SIMPLYP_EINVAL, "nsga2: null state pointer%s");
+  if (st->workspace_bytes < Nsga2Ws::bytes(*ns)) return fail(SIMPLYP_EINVAL, "nsga2: workspace smaller than simplyp_nsga2_workspace_bytes%s");
+  return SIMPLYP_OK;
+}
+
+// The survival (init = 0: over parents and offspring) or the ranking of the initial population (init = 1).
+int nsga2_survive(const SimplypNsga2* ns, const SimplypNsga2State* st, const double* y, const int64_t* diag,
+                  void* stream, int init) {
+  const int rc = check_nsga2(ns, st);
+  if (rc) return rc;
+  if (!y || !diag) return fail(SIMPLYP_EINVAL, "nsga2: null objective rows or diag%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  const int N = ns->n_population, n = init ? N : 2 * N;
+  const unsigned blocks = (unsigned)((n + NS_THREADS - 1) / NS_THREADS);
+  cudaStream_t s = static_cast<cudaStream_t>(stream);
+  nsga2_load_kernel<<<blocks, NS_THREADS, 0, s>>>(*ns, *st, y, diag, init);
+  // the cooperative grid: every block must be resident at once
+  int dev = 0, sms = 0, per_sm = 0;
+  SP_CUDA(cudaGetDevice(&dev));
+  SP_CUDA(cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev));
+  SP_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, nsga2_rank_kernel, NS_THREADS, 0));
+  const unsigned resident = (unsigned)(per_sm * sms);
+  if (resident < 1) return fail(SIMPLYP_ECUDA, "nsga2: the rank kernel cannot be resident%s");
+  SimplypNsga2 a0 = *ns;
+  SimplypNsga2State a1 = *st;
+  int a2 = n;
+  void* args[] = {&a0, &a1, &a2};
+  SP_CUDA(cudaLaunchCooperativeKernel((const void*)nsga2_rank_kernel, dim3(blocks < resident ? blocks : resident),
+                                      dim3(NS_THREADS), args, 0, s));
+  nsga2_crowd_kernel<<<blocks, NS_THREADS, 0, s>>>(*ns, *st, n);
+  nsga2_select_kernel<<<blocks, NS_THREADS, 0, s>>>(*ns, *st, n);
+  nsga2_compact_kernel<<<1, NS_SCAN, 0, s>>>(*ns, *st, n, init);
+  nsga2_scatter_kernel<<<blocks, NS_THREADS, 0, s>>>(*ns, *st, n);
+  nsga2_commit_kernel<<<(N + NS_THREADS - 1) / NS_THREADS, NS_THREADS, 0, s>>>(*ns, *st);
+  g_launches.fetch_add(7);
+  SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
 }  // namespace
 
 // ============================================================================================ C-ABI
@@ -3068,6 +3459,37 @@ int simplyp_de_scale_device(const SimplypDe* de, const double* unit, int64_t n, 
   g_launches.fetch_add(1);
   SP_CUDA(cudaGetLastError());
   return SIMPLYP_OK;
+}
+
+int64_t simplyp_nsga2_workspace_bytes(const SimplypNsga2* ns) {
+  if (!ns || ns->n_population < 4 || ns->n_population > (1 << 29) || ns->n_free < 1 ||
+      ns->n_free > SIMPLYP_MCMC_MAX_FREE || ns->n_objectives < 2 || ns->n_objectives > SIMPLYP_NSGA2_MAX_OBJECTIVES)
+    return fail(SIMPLYP_EINVAL, "nsga2_workspace_bytes: bad n_population / n_free / n_objectives%s");
+  return Nsga2Ws::bytes(*ns);
+}
+
+int simplyp_nsga2_init_device(const SimplypNsga2* ns, const SimplypNsga2State* state, const double* y,
+                              const int64_t* diag, void* stream) {
+  return nsga2_survive(ns, state, y, diag, stream, 1);
+}
+
+int simplyp_nsga2_offspring_device(const SimplypNsga2* ns, const SimplypNsga2State* state, double* member_params,
+                                   double* sc_params, void* stream) {
+  const int rc = check_nsga2(ns, state);
+  if (rc) return rc;
+  if (!member_params || !sc_params) return fail(SIMPLYP_EINVAL, "nsga2: null parameter rows%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  const int pairs = ns->n_population / 2;
+  nsga2_offspring_kernel<<<(pairs + 127) / 128, 128, 0, static_cast<cudaStream_t>(stream)>>>(*ns, *state,
+                                                                                            member_params, sc_params);
+  g_launches.fetch_add(1);
+  SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
+int simplyp_nsga2_survive_device(const SimplypNsga2* ns, const SimplypNsga2State* state, const double* y,
+                                 const int64_t* diag, void* stream) {
+  return nsga2_survive(ns, state, y, diag, stream, 0);
 }
 
 void simplyp_release_cache(void) {

@@ -309,6 +309,22 @@ class Engine:
         (``simplyp_de_init_device``).  Asynchronous."""
         self._call(_cabi.de_init_device, de, state, y.data_ptr(), diag.data_ptr())
 
+    # ------------------------------------------------------------------ NSGA-II
+    def nsga2_init(self, ns, state, y, diag):
+        """Objectives, ranks, crowding and history row 0 of the population from its objective rows ``y`` [M][N] and
+        ``diag`` [N][S][4] (``simplyp_nsga2_init_device``).  Asynchronous."""
+        self._call(_cabi.nsga2_init_device, ns, state, y.data_ptr(), diag.data_ptr())
+
+    def nsga2_offspring(self, ns, state, member_params, sc_params):
+        """Enqueue the offspring of one NSGA-II generation into ``state.offspring`` and the target columns of
+        ``member_params`` [N][NP_MEMBER] / ``sc_params`` ([N] or [1])[S][NP_SC] (``simplyp_nsga2_offspring_device``)."""
+        self._call(_cabi.nsga2_offspring_device, ns, state, member_params.data_ptr(), sc_params.data_ptr())
+
+    def nsga2_survive(self, ns, state, y, diag):
+        """Enqueue the survival of one NSGA-II generation from the offspring's objective rows ``y`` [M][N] and ``diag``
+        [N][S][4] (``simplyp_nsga2_survive_device``).  Asynchronous."""
+        self._call(_cabi.nsga2_survive_device, ns, state, y.data_ptr(), diag.data_ptr())
+
     # ------------------------------------------------------------------ Thornthwaite PET
     def thornthwaite_pet(self, t_air, month_start, year_is_leap, latitude_deg, out=None, out_stride=1):
         """Reference ``daily_PET`` (``inputs.py:232-312``) on the device: ``t_air`` [D] (device or host),
