@@ -20,7 +20,6 @@ struct IO {
     if (k <= cap) { Rec& r = rec[(size_t)day * cap + (k - 1)]; r.t = (float)t; r.h = (float)hh; r.en2 = (float)en2; r.k = (int16_t)k; r.acc = acc; }
     nrec[day] = k;
   }
-  static constexpr bool kAllLanesEmit = false;
   template <class Q> void emit(const Q&, int, const double (&)[NL], double, const double (&)[NA], const double (&)[13], const Cold&) {}
 };
 extern "C" int steps_attempts(int M, int D, int cap, const double* forcing, const double* mp, const double* scp, double rtol, double atol,

@@ -12,7 +12,6 @@ struct IO {
   void upstream(int, double (&us)[4]) const { us[0]=us[1]=us[2]=us[3]=0; }
   bool wants_vr() const { return false; }
   void publish(int) const {}
-  static constexpr bool kAllLanesEmit = false;
   template <class Q> void emit(const Q&, int, const double (&)[NL], double, const double (&acc)[NA], const double (&)[13], const Cold&) { chk += acc[0]; }
   double chk = 0;
 };

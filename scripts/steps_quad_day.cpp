@@ -15,7 +15,6 @@ struct IO {
   bool wants_vr() const { return false; }
   void publish(int) const {}
   void hook(int day, unsigned n) { steps[day] = (uint16_t)(n - last); last = n; }
-  static constexpr bool kAllLanesEmit = false;
   template <class Q> void emit(const Q&, int day, const double (&)[NL], double, const double (&acc)[NA], const double (&)[13], const Cold&) {}
 };
 extern "C" int steps_quad_day(int M, int D, const double* forcing, const double* mp, const double* scp, double rtol, double atol, uint16_t* steps) {

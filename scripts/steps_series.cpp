@@ -18,7 +18,6 @@ struct IO {
   void forcing(int day, double& P, double& E, double& doy, double& T) const { P = f[4*day]; E = f[4*day+1]; doy = f[4*day+2]; T = f[4*day+3]; }
   void upstream(int, double (&us)[4]) const { us[0]=us[1]=us[2]=us[3]=0; }
   void publish(int) const {}
-  static constexpr bool kAllLanesEmit = false;
   template <class Q> void emit(const Q&, int day, const double (&y)[NL], double Vr, const double (&acc)[NA], const double (&)[13], const Cold&) {
     double* o = out + (size_t)day * 12;
     for (int i = 0; i < 4; ++i) o[i] = acc[i];

@@ -94,6 +94,9 @@ struct ThreadOptions {
 struct ThreadCounters {
   long long steps, rejected, rhs_evals;
   int status;
+#ifdef SP_LAT_PROBE
+  long long lat[8];     // analysis builds: SM cycles of the warp by section of the day loop (simplyp_quad.cuh, LatProbe)
+#endif
 };
 
 // ------------------------------------------------------------------------------------------
@@ -575,27 +578,29 @@ SP_CONST double kRK[RK_N] = {
     dp::a61, dp::a62, dp::a63, dp::a64, dp::a65, dp::b1, dp::b2, dp::b3, dp::b4, dp::b5, dp::b6,
     dp::e1, dp::e2, dp::e3, dp::e4, dp::e5, dp::e6, dp::e7};
 
-// The same controller on the MEAN SQUARE of the scaled error (no square root): 0.9*(en^2)^(-1/10) in [0.2, 5].
+// The same controller on the MEAN SQUARE of the scaled error (no square root): 0.9*(en^2)^(-1/10) in [0.2, cap], cap <= 5
+// (the caller passes 1 where the step must not grow: after a rejection and on the step after one).
 // Device: fp32 lg2/ex2 with flush-to-zero and no range branches — an underflowing en^2 gives lg2 = -inf, hence
-// +inf, clamped to 5; an overflowing one gives 0, clamped to 0.2 (en^2 is never NaN here).
+// +inf, clamped to cap; an overflowing one gives 0, and a NaN gives NaN, both clamped to 0.2 (fmaxf drops the NaN).
 // `expo` = -1/(2p) for an estimate of order p-1 ... i.e. -0.1 for the 5(4) pair, -0.125 for Kaps-Rentrop 4(3).
 #ifndef SP_CTRL_SAFETY
 #define SP_CTRL_SAFETY 0.9     // scripts/controller_exp.py: 0.95 saves 2.8 % attempts at the price of 1.5x the rejections
 #define SP_CTRL_MAXGROW 5.0
 #endif
-SP_HD double step_factor_sq(double en2, double expo = -0.1) {
+SP_HD double step_factor_sq(double en2, double expo = -0.1, double cap = SP_CTRL_MAXGROW) {
 #if defined(__CUDA_ARCH__)
   float l, f;
   const float x = __double2float_rn(en2);
   asm("lg2.approx.ftz.f32 %0, %1;" : "=f"(l) : "f"(x));
   l *= (float)expo;
   asm("ex2.approx.ftz.f32 %0, %1;" : "=f"(f) : "f"(l));
-  return (double)fminf(fmaxf((float)SP_CTRL_SAFETY * f, 0.2f), (float)SP_CTRL_MAXGROW);
+  return (double)fminf(fmaxf((float)SP_CTRL_SAFETY * f, 0.2f), (float)cap);
 #else
-  if (!(en2 > 1e-38)) return SP_CTRL_MAXGROW;
+  if (en2 != en2) return 0.2;
+  if (!(en2 > 1e-38)) return cap;
   if (!(en2 < 1e38)) return 0.2;
   const double f = SP_CTRL_SAFETY * exp(expo * log(en2));
-  return sp_min(SP_CTRL_MAXGROW, sp_max(0.2, f));
+  return sp_min(cap, sp_min(SP_CTRL_MAXGROW, sp_max(0.2, f)));
 #endif
 }
 

@@ -335,7 +335,6 @@ struct RunIO : IOBase<ROUTED> {
   // store it together: lane l writes columns l, l+4, l+8, ... — each store instruction of the warp moves eight
   // contiguous 32-byte pieces (one per quad) instead of eight single doubles, 7 store instructions per day instead
   // of 25 by the leader alone.  The column a lane stores is chosen with selects, not by indexing a register array.
-  static constexpr bool kAllLanesEmit = true;
   template <class Q>
   __device__ __forceinline__ void emit(const Q& q, int day, const double (&y)[NL], double Vr, const double (&acc)[NA],
                                        const double (&non)[13], const Cold&) const {
@@ -393,11 +392,14 @@ struct CalIO : IOBase<ROUTED> {
       }
     }
   }
-  static constexpr bool kAllLanesEmit = false;
+  // Called by every lane of the quad (each holds the whole day, see RunIO::emit).  The leader stores the flux row that
+  // it publishes; an ensemble item's observed series are dealt to the lanes — slot k to lane k mod 4 — so that
+  // the lanes update their series side by side instead of the leader updating all of them in turn.  A series always
+  // goes to the same lane and its sums get the same operations in the same order as on any other lane: no bit moves.
   template <class Q>
-  __device__ __forceinline__ void emit(const Q&, int day, const double (&)[NL], double, const double (&acc)[NA],
+  __device__ __forceinline__ void emit(const Q& q, int day, const double (&)[NL], double, const double (&acc)[NA],
                                        const double (&)[13], const Cold& c) const {
-    if (a.flux != nullptr) {
+    if (a.flux != nullptr && q.leader()) {
       double* row = a.flux + (((size_t)m * a.S + s) * a.D + day) * 4;
       row[0] = acc[0]; row[1] = acc[1]; row[2] = acc[2]; row[3] = acc[3];
     }
@@ -410,10 +412,21 @@ struct CalIO : IOBase<ROUTED> {
     // subroutine into the kernel: its mere presence, never executed, cost 2-3 % of the run time (A/B on one box).
     const double A = c.A_catch;
     const double rQ = sp_rcp(acc[0]), rA = sp_rcp(A);
-    int slot = 0;
-    for (int v = 0; v < a.V; ++v) {
-      if (__ldg(a.obs_desc + 2 * v) != s) continue;
-      const int k = slot++;
+    // One pass over the series: each round the lanes walk the next four series of the item together (the cursor is the
+    // same on all four) and each keeps the one of its slot; then they update those side by side.  (A lane that
+    // updated its series inside the walk would leave the other three waiting in every iteration.)
+    // Networks (ROUTED) keep the leader alone on the series: their 3-blocks-per-SM build at 168 registers spills 24 B
+    // more with the series spread over the lanes.
+    constexpr int kLanes = ROUTED ? 1 : 4;
+    if (ROUTED && !q.leader()) return;
+    for (int cur = 0, slot = 0;;) {
+      int v = -1, k = 0;
+      for (int n = 0; n < kLanes && cur < a.V; ++cur) {
+        if (__ldg(a.obs_desc + 2 * cur) != s) continue;
+        if (n++ == q.ql) { v = cur; k = slot; }
+        ++slot;
+      }
+      if (v < 0) break;                      // the series ran out before this lane's slot of the round
       const double o = __ldg(a.obs + (size_t)v * a.D + day);
       if (o != o) continue;  // no observation that day
       const int kind = __ldg(a.obs_desc + 2 * v + 1);
@@ -688,6 +701,9 @@ __global__ void __launch_bounds__(128, MINB) simplyp_quad_kernel(const KArgs a) 
           for (int i = 0; i < STAT_SLOTS * RS_COUNT; ++i) dst[i] = sacc[i];
         } else {
           io.finalise();
+#if defined(SP_LAT_PROBE) && defined(__CUDA_ARCH__)   // analysis builds: the section cycles replace the statistics
+          for (int i = 0; i < LP_N && i < a.V * SIMPLYP_NSTAT; ++i) a.stats[(size_t)m * a.V * SIMPLYP_NSTAT + i] = (double)cnt.lat[i];
+#endif
         }
       }
       cnt.status |= io.wait_status;

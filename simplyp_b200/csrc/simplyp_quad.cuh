@@ -87,6 +87,36 @@
 
 namespace simplyp {
 
+// ------------------------------------------------------------------------------------------ section probe
+// Analysis builds (-DSP_LAT_PROBE, scripts/exp_lat_sections.py): every warp reads clock64() at the section boundaries of
+// its day loop and adds the cycles between two reads to the section the second one closes.  A boundary is where the
+// read ISSUES: a result still in flight there is charged to the section that waits for it.  Without the macro the
+// marks are empty and the product build is unchanged.
+#if defined(SP_LAT_PROBE) && defined(__CUDA_ARCH__)
+enum { LP_RHS = 0,   // step loop top -> the attempt's sixth RHS evaluation (stage arguments included)
+       LP_ERR,       // -> the error norm en2
+       LP_CTRL,      // -> the end of the loop body: controller, accept/reject bookkeeping
+       LP_END,       // step loop exit (last vote) -> end of the day: state gather, end_day, statistics, barriers
+       LP_START,     // -> entry of tomorrow's step loop: wait / forcing, begin_day, quad_daily_coef, first RHS + Jacobian
+       LP_ITERS,     // step-loop iterations of the warp (attempts in lock-step)
+       LP_DAYS,      // day boundaries
+       LP_N };
+static_assert(LP_N <= 8, "ThreadCounters::lat");
+struct LatProbe {
+  long long t, acc[LP_N];
+  __device__ __forceinline__ void mark(int sec) { const long long c = clock64(); acc[sec] += c - t; t = c; }
+};
+#define SP_LAT_PARAM , LatProbe& lp
+#define SP_LAT_ARG , lp
+#define SP_LAT_MARK(sec) lp.mark(sec)
+#define SP_LAT_COUNT(i) (++lp.acc[i])
+#else
+#define SP_LAT_PARAM
+#define SP_LAT_ARG
+#define SP_LAT_MARK(sec) ((void)0)
+#define SP_LAT_COUNT(i) ((void)0)
+#endif
+
 // ------------------------------------------------------------------------------------------ 4-lane host value
 struct V4 { double v[4]; };
 #define SP_V4_BIN(op)                                                                                             \
@@ -152,10 +182,14 @@ struct QuadDev {
     return __hiloint2double(hi, lo);
 #endif
   }
+  // (x + x^1) + (x^2 + x^3): the butterfly's value on every lane (fp addition commutes bitwise, so lane 2's
+  // (x2 + x3) + (x0 + x1) is lane 0's sum), but the three fetches are independent — one shuffle round trip on the
+  // error norm's dependent path instead of two
   __device__ __forceinline__ T sum(T x) const {
-    x += __shfl_xor_sync(0xffffffffu, x, 1);
-    x += __shfl_xor_sync(0xffffffffu, x, 2);
-    return x;
+    const T x1 = __shfl_xor_sync(0xffffffffu, x, 1);
+    const T x2 = __shfl_xor_sync(0xffffffffu, x, 2);
+    const T x3 = __shfl_xor_sync(0xffffffffu, x, 3);
+    return (x + x1) + (x2 + x3);
   }
   __device__ __forceinline__ double first(T x) const { return x; }
   __device__ __forceinline__ T sel3(T on3, T other) const { return ql == 3 ? on3 : other; }
@@ -259,7 +293,7 @@ struct QuadState {
 template <class Q>
 SP_HD double quad_attempt(const Q& q, const QuadCoef<Q>& c, const QuadState<Q>& s, double hh, double rtol, double atol,
                           typename Q::T& ynA, typename Q::T& ynB, typename Q::T& accn, typename Q::T& k7A,
-                          typename Q::T& k7B, typename Q::T& a7, typename Q::T& e7o) {
+                          typename Q::T& k7B, typename Q::T& a7, typename Q::T& e7o SP_LAT_PARAM) {
   using T = typename Q::T;
   T kA2, kA3, kA4, kA5, kA6, kB2, kB3, kB4, kB5, kB6, da, ee;
   T sb = kRK[RB1] * s.a1, se = kRK[RE1] * s.a1;
@@ -279,6 +313,7 @@ SP_HD double quad_attempt(const Q& q, const QuadCoef<Q>& c, const QuadState<Q>& 
   ynA = qfma(hh, qfma(kRK[RB6], kA6, qfma(kRK[RB5], kA5, qfma(kRK[RB4], kA4, qfma(kRK[RB3], kA3, qfma(kRK[RB2], kA2, kRK[RB1] * s.k1A))))), s.yA);
   ynB = qfma(hh, qfma(kRK[RB6], kB6, qfma(kRK[RB5], kB5, qfma(kRK[RB4], kB4, qfma(kRK[RB3], kB3, qfma(kRK[RB2], kB2, kRK[RB1] * s.k1B))))), s.yB);
   quad_rhs(q, c, ynA, ynB, k7A, k7B, a7, e7o);
+  SP_LAT_MARK(LP_RHS);
   accn = qfma(hh, sb, s.acc);
   const T eA = hh * qfma(kRK[RE7], k7A, qfma(kRK[RE6], kA6, qfma(kRK[RE5], kA5, qfma(kRK[RE4], kA4, qfma(kRK[RE3], kA3, qfma(kRK[RE2], kA2, kRK[RE1] * s.k1A))))));
   const T eB = hh * qfma(kRK[RE7], k7B, qfma(kRK[RE6], kB6, qfma(kRK[RE5], kB5, qfma(kRK[RE4], kB4, qfma(kRK[RE3], kB3, qfma(kRK[RE2], kB2, kRK[RE1] * s.k1B))))));
@@ -290,8 +325,9 @@ SP_HD double quad_attempt(const Q& q, const QuadCoef<Q>& c, const QuadState<Q>& 
   const T qA = (eA * wA) * qrcp_fast(qfma(rtol, sA, atol));
   const T qB = (eB * SP_W_B) * qrcp_fast(qfma(rtol, qmax(qabs(s.yB), qabs(ynB)), atol));
   const T qc = (ec * SP_W_ACC) * qrcp_fast(qfma(rtol, qmax(qabs(s.acc), qabs(accn)), atol));
-  const double en2 = q.first(q.sum(qfma(qA, qA, qfma(qB, qB, qc * qc)))) * (1.0 / 12.0);
-  return (en2 == en2) ? en2 : INFINITY;   // NaN -> reject
+  // (a NaN is returned as it is: it rejects like +inf, and step_factor_sq gives both the smallest factor — no select
+  // on the controller's dependent path)
+  return q.first(q.sum(qfma(qA, qA, qfma(qB, qB, qc * qc)))) * (1.0 / 12.0);
 }
 
 // ------------------------------------------------------------------------------------------ stiff reaches
@@ -475,9 +511,8 @@ struct QuadCarry {
 //   void forcing(int day, double& P, double& E, double& doy, double& T_air);
 //   void upstream(int day, double (&us)[4]);
 //   void emit(const Q& q, int day, const double (&y)[NL], double Vr, const double (&acc)[NA], const double (&non)[13],
-//             const Cold& c);                    // kAllLanesEmit: called by every lane, else by the leader only
-//   static constexpr bool kAllLanesEmit;
-//   void publish(int day);                       // leader only
+//             const Cold& c);                    // called by every lane (device: the lanes share the work)
+//   void publish(int day);                       // leader only, after the emit of every lane
 //
 // The whole record of one (member, sub-catchment) item: replaces model.py:491-724 for it.
 // STIFF compiles the Rosenbrock path in (networks); without it every day takes the explicit pair (ensembles of one
@@ -504,6 +539,10 @@ SP_HD void run_quad(const Q& q, const double* mp, const double* sp, double A_qr0
     q.sync();
   }
   unsigned n_steps = 0, n_rej = 0, n_rhs = 0;
+#if defined(SP_LAT_PROBE) && defined(__CUDA_ARCH__)
+  LatProbe lp = {};
+  lp.t = clock64();
+#endif
 #ifdef SP_TIMELINE
   unsigned sp_lockstep_iters = 0;
 #endif
@@ -567,6 +606,11 @@ SP_HD void run_quad(const Q& q, const double* mp, const double* sp, double A_qr0
     bool active = true;
     hstep = sp_min(hstep * SP_DAYSTART_FAC, T1);  // the forcing jumps at midnight
     if (stiff) hstep = sp_min(hstep, SP_H0_STIFF_C * sp_rcp(day_rate));
+    // hstep * 1.0000001 (the test for the day's last step), carried beside hstep: after an accepted step it is formed
+    // from the new step beside the comparison that chooses it, not after it, off the controller's dependent path (the
+    // network builds, STIFF, form it from hstep where it is used: their 3-blocks build would spill the extra register)
+    double hlim = hstep * 1.0000001;
+    SP_LAT_MARK(LP_START);
 
     // ---- step loop: lock-step over the quads of a warp ------------------------------------------
     while (q.any(active)) {
@@ -577,14 +621,15 @@ SP_HD void run_quad(const Q& q, const double* mp, const double* sp, double A_qr0
       ++sp_lockstep_iters;                        // analysis builds: attempts the WARP executed (lock-step)
 #endif
       const double rem = T1 - t;
-      const bool last = hstep * 1.0000001 >= rem;
+      const bool last = (STIFF ? hstep * 1.0000001 : hlim) >= rem;   // (networks: one register fewer, no spill)
       const double hh = active ? (last ? rem : hstep) : hstep;
       const bool do_rk = active && !stiff, do_ros = active && stiff;
       T ynA, ynB, accn;
       double en2 = 0.0, expo = -0.1;
       if (!STIFF || q.any(do_rk) || !q.any(do_ros)) {
         T k7A, k7B, a7, e7;
-        const double e2 = quad_attempt(q, qc, s, hh, opt.rtol, opt.atol, ynA, ynB, accn, k7A, k7B, a7, e7);
+        const double e2 = quad_attempt(q, qc, s, hh, opt.rtol, opt.atol, ynA, ynB, accn, k7A, k7B, a7, e7 SP_LAT_ARG);
+        SP_LAT_MARK(LP_ERR);
         if (do_rk) {
           en2 = e2 * tol_inv2;
           n_rhs += 6;
@@ -618,7 +663,9 @@ SP_HD void run_quad(const Q& q, const double* mp, const double* sp, double A_qr0
           accept = true;                          // forward-progress guard
           status |= 1;
         }
-        double fac = step_factor_sq(en2, expo);
+        // the factor's cap (1 after a rejection and on the step after one) is known before the factor: it is applied
+        // inside the fp32 clamp instead of as a double min after it
+        const double fac = step_factor_sq(en2, expo, (accept && grow_ok) ? SP_CTRL_MAXGROW : 1.0);
 #ifdef SP_ATTEMPT_HOOK
         SP_ATTEMPT_HOOK(io, day, day_steps, t, hh, en2, accept);   // analysis builds only (scripts/)
 #endif
@@ -626,17 +673,21 @@ SP_HD void run_quad(const Q& q, const double* mp, const double* sp, double A_qr0
           t += hh;
           s.yA = ynA; s.yB = ynB; s.acc = accn;
           if (stiff) jac_fresh = false;           // (the explicit path took its FSAL derivative above)
-          if (!grow_ok) fac = sp_min(fac, 1.0);
           grow_ok = true;
           const double hnew = hh * fac;
-          hstep = (last && hnew < hstep) ? hstep : hnew;
+          const bool keep = last && hnew < hstep;
+          hlim = keep ? hlim : hnew * 1.0000001;
+          hstep = keep ? hstep : hnew;
           if (last) active = false;
         } else {
           n_rej += 1;
-          hstep = hh * sp_min(fac, 1.0);
+          hstep = hh * fac;
+          hlim = hstep * 1.0000001;
           grow_ok = false;
         }
       }
+      SP_LAT_MARK(LP_CTRL);
+      SP_LAT_COUNT(LP_ITERS);
     }
 
     // ---- end of the day: post-ODE algebra (:643-724), output --------------------------------------
@@ -664,25 +715,16 @@ SP_HD void run_quad(const Q& q, const double* mp, const double* sp, double A_qr0
       // along that direction is never damped and would random-walk over a 30-year record, so the volume carried
       // into the next day is put back on the curve (the reported Vr is the integrated one).
       s.yB = q.pick(y[iMsus], y[iTDPr], y[iPPr], sp_exp((1.0 - h.bQ) * u_end) * sp_rcp(h.cR));
-      if (IO::kAllLanesEmit) {                     // full output: the row is stored by all four lanes of the quad
-        if (valid) io.emit(q, day, yraw, Vr, acc, non, c);
-        q.sync();                                 // the row is complete before the leader publishes the day
-        if (q.leader()) {
-          qm.c = c;
-          if (valid) io.publish(day);
-        }
-      } else {                                    // calibration: the leader alone updates the statistics
-        q.sync();
-        if (q.leader()) {
-          qm.c = c;
-          if (valid) {
-            io.emit(q, day, yraw, Vr, acc, non, c);
-            io.publish(day);
-          }
-        }
+      if (valid) io.emit(q, day, yraw, Vr, acc, non, c);   // by every lane: the lanes share the row / the series
+      q.sync();                                   // every lane has read qm.c (above) and stored its part of the row
+      if (q.leader()) {                           // before the leader rewrites qm.c and publishes the day
+        qm.c = c;
+        if (valid) io.publish(day);
       }
-      q.sync();
+      q.sync();                                   // tomorrow's begin_day of every lane reads the new qm.c
     }
+    SP_LAT_MARK(LP_END);
+    SP_LAT_COUNT(LP_DAYS);
   }
   if (hand_over) {
     const double a0 = q.first(q.bcast(s.yA, 0)), a1 = q.first(q.bcast(s.yA, 1)), a2 = q.first(q.bcast(s.yA, 2)),
@@ -705,6 +747,9 @@ SP_HD void run_quad(const Q& q, const double* mp, const double* sp, double A_qr0
 #endif
   cnt.rhs_evals = n_rhs;
   cnt.status = status;
+#if defined(SP_LAT_PROBE) && defined(__CUDA_ARCH__)
+  for (int i = 0; i < LP_N; ++i) cnt.lat[i] = lp.acc[i];
+#endif
   (void)Kf;
 }
 
