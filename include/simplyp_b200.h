@@ -490,6 +490,51 @@ int simplyp_sobol_indices_device(const SimplypSobol* sb, const double* y, int64_
                                  double* ST_conf, double* S2, double* S2_conf, double* mean, double* var,
                                  int64_t* n_used, void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- Morris elementary-effects screening ---------------------------------------------------------------------------
+ * SALib's morris.sample / morris.analyze on the device.  K free parameters (the sampler's targets and boxes,
+ * SimplypMcmcParam), p = num_levels, r = n_trajectories of K + 1 design members each; Delta = p / (2 (p - 1)).
+ * Trajectories, levels, the Philox counters (c, q, 0, 6) and (b, q, 1, 6) and the distance of the optimised selection
+ * are documented in csrc/simplyp_morris.cuh.
+ *
+ * simplyp_morris_select_device (n_candidates > 0 only): the r trajectories of the Campolongo spread criterion among
+ *   candidates 0..n_candidates-1 by Ruano et al.'s greedy search (not SALib's routine): selected[r] int32 on the
+ *   device, in the order they were chosen.  Needs simplyp_morris_workspace_bytes(mo, 0) bytes of workspace.
+ * simplyp_morris_design_device: overwrites the target columns of design members [member_offset, member_offset + n)
+ *   of member_params [r (K+1)][NP_MEMBER] and sc_params [r (K+1)][S][NP_SC] (or [1][S][NP_SC] without SC targets).
+ *   Member m = i (K+1) + s is point s of trajectory i, which is candidate selected[i] (candidate i when n_candidates
+ *   is 0; selected may then be NULL).  Value = min(lo + (hi - lo) (level / (p - 1)), hi), each operation rounded.
+ * simplyp_morris_effects_device: per row of Y[n_rows][r (K+1)] (member-major, as the design; the outputs of
+ *   simplyp_sobol_outputs_device or of simplyp_predictive_draws_device), trajectory i used when its K+1 values are all
+ *   finite (n used).  EE_ij = (y at the higher point - y at the lower point) / Delta for the step that moves j;
+ *   mu, mu_star = means of EE and |EE| over the used trajectories, sigma = std (ddof 1) of EE; mu_star_conf = conf_z
+ *   std (ddof 1) of mu_star over n_boot resamples of the used trajectories, drawn with the struct's seed.  NaN where
+ *   n < 2, and mu_star_conf NaN with n_boot < 2.  Outputs [n_rows][K], n_used [n_rows].  Sums run in a fixed order: results are bitwise
+ *   reproducible.  Needs simplyp_morris_workspace_bytes(mo, n_rows) bytes of workspace.
+ * All three only enqueue work on `stream` (no allocation, no synchronisation), so they can be captured into a graph. */
+#define SIMPLYP_MORRIS_MAX_CANDIDATES 8192
+typedef struct {
+  int32_t n_free;           /* K: 1..SIMPLYP_MCMC_MAX_FREE */
+  int32_t n_sc;             /* S of the design's runs */
+  int32_t sc_per_member;    /* sc_params is [r (K+1)][S][NP_SC] (required by the SC targets) */
+  int32_t num_levels;       /* p: even, 2..16 */
+  int32_t n_trajectories;   /* r >= 2 */
+  int32_t n_candidates;     /* 0 (trajectory i is candidate i) or r < n_candidates <= SIMPLYP_MORRIS_MAX_CANDIDATES */
+  uint64_t seed;            /* Philox key: (low word, high word) */
+  SimplypMcmcParam param[SIMPLYP_MCMC_MAX_FREE];
+} SimplypMorris;
+
+/* Workspace bytes that both simplyp_morris_select_device and simplyp_morris_effects_device over n_rows rows can use
+ * (the larger of their needs; n_rows = 0: the selection alone). */
+int64_t simplyp_morris_workspace_bytes(const SimplypMorris* mo, int64_t n_rows);
+int simplyp_morris_select_device(const SimplypMorris* mo, int32_t* selected, void* workspace, int64_t workspace_bytes,
+                                 void* stream);
+int simplyp_morris_design_device(const SimplypMorris* mo, const int32_t* selected, int64_t member_offset,
+                                 int64_t n_members, double* member_params, double* sc_params, void* stream);
+int simplyp_morris_effects_device(const SimplypMorris* mo, const int32_t* selected, const double* y, int64_t n_rows,
+                                  int32_t n_boot, double conf_z, double* mu, double* mu_star,
+                                  double* sigma, double* mu_star_conf, int64_t* n_used, void* workspace,
+                                  int64_t workspace_bytes, void* stream);
+
 /* ---- differential evolution ---------------------------------------------------------------------------------------
  * scipy.optimize.differential_evolution(updating='deferred', polish=False) over the fit statistics: the best parameter
  * set of K free parameters (the sampler's targets and boxes, SimplypMcmcParam) in a population of N members.  The

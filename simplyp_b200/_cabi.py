@@ -31,6 +31,8 @@ EXPORTS = [
     "simplyp_de_select_device", "simplyp_de_init_device", "simplyp_period_aggregates_device",
     "simplyp_calibrate_ar1_device", "simplyp_de_scale_device", "simplyp_nsga2_workspace_bytes",
     "simplyp_nsga2_init_device", "simplyp_nsga2_offspring_device", "simplyp_nsga2_survive_device",
+    "simplyp_morris_workspace_bytes", "simplyp_morris_select_device", "simplyp_morris_design_device",
+    "simplyp_morris_effects_device",
 ]
 MAX_RANKS = 8
 
@@ -63,6 +65,7 @@ MCMC_MEMBER, MCMC_SC_ALL, MCMC_SC_AT, MCMC_ERROR_MODEL = 0, 1, 2, 3
 AR1_MAX_SERIES = 64
 DE_STRATEGIES = {"best1bin": 0, "rand1bin": 1}
 NSGA2_MAX_OBJECTIVES = 16
+MORRIS_MAX_CANDIDATES = 8192
 
 
 class SimplypMcmcParam(C.Structure):
@@ -85,6 +88,12 @@ class SimplypMcmcState(C.Structure):
 class SimplypSobol(C.Structure):
     _fields_ = [("n_free", C.c_int32), ("n_sc", C.c_int32), ("sc_per_member", C.c_int32), ("second_order", C.c_int32),
                 ("n_base", C.c_int64), ("skip", C.c_int64), ("param", SimplypMcmcParam * MCMC_MAX_FREE)]
+
+
+class SimplypMorris(C.Structure):
+    _fields_ = [("n_free", C.c_int32), ("n_sc", C.c_int32), ("sc_per_member", C.c_int32), ("num_levels", C.c_int32),
+                ("n_trajectories", C.c_int32), ("n_candidates", C.c_int32), ("seed", C.c_uint64),
+                ("param", SimplypMcmcParam * MCMC_MAX_FREE)]
 
 
 class SimplypDe(C.Structure):
@@ -227,6 +236,16 @@ def load():
     for name in ("simplyp_nsga2_init_device", "simplyp_nsga2_offspring_device", "simplyp_nsga2_survive_device"):
         getattr(lib, name).argtypes = [nsp, nssp, vp, vp, vp]
         getattr(lib, name).restype = C.c_int
+    mop = C.POINTER(SimplypMorris)
+    lib.simplyp_morris_workspace_bytes.argtypes = [mop, C.c_int64]
+    lib.simplyp_morris_workspace_bytes.restype = C.c_int64
+    lib.simplyp_morris_select_device.argtypes = [mop, vp, vp, C.c_int64, vp]
+    lib.simplyp_morris_select_device.restype = C.c_int
+    lib.simplyp_morris_design_device.argtypes = [mop, vp, C.c_int64, C.c_int64, vp, vp, vp]
+    lib.simplyp_morris_design_device.restype = C.c_int
+    lib.simplyp_morris_effects_device.argtypes = [mop, vp, vp, C.c_int64, C.c_int32, C.c_double, vp, vp, vp, vp, vp,
+                                                  vp, C.c_int64, vp]
+    lib.simplyp_morris_effects_device.restype = C.c_int
     if lib.simplyp_abi_version() != 4:
         raise SimplypError("ABI version mismatch")
     _lib = lib
@@ -452,8 +471,8 @@ def _u64(seed):
 
 
 def _free_params(spec, targets, lo, hi):
-    """``spec`` (SimplypMcmc, SimplypSobol, SimplypDe or SimplypNsga2) with ``n_free`` and ``param`` set to the free
-    parameters ``targets`` [(kind, index, pos)] (``MCMC_MEMBER`` / ``MCMC_SC_ALL`` / ``MCMC_SC_AT`` /
+    """``spec`` (SimplypMcmc, SimplypSobol, SimplypMorris, SimplypDe or SimplypNsga2) with ``n_free`` and ``param``
+    set to the free parameters ``targets`` [(kind, index, pos)] (``MCMC_MEMBER`` / ``MCMC_SC_ALL`` / ``MCMC_SC_AT`` /
     ``MCMC_ERROR_MODEL``) and their boxes ``[lo[k], hi[k]]``."""
     if not 1 <= len(targets) <= MCMC_MAX_FREE:
         raise ValueError("1..%d free parameters" % MCMC_MAX_FREE)
@@ -581,6 +600,41 @@ def sobol_indices_device(sb, y_ptr, n_rows, n_boot, conf_z, seed, S1, ST, S1_con
     _check(lib.simplyp_sobol_indices_device(C.byref(sb), y_ptr, int(n_rows), int(n_boot), float(conf_z),
                                             _u64(seed), S1, ST, S1_conf, ST_conf, S2, S2_conf,
                                             mean, var, n_used, ws_ptr, int(ws_bytes), stream_ptr))
+
+
+def make_morris(targets, lo, hi, n_sc, n_trajectories, num_levels=4, n_candidates=0, sc_per_member=False, seed=0):
+    """SimplypMorris for ``targets`` [(kind, index, pos)] (as :func:`make_mcmc`) with the boxes ``[lo[k], hi[k]]``;
+    ``n_candidates`` 0 takes trajectory i from candidate i."""
+    mo = _free_params(SimplypMorris(), targets, lo, hi)
+    mo.n_sc, mo.sc_per_member, mo.num_levels = int(n_sc), 1 if sc_per_member else 0, int(num_levels)
+    mo.n_trajectories, mo.n_candidates, mo.seed = int(n_trajectories), int(n_candidates or 0), _u64(seed)
+    return mo
+
+
+def morris_workspace_bytes(mo, n_rows):
+    n = load().simplyp_morris_workspace_bytes(C.byref(mo), int(n_rows))
+    if n < 0:
+        _check(int(n))
+    return int(n)
+
+
+def morris_select_device(mo, selected_ptr, ws_ptr, ws_bytes, stream_ptr):
+    """Indices selected [r] int32 of the optimised trajectories; asynchronous on ``stream_ptr``."""
+    _check(require_device().simplyp_morris_select_device(C.byref(mo), selected_ptr, ws_ptr, int(ws_bytes), stream_ptr))
+
+
+def morris_design_device(mo, selected_ptr, member_offset, n_members, member_ptr, sc_ptr, stream_ptr):
+    """Target columns of design members [member_offset, member_offset + n_members); asynchronous on ``stream_ptr``."""
+    _check(require_device().simplyp_morris_design_device(C.byref(mo), selected_ptr, int(member_offset), int(n_members),
+                                                         member_ptr, sc_ptr, stream_ptr))
+
+
+def morris_effects_device(mo, selected_ptr, y_ptr, n_rows, n_boot, conf_z, mu, mu_star, sigma, mu_star_conf, n_used,
+                          ws_ptr, ws_bytes, stream_ptr):
+    """Elementary-effect statistics of every row of Y [n_rows][r (K + 1)]; asynchronous on ``stream_ptr``."""
+    _check(require_device().simplyp_morris_effects_device(C.byref(mo), selected_ptr, y_ptr, int(n_rows), int(n_boot),
+                                                          float(conf_z), mu, mu_star, sigma, mu_star_conf, n_used,
+                                                          ws_ptr, int(ws_bytes), stream_ptr))
 
 
 def make_de(n_population, targets, lo, hi, n_sc, n_rows, sc_per_member=False, strategy="best1bin",

@@ -46,6 +46,7 @@
 #include "simplyp_de.cuh"
 #include "simplyp_nsga2.cuh"
 #include "simplyp_ar1.cuh"
+#include "simplyp_morris.cuh"
 
 using namespace simplyp;
 
@@ -2268,6 +2269,371 @@ int64_t sobol_pass_rows(const SimplypSobol& sb, int64_t n_rows) {
   return rows < n_rows ? rows : n_rows;
 }
 
+// ------------------------------------------------------------------------------------------ Morris screening
+// Selection (simplyp_morris.cuh holds the trajectory and distance arithmetic).  The candidates' stored trajectories
+// go to the workspace once; the all-pairs pass gives each block a 32 x 32 tile of pairs; every greedy step adds the
+// newest selected candidate's squared distances to the scores of the others.  Both passes end with the last block
+// to finish (a ticket counter) reducing the blocks' best entries to the next selected index, so a step is one
+// launch.  The order of (value desc, index asc) is total, so the reduction order does not change the result.
+constexpr int MO_THREADS = 256;
+constexpr int MO_TILE = 32;
+constexpr int MO_GROUPS = 8;                         // bootstrap blocks a row
+constexpr int MO_SLOTS = MO_GROUPS * (MO_THREADS / 32);
+
+struct MorrisSelectWs {
+  uint8_t* traj;      // [nc][4K]
+  double* score;      // [nc]
+  uint8_t* flag;      // [nc] 1: selected
+  double* best_v;     // [blocks]
+  long long* best_k;  // [blocks]
+  unsigned* ticket;
+  static int64_t up8(int64_t b) { return (b + 7) & ~7ll; }
+  static int64_t tiles(int nc) { return (nc + MO_TILE - 1) / MO_TILE; }
+  static int64_t blocks(int nc) {
+    const int64_t t = tiles(nc), s = (nc + MO_THREADS - 1) / MO_THREADS;
+    return t * t > s ? t * t : s;
+  }
+  static int64_t bytes(int nc, int K) {
+    return up8((int64_t)nc * 4 * K) + 8ll * nc + up8(nc) + 16 * blocks(nc) + 8;
+  }
+  MorrisSelectWs(void* ws, int nc, int K) {
+    char* p = static_cast<char*>(ws);
+    traj = reinterpret_cast<uint8_t*>(p);
+    p += up8((int64_t)nc * 4 * K);
+    score = reinterpret_cast<double*>(p);
+    p += 8ll * nc;
+    flag = reinterpret_cast<uint8_t*>(p);
+    p += up8(nc);
+    best_v = reinterpret_cast<double*>(p);
+    p += 8 * blocks(nc);
+    best_k = reinterpret_cast<long long*>(p);
+    p += 8 * blocks(nc);
+    ticket = reinterpret_cast<unsigned*>(p);
+  }
+};
+
+__device__ __forceinline__ bool mo_better(double v, long long k, double bv, long long bk) {
+  return v > bv || (v == bv && k < bk);
+}
+
+// Best (value, index) of the block into the thread 0's v, k.
+__device__ void mo_block_best(double& v, long long& k) {
+  __shared__ double sv[MO_THREADS / 32];
+  __shared__ long long sk[MO_THREADS / 32];
+  for (int o = 16; o > 0; o >>= 1) {
+    const double ov = __shfl_xor_sync(0xffffffffu, v, o);
+    const long long ok = __shfl_xor_sync(0xffffffffu, k, o);
+    if (mo_better(ov, ok, v, k)) v = ov, k = ok;
+  }
+  const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
+  __syncthreads();
+  if (lane == 0) sv[warp] = v, sk[warp] = k;
+  __syncthreads();
+  if (threadIdx.x == 0)
+    for (int w = 1; w < MO_THREADS / 32; ++w)
+      if (mo_better(sv[w], sk[w], v, k)) v = sv[w], k = sk[w];
+}
+
+// Publishes the block's best; true in every thread of the last block to finish, which then reduces all of them.
+__device__ bool mo_publish(const MorrisSelectWs& w, double v, long long k) {
+  __shared__ bool last;
+  mo_block_best(v, k);
+  const unsigned nb = gridDim.x * gridDim.y, b = blockIdx.y * gridDim.x + blockIdx.x;
+  if (threadIdx.x == 0) {
+    w.best_v[b] = v;
+    w.best_k[b] = k;
+    __threadfence();
+    last = atomicAdd(w.ticket, 1u) == nb - 1;
+  }
+  __syncthreads();
+  return last;
+}
+
+// The last block's reduction of the published bests: the overall best index (-1 if none).
+__device__ long long mo_final(const MorrisSelectWs& w) {
+  __threadfence();
+  double v = -1.0;
+  long long k = LLONG_MAX;
+  const unsigned nb = gridDim.x * gridDim.y;
+  for (unsigned b = threadIdx.x; b < nb; b += MO_THREADS) {
+    const double bv = __ldcg(w.best_v + b);
+    const long long bk = __ldcg(w.best_k + b);
+    if (mo_better(bv, bk, v, k)) v = bv, k = bk;
+  }
+  mo_block_best(v, k);
+  return v >= 0.0 ? k : -1;
+}
+
+__global__ void morris_traj_kernel(const SimplypMorris mo, MorrisSelectWs w) {
+  const int c = blockIdx.x * blockDim.x + threadIdx.x;
+  if (c == 0) *w.ticket = 0u;
+  if (c >= mo.n_candidates) return;
+  morris_traj_pack(mo.seed, (uint32_t)c, mo.n_free, mo.num_levels, w.traj + (size_t)c * 4 * mo.n_free);
+  w.score[c] = 0.0;
+  w.flag[c] = 0;
+}
+
+__global__ void __launch_bounds__(MO_THREADS) morris_pairs_kernel(const SimplypMorris mo, MorrisSelectWs w,
+                                                                  int32_t* selected) {
+  __shared__ uint8_t tile[2][MO_TILE][4 * SIMPLYP_MCMC_MAX_FREE];
+  const int K = mo.n_free, nc = mo.n_candidates, h = mo.num_levels / 2, row = 4 * K;
+  const int m0 = blockIdx.y * MO_TILE, l0 = blockIdx.x * MO_TILE;
+  double v = -1.0;
+  long long k = LLONG_MAX;
+  if (l0 + MO_TILE - 1 > m0) {
+    for (int q = threadIdx.x; q < 2 * MO_TILE * row; q += MO_THREADS) {
+      const int side = q / (MO_TILE * row), rem = q % (MO_TILE * row), t = rem / row, b = rem % row;
+      const int c = (side ? l0 : m0) + t;
+      tile[side][t][b] = c < nc ? w.traj[(size_t)c * row + b] : 0;
+    }
+    __syncthreads();
+    for (int q = threadIdx.x; q < MO_TILE * MO_TILE; q += MO_THREADS) {
+      const int m = m0 + q / MO_TILE, l = l0 + q % MO_TILE;
+      if (m < l && l < nc) {
+        const double d = morris_distance(tile[0][q / MO_TILE], tile[1][q % MO_TILE], K, h);
+        const long long key = (long long)m * nc + l;
+        if (mo_better(d, key, v, k)) v = d, k = key;
+      }
+    }
+  }
+  if (!mo_publish(w, v, k)) return;
+  const long long best = mo_final(w);
+  if (threadIdx.x == 0) {
+    const int m = (int)(best / nc), l = (int)(best % nc);
+    selected[0] = m;
+    selected[1] = l;
+    w.flag[m] = w.flag[l] = 1;
+    *w.ticket = 0u;
+  }
+}
+
+// Greedy step: scores += d(c, selected[step])^2, then (pick) selected[step + 1] = the best unselected candidate.
+__global__ void __launch_bounds__(MO_THREADS) morris_step_kernel(const SimplypMorris mo, MorrisSelectWs w,
+                                                                 int32_t* selected, int step, int pick) {
+  __shared__ uint8_t ts[4 * SIMPLYP_MCMC_MAX_FREE];
+  const int K = mo.n_free, nc = mo.n_candidates, h = mo.num_levels / 2, row = 4 * K;
+  const int s = selected[step];
+  for (int b = threadIdx.x; b < row; b += MO_THREADS) ts[b] = w.traj[(size_t)s * row + b];
+  __syncthreads();
+  const int c = blockIdx.x * MO_THREADS + threadIdx.x;
+  double v = -1.0;
+  long long k = LLONG_MAX;
+  if (c < nc && !w.flag[c]) {
+    const uint8_t* tc = w.traj + (size_t)c * row;
+    const double d = c < s ? morris_distance(tc, ts, K, h) : morris_distance(ts, tc, K, h);
+    v = mc_add(w.score[c], mc_mul(d, d));
+    w.score[c] = v;
+    k = c;
+  }
+  if (!pick || !mo_publish(w, v, k)) return;
+  const long long best = mo_final(w);
+  if (threadIdx.x == 0) {
+    selected[step + 1] = (int32_t)best;
+    w.flag[best] = 1;
+    *w.ticket = 0u;
+  }
+}
+
+// Design: one thread per member row.
+__global__ void morris_design_kernel(const SimplypMorris mo, const int32_t* selected, long long member_offset,
+                                     long long n, double* member_params, double* sc_params) {
+  const long long idx = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= n) return;
+  const long long m = member_offset + idx;
+  const int K = mo.n_free, S = mo.n_sc, p = mo.num_levels;
+  const long long i = m / (K + 1);
+  const int s = (int)(m - i * (K + 1));
+  uint8_t t[4 * SIMPLYP_MCMC_MAX_FREE];
+  morris_traj_pack(mo.seed, (uint32_t)(selected ? selected[i] : i), K, p, t);
+  double* mrow = member_params + (size_t)m * SIMPLYP_NP_MEMBER;
+  double* srow = sc_params + (mo.sc_per_member ? (size_t)m * S * SIMPLYP_NP_SC : 0);
+  for (int j = 0; j < K; ++j)
+    mcmc_write_target(mo.param[j], S, morris_value(mo.param[j], morris_level(t, K, p / 2, s, j), p), mrow, srow);
+}
+
+// Effects.  steps[i][2K]: the parameter moved by step s + 1 of trajectory i and whether it moved down.
+__global__ void morris_steps_kernel(const SimplypMorris mo, const int32_t* selected, uint8_t* steps) {
+  const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= mo.n_trajectories) return;
+  const int K = mo.n_free;
+  uint8_t t[4 * SIMPLYP_MCMC_MAX_FREE];
+  morris_traj_pack(mo.seed, (uint32_t)(selected ? selected[i] : i), K, mo.num_levels, t);
+  for (int s = 0; s < K; ++s) {
+    const int j = t[2 * K + s];
+    steps[(size_t)i * 2 * K + s] = (uint8_t)j;
+    steps[(size_t)i * 2 * K + K + s] = t[3 * K + j];
+  }
+}
+
+// One block a row: the used trajectories (in order) into used_ws, their EE into ee_ws [r][K], and the point
+// statistics.  Parameter j's sums split the used trajectories into MO_THREADS / 64 contiguous parts, added in order.
+__global__ void __launch_bounds__(MO_THREADS) morris_point_kernel(const SimplypMorris mo, const double* y,
+                                                                  long long row0, const uint8_t* steps, int* used_ws,
+                                                                  double* ee_ws, double* mu, double* mu_star,
+                                                                  double* sigma, int64_t* n_used) {
+  constexpr int PARTS = MO_THREADS / SIMPLYP_MCMC_MAX_FREE;
+  __shared__ int wcount[MO_THREADS / 32];
+  __shared__ double part[3][PARTS][SIMPLYP_MCMC_MAX_FREE];
+  const int K = mo.n_free, P = K + 1, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const long long N = mo.n_trajectories, rl = blockIdx.x, r = row0 + rl;
+  const double* yr = y + (size_t)r * N * P;
+  int* used = used_ws + (size_t)rl * N;
+  double* ee = ee_ws + (size_t)rl * N * K;
+  const double delta = morris_delta(mo.num_levels);
+  long long n = 0;
+  for (long long i0 = 0; i0 < N; i0 += MO_THREADS) {
+    const long long i = i0 + tid;
+    bool ok = i < N;
+    for (int e = 0; ok && e < P; ++e) ok = isfinite(yr[(size_t)i * P + e]);
+    if (ok) {
+      const uint8_t* st = steps + (size_t)i * 2 * K;
+      for (int s = 1; s <= K; ++s) {
+        const double a = yr[(size_t)i * P + s - 1], b = yr[(size_t)i * P + s];
+        ee[(size_t)i * K + st[s - 1]] = mc_div(st[K + s - 1] ? mc_sub(a, b) : mc_sub(b, a), delta);
+      }
+    }
+    const unsigned mask = __ballot_sync(0xffffffffu, ok);
+    if (lane == 0) wcount[warp] = __popc(mask);
+    __syncthreads();
+    long long off = n;
+    int total = 0;
+    for (int w = 0; w < MO_THREADS / 32; ++w) {
+      if (w < warp) off += wcount[w];
+      total += wcount[w];
+    }
+    if (ok) used[off + __popc(mask & ((1u << lane) - 1u))] = (int)i;
+    n += total;
+    __syncthreads();
+  }
+  const int j = tid % SIMPLYP_MCMC_MAX_FREE, pt = tid / SIMPLYP_MCMC_MAX_FREE;
+  const long long q0 = n * pt / PARTS, q1 = n * (pt + 1) / PARTS;
+  double s1 = 0.0, sa = 0.0;
+  if (j < K)
+    for (long long q = q0; q < q1; ++q) {
+      const double e = ee[(size_t)used[q] * K + j];
+      s1 += e;
+      sa += fabs(e);
+    }
+  part[0][pt][j] = s1;
+  part[1][pt][j] = sa;
+  __syncthreads();
+  double m1 = 0.0, ma = 0.0;
+  for (int u = 0; u < PARTS; ++u) {
+    m1 += part[0][u][j];
+    ma += part[1][u][j];
+  }
+  m1 /= (double)n;
+  double s2 = 0.0;
+  if (j < K)
+    for (long long q = q0; q < q1; ++q) {
+      const double d = ee[(size_t)used[q] * K + j] - m1;
+      s2 += d * d;
+    }
+  part[2][pt][j] = s2;
+  __syncthreads();
+  if (pt == 0 && j < K) {
+    double v = 0.0;
+    for (int u = 0; u < PARTS; ++u) v += part[2][u][j];
+    const bool ok = n >= 2;
+    mu[(size_t)r * K + j] = ok ? m1 : NAN;
+    mu_star[(size_t)r * K + j] = ok ? ma / (double)n : NAN;
+    sigma[(size_t)r * K + j] = ok ? sqrt(v / (double)(n - 1)) : NAN;
+  }
+  if (tid == 0) n_used[r] = n;
+}
+
+// Grid (MO_GROUPS, rows of the pass): warp slot u takes resamples u, u + MO_SLOTS, ...; lane l owns the parameters l
+// and l + 32.  part[row][u][2][K]: sums of e and e^2, e = resampled mu_star - mu_star.
+__global__ void __launch_bounds__(MO_THREADS) morris_boot_kernel(const SimplypMorris mo, long long row0,
+                                                                 const int* used_ws, const double* ee_ws, int n_boot,
+                                                                 const double* mu_star, const int64_t* n_used,
+                                                                 double* part) {
+  const int K = mo.n_free, lane = threadIdx.x & 31, u = blockIdx.x * (MO_THREADS / 32) + (threadIdx.x >> 5);
+  const long long N = mo.n_trajectories, rl = blockIdx.y, r = row0 + rl, n = n_used[r];
+  const int* used = used_ws + (size_t)rl * N;
+  const double* ee = ee_ws + (size_t)rl * N * K;
+  double d[2] = {0.0, 0.0}, dd[2] = {0.0, 0.0}, ms[2];
+#pragma unroll
+  for (int hh = 0; hh < 2; ++hh) ms[hh] = lane + 32 * hh < K ? mu_star[(size_t)r * K + lane + 32 * hh] : 0.0;
+  for (int t = u; n >= 2 && t < n_boot; t += MO_SLOTS) {
+    double acc[2] = {0.0, 0.0};
+    for (long long base = 0; base < n; base += 128) {
+      uint32_t w[4], pos[4];
+      morris_words(mo.seed, (uint32_t)t, (uint32_t)(base >> 2) + lane, 1u, w);
+#pragma unroll
+      for (int q = 0; q < 4; ++q) pos[q] = morris_pick(w[q], (uint32_t)n);
+      const int cnt = (int)(n - base < 128 ? n - base : 128);
+      for (int src = 0; src * 4 < cnt; ++src) {
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          const uint32_t pq = __shfl_sync(0xffffffffu, pos[q], src);
+          if (src * 4 + q < cnt) {
+            const double* e = ee + (size_t)used[pq] * K;
+#pragma unroll
+            for (int hh = 0; hh < 2; ++hh)
+              if (lane + 32 * hh < K) acc[hh] += fabs(e[lane + 32 * hh]);
+          }
+        }
+      }
+    }
+#pragma unroll
+    for (int hh = 0; hh < 2; ++hh) {
+      const double e = acc[hh] / (double)n - ms[hh];
+      d[hh] += e;
+      dd[hh] += e * e;
+    }
+  }
+  double* p = part + ((size_t)rl * MO_SLOTS + u) * 2 * K;
+#pragma unroll
+  for (int hh = 0; hh < 2; ++hh)
+    if (lane + 32 * hh < K) {
+      p[lane + 32 * hh] = d[hh];
+      p[K + lane + 32 * hh] = dd[hh];
+    }
+}
+
+// mu_star_conf = z std(ddof 1) over the resamples, from the per-slot sums added in slot order.
+__global__ void morris_conf_kernel(const SimplypMorris mo, long long row0, int n_boot, double z, const int64_t* n_used,
+                                   const double* part, double* conf) {
+  const int K = mo.n_free, j = threadIdx.x;
+  const long long rl = blockIdx.x, r = row0 + rl;
+  if (j >= K) return;
+  double d = 0.0, dd = 0.0;
+  for (int u = 0; u < MO_SLOTS; ++u) {
+    const double* p = part + ((size_t)rl * MO_SLOTS + u) * 2 * K;
+    d += p[j];
+    dd += p[K + j];
+  }
+  const double nb = (double)n_boot, v = (dd - d * d / nb) / (nb - 1.0);
+  conf[(size_t)r * K + j] = (n_boot >= 2 && n_used[r] >= 2) ? z * sqrt(v > 0.0 ? v : 0.0) : NAN;
+}
+
+int check_morris(const SimplypMorris* mo) {
+  if (!mo) return fail(SIMPLYP_EINVAL, "morris: null argument%s");
+  const int K = mo->n_free, p = mo->num_levels, r = mo->n_trajectories, nc = mo->n_candidates;
+  if (K < 1 || K > SIMPLYP_MCMC_MAX_FREE) return fail(SIMPLYP_EINVAL, "morris: 1..SIMPLYP_MCMC_MAX_FREE free parameters%s");
+  if (mo->n_sc < 1 || (mo->sc_per_member != 0 && mo->sc_per_member != 1))
+    return fail(SIMPLYP_EINVAL, "morris: bad n_sc / sc_per_member%s");
+  if (p < 2 || p > 16 || p % 2 != 0) return fail(SIMPLYP_EINVAL, "morris: num_levels must be even, 2..16%s");
+  if (r < 2) return fail(SIMPLYP_EINVAL, "morris: n_trajectories must be >= 2%s");
+  if (nc != 0 && (nc <= r || nc > SIMPLYP_MORRIS_MAX_CANDIDATES))
+    return fail(SIMPLYP_EINVAL, "morris: n_candidates must be 0 or in n_trajectories + 1 .. SIMPLYP_MORRIS_MAX_CANDIDATES%s");
+  return check_targets(mo->param, K, mo->n_sc, mo->sc_per_member, "morris");
+}
+
+// Effects workspace: the steps table, then per row of a pass the used list, the EE matrix and the bootstrap sums.
+int64_t morris_steps_bytes(const SimplypMorris& mo) { return ((int64_t)mo.n_trajectories * 2 * mo.n_free + 7) & ~7ll; }
+int64_t morris_row_bytes(const SimplypMorris& mo) {
+  const int64_t N = mo.n_trajectories, K = mo.n_free;
+  return ((4 * N + 7) & ~7ll) + 8 * N * K + 8ll * MO_SLOTS * 2 * K;
+}
+int64_t morris_pass_rows(const SimplypMorris& mo, int64_t n_rows) {
+  int64_t rows = SB_PASS_BYTES / morris_row_bytes(mo);
+  if (rows < 1) rows = 1;
+  if (rows > 65535) rows = 65535;
+  return rows < n_rows ? rows : n_rows;
+}
+
 // ------------------------------------------------------------------------------------------ differential evolution
 // One thread per member (simplyp_de.cuh holds the arithmetic); once converged is set every kernel returns at once.
 __global__ void de_trial_kernel(const SimplypDe de, const SimplypDeState st, double* member_params, double* sc_params) {
@@ -3506,6 +3872,97 @@ int simplyp_nsga2_offspring_device(const SimplypNsga2* ns, const SimplypNsga2Sta
 int simplyp_nsga2_survive_device(const SimplypNsga2* ns, const SimplypNsga2State* state, const double* y,
                                  const int64_t* diag, void* stream) {
   return nsga2_survive(ns, state, y, diag, stream, 0);
+}
+
+int64_t simplyp_morris_workspace_bytes(const SimplypMorris* mo, int64_t n_rows) {
+  const int rc = check_morris(mo);
+  if (rc) return rc;
+  if (n_rows < 0) return fail(SIMPLYP_EINVAL, "morris: negative row count%s");
+  const int64_t sel = mo->n_candidates ? MorrisSelectWs::bytes(mo->n_candidates, mo->n_free) : 0;
+  const int64_t eff = n_rows ? morris_steps_bytes(*mo) + morris_pass_rows(*mo, n_rows) * morris_row_bytes(*mo) : 0;
+  return sel > eff ? sel : eff;
+}
+
+int simplyp_morris_select_device(const SimplypMorris* mo, int32_t* selected, void* workspace, int64_t workspace_bytes,
+                                 void* stream) {
+  const int rc = check_morris(mo);
+  if (rc) return rc;
+  if (mo->n_candidates == 0) return fail(SIMPLYP_EINVAL, "morris select: n_candidates is 0, nothing to select%s");
+  if (!selected) return fail(SIMPLYP_EINVAL, "morris select: null selected%s");
+  const int nc = mo->n_candidates, K = mo->n_free, r = mo->n_trajectories;
+  if (!workspace || workspace_bytes < MorrisSelectWs::bytes(nc, K))
+    return fail(SIMPLYP_EINVAL, "morris select: workspace smaller than simplyp_morris_workspace_bytes%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  MorrisSelectWs w(workspace, nc, K);
+  const unsigned tiles = (unsigned)MorrisSelectWs::tiles(nc), blocks = (unsigned)((nc + MO_THREADS - 1) / MO_THREADS);
+  morris_traj_kernel<<<blocks, MO_THREADS, 0, st>>>(*mo, w);
+  morris_pairs_kernel<<<dim3(tiles, tiles), MO_THREADS, 0, st>>>(*mo, w, selected);
+  g_launches.fetch_add(2);
+  SP_CUDA(cudaGetLastError());
+  for (int k = 0; r > 2 && k < r - 1; ++k) {
+    morris_step_kernel<<<blocks, MO_THREADS, 0, st>>>(*mo, w, selected, k, k >= 1);
+    g_launches.fetch_add(1);
+    SP_CUDA(cudaGetLastError());
+  }
+  return SIMPLYP_OK;
+}
+
+int simplyp_morris_design_device(const SimplypMorris* mo, const int32_t* selected, int64_t member_offset,
+                                 int64_t n_members, double* member_params, double* sc_params, void* stream) {
+  const int rc = check_morris(mo);
+  if (rc) return rc;
+  if (!member_params || !sc_params || (mo->n_candidates && !selected))
+    return fail(SIMPLYP_EINVAL, "morris design: null parameter rows or selected indices%s");
+  const int64_t total = (int64_t)mo->n_trajectories * (mo->n_free + 1);
+  if (member_offset < 0 || n_members < 0 || member_offset + n_members > total)
+    return fail(SIMPLYP_EINVAL, "morris design: members outside 0 .. n_trajectories * (K + 1) - 1%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  if (n_members == 0) return SIMPLYP_OK;
+  morris_design_kernel<<<(unsigned)((n_members + 127) / 128), 128, 0, static_cast<cudaStream_t>(stream)>>>(
+      *mo, mo->n_candidates ? selected : nullptr, member_offset, n_members, member_params, sc_params);
+  g_launches.fetch_add(1);
+  SP_CUDA(cudaGetLastError());
+  return SIMPLYP_OK;
+}
+
+int simplyp_morris_effects_device(const SimplypMorris* mo, const int32_t* selected, const double* y, int64_t n_rows,
+                                  int32_t n_boot, double conf_z, double* mu, double* mu_star, double* sigma,
+                                  double* mu_star_conf, int64_t* n_used, void* workspace, int64_t workspace_bytes,
+                                  void* stream) {
+  const int rc = check_morris(mo);
+  if (rc) return rc;
+  if (!y || !mu || !mu_star || !sigma || !mu_star_conf || !n_used || (mo->n_candidates && !selected))
+    return fail(SIMPLYP_EINVAL, "morris effects: null argument%s");
+  if (n_rows < 0 || n_boot < 0 || n_boot > 10000 || !(conf_z >= 0.0 && conf_z < INFINITY))
+    return fail(SIMPLYP_EINVAL, "morris effects: need n_rows >= 0, n_boot in 0..10^4 and a finite conf_z >= 0%s");
+  const int64_t need = n_rows ? morris_steps_bytes(*mo) + morris_pass_rows(*mo, n_rows) * morris_row_bytes(*mo) : 0;
+  if (need > 0 && (!workspace || workspace_bytes < need))
+    return fail(SIMPLYP_EINVAL, "morris effects: workspace smaller than simplyp_morris_workspace_bytes%s");
+  if (simplyp_device_count() <= 0) return fail(SIMPLYP_ENODEVICE, "no CUDA device%s");
+  if (n_rows == 0) return SIMPLYP_OK;
+  const int64_t N = mo->n_trajectories, K = mo->n_free, rows = morris_pass_rows(*mo, n_rows);
+  const int32_t* sel = mo->n_candidates ? selected : nullptr;
+  char* ws = static_cast<char*>(workspace);
+  uint8_t* steps = reinterpret_cast<uint8_t*>(ws);
+  int* used = reinterpret_cast<int*>(ws + morris_steps_bytes(*mo));
+  double* ee = reinterpret_cast<double*>(reinterpret_cast<char*>(used) + rows * ((4 * N + 7) & ~7ll));
+  double* part = ee + (size_t)rows * N * K;
+  cudaStream_t st = static_cast<cudaStream_t>(stream);
+  morris_steps_kernel<<<(unsigned)((N + 127) / 128), 128, 0, st>>>(*mo, sel, steps);
+  g_launches.fetch_add(1);
+  SP_CUDA(cudaGetLastError());
+  for (int64_t r0 = 0; r0 < n_rows; r0 += rows) {
+    const int64_t nr = n_rows - r0 < rows ? n_rows - r0 : rows;
+    morris_point_kernel<<<(unsigned)nr, MO_THREADS, 0, st>>>(*mo, y, r0, steps, used, ee, mu, mu_star, sigma, n_used);
+    morris_boot_kernel<<<dim3(MO_GROUPS, (unsigned)nr), MO_THREADS, 0, st>>>(*mo, r0, used, ee, n_boot, mu_star,
+                                                                               n_used, part);
+    morris_conf_kernel<<<(unsigned)nr, SIMPLYP_MCMC_MAX_FREE, 0, st>>>(*mo, r0, n_boot, conf_z, n_used, part,
+                                                                       mu_star_conf);
+    g_launches.fetch_add(3);
+    SP_CUDA(cudaGetLastError());
+  }
+  return SIMPLYP_OK;
 }
 
 void simplyp_release_cache(void) {

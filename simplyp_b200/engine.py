@@ -287,6 +287,49 @@ class Engine:
                    ws.data_ptr(), need)
         return out
 
+    # ------------------------------------------------------------------ Morris screening
+    def morris_select(self, mo, selected=None):
+        """Indices [r] int32 (device) of the trajectories the greedy spread search picks among the
+        :class:`_cabi.SimplypMorris` ``mo``'s candidates (``simplyp_morris_select_device``).  Asynchronous."""
+        torch = _torch()
+        if selected is None:
+            selected = torch.empty(mo.n_trajectories, dtype=torch.int32, device=self.device)
+        need = _cabi.morris_workspace_bytes(mo, 0)
+        ws = self._workspace(need)
+        self._call(_cabi.morris_select_device, mo, selected.data_ptr(), ws.data_ptr(), need)
+        return selected
+
+    def morris_design(self, mo, member_params, sc_params, selected=None, member_offset=0, n_members=None):
+        """Write the target columns of design members ``member_offset .. member_offset + n_members`` (default: to the
+        end) of ``member_params`` [r (K+1)][NP_MEMBER] and ``sc_params`` ([r (K+1)] or [1])[S][NP_SC]; ``selected``
+        (from :meth:`morris_select`) is needed when ``mo`` has candidates (``simplyp_morris_design_device``).
+        Asynchronous."""
+        if n_members is None:
+            n_members = member_params.shape[0] - member_offset
+        self._call(_cabi.morris_design_device, mo, selected.data_ptr() if selected is not None else None,
+                   member_offset, n_members, member_params.data_ptr(), sc_params.data_ptr())
+        return member_params, sc_params
+
+    def morris_effects(self, mo, y, n_boot, conf_z, selected=None, out=None):
+        """Elementary-effect statistics of every row of ``y`` [R][r (K+1)] (``simplyp_morris_effects_device``).
+        Returns a dict of device tensors mu, mu_star, sigma, mu_star_conf [R][K] and n_used [R]; ``out`` may give them
+        preallocated.  Asynchronous."""
+        torch = _torch()
+        if y.dim() != 2 or y.dtype != torch.float64 or not y.is_contiguous():
+            raise ValueError("morris_effects takes a contiguous [R][r (K + 1)] float64 matrix")
+        R, K = y.shape[0], mo.n_free
+        if out is None:
+            out = {k: torch.empty((R, K), dtype=torch.float64, device=self.device)
+                   for k in ("mu", "mu_star", "sigma", "mu_star_conf")}
+            out["n_used"] = torch.empty(R, dtype=torch.int64, device=self.device)
+        need = _cabi.morris_workspace_bytes(mo, R)
+        ws = self._workspace(need)
+        self._call(_cabi.morris_effects_device, mo, selected.data_ptr() if selected is not None else None,
+                   y.data_ptr(), R, n_boot, conf_z, out["mu"].data_ptr(), out["mu_star"].data_ptr(),
+                   out["sigma"].data_ptr(), out["mu_star_conf"].data_ptr(), out["n_used"].data_ptr(), ws.data_ptr(),
+                   need)
+        return out
+
     # ------------------------------------------------------------------ differential evolution
     def de_trial(self, de, state, member_params, sc_params):
         """Trials of the :class:`_cabi.SimplypDe` population ``state`` into its trial buffer and the target columns of
